@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — mapped reads/s of the `pandora map` hot path (BASELINE.json metric) on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl ours|reference] [--no-extras]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl ours|reference] [--no-extras] [--dump-outputs DIR]
 
 Workload = BASELINE config 3, the configuration the metric ("mapped reads/sec at 1/2/4/8 B200") is quoted on: the
 config-2 panel and genome with 30 M simulated 150 bp reads (~1000x panel depth), STRONG-scaled: the same 30 M reads are
@@ -164,6 +164,28 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def strip_file_date(vcf_text):
+    """the VCF text without its ##fileDate line, the one line that differs between two runs on the same reads"""
+    return b"\n".join(l for l in vcf_text.splitlines() if not l.startswith(b"##fileDate"))
+
+
+def dump_outputs(out_dir, ix, vcf_text, st):
+    """Writes what the last timed step computed as DIR/<name>.npy, so that two builds can be compared output for output:
+    the VCF text (byte codes as float32, without ##fileDate: its SHA-1 is the run's `vcf_sha1`), the hit counts of the map
+    step (hits, kept hits, bases, reads), the k-mer coverage the genotype step started from, the fitted parameters (in the
+    order of lib.Index.params()) and every per-record and per-allele array behind the VCF (float64).  All arrays are sized
+    by the panel, not by the reads (~38 k k-mer nodes, ~4.5 k sites, ~5 MB in all), so they are written whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    cov = ix.coverage()
+    out = {"vcf_text": np.frombuffer(strip_file_date(vcf_text), np.uint8).astype(np.float32),
+           "map_totals": np.array([st["hits"][-1], st["kept"][-1], cov["total_bases"], cov["n_reads"]], np.float64),
+           "coverage_fwd": cov["fwd"], "coverage_rev": cov["rev"], "locus_reads": cov["locus_reads"],
+           "gt_params": np.array(list(ix.params().values()), np.float64)}
+    out.update({"gt_" + k: v for k, v in ix.gt_records().items()})
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def extras_single_gpu(lib, workload, sim, wl, ix, opts, torch, flush):
     """the other BASELINE configurations and the file-level plugin call, measured on one GPU (bounded: a few seconds)"""
     out = {}
@@ -280,7 +302,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -352,6 +379,7 @@ def main():
         for k_, v_ in t.items():
             stats.setdefault(k_, []).append(v_)
         stats.setdefault("hits", []).append(nh)
+        stats.setdefault("kept", []).append(nk)
         if world > 1:
             if reduce_mode == "fused":
                 if rank != 0:          # this rank's coverage is already in the root's accumulator: report the arrival
@@ -412,6 +440,9 @@ def main():
         sampler.start()
     ms_step, launches, vcf_text, st = timed(step_resident, args.steps, args.warmup)
     clocks = sampler.stop()
+    vcf_text = bytes(vcf_text) if vcf_text is not None else b""  # a copy: the next genotype call reuses the library's buffer
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ix, vcf_text, st)
     ms_e2e, _, _, _ = timed(step_e2e, max(3, args.steps // 2), args.warmup)
 
     total_reads = wl.total_reads
@@ -426,7 +457,6 @@ def main():
     achieved = alg_bytes / (k_ms * 1e-3) / 1e9
     prof = screen_profile()
     issue_peak = ix.issue_peak() if rank == 0 else 0.0
-    vcf_text = bytes(vcf_text) if vcf_text is not None else b""
     n_records = sum(1 for l in vcf_text.splitlines() if not l.startswith(b"#"))
     h2d = int(total_reads * (workload.STRIDE_WORDS * 4 + 4))  # all ranks together: words + lengths of the 30 M reads
     d2h = int(len(vcf_text) + 4096)
@@ -440,14 +470,14 @@ def main():
                 "reduce": ("none (one GPU)" if world == 1 else
                            "fused: coverage kernel adds into the root accumulator over NVLink (CUDA IPC mapping), device-side arrival flags"
                            if reduce_mode == "fused" else "NCCL allreduce of the accumulator (torch.distributed)"),
-                "vcf_records": n_records, "vcf_sha1": hashlib.sha1(b"\n".join(l for l in vcf_text.splitlines() if not l.startswith(b"##fileDate"))).hexdigest()},
+                "vcf_records": n_records, "vcf_sha1": hashlib.sha1(strip_file_date(vcf_text)).hexdigest()},
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "ms_per_step": ms_e2e,
                 "what": "same steps from pinned host buffers: H2D of every rank's packed shard inside the timed region, VCF text read on the host",
                 "reads_per_rank": "even" if mine_e2e == mine or h2d_gbps is None else
                                   "proportional to each rank's measured concurrent H2D bandwidth: " + ", ".join(f"{g:.0f}" for g in h2d_gbps) + " GB/s"},
         "gpu_launches": int(launches),
         "clocks": clocks,
-        "stage_ms": {k_: float(np.mean(v_)) for k_, v_ in st.items() if k_ != "hits"},
+        "stage_ms": {k_: float(np.mean(v_)) for k_, v_ in st.items() if k_ not in ("hits", "kept")},
     }
     roof = {"bound": "hbm", "kernel": "screen_kernel<15,10> + resolve_kernel<11,15> (S1+S2: k-mer screen of every read, then hash/probe/minimizer test of the flagged positions)",
             "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak, "traffic": None, "peak_source": peak_src,
