@@ -64,10 +64,11 @@ struct ModelParams {  // S6 output, computed on the host
 uint64_t launch_count();
 
 // S1+S2: sketch every read and probe the index; hits appended (unordered) through *hit_count
-// With a screen workspace (d_queue + d_queue_kmer: queue_cap entries each, d_screen_counters: {queue length, ticket, largest queue length
-// wanted}) and a screenable index (k = 15), a k-mer screen queues the positions whose k-mer may be indexed and only
-// those are hashed, probed and tested for minimizer status (identical hits).  The queue overflowed when
-// d_screen_counters[2] > queue_cap (the caller zeroes [2] before a batch and redoes the batch with a larger queue).
+// With a screen workspace (d_queue + d_queue_kmer: queue_cap entries each, d_screen_counters: the batch counters from CTR_QUEUE on,
+// i.e. {queue length, ticket, largest queue length wanted, ..., probe survivors at CTR_SURVIVORS}) and a screenable index (k = 15),
+// a k-mer screen queues the positions whose k-mer may be indexed and only those are hashed, probed and tested for minimizer
+// status (identical hits).  The queue overflowed when d_screen_counters[2] > queue_cap (the caller zeroes the counters before a
+// batch and redoes the batch with a larger queue).
 void launch_sketch_lookup(const DevReads& R, const DevTable& T, uint32_t w, uint32_t k, unsigned long long* d_hi,
                           unsigned long long* d_lo, unsigned long long* d_hit_count, uint64_t hit_cap, int sm_count,
                           uint32_t max_len, cudaStream_t st, unsigned long long* d_queue = nullptr, uint64_t queue_cap = 0,
@@ -93,6 +94,7 @@ enum : int {
     CTR_CURSOR = 6,      // grouped-hit slices handed out
     CTR_BIG = 7,         // active reads with more than CLUSTER_WARP_MAX hits
     CTR_LKOVF = 8,       // locus keys beyond two kept clusters per read
+    CTR_SURVIVORS = 9,   // k-mer screen: queue entries whose k-mer is in the index (summed over the chunks)
     CTR_COUNT = 16
 };
 constexpr uint32_t CLUSTER_WARP_MAX = 64;  // hits of a read one warp sorts in registers; longer reads get a CTA

@@ -548,10 +548,11 @@ static bool launch_short(const DevReads& R, const DevTable& T, uint32_t w, uint3
 //                   words in registers) and tests each k-mer against a blocked 2-bit Bloom filter held in
 //                   shared memory: one multiply, one LDS, two shifts, ~10 instructions per position.  The
 //                   flagged positions (~1 % false positives + the real ones) are appended to a queue.
-//   resolve_kernel  one thread per queued (read, position): canonical hash of that k-mer, index probe (exact,
-//                   drops the false positives), then the minimizer test restricted to that position — it is a
-//                   (w,k)-minimizer with pandora's "all ties kept" rule iff the run of neighbours whose hash
-//                   is >= its own covers a whole window — and the hit records.
+//   resolve_kernel  persistent warps, several queued (read, position) pairs per lane: canonical hash of each k-mer,
+//                   index probes side by side (exact, drops the false positives), survivors collected in a per-warp
+//                   shared-memory ring and tested 32 at a time — a position is a (w,k)-minimizer with pandora's
+//                   "all ties kept" rule iff the run of neighbours whose hash is >= its own covers a whole window —
+//                   then the hit records (details above the kernel).
 // The hits are the same set the full sketch + lookup kernels emit; only ~2 % of the positions ever get hashed.
 // ============================================================================================
 constexpr int SCREEN_THREADS = 1024;
@@ -730,35 +731,44 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
     }
 }
 
-// Resolve the flagged (read, position) pairs.  Phase 1, one thread per queue entry: canonical hash of the k-mer, index
-// probe — exact, so the Bloom filter's false positives (~80 % of the queue) end here; the survivors are compacted into
-// shared memory.  Phase 2, one thread per survivor in dense warps: the minimizer test restricted to that position.
+// Resolve the flagged (read, position) pairs: persistent warps, no CTA barrier.  A warp takes tiles of RESOLVE_PER_LANE
+// queue entries per lane (lane-strided, so the queue loads stay coalesced), computes the canonical hash of every queued
+// k-mer and issues the index probes of all of them before it uses any result: RESOLVE_PER_LANE independent L2 chains per
+// thread.  The probe is exact, so the Bloom filter's false positives (~80 % of the queue) end here.  The survivors are
+// appended by ballot to a ring in the warp's own shared memory; whenever it holds 32 of them the warp runs the minimizer
+// test restricted to those positions with every lane busy, and after its last tile it tests what is left.
 //   W > 0: compile-time window (2W-2+K bases around the position fit three aligned words): the words are fetched once,
 //          shifted so that every neighbour sits at a static offset, and all 2W-1 canonical hashes are computed branch-free;
 //   W == 0: any window, neighbours fetched one by one with early exit.
-constexpr int RESOLVE_THREADS = 256;
+constexpr int RESOLVE_WARPS = 8;
+constexpr int RESOLVE_PER_LANE = 4;
+constexpr uint32_t RESOLVE_TILE = 32 * RESOLVE_PER_LANE;
+constexpr int RESOLVE_RING = 31 + RESOLVE_TILE;  // < 32 untested survivors + one tile's
 template <int W, int K>
-__global__ void __launch_bounds__(RESOLVE_THREADS) resolve_kernel(DevReads R, DevTable T, uint32_t w_rt, uint32_t k_rt,
-                                                                  const unsigned long long* __restrict__ queue,
-                                                                  const uint32_t* __restrict__ queue_kmer,
-                                                                  const unsigned long long* __restrict__ queue_count,
-                                                                  unsigned long long queue_cap,
-                                                                  unsigned long long* __restrict__ queue_need,
-                                                                  unsigned long long* __restrict__ out_a,
-                                                                  unsigned long long* __restrict__ out_b,
-                                                                  unsigned long long* __restrict__ out_count,
-                                                                  unsigned long long cap) {
+__global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R, DevTable T, uint32_t w_rt, uint32_t k_rt,
+                                                                     const unsigned long long* __restrict__ queue,
+                                                                     const uint32_t* __restrict__ queue_kmer,
+                                                                     const unsigned long long* __restrict__ queue_count,
+                                                                     unsigned long long queue_cap,
+                                                                     unsigned long long* __restrict__ queue_need,
+                                                                     unsigned long long* __restrict__ survivors,
+                                                                     unsigned long long* __restrict__ out_a,
+                                                                     unsigned long long* __restrict__ out_b,
+                                                                     unsigned long long* __restrict__ out_count,
+                                                                     unsigned long long cap) {
     static_assert(W == 0 || 2 * W - 2 + K <= 48, "window + k-mer must fit three aligned words");
-    __shared__ unsigned long long s_q[RESOLVE_THREADS];
-    __shared__ uint32_t s_rec[RESOLVE_THREADS];
-    __shared__ uint32_t s_n;
+    __shared__ unsigned long long s_q[RESOLVE_WARPS][RESOLVE_RING];
+    __shared__ uint32_t s_rec[RESOLVE_WARPS][RESOLVE_RING];
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicMax(queue_need, *queue_count);  // sticky over the chunks of a batch: the host regrows and redoes
     if (*queue_count > queue_cap) return;  // overflow: the queue has unwritten slots and the batch is redone anyway
     const unsigned long long n = *queue_count;
     const uint32_t w = W ? (uint32_t)W : w_rt, k = W ? (uint32_t)K : k_rt;
     const uint32_t S = 32 - 2 * k;
     const uint32_t hm = (S == 0) ? 0xffffffffu : ~((1u << S) - 1u);
-    const int tid = threadIdx.x, lane = tid & 31;
+    const uint32_t smask = (1u << T.slot_bits) - 1u;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    unsigned long long* ring_q = s_q[wid];
+    uint32_t* ring_rec = s_rec[wid];
     auto canon_of = [&](uint32_t v, uint32_t& strand) {  // v: 32 bits starting at the k-mer's first base
         const uint32_t F = v & hm;
         uint32_t y = __brev(~v & hm);
@@ -767,50 +777,70 @@ __global__ void __launch_bounds__(RESOLVE_THREADS) resolve_kernel(DevReads R, De
         strand = hf <= hr ? 1u : 0u;
         return min(hf, hr);
     };
-    for (unsigned long long base = (unsigned long long)blockIdx.x * RESOLVE_THREADS; base < n;
-         base += (unsigned long long)gridDim.x * RESOLVE_THREADS) {  // CTA-uniform trip count
-        if (tid == 0) s_n = 0;
-        __syncthreads();
-        // ---- phase 1
-        {
-            const unsigned long long e = base + tid;
-            uint32_t rec = 0;
-            unsigned long long q = 0;
-            if (e < n) {
-                q = queue[e];
+    const unsigned long long n_tiles = (n + RESOLVE_TILE - 1) / RESOLVE_TILE;
+    const unsigned long long n_warps = (unsigned long long)gridDim.x * RESOLVE_WARPS;
+    uint32_t ring_n = 0;              // survivors in the ring (warp-uniform)
+    unsigned long long n_surv = 0;    // survivors this warp found (warp-uniform)
+    for (unsigned long long tile = (unsigned long long)blockIdx.x * RESOLVE_WARPS + wid;; tile += n_warps) {
+        const bool more = tile < n_tiles;  // warp-uniform
+        if (more) {
+            unsigned long long q[RESOLVE_PER_LANE];
+            uint32_t km[RESOLVE_PER_LANE], hv[RESOLVE_PER_LANE], slot[RESOLVE_PER_LANE], rec[RESOLVE_PER_LANE];
+            uint32_t pending = 0;  // bit i: entry i still walks its probe chain
+#pragma unroll
+            for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
+                const unsigned long long e = tile * RESOLVE_TILE + i * 32 + lane;
+                q[i] = 0;
+                km[i] = 0;
+                rec[i] = 0;
+                if (e < n) {
+                    q[i] = queue[e];
+                    km[i] = queue_kmer[e];
+                    pending |= 1u << i;
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
                 uint32_t strand;
-                const uint32_t hv = canon_of(queue_kmer[e] << S, strand) >> S;  // the queued k-mer, left aligned
-                uint32_t slot = table_slot(hv, T.slot_bits);
-                const uint32_t smask = (1u << T.slot_bits) - 1u;
-                while (true) {
-                    const uint2 ent = __ldg(T.slots + slot);
-                    if (ent.y == 0u) break;
-                    if (ent.x == hv) {
-                        rec = ent.y;  // rec_begin | rec_count << 24, count >= 1
-                        break;
+                hv[i] = canon_of(km[i] << S, strand) >> S;  // the queued k-mer, left aligned
+                slot[i] = table_slot(hv[i], T.slot_bits);
+            }
+            // one slot of every unfinished chain per round: the loads of a round are independent of each other
+            while (pending) {
+                uint2 ent[RESOLVE_PER_LANE];
+#pragma unroll
+                for (int i = 0; i < RESOLVE_PER_LANE; ++i) ent[i] = (pending >> i & 1u) ? __ldg(T.slots + slot[i]) : make_uint2(0u, 0u);
+#pragma unroll
+                for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
+                    if (!(pending >> i & 1u)) continue;
+                    if (ent[i].y == 0u || ent[i].x == hv[i]) {
+                        rec[i] = ent[i].y;  // rec_begin | rec_count << 24 (count >= 1), or 0: not indexed
+                        pending &= ~(1u << i);
+                    } else {
+                        slot[i] = (slot[i] + 1) & smask;
                     }
-                    slot = (slot + 1) & smask;
                 }
             }
-            const uint32_t bal = __ballot_sync(FULL, rec != 0u);
-            if (bal) {
-                uint32_t o = 0;
-                if (lane == 0) o = atomicAdd(&s_n, (uint32_t)__popc(bal));
-                o = __shfl_sync(FULL, o, 0) + __popc(bal & ((1u << lane) - 1u));
-                if (rec) {
-                    s_q[o] = q;
-                    s_rec[o] = rec;
+#pragma unroll
+            for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
+                const uint32_t bal = __ballot_sync(FULL, rec[i] != 0u);
+                if (rec[i]) {
+                    const uint32_t o = ring_n + __popc(bal & ((1u << lane) - 1u));
+                    ring_q[o] = q[i];
+                    ring_rec[o] = rec[i];
                 }
+                ring_n += __popc(bal);
+                n_surv += __popc(bal);
             }
+            __syncwarp();
         }
-        __syncthreads();
-        // ---- phase 2
-        const uint32_t nf = s_n;
-        if ((uint32_t)(tid & ~31) < nf) {  // warp-uniform
+        // minimizer tests, 32 survivors at a time; after the last tile also the partial batch
+        uint32_t done = 0;
+        for (; done + 32 <= ring_n || (!more && done < ring_n); done += 32) {
             uint32_t emit_n = 0, rec_begin = 0, read_strand = 0, r = 0, pos = 0;
-            if ((uint32_t)tid < nf) {
-                const unsigned long long q = s_q[tid];
-                const uint32_t rec = s_rec[tid];
+            if (done + lane < ring_n) {
+                const unsigned long long q = ring_q[done + lane];
+                const uint32_t rec = ring_rec[done + lane];
                 r = (uint32_t)(q >> 32);
                 pos = (uint32_t)q;
                 uint32_t rec_n;
@@ -891,8 +921,26 @@ __global__ void __launch_bounds__(RESOLVE_THREADS) resolve_kernel(DevReads R, De
                 }
             }
         }
-        __syncthreads();
+        if (!more) break;
+        // the < 32 untested survivors move to the front of the ring
+        if (done) {
+            const uint32_t left = ring_n - done;
+            unsigned long long q = 0;
+            uint32_t rec = 0;
+            if ((uint32_t)lane < left) {
+                q = ring_q[done + lane];
+                rec = ring_rec[done + lane];
+            }
+            __syncwarp();
+            if ((uint32_t)lane < left) {
+                ring_q[lane] = q;
+                ring_rec[lane] = rec;
+            }
+            __syncwarp();
+            ring_n = left;
+        }
     }
+    if (lane == 0 && n_surv) atomicAdd(survivors, n_surv);
 }
 
 template <int K, int CW, int V>
@@ -927,7 +975,29 @@ static void launch_screen_one(const DevReads& R, const DevTable& T, uint32_t wk,
     }
 }
 
-// screen + resolve; counters = {queue length, ticket, largest queue length wanted (not reset here)}
+// counters = the CTR_QUEUE.. slots of the batch counters
+template <int W, int K>
+static void launch_resolve(const DevReads& R, const DevTable& T, uint32_t w, const unsigned long long* queue, const uint32_t* queue_kmer,
+                           uint64_t queue_cap, unsigned long long* counters, unsigned long long* a, unsigned long long* b,
+                           unsigned long long* cnt, uint64_t cap, int sm_count, uint32_t max_len, cudaStream_t st) {
+    static const int per_sm = [] {
+        int n = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, resolve_kernel<W, K>, RESOLVE_WARPS * 32, 0);
+        return std::max(n, 1);
+    }();
+    // persistent warps at full occupancy; the queue length is only known on the device, but it cannot exceed the number of
+    // k-mer positions, which caps the grid of a small batch
+    const unsigned long long positions = (R.seg_read ? R.n_segs * R.seg_len : R.n_reads * max_len) + 1;
+    const unsigned long long want = (positions + RESOLVE_TILE * RESOLVE_WARPS - 1) / (RESOLVE_TILE * RESOLVE_WARPS);
+    const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)per_sm * (unsigned)sm_count);
+    resolve_kernel<W, K><<<grid, RESOLVE_WARPS * 32, 0, st>>>(R, T, w, K, queue, queue_kmer, counters, queue_cap,
+                                                              counters + (CTR_QUEUE_NEED - CTR_QUEUE), counters + (CTR_SURVIVORS - CTR_QUEUE),
+                                                              a, b, cnt, cap);
+    ++g_launches;
+}
+
+// screen + resolve; counters = the CTR_QUEUE.. slots of the batch counters: {queue length, ticket, largest queue length
+// wanted, ...} (only the first two are reset here)
 template <int K>
 static void launch_screened(const DevReads& R, const DevTable& T, uint32_t w, unsigned long long* a, unsigned long long* b,
                             unsigned long long* cnt, uint64_t cap, int sm_count, uint32_t max_len,
@@ -936,13 +1006,9 @@ static void launch_screened(const DevReads& R, const DevTable& T, uint32_t w, un
     cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned long long), st);
     if (!R.seg_read && max_len >= (uint32_t)K && max_len - K + 1 <= 10 * 16) launch_screen_one<K, 10>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
     else launch_screen_one<K, 8>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
-    // ~2 queue entries per read; the grid-stride loop reads the real length on the device
-    const unsigned long long n_items = R.seg_read ? R.n_segs : R.n_reads;
-    const unsigned grid = (unsigned)std::min<unsigned long long>((n_items * 2 + 255) / 256 + 1, 8ull * (unsigned)sm_count);
-    if (w == 11) resolve_kernel<11, K><<<grid, RESOLVE_THREADS, 0, st>>>(R, T, w, K, queue, queue_kmer, counters, queue_cap, counters + 2, a, b, cnt, cap);
-    else if (w == 14) resolve_kernel<14, K><<<grid, RESOLVE_THREADS, 0, st>>>(R, T, w, K, queue, queue_kmer, counters, queue_cap, counters + 2, a, b, cnt, cap);
-    else resolve_kernel<0, K><<<grid, RESOLVE_THREADS, 0, st>>>(R, T, w, K, queue, queue_kmer, counters, queue_cap, counters + 2, a, b, cnt, cap);
-    ++g_launches;
+    if (w == 11) launch_resolve<11, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);
+    else if (w == 14) launch_resolve<14, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);
+    else launch_resolve<0, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);
 }
 
 static int grid_for(int sm_count, uint64_t n_reads) {
