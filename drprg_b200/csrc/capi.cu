@@ -215,9 +215,7 @@ struct drprg_index {
     uint32_t* d_kfilter = nullptr;
     uint32_t *d_filter = nullptr, *d_knode_base = nullptr, *d_edge_off = nullptr, *d_edges = nullptr;
     uint8_t *d_is_terminal = nullptr, *d_needs_mean = nullptr;
-    uint32_t *d_locus_unit_off = nullptr, *d_unit_start = nullptr, *d_unit_nodes = nullptr;
     uint32_t *d_locus_level_off = nullptr, *d_level_start = nullptr, *d_level_nodes = nullptr, *d_level_singles = nullptr;
-    float mean_run_len = 0.f;
     uint32_t table_slots = 0, filter_words = 0;
     uint64_t n_edges = 0, n_ivs = 0;
     // accumulators: [2*N coverage | P locus reads | 4 scalars]
@@ -330,7 +328,7 @@ struct drprg_index {
         cudaSetDevice(device);
         if (ipc_mapping) cudaIpcCloseMemHandle(ipc_mapping);
         for (void* p : {(void*)d_slots, (void*)d_recs, (void*)d_filter, (void*)d_knode_base, (void*)d_edge_off, (void*)d_edges,
-                        (void*)d_is_terminal, (void*)d_needs_mean, (void*)d_locus_unit_off, (void*)d_unit_start, (void*)d_unit_nodes, (void*)d_accum, (void*)d_thresh, (void*)d_counters, (void*)d_rec_off,
+                        (void*)d_is_terminal, (void*)d_needs_mean, (void*)d_accum, (void*)d_thresh, (void*)d_counters, (void*)d_rec_off,
                         (void*)d_allele_off, (void*)d_allele_kn, (void*)d_knode_locus, (void*)d_hist, (void*)d_kfilter, (void*)d_locus_level_off, (void*)d_level_start, (void*)d_level_nodes, (void*)d_level_singles})
             if (p) cudaFree(p);
         if (h_counters) cudaFreeHost(h_counters);
@@ -476,50 +474,6 @@ void upload_index(drprg_index* X) {
                     for (uint32_t o : L.kout[r]) needs[base + o] = 1;
         }
         X->d_needs_mean = to_device(needs);
-    }
-    {   // processing units of the ML-path kernel: a node with a choice (or none), or a run of <= 32 single-successor nodes
-        std::vector<uint32_t> locus_unit_off(1, 0), unit_start(1, 0), unit_nodes;
-        for (size_t l = 0; l < H.loci.size(); ++l) {
-            const Locus& L = H.loci[l];
-            const uint32_t n = (uint32_t)L.kpath.size();
-            std::vector<std::vector<uint32_t>> preds(n);
-            for (uint32_t r = 0; r < n; ++r)
-                for (uint32_t o : L.kout[r]) preds[o].push_back(r);
-            std::vector<char> done(n, 0);
-            for (uint32_t r = n >= 2 ? n - 1 : 0; r-- > 0;) {  // n-2 .. 0 (the terminus is not a unit)
-                if (done[r]) continue;
-                done[r] = 1;
-                unit_nodes.push_back(r);
-                if (L.kout[r].size() == 1) {
-                    uint32_t cur = r, len = 1;
-                    while (len < 32) {
-                        uint32_t best = UINT32_MAX;
-                        for (uint32_t p : preds[cur])
-                            if (!done[p] && L.kout[p].size() == 1 && (best == UINT32_MAX || p > best)) best = p;
-                        if (best == UINT32_MAX) break;
-                        done[best] = 1;
-                        unit_nodes.push_back(best);
-                        cur = best;
-                        ++len;
-                    }
-                }
-                unit_start.push_back((uint32_t)unit_nodes.size());
-            }
-            locus_unit_off.push_back((uint32_t)unit_start.size() - 1);
-        }
-        {
-            uint64_t runs = 0, run_nodes = 0;
-            for (size_t l = 0; l < H.loci.size(); ++l)
-                for (uint32_t uu = locus_unit_off[l]; uu < locus_unit_off[l + 1]; ++uu)
-                    if (H.loci[l].kout[unit_nodes[unit_start[uu]]].size() == 1) {
-                        ++runs;
-                        run_nodes += unit_start[uu + 1] - unit_start[uu];
-                    }
-            X->mean_run_len = runs ? (float)run_nodes / (float)runs : 0.f;
-        }
-        X->d_locus_unit_off = to_device(locus_unit_off);
-        X->d_unit_start = to_device(unit_start);
-        X->d_unit_nodes = to_device(unit_nodes);
     }
     {   // level order for the level-parallel ML-path kernel: level = 1 + max level of the successors (terminus = 0)
         std::vector<uint32_t> locus_level_off(1, 0), level_start(1, 0), level_nodes, level_singles;
@@ -940,11 +894,11 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
     CK(cudaEventRecord(X->ev_ml[0], X->st_ml));
     // The level-parallel kernel writes every locus's path straight into pinned host memory (UVA: the same pointers
     // are valid on the device) and raises a per-locus flag, so the host can verify the small loci while the big ones
-    // are still running; the older kernels leave the paths in device memory and are copied back as a whole.
+    // are still running; the generic kernel leaves the paths in device memory and they are copied back as a whole.
     const bool ml_streamed = launch_mlpath(
         P, X->d_knode_base, X->d_edge_off, X->d_edges, X->d_prob.p, X->d_accum + 2ull * N, MP, X->d_M.p, X->d_len.p, X->d_up.p, N,
-        X->d_path.p, X->d_path_len.p, X->max_locus_knodes, X->max_locus_edges, X->d_needs_mean, X->d_locus_unit_off, X->d_unit_start,
-        X->d_unit_nodes, X->mean_run_len, X->st_ml, X->d_locus_level_off, X->d_level_start, X->d_level_nodes, X->d_level_singles,
+        X->d_path.p, X->d_path_len.p, X->max_locus_knodes, X->max_locus_edges, X->d_needs_mean, X->st_ml,
+        X->d_locus_level_off, X->d_level_start, X->d_level_nodes, X->d_level_singles,
         X->h_path.data(), X->h_plen.data(), X->h_done.data(), X->d_thresh_f64);
     X->ml_in_flight = true;
     CK(cudaEventRecord(X->ev_ml[1], X->st_ml));

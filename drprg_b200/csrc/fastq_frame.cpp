@@ -7,7 +7,6 @@
 
 #include <immintrin.h>
 
-#include <sys/mman.h>
 #include <unistd.h>
 
 #include <atomic>
@@ -253,44 +252,26 @@ bool fastq_frame_text(const TextSource& src, uint32_t threads, char* seq_buf, st
             size_t used = 0;
             ok = F.feed(src.mem + lo, hi - lo, used) && F.finish(src.mem + lo + used, hi - lo - used, hi == src.size);
         } else {
-            // default: pread into an L2-resident bounce buffer.  DRPRG_FRAME_MMAP=1 maps the slice instead (populated in one
-            // call, framed in place): it saves the copy, but mapping, populating and unmapping page-cache (tmpfs) pages
-            // from 16 threads costs far more — 10 M reads from a 3.15 GB file: 64 ms with pread, 134-191 ms mapped (1, 4
-            // and 16 MB slices; tools/frame_mmap_ab.sh)
-            static const bool use_mmap = getenv("DRPRG_FRAME_MMAP") && atoi(getenv("DRPRG_FRAME_MMAP")) != 0;
-            static const size_t page = (size_t)sysconf(_SC_PAGESIZE);
-            void* map = MAP_FAILED;
-            size_t map_lo = 0, map_len = 0;
-            if (use_mmap) {
-                map_lo = (src.origin + lo) / page * page;
-                map_len = src.origin + hi - map_lo;
-                map = mmap(nullptr, map_len, PROT_READ, MAP_PRIVATE | MAP_POPULATE, src.fd, (off_t)map_lo);
-            }
-            if (map != MAP_FAILED) {
-                const char* t = (const char*)map + (src.origin + lo - map_lo);
-                size_t used = 0;
-                ok = F.feed(t, hi - lo, used) && F.finish(t + used, hi - lo - used, hi == src.size);
-                munmap(map, map_len);
-            } else {
-                constexpr size_t CH = 512u << 10;  // stays in the core's L2
-                if (buf.size() < 2 * CH) buf.resize(2 * CH);
-                size_t at = lo, carry = 0;
-                while (ok && at < hi) {
-                    const size_t want = std::min(CH, hi - at);
-                    if (buf.size() < carry + want) buf.resize(std::max(buf.size() * 2, carry + want));
-                    if (src.read(buf.data() + carry, at, want) != want) {
-                        Z.state = -2;
-                        failed = true;
-                        return;
-                    }
-                    at += want;
-                    size_t used = 0;
-                    ok = F.feed(buf.data(), carry + want, used);
-                    carry = carry + want - used;
-                    if (ok && carry) memmove(buf.data(), buf.data() + used, carry);
+            // pread into an L2-resident bounce buffer: mapping the slices instead saves the copy but was measured 2-3x
+            // slower from 16 threads (10 M reads from a 3.15 GB file: 64 ms with pread, 134-191 ms mapped with 1-16 MB slices)
+            constexpr size_t CH = 512u << 10;  // stays in the core's L2
+            if (buf.size() < 2 * CH) buf.resize(2 * CH);
+            size_t at = lo, carry = 0;
+            while (ok && at < hi) {
+                const size_t want = std::min(CH, hi - at);
+                if (buf.size() < carry + want) buf.resize(std::max(buf.size() * 2, carry + want));
+                if (src.read(buf.data() + carry, at, want) != want) {
+                    Z.state = -2;
+                    failed = true;
+                    return;
                 }
-                ok = ok && F.finish(buf.data(), carry, hi == src.size);
+                at += want;
+                size_t used = 0;
+                ok = F.feed(buf.data(), carry + want, used);
+                carry = carry + want - used;
+                if (ok && carry) memmove(buf.data(), buf.data() + used, carry);
             }
+            ok = ok && F.finish(buf.data(), carry, hi == src.size);
         }
         if (!ok) {
             Z.state = -1;

@@ -143,8 +143,7 @@ bool launch_mlpath(uint32_t n_loci, const uint32_t* d_knode_base, const uint32_t
                    const double* d_prob, const int32_t* d_locus_reads, ModelParams P, double* d_M, uint32_t* d_len,
                    uint32_t* d_up, uint32_t total_knodes, uint32_t* d_path, uint32_t* d_path_len,
                    uint32_t max_locus_knodes, uint32_t max_locus_edges, const uint8_t* d_needs_mean,
-                   const uint32_t* d_locus_unit_off, const uint32_t* d_unit_start, const uint32_t* d_unit_nodes,
-                   float mean_run_len, cudaStream_t st, const uint32_t* d_locus_level_off = nullptr,
+                   cudaStream_t st, const uint32_t* d_locus_level_off = nullptr,
                    const uint32_t* d_level_start = nullptr, const uint32_t* d_level_nodes = nullptr,
                    const uint32_t* d_level_singles = nullptr, uint32_t* h_path = nullptr, uint32_t* h_path_len = nullptr,
                    uint32_t* h_done = nullptr, const double* d_thresh = nullptr);

@@ -256,15 +256,23 @@ __global__ void mlpath_kernel(uint32_t n_loci, const uint32_t* __restrict__ knod
     path_len[l] = cnt;
 }
 
-// ---- fast variant: 64-byte node records addressed by their shared-memory address ---------------------------
-// The generic kernel above spends ~160 instructions and ~1000 cycles per node, two thirds of it address
-// arithmetic and dependent-issue waits (ncu: stall_wait 2.4, stall_short_scoreboard 2.6 per issued instruction).
-// Here every pointer the chain follows (successor, lifting pointers, edge targets) is stored as the 32-bit
-// shared-memory ADDRESS of the target's 64-byte record, so one hop is a single LDS with an immediate offset.
-constexpr uint32_t REC = 64, R_M = 0, R_MEAN = 8, R_PR = 16, R_LEN = 24, R_EOFF = 28, R_UP = 32, R_T = 60;
-// record: sum f64 | mean f64 | score f64 | len u32 | edge-list address u32 | lifting pointers up[0..6] | T
-// T = the node window-1 steps down the chosen path (what a predecessor subtracts when its window is full)
-
+// ---- level-parallel kernel ---------------------------------------------------------------------------------
+// A node only needs its successors' finished records, so all nodes at the same distance-to-sink ("level": 1 + the
+// largest level among the successors) are independent: the alleles of a bubble advance side by side.  The host
+// sorts every locus by level, single-successor nodes first within a level.  A locus gets a CTA of four warps: warps
+// 0-1 take the level's single-successor nodes, warps 2-3 the nodes with a choice, one node per lane, so the two code
+// paths run on different schedulers instead of serialising inside one warp (a lone warp issues one instruction every
+// ~6 cycles here: the kernel is bound by its own instruction latency, not by shared memory).  Each node runs the
+// per-node step of the generic kernel's chain (successors still visited in rank order, so pandora's order-dependent
+// tie-breaking is unchanged); the CTA synchronises between levels.  The serial chain shrinks from the number of nodes
+// to the number of levels (benchmark panel: 38 251 nodes -> 15 128 levels, widest level 22 nodes).
+//
+// Node records are 64 bytes of shared memory, and every pointer the DP follows (successor, lifting pointers, window
+// tail, edge targets, level lists) is stored as the 32-bit shared-memory ADDRESS of the target's record, so one hop is
+// a single LDS with an immediate offset.  The generic kernel above spends ~160 instructions and ~1000 cycles per node,
+// two thirds of it address arithmetic and dependent-issue waits (ncu: stall_wait 2.4, stall_short_scoreboard 2.6 per
+// issued instruction).
+constexpr uint32_t REC = 64;
 __device__ __forceinline__ uint32_t lds32(uint32_t a) {
     uint32_t v;
     asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
@@ -278,310 +286,6 @@ __device__ __forceinline__ double lds64(uint32_t a) {
 __device__ __forceinline__ void sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v)); }
 __device__ __forceinline__ void sts64(uint32_t a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v)); }
 
-// After the successor v of node a is known, two pointer chases remain, both through tables of OLDER nodes only and
-// therefore independent of each other and of the fp chain: the lifting pointers of a (level l of a = level l-1 of
-// the node 2^(l-1) steps down) and T(a) = succ^(window-2)(v).  Their loads are issued interleaved so the two chains
-// overlap instead of adding up (volatile asm keeps this order).
-__device__ __forceinline__ void mlpath_link(uint32_t a, uint32_t v, uint32_t steps2) {
-    sts32(a + R_UP, v);
-    uint32_t x = v, t = v;
-#pragma unroll
-    for (int l = 0; l < 7; ++l) {
-        const uint32_t xn = (l < 6) ? lds32(x + R_UP + 4 * l) : 0u;          // level l+1 of a
-        const uint32_t tn = ((steps2 >> l) & 1u) ? lds32(t + R_UP + 4 * l) : t;  // walk window-2 steps from v
-        if (l < 6) {
-            sts32(a + R_UP + 4 * (l + 1), xn);
-            x = xn;
-        }
-        t = tn;
-    }
-    sts32(a + R_T, t);
-}
-
-__global__ void mlpath_rec_kernel(uint32_t n_loci, const uint32_t* __restrict__ knode_base, const uint32_t* __restrict__ edge_off,
-                                  const uint32_t* __restrict__ edges, const double* __restrict__ prob,
-                                  const int32_t* __restrict__ locus_reads, const uint8_t* __restrict__ needs_mean,
-                                  ModelParams P, uint32_t* __restrict__ path, uint32_t* __restrict__ path_len,
-                                  uint32_t max_nodes) {
-    extern __shared__ double s_dyn[];
-    const uint32_t l = blockIdx.x;
-    if (l >= n_loci) return;
-    const uint32_t base = knode_base[l], n = knode_base[l + 1] - base;
-    if (locus_reads[l] <= 0 || n < 2) {
-        if (threadIdx.x == 0) path_len[l] = 0xffffffffu;
-        return;
-    }
-    const uint32_t e_base = edge_off[base], n_edges = edge_off[base + n] - e_base;
-    const uint32_t recs = (uint32_t)__cvta_generic_to_shared(s_dyn);  // n + 1 records (the extra one carries the edge end)
-    const uint32_t edg = recs + (max_nodes + 1) * REC;                // successor record addresses
-    for (uint32_t i = threadIdx.x; i <= n; i += blockDim.x) {
-        const uint32_t a = recs + i * REC;
-        if (i < n) sts64(a + R_PR, prob[base + i]);
-        // edge list address (4-byte aligned) | bit0: some predecessor has a choice, so this node's mean is compared
-        sts32(a + R_EOFF, (edg + (edge_off[base + i] - e_base) * 4u) | (i < n ? (uint32_t)needs_mean[base + i] : 0u));
-    }
-    for (uint32_t i = threadIdx.x; i < n_edges; i += blockDim.x) sts32(edg + i * 4u, recs + edges[e_base + i] * REC);
-    __syncwarp();
-    if (threadIdx.x != 0) return;
-    const double tol = 0.000001;
-    const uint32_t term = recs + (n - 1) * REC;
-    const uint32_t steps2 = P.window - 2;  // T(a) = succ^(window-1)(a) = succ^(window-2)(chosen successor)
-    sts64(term + R_M, 0.0);
-    sts32(term + R_LEN, 0u);
-#pragma unroll
-    for (int v = 0; v < 8; ++v) sts32(term + R_UP + 4 * v, term);  // includes R_T
-    for (uint32_t a = term - REC; a + REC > recs; a -= REC) {  // nodes n-2 .. 0
-        double Mj = 0.0;
-        uint32_t lenj = 0, prevj = term;
-        const double pj = lds64(a + R_PR);
-        const uint32_t e1 = lds32(a + REC + R_EOFF) & ~3u;
-        const uint32_t e0w = lds32(a + R_EOFF);
-        const uint32_t e0 = e0w & ~3u;
-        if (e1 - e0 == 4u) {
-            // single successor (most nodes): no choice to make.  pandora's comparison against the initial
-            // -FLT_MAX accepts any successor with a real mean, i.e. any successor that is not a dead end.
-            const uint32_t v = lds32(e0);
-            const uint32_t lv = lds32(v + R_LEN);
-            const uint32_t tv = lds32(v + R_T);
-            const double Mv = lds64(v + R_M);
-            if (v == term || lv > 0u) {
-                mlpath_link(a, v, steps2);  // independent of the sums below: overlaps them
-                prevj = v;
-                lenj = 1 + lv;
-                Mj = pj + Mv;
-                if (lenj > P.window) {
-                    Mj -= lds64(tv + R_PR);
-                    lenj -= 1;
-                }
-            }
-        } else {
-            double max_mean = -(double)FLT_MAX;
-            uint32_t max_len = 0;
-            for (uint32_t e = e0; e < e1; e += 4u) {
-                const uint32_t v = lds32(e);
-                const bool is_term = (v == term);
-                const uint32_t lv = lds32(v + R_LEN);
-                const uint32_t tv = lds32(v + R_T);
-                const double mean_v = lds64(v + R_MEAN);
-                const double Mv = lds64(v + R_M);
-                const bool take = is_term ? (P.thresh > max_mean + tol)
-                                          : ((mean_v > max_mean + tol) || (max_mean - mean_v <= tol && lv > max_len));
-                if (!take) continue;
-                Mj = pj + Mv;
-                lenj = 1 + lv;
-                prevj = v;
-                if (lenj > P.window) {
-                    Mj -= lds64(tv + R_PR);
-                    lenj -= 1;
-                }
-                max_mean = is_term ? P.thresh : mean_v;
-                if (!is_term) max_len = lv;
-            }
-            if (lenj) mlpath_link(a, prevj, steps2);
-        }
-        if (!lenj) {  // dead end (or no acceptable successor): points at the terminus like pandora's default
-#pragma unroll
-            for (int v = 0; v < 8; ++v) sts32(a + R_UP + 4 * v, term);
-        }
-        sts64(a + R_M, Mj);
-        sts32(a + R_LEN, lenj);
-        if (e0w & 1u) sts64(a + R_MEAN, Mj / (double)lenj);  // 0/0 = NaN for a dead end: never chosen, like pandora
-    }
-    uint32_t cnt = 0, p = lds32(recs + R_UP);
-    while (p != term && cnt < n) {
-        path[base + cnt++] = (p - recs) / REC;
-        p = lds32(p + R_UP);
-    }
-    path_len[l] = cnt;
-}
-
-// ---- run-parallel variant ---------------------------------------------------------------------------------
-// Most k-mer nodes have a single successor, so which node follows them is known from the graph alone; only the
-// running sums are sequential.  The host cuts every locus into UNITS in processing order: a node with a choice (or
-// none), or a RUN of up to 32 single-successor nodes j_1 <- j_2 <- ... hanging off an already finished node b.  For
-// a run every pointer a node needs (lifting pointers, window tail T, the node whose score leaves the window) is
-// succ^m(j_i) = j_(i-m) inside the run or a walk of m-i steps from b through finished tables: all 32 lanes resolve
-// their node's pointers at once (independent loads, no stores in between), then lane 0 adds up the sums in pandora's
-// order from staged operands (two dependent DADDs per node instead of ~10 dependent shared-memory hops).
-struct MlUnitsDev {
-    const uint32_t* locus_unit_off;  // n_loci + 1
-    const uint32_t* unit_start;      // n_units + 1 -> unit_nodes
-    const uint32_t* unit_nodes;      // ranks within the locus, chain order (highest rank first)
-};
-
-__device__ __forceinline__ uint32_t ldsx32(uint32_t a, uint32_t token) {  // reorderable load, tied to the unit by `token`
-    uint32_t v;
-    asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a), "r"(token));
-    return v;
-}
-__device__ __forceinline__ double ldsx64(uint32_t a, uint32_t token) {
-    double v;
-    asm("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a), "r"(token));
-    return v;
-}
-__device__ __forceinline__ uint32_t ml_walk(uint32_t x, uint32_t steps, uint32_t token) {
-#pragma unroll
-    for (int l = 0; l < 7; ++l)
-        if ((steps >> l) & 1u) x = ldsx32(x + R_UP + 4 * l, token);
-    return x;
-}
-
-__global__ void mlpath_unit_kernel(uint32_t n_loci, const uint32_t* __restrict__ knode_base, const uint32_t* __restrict__ edge_off,
-                                   const uint32_t* __restrict__ edges, const double* __restrict__ prob,
-                                   const int32_t* __restrict__ locus_reads, const uint8_t* __restrict__ needs_mean,
-                                   MlUnitsDev U, ModelParams P, uint32_t* __restrict__ path, uint32_t* __restrict__ path_len,
-                                   uint32_t max_nodes, uint32_t max_edges) {
-    extern __shared__ double s_dyn[];
-    const uint32_t l = blockIdx.x;
-    if (l >= n_loci) return;
-    const uint32_t lane = threadIdx.x;
-    const uint32_t base = knode_base[l], n = knode_base[l + 1] - base;
-    if (locus_reads[l] <= 0 || n < 2) {
-        if (lane == 0) path_len[l] = 0xffffffffu;
-        return;
-    }
-    const uint32_t e_base = edge_off[base], n_edges = edge_off[base + n] - e_base;
-    const uint32_t recs = (uint32_t)__cvta_generic_to_shared(s_dyn);
-    const uint32_t edg = recs + (max_nodes + 1) * REC;
-    const uint32_t scr = (edg + (max_edges + 1) * 4u + 7u) & ~7u;  // staging: 32 x {p f64, q f64, node u32}
-    const uint32_t s_p = scr, s_q = scr + 256, s_n = scr + 512;
-    for (uint32_t i = lane; i <= n; i += 32) {
-        const uint32_t a = recs + i * REC;
-        if (i < n) sts64(a + R_PR, prob[base + i]);
-        sts32(a + R_EOFF, (edg + (edge_off[base + i] - e_base) * 4u) | (i < n ? (uint32_t)needs_mean[base + i] : 0u));
-    }
-    for (uint32_t i = lane; i < n_edges; i += 32) sts32(edg + i * 4u, recs + edges[e_base + i] * REC);
-    const double tol = 0.000001;
-    const uint32_t term = recs + (n - 1) * REC;
-    const uint32_t W = P.window;
-    if (lane == 0) {
-        sts64(term + R_M, 0.0);
-        sts32(term + R_LEN, 0u);
-#pragma unroll
-        for (int v = 0; v < 8; ++v) sts32(term + R_UP + 4 * v, term);  // includes R_T
-    }
-    __syncwarp();
-    const uint32_t u0 = U.locus_unit_off[l], u1 = U.locus_unit_off[l + 1];
-    for (uint32_t u = u0; u < u1; ++u) {
-        const uint32_t s0 = U.unit_start[u], k = U.unit_start[u + 1] - s0;
-        const uint32_t a1 = recs + U.unit_nodes[s0] * REC;
-        const uint32_t e0w = lds32(a1 + R_EOFF);
-        const uint32_t e0 = e0w & ~3u, e1 = lds32(a1 + REC + R_EOFF) & ~3u;
-        if (e1 - e0 != 4u) {
-            // ---- a node with a choice (or a dead end): pandora's sequential comparison, one lane
-            if (lane == 0) {
-                const uint32_t a = a1;
-                double Mj = 0.0, max_mean = -(double)FLT_MAX;
-                uint32_t lenj = 0, prevj = term, max_len = 0;
-                const double pj = lds64(a + R_PR);
-                for (uint32_t e = e0; e < e1; e += 4u) {
-                    const uint32_t v = lds32(e);
-                    const bool is_term = (v == term);
-                    const uint32_t lv = lds32(v + R_LEN);
-                    const uint32_t tv = lds32(v + R_T);
-                    const double mean_v = lds64(v + R_MEAN);
-                    const double Mv = lds64(v + R_M);
-                    const bool take = is_term ? (P.thresh > max_mean + tol)
-                                              : ((mean_v > max_mean + tol) || (max_mean - mean_v <= tol && lv > max_len));
-                    if (!take) continue;
-                    Mj = pj + Mv;
-                    lenj = 1 + lv;
-                    prevj = v;
-                    if (lenj > W) {
-                        Mj -= lds64(tv + R_PR);
-                        lenj -= 1;
-                    }
-                    max_mean = is_term ? P.thresh : mean_v;
-                    if (!is_term) max_len = lv;
-                }
-                if (lenj) {
-                    mlpath_link(a, prevj, W - 2);
-                } else {
-#pragma unroll
-                    for (int v = 0; v < 8; ++v) sts32(a + R_UP + 4 * v, term);
-                }
-                sts64(a + R_M, Mj);
-                sts32(a + R_LEN, lenj);
-                if (e0w & 1u) sts64(a + R_MEAN, Mj / (double)lenj);
-            }
-            __syncwarp();
-            continue;
-        }
-        // ---- a run of k single-successor nodes hanging off b
-        const uint32_t b = lds32(e0);
-        const uint32_t lb = lds32(b + R_LEN);
-        const double Mb = lds64(b + R_M);
-        const bool active = lane < k;
-        const uint32_t me = active ? recs + U.unit_nodes[s0 + lane] * REC : term;
-        if (b != term && lb == 0u) {  // hanging off a dead end: the whole run is dead (pandora never takes a NaN mean)
-            if (active) {
-#pragma unroll
-                for (int v = 0; v < 8; ++v) sts32(me + R_UP + 4 * v, term);
-                sts64(me + R_M, 0.0);
-                sts32(me + R_LEN, 0u);
-                if (lds32(me + R_EOFF) & 1u) sts64(me + R_MEAN, 0.0 / 0.0);
-            }
-            __syncwarp();
-            continue;
-        }
-        if (active) {
-            const uint32_t i = lane + 1;  // j_i
-            auto succ = [&](uint32_t m) -> uint32_t {  // succ^m(j_i), m >= 1
-                return (m < i) ? recs + U.unit_nodes[s0 + lane - m] * REC : ml_walk(b, m - i, u);
-            };
-            uint32_t up[7];
-#pragma unroll
-            for (int lv = 0; lv < 7; ++lv) up[lv] = succ(1u << lv);
-            const uint32_t T = succ(W - 1);
-            const uint32_t qn = succ(W);  // = T(successor of j_i): its score leaves the window when j_i joins a full one
-            const double p = ldsx64(me + R_PR, u), q = ldsx64(qn + R_PR, u);
-#pragma unroll
-            for (int lv = 0; lv < 7; ++lv) sts32(me + R_UP + 4 * lv, up[lv]);
-            sts32(me + R_T, T);
-            sts64(s_p + 8 * lane, p);
-            sts64(s_q + 8 * lane, q);
-            sts32(s_n + 4 * lane, me);
-        }
-        __syncwarp();
-        if (lane == 0) {
-            double M = Mb;
-            uint32_t len = lb;
-            for (uint32_t i = 0; i < k; ++i) {
-                const uint32_t node = lds32(s_n + 4 * i);
-                M = lds64(s_p + 8 * i) + M;
-                len += 1;
-                if (len > W) {
-                    M -= lds64(s_q + 8 * i);
-                    len = W;
-                }
-                sts64(node + R_M, M);
-                sts32(node + R_LEN, len);
-            }
-        }
-        __syncwarp();
-        if (active && (lds32(me + R_EOFF) & 1u)) sts64(me + R_MEAN, lds64(me + R_M) / (double)lds32(me + R_LEN));
-        __syncwarp();
-    }
-    if (lane == 0) {
-        uint32_t cnt = 0, p = lds32(recs + R_UP);
-        while (p != term && cnt < n) {
-            path[base + cnt++] = (p - recs) / REC;
-            p = lds32(p + R_UP);
-        }
-        path_len[l] = cnt;
-    }
-}
-
-// ---- level-parallel variant --------------------------------------------------------------------------------
-// A node only needs its successors' finished records, so all nodes at the same distance-to-sink ("level": 1 + the
-// largest level among the successors) are independent: the alleles of a bubble advance side by side.  The host
-// sorts every locus by level, single-successor nodes first within a level.  A locus gets a CTA of four warps: warps
-// 0-1 take the level's single-successor nodes, warps 2-3 the nodes with a choice, one node per lane, so the two code
-// paths run on different schedulers instead of serialising inside one warp (a lone warp issues one instruction every
-// ~6 cycles here: the kernel is bound by its own instruction latency, not by shared memory).  Each node runs exactly
-// the per-node step of mlpath_rec_kernel (successors still visited in rank order, so pandora's order-dependent
-// tie-breaking is unchanged); the CTA synchronises between levels.  The serial chain shrinks from the number of nodes
-// to the number of levels (benchmark panel: 38 251 nodes -> 15 128 levels, widest level 22 nodes).
 // sum / length on the level kernel's critical path.  The length is an integer <= 128, so the correctly rounded quotient
 // comes from a table of correctly rounded reciprocals and two Markstein corrections (q += fma(-q, n, a) * y): five
 // dependent FP64 operations instead of the ~15 of the generic division sequence.  The first correction makes q
@@ -610,7 +314,7 @@ __device__ __forceinline__ double div_small(double a, uint32_t n) {
     return q;
 }
 
-// The level kernel's own record layout (64 B), arranged for vector shared-memory accesses: a lone warp per scheduler
+// The record layout (64 B), arranged for vector shared-memory accesses: a lone warp per scheduler
 // pays ~6 cycles per instruction, so fewer, wider accesses matter more than anything else here.
 //   0 sum f64 | 8 mean f64 | 16 score f64 | 24 len u32 | 28 T u32 | 32 edge-list address u32 | 36 up[0..6] u32
 // sum+mean come with one LDS.128, len+T with one LDS.64; up[1..6] sit at 40/48/56 and are stored as three STS.64.
@@ -625,8 +329,10 @@ __device__ __forceinline__ void lds_len_t(uint32_t a, uint32_t& len, uint32_t& t
 __device__ __forceinline__ void sts_pair32(uint32_t addr, uint32_t x, uint32_t y) {
     asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(x), "r"(y));
 }
-// lifting pointers of a (successor v) and T(a) = succ^(window-2)(v): the two pointer chases are issued interleaved like
-// mlpath_link; the stores are batched: up[0] | (up[1],up[2]) | (up[3],up[4]) | (up[5],up[6]); T is returned
+// After the successor v of node a is known, two pointer chases remain, both through the records of finished nodes only
+// and therefore independent of each other and of the fp chain: the lifting pointers of a (level l of a = level l-1 of the
+// node 2^(l-1) steps down) and T(a) = succ^(window-2)(v).  Their loads are issued interleaved so the two chains overlap
+// instead of adding up.  The stores are batched: up[0] | (up[1],up[2]) | (up[3],up[4]) | (up[5],up[6]); T is returned.
 __device__ __forceinline__ uint32_t level_link(uint32_t a, uint32_t v, uint32_t steps2) {
     uint32_t up[7];
     up[0] = v;
@@ -648,12 +354,20 @@ __device__ __forceinline__ uint32_t level_link(uint32_t a, uint32_t v, uint32_t 
     return t;
 }
 
+// The level order built at index load: the levels of locus l are locus_level_off[l] .. locus_level_off[l + 1] - 1, and
+// level u holds the nodes level_nodes[level_start[u] .. level_start[u + 1]), single-successor nodes first.
+struct MlLevelsDev {
+    const uint32_t* locus_level_off;  // n_loci + 1 -> levels
+    const uint32_t* level_start;      // n_levels + 1 -> level_nodes
+    const uint32_t* level_nodes;      // ranks within the locus
+};
+
 constexpr int ML_LEVEL_THREADS = 128;
 constexpr uint32_t ML_FAN = 4;  // successors whose records are fetched side by side (nodes with more take the serial loop)
 __global__ void __launch_bounds__(ML_LEVEL_THREADS) mlpath_level_kernel(
     uint32_t n_loci, const uint32_t* __restrict__ knode_base, const uint32_t* __restrict__ edge_off,
     const uint32_t* __restrict__ edges, const double* __restrict__ prob, const int32_t* __restrict__ locus_reads,
-    const uint8_t* __restrict__ needs_mean, MlUnitsDev L, const uint32_t* __restrict__ level_singles, ModelParams P,
+    const uint8_t* __restrict__ needs_mean, MlLevelsDev L, const uint32_t* __restrict__ level_singles, ModelParams P,
     uint32_t* __restrict__ path, uint32_t* __restrict__ path_len, uint32_t max_nodes, uint32_t max_edges,
     volatile uint32_t* done,     // done != nullptr: path / path_len are host-mapped and done[l] tells the host that locus l is there
     const double* d_thresh) {    // != nullptr: the probability threshold is read from device memory (computed by prob_thresh_kernel)
@@ -706,14 +420,14 @@ __global__ void __launch_bounds__(ML_LEVEL_THREADS) mlpath_level_kernel(
         for (uint32_t u = 0; u < UNR; ++u)
             if (i0 + u * ML_LEVEL_THREADS < n_edges) sts32(edg + (i0 + u * ML_LEVEL_THREADS) * 4u, recs + e[u] * REC);
     }
-    const uint32_t u0 = L.locus_unit_off[l], n_levels = L.locus_unit_off[l + 1] - u0;
-    const uint32_t s00 = L.unit_start[u0];
+    const uint32_t u0 = L.locus_level_off[l], n_levels = L.locus_level_off[l + 1] - u0;
+    const uint32_t s00 = L.level_start[u0];
     for (uint32_t i0 = tid; i0 <= n_levels; i0 += STEP) {
         uint32_t us[UNR], ls[UNR];
 #pragma unroll
         for (uint32_t u = 0; u < UNR; ++u) {
             const uint32_t i = i0 + u * ML_LEVEL_THREADS;
-            us[u] = i <= n_levels ? L.unit_start[u0 + i] : 0u;
+            us[u] = i <= n_levels ? L.level_start[u0 + i] : 0u;
             ls[u] = i < n_levels ? level_singles[u0 + i] : 0u;
         }
 #pragma unroll
@@ -725,7 +439,7 @@ __global__ void __launch_bounds__(ML_LEVEL_THREADS) mlpath_level_kernel(
     for (uint32_t i0 = tid; i0 + 1 < n; i0 += STEP) {
         uint32_t un[UNR];
 #pragma unroll
-        for (uint32_t u = 0; u < UNR; ++u) un[u] = i0 + u * ML_LEVEL_THREADS + 1 < n ? L.unit_nodes[s00 + i0 + u * ML_LEVEL_THREADS] : 0u;
+        for (uint32_t u = 0; u < UNR; ++u) un[u] = i0 + u * ML_LEVEL_THREADS + 1 < n ? L.level_nodes[s00 + i0 + u * ML_LEVEL_THREADS] : 0u;
 #pragma unroll
         for (uint32_t u = 0; u < UNR; ++u)
             if (i0 + u * ML_LEVEL_THREADS + 1 < n) sts32(lvn + 4u * (i0 + u * ML_LEVEL_THREADS), recs + un[u] * REC);
@@ -893,56 +607,32 @@ __global__ void __launch_bounds__(ML_LEVEL_THREADS) mlpath_level_kernel(
 bool launch_mlpath(uint32_t n_loci, const uint32_t* d_knode_base, const uint32_t* d_edge_off, const uint32_t* d_edges,
                    const double* d_prob, const int32_t* d_locus_reads, ModelParams P, double* d_M, uint32_t* d_len,
                    uint32_t* d_up, uint32_t total_knodes, uint32_t* d_path, uint32_t* d_path_len,
-                   uint32_t max_locus_knodes, uint32_t max_locus_edges, const uint8_t* d_needs_mean,
-                   const uint32_t* d_locus_unit_off, const uint32_t* d_unit_start, const uint32_t* d_unit_nodes,
-                   float mean_run_len, cudaStream_t st, const uint32_t* d_locus_level_off, const uint32_t* d_level_start,
-                   const uint32_t* d_level_nodes, const uint32_t* d_level_singles, uint32_t* h_path, uint32_t* h_path_len,
-                   uint32_t* h_done, const double* d_thresh) {
+                   uint32_t max_locus_knodes, uint32_t max_locus_edges, const uint8_t* d_needs_mean, cudaStream_t st,
+                   const uint32_t* d_locus_level_off, const uint32_t* d_level_start, const uint32_t* d_level_nodes,
+                   const uint32_t* d_level_singles, uint32_t* h_path, uint32_t* h_path_len, uint32_t* h_done,
+                   const double* d_thresh) {
     if (!n_loci) return false;
-    {   // default: level-parallel kernel (any of the older switches selects the older kernels)
-        static const bool levels_on = [] {
-            const char* e = getenv("DRPRG_MLPATH_LEVELS");
-            if (e) return atoi(e) != 0;
-            return !getenv("DRPRG_MLPATH_UNITS") && !getenv("DRPRG_MLPATH_GENERIC");
-        }();
-        const size_t lvl_smem = ((size_t)max_locus_knodes + 1) * REC + (size_t)(max_locus_edges + 1) * 4 + (size_t)max_locus_knodes * 12 + 32;
-        if (levels_on && d_level_nodes && d_level_singles && d_needs_mean && P.window >= 2 && P.window <= 128 && lvl_smem <= 220u * 1024u) {
-            ensure_dyn_smem(mlpath_level_kernel, lvl_smem);
-            MlUnitsDev L{d_locus_level_off, d_level_start, d_level_nodes};
-            upload_rcp_table();
-            const bool streamed = h_path && h_path_len && h_done;  // results straight into host-mapped memory, locus by locus
-            mlpath_level_kernel<<<n_loci, ML_LEVEL_THREADS, lvl_smem, st>>>(
-                n_loci, d_knode_base, d_edge_off, d_edges, d_prob, d_locus_reads, d_needs_mean, L, d_level_singles, P,
-                streamed ? h_path : d_path, streamed ? h_path_len : d_path_len, max_locus_knodes, max_locus_edges,
-                streamed ? h_done : nullptr, d_thresh);
-            ++g_launches;
-            return streamed;
-        }
+    // the level-parallel kernel when the largest locus fits in shared memory; otherwise the generic kernel below, which
+    // DRPRG_MLPATH_GENERIC also forces
+    static const bool force_generic = getenv("DRPRG_MLPATH_GENERIC") != nullptr;
+    const size_t lvl_smem = ((size_t)max_locus_knodes + 1) * REC + (size_t)(max_locus_edges + 1) * 4 + (size_t)max_locus_knodes * 12 + 32;
+    if (!force_generic && d_level_nodes && d_level_singles && d_needs_mean && P.window >= 2 && P.window <= 128 && lvl_smem <= 220u * 1024u) {
+        ensure_dyn_smem(mlpath_level_kernel, lvl_smem);
+        MlLevelsDev L{d_locus_level_off, d_level_start, d_level_nodes};
+        upload_rcp_table();
+        const bool streamed = h_path && h_path_len && h_done;  // results straight into host-mapped memory, locus by locus
+        mlpath_level_kernel<<<n_loci, ML_LEVEL_THREADS, lvl_smem, st>>>(
+            n_loci, d_knode_base, d_edge_off, d_edges, d_prob, d_locus_reads, d_needs_mean, L, d_level_singles, P,
+            streamed ? h_path : d_path, streamed ? h_path_len : d_path_len, max_locus_knodes, max_locus_edges,
+            streamed ? h_done : nullptr, d_thresh);
+        ++g_launches;
+        return streamed;
     }
-    if (d_thresh) {  // the older kernels take the threshold by value: one small read-back
+    if (d_thresh) {  // the generic kernel takes the threshold by value: one small read-back
         double t = P.thresh;
         cudaMemcpyAsync(&t, d_thresh, sizeof t, cudaMemcpyDeviceToHost, st);
         cudaStreamSynchronize(st);
         P.thresh = t;
-    }
-    // The run-parallel kernel pays ~1.5k cycles of per-unit overhead (warp syncs, ~50 loads per lane): it wins when
-    // runs of single-successor nodes are long (sparse panels) and loses on bubble-dense graphs (the benchmark panel:
-    // 32 % of the nodes have a choice, mean run 2.6 nodes: 1.23 ms vs 0.78 ms for the chain kernel), so among the older
-    // kernels it is chosen by run length; the level-parallel kernel above is the default.
-    static const char* force_units = getenv("DRPRG_MLPATH_UNITS");
-    const bool want_units = force_units ? atoi(force_units) != 0 : mean_run_len >= 8.0f;
-    if (want_units) {
-        const size_t unit_smem = ((size_t)max_locus_knodes + 1) * REC + (size_t)(max_locus_edges + 1) * 4 + 8 + 32 * 20;
-        static const bool no_units = getenv("DRPRG_MLPATH_GENERIC") != nullptr;
-        if (P.window >= 2 && P.window <= 127 && unit_smem <= 220u * 1024u && !no_units && d_needs_mean && d_unit_nodes) {
-            ensure_dyn_smem(mlpath_unit_kernel, unit_smem);
-            MlUnitsDev U{d_locus_unit_off, d_unit_start, d_unit_nodes};
-            mlpath_unit_kernel<<<n_loci, 32, unit_smem, st>>>(n_loci, d_knode_base, d_edge_off, d_edges, d_prob, d_locus_reads,
-                                                             d_needs_mean, U, P, d_path, d_path_len, max_locus_knodes,
-                                                             max_locus_edges);
-            ++g_launches;
-            return false;
-        }
     }
     // shared memory: per k-mer node sum, mean, score (f64), length, LV lifting pointers, edge offset (u32);
     // per edge one u32.  Up to the 227 KB a CTA may own; larger loci fall back to global memory.
@@ -957,17 +647,6 @@ bool launch_mlpath(uint32_t n_loci, const uint32_t* d_knode_base, const uint32_t
         smem_edges = (uint32_t)((budget / 2) / 4);
     }
     const size_t smem = (size_t)smem_nodes * per_node + 16 + 4 * (size_t)smem_edges;
-    {
-        const size_t rec_smem = ((size_t)max_locus_knodes + 1) * REC + (size_t)(max_locus_edges + 1) * 4;
-        static const bool force_generic = getenv("DRPRG_MLPATH_GENERIC") != nullptr;
-        if (P.window >= 2 && P.window <= 128 && rec_smem <= budget && !force_generic && d_needs_mean) {
-            ensure_dyn_smem(mlpath_rec_kernel, rec_smem);
-            mlpath_rec_kernel<<<n_loci, 32, rec_smem, st>>>(n_loci, d_knode_base, d_edge_off, d_edges, d_prob, d_locus_reads,
-                                                           d_needs_mean, P, d_path, d_path_len, max_locus_knodes);
-            ++g_launches;
-            return false;
-        }
-    }
     auto go = [&](auto kernel) {
         ensure_dyn_smem(kernel, smem);
         kernel<<<n_loci, 32, smem, st>>>(n_loci, d_knode_base, d_edge_off, d_edges, d_prob, d_locus_reads, P, d_M, d_len, d_up,

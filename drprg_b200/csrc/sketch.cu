@@ -271,11 +271,8 @@ __global__ void __launch_bounds__(WARPS * 32) sketch_kernel(DevReads R, DevTable
 // ============================================================================================
 constexpr int SHORT_THREADS = 512;
 constexpr uint32_t SMEM_FILTER_BITS = 14;  // a pre-filter of <= 2^14 words (64 KB) is copied into shared memory
-#ifndef DRPRG_DEFAULT_VARIANT
-#define DRPRG_DEFAULT_VARIANT 3
-#endif
 
-template <int W, int K, bool LOOKUP, int VARIANT, bool SMEM_FILTER, int THREADS>
+template <int W, int K, bool LOOKUP, bool SMEM_FILTER, int THREADS>
 __global__ void __launch_bounds__(THREADS) sketch_short_kernel(DevReads R, DevTable T,
                                                                      unsigned long long* __restrict__ out_a,
                                                                      unsigned long long* __restrict__ out_b,
@@ -367,14 +364,13 @@ __global__ void __launch_bounds__(THREADS) sketch_short_kernel(DevReads R, DevTa
         uint32_t* sh = &s_h[b & 1][0][tid];
         refill();
         avail -= (uint32_t)W;
-        // blocks that lie inside every lane's read (all but the last one or two) may skip the per-position padding select
+        // strand and minimizer flags are set by predicated ORs, and full blocks skip the padding select below: of the four
+        // combinations measured in round 1 (with and without each), this one was the fastest
         auto strand_bit = [&](uint32_t hf, uint32_t hr, int j) {
-            if (VARIANT & 1)
-                asm("{\n\t.reg .pred p;\n\tsetp.gt.u32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(not_strand) : "r"(hf), "r"(hr), "r"(1u << (W - 1 - j)));
-            else
-                not_strand |= (hf > hr ? 1u : 0u) << (W - 1 - j);
+            asm("{\n\t.reg .pred p;\n\tsetp.gt.u32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(not_strand) : "r"(hf), "r"(hr), "r"(1u << (W - 1 - j)));
         };
-        if ((VARIANT & 2) && p0 + W <= nk_min) {
+        // blocks that lie inside every lane's read (all but the last one or two) may skip the per-position padding select
+        if (p0 + W <= nk_min) {
 #pragma unroll
             for (int j = 0; j < W; ++j) {
                 next_base();
@@ -416,10 +412,7 @@ __global__ void __launch_bounds__(THREADS) sketch_short_kernel(DevReads R, DevTa
             for (int j = 0; j < W; ++j) {
                 pmax = max(pmax, wm[j]);
                 const uint32_t best = max(pmax, SXo[j + 1]);
-                if (VARIANT & 1)
-                    asm("{\n\t.reg .pred p;\n\tsetp.eq.u32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(flags) : "r"(hp[j]), "r"(best), "r"(1u << j));
-                else
-                    flags |= (hp[j] == best ? 1u : 0u) << j;
+                asm("{\n\t.reg .pred p;\n\tsetp.eq.u32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(flags) : "r"(hp[j]), "r"(best), "r"(1u << j));
             }
         }
         if (b > 0) {
@@ -495,46 +488,32 @@ __global__ void __launch_bounds__(THREADS) sketch_short_kernel(DevReads R, DevTa
     }  // persistent tile loop
 }
 
-template <int W, int K, bool LOOKUP, int V, bool SF>
+template <int W, int K, bool LOOKUP, bool SF>
 static void launch_short_one(const DevReads& R, const DevTable& T, unsigned long long* a, unsigned long long* b,
                              unsigned long long* cnt, uint64_t cap, int sm_count, cudaStream_t st) {
     const size_t smem = (size_t)2 * W * SHORT_THREADS * 4 + (SF ? (size_t)4 << T.filter_bits : 0);
-    ensure_dyn_smem(sketch_short_kernel<W, K, LOOKUP, V, SF, SHORT_THREADS>, (size_t)(2 * W * SHORT_THREADS * 4 + (SF ? (4u << SMEM_FILTER_BITS) : 0)));
+    ensure_dyn_smem(sketch_short_kernel<W, K, LOOKUP, SF, SHORT_THREADS>, (size_t)(2 * W * SHORT_THREADS * 4 + (SF ? (4u << SMEM_FILTER_BITS) : 0)));
     // persistent CTAs: two per SM (register file: 2 x 512 threads x 62 registers), each loops over read tiles
     const unsigned long long n_items = R.seg_read ? R.n_segs : R.n_reads;
     const unsigned long long n_tiles = (n_items + SHORT_THREADS - 1) / SHORT_THREADS;
     const unsigned grid = (unsigned)std::min<unsigned long long>(n_tiles, 2ull * (unsigned)sm_count);
-    sketch_short_kernel<W, K, LOOKUP, V, SF, SHORT_THREADS><<<grid, SHORT_THREADS, smem, st>>>(R, T, a, b, cnt, cap);
+    sketch_short_kernel<W, K, LOOKUP, SF, SHORT_THREADS><<<grid, SHORT_THREADS, smem, st>>>(R, T, a, b, cnt, cap);
     ++g_launches;
 }
 
 template <bool LOOKUP>
 static bool launch_short(const DevReads& R, const DevTable& T, uint32_t w, uint32_t k, unsigned long long* a,
                          unsigned long long* b, unsigned long long* cnt, uint64_t cap, int sm_count, cudaStream_t st) {
-    // two instantiations per (w,k): the default (predicated-OR flag accumulation + padding-free fast path, the fastest
-    // of the four variants measured in round 1) and the plain one as the fallback / second implementation
-    // (DRPRG_SKETCH_VARIANT=0, exercised by the parity tests)
-    static const bool plain = [] {
-        const char* e = getenv("DRPRG_SKETCH_VARIANT");
-        return e && atoi(e) == 0;
-    }();
     const bool sf = LOOKUP && T.filter_bits <= SMEM_FILTER_BITS;
-#define DRPRG_SHORT_V(WW, KK, VV)                                                                             \
-    {                                                                                                         \
-        if (!LOOKUP) launch_short_one<WW, KK, LOOKUP, VV, false>(R, T, a, b, cnt, cap, sm_count, st);         \
-        else if (sf) launch_short_one<WW, KK, LOOKUP, VV, LOOKUP>(R, T, a, b, cnt, cap, sm_count, st);        \
-        else launch_short_one<WW, KK, LOOKUP, VV, false>(R, T, a, b, cnt, cap, sm_count, st);                 \
-        return true;                                                                                          \
-    }
-#define DRPRG_SHORT(WW, KK)                                 \
-    if (w == WW && k == KK) {                               \
-        if (plain && LOOKUP) DRPRG_SHORT_V(WW, KK, 0)       \
-        DRPRG_SHORT_V(WW, KK, DRPRG_DEFAULT_VARIANT)        \
+#define DRPRG_SHORT(WW, KK)                                                                        \
+    if (w == WW && k == KK) {                                                                      \
+        if (sf) launch_short_one<WW, KK, LOOKUP, LOOKUP>(R, T, a, b, cnt, cap, sm_count, st);      \
+        else launch_short_one<WW, KK, LOOKUP, false>(R, T, a, b, cnt, cap, sm_count, st);          \
+        return true;                                                                               \
     }
     DRPRG_SHORT(11, 15)  // drprg defaults (src/builder.rs:40-41)
     DRPRG_SHORT(14, 15)  // pandora's default w, used by the reference's build tests (src/builder.rs:1181)
 #undef DRPRG_SHORT
-#undef DRPRG_SHORT_V
     return false;
 }
 
@@ -564,13 +543,14 @@ void screen_filter_insert(uint32_t* filter, uint32_t n_words, uint32_t kmer, uin
     filter[idx] |= (1u << (kmer & 31u)) | (1u << ((p >> 11) & 31u));
 }
 
-// V: pipe-balance variants (the ALU pipe — SHF/LOP3/LEA — binds first, the multiplier pipe has room):
-//   bit 0: shared-memory address by IMAD with a run-time 4 instead of LEA;  bit 1: the second bit index by
-//   multiply-high with a run-time 2^21 instead of a shift;  bit 2: the flag of a position shifted into its word by a
-//   multiply-add instead of a compare + predicated OR.  Default 5 (bits 0 and 2): measured 0.152 ms against 0.155 for 1
-//   and 0.159 for 0 per million reads; bit 1 never paid.
-struct ScreenConsts { uint32_t four, two21, prefetch, two; };
-template <int K, int CW, int V>
+// Pipe balance: the ALU pipe (SHF/LOP3/LEA) binds first and the multiplier pipe has room, so two per-position steps are
+// moved onto the multiplier: the filter word's shared-memory address is a multiply-add by `four` instead of an LEA, and a
+// position's flag is shifted into its word by a multiply-add by `two` instead of a compare + predicated OR.  Both
+// constants are KERNEL ARGUMENTS on purpose: as compile-time values the compiler folds them straight back into LEA and
+// shifts on the ALU pipe.  Measured 0.152 ms per million reads against 0.155 with the address step alone and 0.159 with
+// neither; a multiply-high for the second bit index as well never paid.
+struct ScreenConsts { uint32_t four, two; };
+template <int K, int CW>
 __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, DevTable T, uint32_t wk, ScreenConsts SC,
                                                                    unsigned long long* __restrict__ queue,
                                                                    uint32_t* __restrict__ queue_kmer,
@@ -590,8 +570,7 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
     const unsigned long long n_tiles = (n_items + 31) / 32;
     const bool wide = R.stride_words && !(R.stride_words & 1u) && !R.seg_read &&
                       (reinterpret_cast<unsigned long long>(R.words) & 7ull) == 0ull;  // every read starts 8-byte aligned
-    // tickets are drawn two tiles ahead: the next tile's id is known when a tile starts, so its words can be
-    // prefetched into L2 while this tile is screened (a cold read otherwise costs the full HBM latency per tile)
+    // tickets are drawn two tiles ahead, so the atomic for the tile after next is in flight while this tile is screened
     unsigned long long tile = 0, next_tile = 0;
     if (lane == 0) {
         tile = atomicAdd(ticket, 1ull);
@@ -602,12 +581,6 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
     while (tile < n_tiles) {
         unsigned long long after_next = 0;
         if (lane == 0) after_next = atomicAdd(ticket, 1ull);  // lands while this tile is screened
-        if (SC.prefetch && !R.seg_read && R.stride_words && next_tile * 32 + lane < n_items) {
-            const uint32_t* np = R.words + (next_tile * 32 + lane) * R.stride_words;
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(np));
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(np + R.stride_words - 1));
-            if (lane == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(R.lens + next_tile * 32));
-        }
         const unsigned long long item = tile * 32 + lane;
         const bool have = item < n_items;
         const unsigned long long r = have ? (R.seg_read ? (unsigned long long)__ldg(R.seg_read + item) : item) : 0ull;
@@ -650,34 +623,19 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
                         const int n = 64 - 2 * (j + K);
                         const uint32_t v = (n >= 32) ? (cw[i] >> ((n - 32) & 31)) : __funnelshift_r(cw[i + 1], cw[i], n & 31);
                         const uint32_t p = v * (SCREEN_MUL << (32 - 2 * K));
-                        uint32_t word;
-                        if (V & 1) {
-                            uint32_t addr;
-                            asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(addr) : "r"(__umulhi(p, n_fw)), "r"(SC.four), "r"(s_base));
-                            asm("ld.shared.u32 %0, [%1];" : "=r"(word) : "r"(addr));
-                        } else {
-                            word = s_kf[__umulhi(p, n_fw)];
-                        }
-                        const uint32_t s2 = (V & 2) ? __umulhi(p, SC.two21) : (p >> 11);
-                        const uint32_t t = __funnelshift_r(word, 0u, v) & __funnelshift_r(word, 0u, s2);
-                        if (V & 4) {
-                            // flags shifted in by a multiply-add (the multiplier pipe has room, the shift/logic pipe does not);
-                            // the word is bit-reversed once at the end
-                            asm("mad.lo.u32 %0, %0, %1, %2;" : "+r"(f[i >> 1]) : "r"(SC.two), "r"(t & 1u));
-                        } else {
-                            asm("{\n\t.reg .pred q;\n\t.reg .b32 t;\n\tand.b32 t, %1, 1;\n\tsetp.ne.u32 q, t, 0;\n\t@q or.b32 %0, %0, %2;\n\t}"
-                                : "+r"(f[i >> 1])
-                                : "r"(t), "r"(1u << ((i & 1) * 16 + j)));
-                        }
+                        uint32_t addr, word;
+                        asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(addr) : "r"(__umulhi(p, n_fw)), "r"(SC.four), "r"(s_base));
+                        asm("ld.shared.u32 %0, [%1];" : "=r"(word) : "r"(addr));
+                        const uint32_t t = __funnelshift_r(word, 0u, v) & __funnelshift_r(word, 0u, p >> 11);
+                        // the flag enters at the bottom of its word; the word is bit-reversed once at the end
+                        asm("mad.lo.u32 %0, %0, %1, %2;" : "+r"(f[i >> 1]) : "r"(SC.two), "r"(t & 1u));
                     }
-                } else if (V & 4) {
+                } else {
                     f[i >> 1] <<= 16;  // a skipped word still occupies its sixteen flag positions
                 }
             }
-            if (V & 4) {
 #pragma unroll
-                for (int i = 0; i < NF; ++i) f[i] = __brev((CW & 1) && i == NF - 1 ? f[i] << 16 : f[i]);
-            }
+            for (int i = 0; i < NF; ++i) f[i] = __brev((CW & 1) && i == NF - 1 ? f[i] << 16 : f[i]);
             // keep the flags of positions inside [seg_s, seg_e), count them, reserve queue space per warp
             uint32_t cnt = 0;
             {
@@ -943,36 +901,15 @@ __global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R,
     if (lane == 0 && n_surv) atomicAdd(survivors, n_surv);
 }
 
-template <int K, int CW, int V>
-static void launch_screen_v(const DevReads& R, const DevTable& T, uint32_t wk, unsigned long long* queue, uint32_t* queue_kmer,
-                            unsigned long long* counters, uint64_t queue_cap, int sm_count, cudaStream_t st) {
-    ensure_dyn_smem(screen_kernel<K, CW, V>, (size_t)SCREEN_MAX_FILTER_WORDS * 4);
-    static const uint32_t prefetch = [] {
-        const char* e = getenv("DRPRG_SCREEN_PREFETCH");  // L2 prefetch of the next tile: measured neutral (cold == warm L2 time), off
-        return e ? (uint32_t)atoi(e) : 0u;
-    }();
+template <int K, int CW>
+static void launch_screen(const DevReads& R, const DevTable& T, uint32_t wk, unsigned long long* queue, uint32_t* queue_kmer,
+                          unsigned long long* counters, uint64_t queue_cap, int sm_count, cudaStream_t st) {
+    ensure_dyn_smem(screen_kernel<K, CW>, (size_t)SCREEN_MAX_FILTER_WORDS * 4);
     const unsigned long long n_items = R.seg_read ? R.n_segs : R.n_reads;
     const unsigned long long n_ctas = (n_items + SCREEN_THREADS - 1) / SCREEN_THREADS;
     const unsigned grid = (unsigned)std::min<unsigned long long>(n_ctas, (unsigned long long)sm_count);  // one persistent CTA per SM
-    screen_kernel<K, CW, V><<<grid, SCREEN_THREADS, (size_t)T.kfilter_words * 4, st>>>(R, T, wk, ScreenConsts{4u, 1u << 21, prefetch, 2u}, queue, queue_kmer, counters, queue_cap, counters + 1);
+    screen_kernel<K, CW><<<grid, SCREEN_THREADS, (size_t)T.kfilter_words * 4, st>>>(R, T, wk, ScreenConsts{4u, 2u}, queue, queue_kmer, counters, queue_cap, counters + 1);
     ++g_launches;
-}
-
-#ifndef DRPRG_SCREEN_DEFAULT_VARIANT
-#define DRPRG_SCREEN_DEFAULT_VARIANT 5
-#endif
-template <int K, int CW>
-static void launch_screen_one(const DevReads& R, const DevTable& T, uint32_t wk, unsigned long long* queue, uint32_t* queue_kmer,
-                              unsigned long long* counters, uint64_t queue_cap, int sm_count, cudaStream_t st) {
-    static const int variant = [] {
-        const char* e = getenv("DRPRG_SCREEN_VARIANT");
-        return e ? atoi(e) & 7 : DRPRG_SCREEN_DEFAULT_VARIANT;
-    }();
-    switch (variant) {  // the default and the plain kernel (second implementation for the parity tests)
-        case 0: return launch_screen_v<K, CW, 0>(R, T, wk, queue, queue_kmer, counters, queue_cap, sm_count, st);
-        case 1: return launch_screen_v<K, CW, 1>(R, T, wk, queue, queue_kmer, counters, queue_cap, sm_count, st);
-        default: return launch_screen_v<K, CW, 5>(R, T, wk, queue, queue_kmer, counters, queue_cap, sm_count, st);
-    }
 }
 
 // counters = the CTR_QUEUE.. slots of the batch counters
@@ -1004,8 +941,8 @@ static void launch_screened(const DevReads& R, const DevTable& T, uint32_t w, un
                             unsigned long long* queue, uint32_t* queue_kmer, uint64_t queue_cap, unsigned long long* counters,
                             cudaStream_t st) {
     cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned long long), st);
-    if (!R.seg_read && max_len >= (uint32_t)K && max_len - K + 1 <= 10 * 16) launch_screen_one<K, 10>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
-    else launch_screen_one<K, 8>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
+    if (!R.seg_read && max_len >= (uint32_t)K && max_len - K + 1 <= 10 * 16) launch_screen<K, 10>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
+    else launch_screen<K, 8>(R, T, w + K, queue, queue_kmer, counters, queue_cap, sm_count, st);
     if (w == 11) launch_resolve<11, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);
     else if (w == 14) launch_resolve<14, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);
     else launch_resolve<0, K>(R, T, w, queue, queue_kmer, queue_cap, counters, a, b, cnt, cap, sm_count, max_len, st);

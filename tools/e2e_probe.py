@@ -17,7 +17,7 @@ if len(sys.argv) > 1 and sys.argv[1] == "run":
                          genotype_ms=round(st["ms_genotype"], 2), n_reads=st["n_reads"], records=st["n_records"])
     import hashlib
     res["vcf_sha1"] = hashlib.sha1(b"".join(l for l in open(os.path.join(out, "pandora_genotyped.vcf"), "rb") if not l.startswith(b"##fileDate"))).hexdigest()[:12]
-    print(json.dumps({"host_ingest": os.environ.get("DRPRG_HOST_INGEST", "0"), "ingest": os.environ.get("DRPRG_INGEST", "framed"), "mmap": os.environ.get("DRPRG_FRAME_MMAP", "0"), **res}))
+    print(json.dumps({"host_ingest": os.environ.get("DRPRG_HOST_INGEST", "0"), "ingest": os.environ.get("DRPRG_INGEST", "framed"), **res}))
 else:
     from drprg_b200 import workload, sim
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 1000000
@@ -35,5 +35,5 @@ else:
     rec[:, 12 + L:12 + 2 * L] = ord("I"); rec[:, 12 + 2 * L] = 10
     rec.tofile(fq)
     subprocess.run(f"gzip -1 -c {fq} > {gz}", shell=True, check=True)
-    for extra in ({}, {"DRPRG_FRAME_MMAP": "1"}, {"DRPRG_INGEST": "device"}, {"DRPRG_HOST_INGEST": "1"}):
+    for extra in ({}, {"DRPRG_INGEST": "device"}, {"DRPRG_HOST_INGEST": "1"}):
         subprocess.run([sys.executable, __file__, "run", fq, gz, wl.prg_path, wl.refs_path], env=dict(os.environ, **extra))

@@ -9,15 +9,15 @@ set -x
 mkdir -p gpurun_out
 ncu --metrics gpu__time_duration.sum --clock-control none --kernel-name-base demangled -k regex:'drprg::' -c 400 --csv --log-file gpurun_out/r2_launches_final.csv \
     python bench.py --steps 2 --warmup 3 --no-extras --no-cpu-baseline > gpurun_out/r2_launches_final.bench 2>&1
-DRPRG_SCREEN=1 DRPRG_SCREEN_VARIANT=5 ncu --set full --import-source on --clock-control none --cache-control none \
+DRPRG_SCREEN=1 ncu --set full --import-source on --clock-control none --cache-control none \
     -k regex:'screen_kernel|resolve_kernel' --launch-skip 10 -c 2 -f -o gpurun_out/r2_screen4m \
     python tools/screen_bench.py run 4000000 > gpurun_out/r2_screen4m.log 2>&1
 ncu -i gpurun_out/r2_screen4m.ncu-rep --page raw --csv > gpurun_out/r2_screen4m_raw.csv 2>/dev/null
-DRPRG_SCREEN=1 DRPRG_SCREEN_VARIANT=5 ncu --set full --clock-control none --cache-control none \
+DRPRG_SCREEN=1 ncu --set full --clock-control none --cache-control none \
     -k regex:'screen_kernel|resolve_kernel' --launch-skip 10 -c 2 -f -o gpurun_out/r2_screen1m_nc \
     python tools/screen_bench.py run 1000000 > gpurun_out/r2_screen1m_nc.log 2>&1
 ncu -i gpurun_out/r2_screen1m_nc.ncu-rep --page raw --csv > gpurun_out/r2_screen1m_nc_raw.csv 2>/dev/null
-DRPRG_SCREEN=1 DRPRG_SCREEN_VARIANT=5 ncu --set full --clock-control none \
+DRPRG_SCREEN=1 ncu --set full --clock-control none \
     -k regex:'screen_kernel|resolve_kernel' --launch-skip 10 -c 2 -f -o gpurun_out/r2_screen1m \
     python tools/screen_bench.py run 1000000 > gpurun_out/r2_screen1m.log 2>&1
 ncu -i gpurun_out/r2_screen1m.ncu-rep --page raw --csv > gpurun_out/r2_screen1m_raw.csv 2>/dev/null

@@ -1,5 +1,5 @@
 """A/B of the k-mer screen inside one gpurun call: sketch+lookup stage time (device-resident batch, one launch per
-kernel) with the screen on / off and across its pipe-balance variants; the hit set must be identical.
+kernel) with the screen off and on; the hit set must be identical.
    python tools/screen_bench.py [n_reads]"""
 import sys, os, subprocess, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -20,10 +20,10 @@ if len(sys.argv) > 1 and sys.argv[1] == "run":
         ix.sample_begin(opts, 150); nh, nk = ix.map_batch(b); cold.append(ix.last_timings()["sketch_lookup"])
     h = ix.last_hits(nh)
     dig = hashlib.sha1(b"".join(np.ascontiguousarray(h[k]).tobytes() for k in ("read", "prg", "fwd", "start", "knode", "kept"))).hexdigest()
-    print(json.dumps({"screen": os.environ.get("DRPRG_SCREEN"), "variant": os.environ.get("DRPRG_SCREEN_VARIANT"), "exact": os.environ.get("DRPRG_SCREEN_EXACT"), "reads": n,
-                      "sketch_ms_min": round(min(ts[2:]), 4), "sketch_ms_med": round(sorted(ts[2:])[len(ts[2:]) // 2], 4), "cold_ms_min": round(min(cold[1:]), 4), "cold_ms_med": round(sorted(cold[1:])[len(cold[1:]) // 2], 4), "prefetch": os.environ.get("DRPRG_SCREEN_PREFETCH"),
+    print(json.dumps({"screen": os.environ.get("DRPRG_SCREEN"), "reads": n,
+                      "sketch_ms_min": round(min(ts[2:]), 4), "sketch_ms_med": round(sorted(ts[2:])[len(ts[2:]) // 2], 4), "cold_ms_min": round(min(cold[1:]), 4), "cold_ms_med": round(sorted(cold[1:])[len(cold[1:]) // 2], 4),
                       "hits": nh, "kept": nk, "sha1": dig[:12]}))
 else:
     n = sys.argv[1] if len(sys.argv) > 1 else "1000000"
-    for s, v, ex in (("0", "5", "0"), ("1", "0", "0"), ("1", "1", "0"), ("1", "5", "0")):
-        subprocess.run([sys.executable, __file__, "run", n], env=dict(os.environ, DRPRG_SCREEN=s, DRPRG_SCREEN_VARIANT=v, DRPRG_SCREEN_EXACT=ex))
+    for s in ("0", "1"):
+        subprocess.run([sys.executable, __file__, "run", n], env=dict(os.environ, DRPRG_SCREEN=s))
