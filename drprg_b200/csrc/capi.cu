@@ -1405,15 +1405,19 @@ void map_batch_any(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_
     else map_batch(X, B, st, n_hits, n_kept);
 }
 
-// A reads file as a device-resident batch.  Strict 4-line FASTQ (plain or gzip) is parsed and packed ON THE DEVICE
-// (ingest.cu); FASTA and anything unusual goes through the host parser and an upload.  DRPRG_HOST_INGEST=1 forces the
-// host parser (tests compare the two).
+// A reads file as a device-resident batch.  Strict 4-line FASTQ (plain or gzip) is framed on the host and packed on the
+// device (ingest.cu); FASTA and anything unusual goes through the host parser and an upload.  DRPRG_HOST_INGEST=1 forces
+// the host parser (tests compare the two).
 struct FileBatch {
     drprg_batch* B = nullptr;
     uint64_t n_dropped = 0;
     uint32_t first_read_len = 0;
-    bool on_device = false;
+    bool on_device = false;  // packed on the device (else: host parser)
 };
+bool host_ingest_forced() {
+    static const bool on = getenv("DRPRG_HOST_INGEST") != nullptr && atoi(getenv("DRPRG_HOST_INGEST")) != 0;
+    return on;
+}
 struct Inflated {  // a gzip reads file inflated ahead of time (batch mode)
     char* p = nullptr;
     size_t n = 0;
@@ -1432,6 +1436,37 @@ struct Inflated {  // a gzip reads file inflated ahead of time (batch mode)
         return *this;
     }
     ~Inflated() { free(p); }
+};
+
+// The whole text of a reads file for the framer: a gzip file is inflated into host memory on all host threads
+// (gzip_inflate.cpp) unless the batch driver has done that already (`pre`); a plain file is read in place with pread.
+struct ReadsText {
+    TextSource src;
+    Inflated local;
+    ReadsText(const char* path, const Inflated* pre) {
+        if (!pre && file_is_gzip(path)) {
+            inflate_file(path, &local.p, &local.n);
+            pre = &local;
+        }
+        if (pre) {
+            src.mem = pre->p;
+            src.size = pre->n;
+            return;
+        }
+        src.fd = open(path, O_RDONLY);
+        if (src.fd < 0) throw std::runtime_error(std::string("cannot open ") + path);
+        src.size = (size_t)lseek(src.fd, 0, SEEK_END);
+    }
+    ReadsText(const ReadsText&) = delete;
+    ReadsText& operator=(const ReadsText&) = delete;
+    ~ReadsText() {
+        if (src.fd >= 0) close(src.fd);
+    }
+    // FASTA, leading blank lines and files too small for one record go to the host parser without being framed
+    bool may_be_fastq() const {
+        char first = 0;
+        return src.size >= 8 && src.read(&first, 0, 1) == 1 && first == '@';
+    }
 };
 
 // the packed reads an ingest left on the device, as a batch of this index
@@ -1456,56 +1491,51 @@ drprg_batch* batch_from_ingest(drprg_index* X, const IngestResult& I, uint32_t r
     return B.release();
 }
 
-FileBatch batch_from_file(drprg_index* X, const char* reads_path, uint32_t threads, const Inflated* pre = nullptr) {
+// the host parser's batch; a multi-GPU handle gets one shard of the reads per GPU
+FileBatch host_parsed_batch(drprg_index* X, const char* reads_path, uint32_t threads) {
     need_device(X);
     CK(cudaSetDevice(X->device));
-    FileBatch F;
-    if (is_multi(X)) {  // one shard of the reads per GPU
-        PackedReads pr;
-        load_reads_packed(reads_path, threads, pr);
-        const uint64_t n = pr.lens.size();
-        if (n > 0xfffffff0ull) throw std::runtime_error("more than 2^32 reads in one sample");
-        F.B = multi_upload(X, pr.words.data(), pr.word_off.data(), 0, pr.lens.data(), n, pr.total_bases, 0);
-        F.n_dropped = pr.n_dropped;
-        F.first_read_len = pr.first_read_len;
-        return F;
-    }
-    static const bool host_only = getenv("DRPRG_HOST_INGEST") != nullptr && atoi(getenv("DRPRG_HOST_INGEST")) != 0;
-    // gzip: the whole stream is inflated on all host threads first (gzip_inflate.cpp; zlib's one-core gzread only for
-    // streams the parallel decoder declines), then the text takes the same device path as a plain file
-    Inflated local;
-    if (!pre && !host_only && file_is_gzip(reads_path)) {
-        inflate_file(reads_path, &local.p, &local.n);
-        pre = &local;
-    }
-    IngestResult I;
-    const int dev = X->device;
-    if (!host_only && ingest_fastq_device(reads_path, X->device, threads, I, 0, [dev](size_t bytes) { return g_pool.get(bytes, dev); },
-                                          pre ? pre->p : nullptr, pre ? pre->n : 0)) {
-        std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(batch_from_ingest(X, I, 0), free_batch);
-        F.B = B.release();
-        F.n_dropped = I.n_dropped;
-        F.first_read_len = I.first_read_len;
-        F.on_device = true;
-        return F;
-    }
     PackedReads pr;
     load_reads_packed(reads_path, threads, pr);
     const uint64_t n = pr.lens.size();
     if (n > 0xfffffff0ull) throw std::runtime_error("more than 2^32 reads in one sample");
-    F.B = upload_batch(X, pr.words.data(), pr.word_off.data(), 0, pr.lens.data(), n, pr.total_bases, 0, 0);
-    CK(cudaStreamSynchronize(0));  // pr dies with this scope
+    FileBatch F;
+    if (is_multi(X)) {
+        F.B = multi_upload(X, pr.words.data(), pr.word_off.data(), 0, pr.lens.data(), n, pr.total_bases, 0);
+    } else {
+        F.B = upload_batch(X, pr.words.data(), pr.word_off.data(), 0, pr.lens.data(), n, pr.total_bases, 0, 0);
+        CK(cudaStreamSynchronize(0));  // pr dies with this scope
+    }
     F.n_dropped = pr.n_dropped;
     F.first_read_len = pr.first_read_len;
     return F;
+}
+
+FileBatch batch_from_file(drprg_index* X, const char* reads_path, uint32_t threads) {
+    need_device(X);
+    if (!is_multi(X) && !host_ingest_forced()) {
+        CK(cudaSetDevice(X->device));
+        const ReadsText T(reads_path, nullptr);
+        IngestResult I;
+        const int dev = X->device;
+        if (T.may_be_fastq() && ingest_fastq_text(T.src, dev, threads, I, 0, [dev](size_t bytes) { return g_pool.get(bytes, dev); })) {
+            FileBatch F;
+            F.B = batch_from_ingest(X, I, 0);
+            F.n_dropped = I.n_dropped;
+            F.first_read_len = I.first_read_len;
+            F.on_device = true;
+            return F;
+        }
+    }
+    return host_parsed_batch(X, reads_path, threads);
 }
 
 // A reads file of any size, mapped wave by wave: plain strict FASTQ (or a gzip file inflated into host memory) is cut at
 // record starts into waves of ~1 GiB of text; every wave is framed on the host, uploaded (sequence lines only), packed and
 // mapped into the sample's accumulators before the next one is read, so a 30 M-read file (9.4 GB of text, BASELINE
 // config 3) needs 0.5 GiB of pinned and 1 GiB of device memory instead of the whole text, and files beyond the 8 GB limit
-// of one ingest still take the fast path.  false = the general path (batch_from_file) must handle the file; a sample
-// that was begun here is begun again there.
+// of one ingest still take the fast path.  false = the host parser must handle the file; a sample that was begun here is
+// begun again there.
 struct WaveTotals {
     uint64_t n = 0, dropped = 0, bases = 0, hits = 0, kept = 0;
     uint32_t first_len = 0;
@@ -1513,12 +1543,7 @@ struct WaveTotals {
     double ms_ingest = 0, ms_map = 0;
 };
 bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_opts* o, const Inflated* pre, WaveTotals& W) {
-    static const bool off = [] {
-        const char* h = getenv("DRPRG_HOST_INGEST");
-        const char* d = getenv("DRPRG_INGEST");
-        return (h && atoi(h) != 0) || (d && std::string(d) == "device");
-    }();
-    if (off) return false;
+    if (host_ingest_forced()) return false;
     // A multi-GPU handle maps the file on its root GPU: a file-fed sample is bound by the host's framing rate (~45 GB/s of
     // text on 16 cores against 1.9 ms of GPU time per 10 M reads), so sharding the waves would leave every GPU idle
     // anyway; read sharding pays for batches that are already packed (drprg_cuda_batch_upload).
@@ -1526,29 +1551,9 @@ bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_o
         const char* e = getenv("DRPRG_WAVE_BYTES");
         return e && atol(e) > 0 ? (size_t)atol(e) : (size_t)(1u << 30);
     }();
-    TextSource F;
-    struct Closer {
-        int fd = -1;
-        ~Closer() {
-            if (fd >= 0) close(fd);
-        }
-    } closer;
-    Inflated local;
-    if (!pre && file_is_gzip(reads_path)) {  // gzip: inflated on all host threads first (gzip_inflate.cpp)
-        inflate_file(reads_path, &local.p, &local.n);
-        pre = &local;
-    }
-    if (pre) {
-        F.mem = pre->p;
-        F.size = pre->n;
-    } else {
-        closer.fd = open(reads_path, O_RDONLY);
-        if (closer.fd < 0) throw std::runtime_error(std::string("cannot open ") + reads_path);
-        F.fd = closer.fd;
-        F.size = (size_t)lseek(closer.fd, 0, SEEK_END);
-    }
-    char first = 0;
-    if (F.size < 8 || F.read(&first, 0, 1) != 1 || first != '@') return false;
+    const ReadsText T(reads_path, pre);
+    if (!T.may_be_fastq()) return false;
+    const TextSource& F = T.src;
     const uint32_t threads = o ? std::max(1u, o->threads) : 1u;
     const int dev = X->device;
     std::vector<char> scratch;
@@ -1599,7 +1604,6 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
         uint64_t n_dropped, total_bases;
     } pr{0, 0};
     uint64_t nh = 0, nk = 0, n = 0;
-    bool on_device = true;
     size_t waves = 0;
     double t1 = t0, wave_ingest_ms = -1, wave_map_ms = 0;
     WaveTotals W;
@@ -1613,11 +1617,12 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
         wave_ingest_ms = W.ms_ingest;  // ingest and map alternate wave by wave
         wave_map_ms = W.ms_map;
     } else {
-        FileBatch F = batch_from_file(X, reads_path, o ? o->threads : 1, pre);
+        // Not strict 4-line FASTQ, or host ingest forced.  Framing the whole file would decline as well: it runs the same
+        // framer over the same records as the waves, and it takes at most 8 GB of text where the waves take any size.
+        FileBatch F = host_parsed_batch(X, reads_path, o ? o->threads : 1);
         std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(F.B, free_batch);
         pr.n_dropped = F.n_dropped;
         pr.total_bases = B->total_bases;
-        on_device = F.on_device;
         t1 = now_ms();
         sample_begin_any(X, o, F.first_read_len);
         n = B->R.n_reads;
@@ -1645,7 +1650,7 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
     if (stats) *stats = s;
     log << "drprg-cuda map: reads=" << n << " dropped=" << pr.n_dropped << " bases=" << pr.total_bases << " hits=" << nh
         << " kept=" << nk << " loci=" << s.n_loci_present << " records=" << s.n_records << " E=" << s.exp_depth_covg
-        << " ingest=" << (waves ? "host-framed, " + std::to_string(waves) + " wave(s)" : on_device ? "device" : "host") << "\nkernel ms: sketch_lookup=" << X->timings[0] << " sort=" << X->timings[1] << " cluster=" << X->timings[2]
+        << " ingest=" << (waves ? "host-framed, " + std::to_string(waves) + " wave(s)" : "host") << "\nkernel ms: sketch_lookup=" << X->timings[0] << " sort=" << X->timings[1] << " cluster=" << X->timings[2]
         << " coverage=" << X->timings[3] << "\nwall ms: ingest=" << s.ms_ingest << " map=" << s.ms_map
         << " genotype=" << s.ms_genotype << " total=" << s.ms_total << "\n";
     return 0;
@@ -1805,19 +1810,12 @@ int drprg_cuda_frame_fastq(const char* path, uint32_t threads, uint8_t** ascii, 
     *lens = nullptr;
     *n_reads = *total_bases = 0;
     *is_fastq = 0;
-    TextSource src;
-    src.fd = open(path, O_RDONLY);
-    if (src.fd < 0) throw std::runtime_error(std::string("cannot open ") + path);
-    struct Closer {
-        int fd;
-        ~Closer() { close(fd); }
-    } closer{src.fd};
-    src.size = (size_t)lseek(src.fd, 0, SEEK_END);
-    char first = 0;
-    if (src.size < 8 || src.read(&first, 0, 1) != 1 || first != '@') return 0;
-    std::vector<char> buf(src.size / 2 + 64);
+    if (file_is_gzip(path)) return 0;  // plain files only
+    const ReadsText T(path, nullptr);
+    if (!T.may_be_fastq()) return 0;
+    std::vector<char> buf(T.src.size / 2 + 64);
     std::vector<FramedSlice> sl;
-    if (!fastq_frame_text(src, threads, buf.data(), sl)) return 0;
+    if (!fastq_frame_text(T.src, threads, buf.data(), sl)) return 0;
     uint64_t n = 0, bases = 0;
     for (const FramedSlice& z : sl) {
         n += z.st.n_reads;

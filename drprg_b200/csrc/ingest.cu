@@ -1,19 +1,12 @@
 // Ingest of 4-line FASTQ (plain, or gzip inflated into host memory), SURVEY.md §8f rank 2: the reads file that `drprg
 // predict` hands to the map step (/root/reference/src/predict.rs:166-170, 288-294) becomes a 2-bit packed batch in HBM.
-// Default path (ingest_fastq_text / ingest_fastq_framed): the record structure is found on the HOST (fastq_frame.cpp),
-// only the sequence lines and a (start, length) table cross PCIe, and the device packs:
+// The record structure is found on the HOST (fastq_frame.cpp), only the sequence lines and a (start, length) table cross
+// PCIe, and the device packs:
 //   pack_stride/ragged  ASCII -> 2-bit words (first base in the top bits), non-ACGT reads flagged
 //   finish_lens         lens[r] = 0 for a flagged read (pandora drops it), dropped-read count
-// Second implementation (ingest_fastq_device with DRPRG_INGEST=device; the round-1 path, kept for A/B and parity): the
-// RAW TEXT goes to the GPU through two pinned staging buffers and is parsed there:
-//   newline_positions   cub::DeviceSelect over the text -> offsets of every '\n'
-//   fastq_records       one thread per record: checks the '@' / '+' framing, sequence start and length ('\r' stripped)
-// Anything that is not strict 4-line FASTQ (FASTA, wrapped records, blank lines) is left to the general host parser
-// (load_reads_packed), which produces the same packed layout.
+// Anything that is not strict 4-line FASTQ (FASTA, wrapped records, blank lines, damaged records) is left to the general
+// host parser (load_reads_packed), which produces the same packed layout.
 #include <cuda_runtime.h>
-#include <fcntl.h>
-#include <unistd.h>
-#include <zlib.h>
 
 #include <algorithm>
 #include <atomic>
@@ -21,9 +14,6 @@
 #include <cstdio>
 #include <cstring>
 #include <functional>
-#include <cub/cub.cuh>
-#include <thrust/iterator/counting_iterator.h>
-#include <thrust/iterator/transform_iterator.h>
 #include <mutex>
 #include <stdexcept>
 #include <string>
@@ -44,27 +34,20 @@ namespace {
             throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e__) + " at " #call); \
     } while (0)
 
-constexpr size_t STAGE_BYTES = 32u << 20;
 double now_ms_i() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-struct Staging {  // process-wide pinned double buffer + grow-only device text / scratch buffers (one ingest at a time)
+struct Staging {  // process-wide grow-only pinned and device buffers (one ingest at a time)
     std::mutex m;
-    char* pinned[2] = {nullptr, nullptr};
-    cudaEvent_t done[2] = {nullptr, nullptr};
     int device = -1;
-    char* d_text = nullptr;
+    char* d_text = nullptr;  // the sequence lines
     size_t text_cap = 0;
-    uint32_t* d_nl = nullptr;
-    size_t nl_cap = 0;
-    void* d_temp = nullptr;
-    size_t temp_cap = 0;
     uint32_t* d_rec = nullptr;  // per record: sequence start | raw length | bad flag (3 x rec_cap)
     size_t rec_cap = 0;
-    unsigned long long* d_scalars = nullptr;  // [0] n newlines, [1] bad framing, [2] max len, [3] total bases, [4] dropped
+    unsigned long long* d_scalars = nullptr;  // [4] dropped reads (finish_lens_kernel)
     unsigned long long* h_scalars = nullptr;
-    char* pinned_seq = nullptr;  // host-framed path: the sequence lines of the whole file
+    char* pinned_seq = nullptr;  // the sequence lines, framed on the host
     size_t seq_cap = 0;
-    uint32_t* h_rec = nullptr;   // host-framed path: sequence start | length per read (2 x hrec_cap)
+    uint32_t* h_rec = nullptr;   // sequence start | length per read (2 x hrec_cap)
     size_t hrec_cap = 0;
     void ensure_seq(size_t bytes) {
         if (bytes <= seq_cap) return;
@@ -84,83 +67,35 @@ struct Staging {  // process-wide pinned double buffer + grow-only device text /
         ICK(cudaMallocHost(&h_rec, want * 2 * sizeof(uint32_t)));
         hrec_cap = want;
     }
-    void ensure_host() {
-        for (int i = 0; i < 2; ++i)
-            if (!pinned[i]) {
-                ICK(cudaMallocHost(&pinned[i], STAGE_BYTES));
-                ICK(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming));
-            }
-        if (!h_scalars) ICK(cudaMallocHost(&h_scalars, 8 * sizeof(unsigned long long)));
-    }
     void ensure_device(int dev, size_t text_bytes) {
         if (dev != device) {  // buffers belong to one device; switching devices starts over
             release_device();
             device = dev;
         }
         if (!d_scalars) ICK(cudaMalloc(&d_scalars, 8 * sizeof(unsigned long long)));
-        if (text_bytes > text_cap) {
-            char* p = nullptr;
+        if (!h_scalars) ICK(cudaMallocHost(&h_scalars, 8 * sizeof(unsigned long long)));
+        if (text_bytes > text_cap) {  // every ingest writes the buffer afresh: nothing to carry over
+            if (d_text) cudaFree(d_text);
+            d_text = nullptr;
+            text_cap = 0;
             const size_t want = text_bytes + text_bytes / 8 + (1u << 20);
-            ICK(cudaMalloc(&p, want));
-            if (d_text) {
-                ICK(cudaMemcpy(p, d_text, text_cap, cudaMemcpyDeviceToDevice));
-                cudaFree(d_text);
-            }
-            d_text = p;
+            ICK(cudaMalloc(&d_text, want));
             text_cap = want;
         }
     }
     void release_device() {
-        for (void* p : {(void*)d_text, (void*)d_nl, d_temp, (void*)d_scalars, (void*)d_rec})
+        for (void* p : {(void*)d_text, (void*)d_scalars, (void*)d_rec})
             if (p) cudaFree(p);
         d_text = nullptr;
-        d_nl = nullptr;
-        d_temp = nullptr;
         d_scalars = nullptr;
         d_rec = nullptr;
-        text_cap = nl_cap = temp_cap = rec_cap = 0;
+        text_cap = rec_cap = 0;
     }
 } g_stage;
-
-struct IsNewline {
-    const char* t;
-    __host__ __device__ bool operator()(uint32_t i) const { return t[i] == '\n'; }
-};
-struct NewlineCount {
-    const char* t;
-    __host__ __device__ unsigned long long operator()(uint32_t i) const { return t[i] == '\n' ? 1ull : 0ull; }
-};
 
 __device__ __forceinline__ uint32_t code4_dev(uint32_t c) {
     c &= 0xdfu;  // fold case (only letters matter)
     return c == 'A' ? 0u : c == 'C' ? 1u : c == 'G' ? 2u : c == 'T' ? 3u : 4u;
-}
-
-// line i spans (nl[i-1], nl[i]); record r = lines 4r .. 4r+3
-__global__ void fastq_records_kernel(const char* __restrict__ text, const uint32_t* __restrict__ nl, uint64_t n_records,
-                                     uint32_t* __restrict__ seq_start, uint32_t* __restrict__ raw_len,
-                                     unsigned long long* __restrict__ scalars) {
-    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t len = 0;
-    bool bad = false;
-    if (r < n_records) {
-        const uint32_t rec = r ? nl[4 * r - 1] + 1 : 0u;
-        const uint32_t s = nl[4 * r] + 1, e = nl[4 * r + 1];
-        const uint32_t plus = e + 1;
-        bad = text[rec] != '@' || text[plus] != '+' || nl[4 * r] == rec;  // header must be non-empty
-        len = e - s;
-        if (len && text[e - 1] == '\r') --len;
-        seq_start[r] = s;
-        raw_len[r] = len;
-    }
-    const uint32_t wmax = __reduce_max_sync(0xffffffffu, len);
-    const uint32_t wsum = __reduce_add_sync(0xffffffffu, len);
-    const uint32_t wbad = __ballot_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) {
-        if (wbad) atomicAdd(scalars + 1, 1ull);
-        atomicMax(scalars + 2, (unsigned long long)wmax);
-        atomicAdd(scalars + 3, (unsigned long long)wsum);
-    }
 }
 
 __device__ __forceinline__ uint32_t pack_word(const char* __restrict__ s, uint32_t n, uint32_t& bad) {
@@ -204,11 +139,6 @@ __global__ void pack_ragged_kernel(const char* __restrict__ text, const uint32_t
     if (__any_sync(0xffffffffu, bad != 0) && lane == 0) bad_flag[r] = 1u;
 }
 
-__global__ void nwords_kernel(const uint32_t* __restrict__ raw_len, uint64_t n, unsigned long long* __restrict__ nw) {
-    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r < n) nw[r] = (raw_len[r] + 15) >> 4;
-}
-
 __global__ void finish_lens_kernel(const uint32_t* __restrict__ raw_len, const uint32_t* __restrict__ bad_flag, uint64_t n,
                                    uint32_t* __restrict__ lens, unsigned long long* __restrict__ scalars) {
     const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -222,81 +152,16 @@ __global__ void finish_lens_kernel(const uint32_t* __restrict__ raw_len, const u
     if ((threadIdx.x & 31) == 0 && b) atomicAdd(scalars + 4, (unsigned long long)__popc(b));
 }
 
-// ---- host side: bytes -> device text ------------------------------------------------------------------------
-struct ByteSource {
-    int fd = -1;
-    gzFile gz = nullptr;
-    const char* mem = nullptr;  // text already in host memory (a gzip file inflated ahead of time by the batch driver)
-    size_t fsize = 0, pos = 0;
-    bool eof = false;
-    ~ByteSource() {
-        if (gz) gzclose(gz);
-        else if (fd >= 0) close(fd);
-    }
-    // fills buf with up to cap bytes; plain files are read by `threads` workers at once
-    size_t fill(char* buf, size_t cap, uint32_t threads) {
-        if (eof) return 0;
-        if (gz) {
-            size_t n = 0;
-            while (n < cap) {
-                const int r = gzread(gz, buf + n, (unsigned)std::min<size_t>(cap - n, 1u << 30));
-                if (r < 0) throw std::runtime_error("gzip read error");
-                if (r == 0) {
-                    eof = true;
-                    break;
-                }
-                n += (size_t)r;
-            }
-            return n;
-        }
-        const size_t want = std::min(cap, fsize - pos);
-        if (want == 0) {
-            eof = true;
-            return 0;
-        }
-        const size_t T = std::max<size_t>(1, std::min<size_t>({(size_t)std::max(1u, threads), (size_t)16, want / (1u << 20) + 1}));
-        std::vector<long long> got(T, 0);
-        parallel_for(T, [&](size_t t) {
-            const size_t lo = want * t / T, hi = want * (t + 1) / T;
-            size_t done = 0;
-            if (mem) {
-                memcpy(buf + lo, mem + pos + lo, hi - lo);
-                done = hi - lo;
-            }
-            while (lo + done < hi) {
-                const ssize_t r = pread(fd, buf + lo + done, hi - lo - done, (off_t)(pos + lo + done));
-                if (r <= 0) break;
-                done += (size_t)r;
-            }
-            got[t] = (long long)done;
-        }, T);
-        for (size_t t = 0; t < T; ++t)
-            if ((size_t)got[t] != want * (t + 1) / T - want * t / T) throw std::runtime_error("short read from the reads file");
-        pos += want;
-        if (pos >= fsize) eof = true;
-        return want;
-    }
-};
-
 // records (sequence start, raw length in g_stage.d_rec) -> 2-bit words, lengths (0 = dropped), dropped-read count
-// h_lens (optional): the raw lengths on the host — the ragged layout's word offsets are then a host prefix sum uploaded
-// with the other tables (the device-parsed path has the lengths on the device only and scans them there)
+// h_lens: the same raw lengths on the host, from which the ragged layout's word offsets are summed
 void pack_records(const char* text, uint64_t n, uint32_t max_len, uint64_t total_bases, uint32_t first_len, IngestResult& out,
-                  cudaStream_t st, const std::function<void*(size_t)>& alloc, const uint32_t* h_lens = nullptr) {
+                  cudaStream_t st, const std::function<void*(size_t)>& alloc, const uint32_t* h_lens) {
     uint32_t *d_start = g_stage.d_rec, *d_rawlen = g_stage.d_rec + g_stage.rec_cap, *d_bad = g_stage.d_rec + 2 * g_stage.rec_cap;
     auto dev_alloc = [&](size_t bytes) -> void* {
         if (alloc) return alloc(bytes);
         void* p = nullptr;
         ICK(cudaMalloc(&p, bytes));
         return p;
-    };
-    auto need_temp = [&](size_t bytes) {
-        if (bytes <= g_stage.temp_cap) return;
-        ICK(cudaStreamSynchronize(st));
-        if (g_stage.d_temp) cudaFree(g_stage.d_temp);
-        g_stage.d_temp = nullptr;
-        g_stage.temp_cap = bytes + bytes / 4 + 1024;
-        ICK(cudaMalloc(&g_stage.d_temp, g_stage.temp_cap));
     };
     try {
         const unsigned rb = (unsigned)((n + 255) / 256);
@@ -320,28 +185,14 @@ void pack_records(const char* text, uint64_t n, uint32_t max_len, uint64_t total
             out.b_off = (n + 1) * 8;
             out.d_word_off = (uint64_t*)dev_alloc(out.b_off);
             unsigned long long total_words = 0;
-            if (h_lens) {
-                std::vector<uint64_t> off(n + 1);
-                for (uint64_t r = 0; r < n; ++r) {
-                    off[r] = total_words;
-                    total_words += (h_lens[r] + 15u) >> 4;
-                }
-                off[n] = total_words;
-                ICK(cudaMemcpyAsync(out.d_word_off, off.data(), (n + 1) * 8, cudaMemcpyHostToDevice, st));
-                ICK(cudaStreamSynchronize(st));  // `off` dies with this scope
-            } else {
-                unsigned long long* d_nw = nullptr;
-                ICK(cudaMalloc(&d_nw, (n + 1) * 8));
-                ICK(cudaMemsetAsync(d_nw + n, 0, 8, st));
-                nwords_kernel<<<rb, 256, 0, st>>>(d_rawlen, n, d_nw);
-                size_t t2 = 0;
-                cub::DeviceScan::ExclusiveSum(nullptr, t2, d_nw, (unsigned long long*)out.d_word_off, (int64_t)(n + 1), st);
-                need_temp(t2);
-                cub::DeviceScan::ExclusiveSum(g_stage.d_temp, t2, d_nw, (unsigned long long*)out.d_word_off, (int64_t)(n + 1), st);
-                ICK(cudaMemcpyAsync(&total_words, out.d_word_off + n, 8, cudaMemcpyDeviceToHost, st));
-                ICK(cudaStreamSynchronize(st));
-                cudaFree(d_nw);
+            std::vector<uint64_t> off(n + 1);
+            for (uint64_t r = 0; r < n; ++r) {
+                off[r] = total_words;
+                total_words += (h_lens[r] + 15u) >> 4;
             }
+            off[n] = total_words;
+            ICK(cudaMemcpyAsync(out.d_word_off, off.data(), (n + 1) * 8, cudaMemcpyHostToDevice, st));
+            ICK(cudaStreamSynchronize(st));  // `off` dies with this scope
             out.b_words = (total_words + 2) * 4;
             out.d_words = (uint32_t*)dev_alloc(out.b_words);
             pack_ragged_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(text, d_start, d_rawlen, n,
@@ -372,21 +223,20 @@ void ensure_records(uint64_t n) {  // grow-only scratch: cudaMalloc / cudaFree p
 
 }  // namespace
 
-// ---- host-framed path: only the sequence lines cross PCIe ------------------------------------------------------------
 // The text (a plain file read in pieces by the pool threads, or a gzip file already inflated into host memory) is cut into
 // slices at record starts; every slice is framed by one thread (fastq_frame.cpp) straight into its own part of a pinned
 // buffer — the sequence lines of the slice [lo, hi) go to offset lo / 2, which cannot collide with the next slice because
 // a record's sequence is less than half of its bytes — and the thread that framed a slice also queues its H2D copy, so
-// the copies overlap the framing of the other slices.  Then (start, length) of every read is uploaded and the same pack
-// kernels as in the device-parsed path run.  false = not strict 4-line FASTQ (nothing is left behind; the caller goes on
-// with the device parser / host parser).
-static bool ingest_fastq_framed(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
-                                const std::function<void*(size_t)>& alloc) {
+// the copies overlap the framing of the other slices.  Then (start, length) of every read is uploaded and the pack
+// kernels run.  false = not strict 4-line FASTQ (nothing is left behind; the caller goes on with the host parser).
+bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
+                       const std::function<void*(size_t)>& alloc) {
+    out = IngestResult();
+    std::lock_guard<std::mutex> lock(g_stage.m);
     static const bool timing = getenv("DRPRG_TIMING") != nullptr;
     const double t0 = now_ms_i();
     if (src.size < 8 || src.size / 2 + 64 >= 0xfff00000ull) return false;  // 32-bit sequence offsets
     ICK(cudaSetDevice(device));
-    g_stage.ensure_host();
     g_stage.ensure_seq(src.size / 2 + 64);
     g_stage.ensure_device(device, src.size / 2 + 64);
     char* const pinned = g_stage.pinned_seq;
@@ -452,145 +302,6 @@ static bool ingest_fastq_framed(const TextSource& src, int device, uint32_t thre
     if (timing)
         fprintf(stderr, "[drprg-cuda] ingest (host-framed): %.1f MB text in %zu slices, frame + queue H2D %.2f ms, record table %.2f ms, "
                         "upload tail + pack %.2f ms\n", src.size / 1e6, S, t1 - t0, t2 - t1, now_ms_i() - t2);
-    return true;
-}
-
-bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
-                       const std::function<void*(size_t)>& alloc) {
-    out = IngestResult();
-    std::lock_guard<std::mutex> lock(g_stage.m);
-    if (ingest_fastq_framed(src, device, threads, out, st, alloc)) return true;
-    out = IngestResult();
-    return false;
-}
-
-bool ingest_fastq_device(const std::string& path, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
-                         const std::function<void*(size_t)>& alloc, const char* mem, size_t mem_size) {
-    out = IngestResult();
-    ByteSource src;
-    unsigned char magic[2] = {0, 0};
-    ssize_t got = 0;
-    if (mem) {
-        src.mem = mem;
-        src.fsize = mem_size;
-        got = (ssize_t)std::min<size_t>(2, mem_size);
-        memcpy(magic, mem, (size_t)got);
-    } else {
-        src.fd = open(path.c_str(), O_RDONLY);
-        if (src.fd < 0) throw std::runtime_error("cannot open " + path);
-        got = pread(src.fd, magic, 2, 0);
-        src.fsize = (size_t)lseek(src.fd, 0, SEEK_END);
-    }
-    const bool is_gz = !mem && got == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
-    if (is_gz) {
-        lseek(src.fd, 0, SEEK_SET);
-        src.gz = gzdopen(src.fd, "rb");
-        if (!src.gz) throw std::runtime_error("cannot open " + path);
-        gzbuffer(src.gz, 1 << 20);
-    } else if (got < 1 || magic[0] != '@') {
-        return false;  // FASTA, leading blank lines, empty file: host parser
-    }
-    std::lock_guard<std::mutex> lock(g_stage.m);
-    static const bool timing = getenv("DRPRG_TIMING") != nullptr;
-    // DRPRG_INGEST=device keeps the device-side parser below (the second implementation; tests compare the two)
-    static const bool framed_on = !(getenv("DRPRG_INGEST") && std::string(getenv("DRPRG_INGEST")) == "device");
-    if (framed_on && !is_gz) {
-        TextSource ts;
-        ts.fd = src.fd;
-        ts.mem = mem;
-        ts.size = src.fsize;
-        if (ingest_fastq_framed(ts, device, threads, out, st, alloc)) return true;
-        out = IngestResult();
-    }
-    const double ti0 = now_ms_i();
-    if (!is_gz && src.fsize >= 0xfff00000ull) return false;  // 32-bit text offsets
-    ICK(cudaSetDevice(device));
-    g_stage.ensure_host();
-    g_stage.ensure_device(device, is_gz ? std::max<size_t>(src.fsize * 4, 1u << 20) : src.fsize + 1);
-    // ---- stream the bytes through the pinned double buffer
-    size_t total = 0;
-    for (int i = 0;; ++i) {
-        const int b = i & 1;
-        if (i >= 2) ICK(cudaEventSynchronize(g_stage.done[b]));  // the copy that last used this buffer has finished
-        const size_t n = src.fill(g_stage.pinned[b], STAGE_BYTES, threads);
-        if (n == 0) break;
-        if (i == 0 && g_stage.pinned[b][0] != '@') return false;  // gzip of something that is not FASTQ
-        if (total + n >= 0xfff00000ull) return false;
-        if (total + n + 1 > g_stage.text_cap) {
-            ICK(cudaStreamSynchronize(st));
-            g_stage.ensure_device(device, (total + n) * 2);
-        }
-        ICK(cudaMemcpyAsync(g_stage.d_text + total, g_stage.pinned[b], n, cudaMemcpyHostToDevice, st));
-        ICK(cudaEventRecord(g_stage.done[b], st));
-        total += n;
-    }
-    if (total == 0) return false;
-    if (timing) ICK(cudaStreamSynchronize(st));
-    const double ti1 = now_ms_i();
-    // ---- newline offsets
-    const char* text = g_stage.d_text;
-    ICK(cudaMemsetAsync(g_stage.d_scalars, 0, 8 * sizeof(unsigned long long), st));
-    thrust::counting_iterator<uint32_t> idx(0);
-    unsigned long long* d_count = g_stage.d_scalars;
-    auto need_temp = [&](size_t bytes) {
-        if (bytes <= g_stage.temp_cap) return;
-        ICK(cudaStreamSynchronize(st));
-        if (g_stage.d_temp) cudaFree(g_stage.d_temp);
-        g_stage.d_temp = nullptr;
-        g_stage.temp_cap = bytes + bytes / 4 + 1024;
-        ICK(cudaMalloc(&g_stage.d_temp, g_stage.temp_cap));
-    };
-    {   // count first: the offsets array is sized for the lines that exist, not for the worst case
-        auto ones = thrust::make_transform_iterator(idx, NewlineCount{text});
-        size_t temp = 0;
-        cub::DeviceReduce::Sum(nullptr, temp, ones, d_count, (int64_t)total, st);
-        need_temp(temp);
-        cub::DeviceReduce::Sum(g_stage.d_temp, temp, ones, d_count, (int64_t)total, st);
-        ICK(cudaMemcpyAsync(g_stage.h_scalars, g_stage.d_scalars, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        ICK(cudaStreamSynchronize(st));
-        const size_t lines = (size_t)g_stage.h_scalars[0] + 8;
-        if (lines > g_stage.nl_cap) {
-            if (g_stage.d_nl) cudaFree(g_stage.d_nl);
-            g_stage.d_nl = nullptr;
-            g_stage.nl_cap = lines + lines / 8 + 1024;
-            ICK(cudaMalloc(&g_stage.d_nl, g_stage.nl_cap * sizeof(uint32_t)));
-        }
-        cub::DeviceSelect::If(nullptr, temp, idx, g_stage.d_nl, d_count, (int64_t)total, IsNewline{text}, st);
-        need_temp(temp);
-        cub::DeviceSelect::If(g_stage.d_temp, temp, idx, g_stage.d_nl, d_count, (int64_t)total, IsNewline{text}, st);
-    }
-    // last byte: a file without a final newline gets a virtual one
-    char last = 0;
-    ICK(cudaMemcpyAsync(g_stage.h_scalars, g_stage.d_scalars, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    ICK(cudaMemcpyAsync(&last, text + total - 1, 1, cudaMemcpyDeviceToHost, st));
-    ICK(cudaStreamSynchronize(st));
-    uint64_t n_lines = g_stage.h_scalars[0];
-    if (last != '\n') {
-        const uint32_t end = (uint32_t)total;
-        ICK(cudaMemcpyAsync(g_stage.d_nl + n_lines, &end, 4, cudaMemcpyHostToDevice, st));
-        ICK(cudaStreamSynchronize(st));
-        ++n_lines;
-    }
-    const double ti2 = now_ms_i();
-    if (n_lines == 0 || (n_lines & 3u)) return false;  // blank or wrapped lines: host parser
-    const uint64_t n = n_lines / 4;
-    if (n > 0xfffffff0ull) throw std::runtime_error("more than 2^32 reads in one sample");
-    // ---- records
-    ensure_records(n);
-    uint32_t *d_start = g_stage.d_rec, *d_rawlen = g_stage.d_rec + g_stage.rec_cap;
-    {
-        const unsigned rb = (unsigned)((n + 255) / 256);
-        fastq_records_kernel<<<rb, 256, 0, st>>>(text, g_stage.d_nl, n, d_start, d_rawlen, g_stage.d_scalars);
-        ICK(cudaMemcpyAsync(g_stage.h_scalars, g_stage.d_scalars, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        uint32_t first_len = 0;
-        ICK(cudaMemcpyAsync(&first_len, d_rawlen, 4, cudaMemcpyDeviceToHost, st));
-        ICK(cudaStreamSynchronize(st));
-        if (g_stage.h_scalars[1]) return false;  // '@' / '+' framing broken somewhere: not strict 4-line FASTQ
-        pack_records(text, n, (uint32_t)g_stage.h_scalars[2], g_stage.h_scalars[3], first_len, out, st, alloc);
-    }
-    if (timing)
-        fprintf(stderr, "[drprg-cuda] ingest: %.1f MB text, read+H2D %.2f ms, newline scan %.2f ms, records+pack %.2f ms\n", total / 1e6,
-                ti1 - ti0, ti2 - ti1, now_ms_i() - ti2);
     return true;
 }
 

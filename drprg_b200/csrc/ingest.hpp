@@ -4,7 +4,6 @@
 
 #include <cstdint>
 #include <functional>
-#include <string>
 
 namespace drprg {
 
@@ -17,16 +16,11 @@ struct IngestResult {  // device buffers from cudaMalloc, owned by the caller
     uint64_t n_reads = 0, total_bases = 0, n_dropped = 0;
 };
 
-// false: the input is not strict 4-line FASTQ below 4 GiB of text (the caller uses the host parser); throws on IO errors
-// `alloc` supplies the output buffers (e.g. from the caller's buffer pool); default: cudaMalloc.  With `mem` the text is
-// taken from host memory instead of the file (a gzip file inflated ahead of time).
-bool ingest_fastq_device(const std::string& path, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
-                         const std::function<void*(size_t)>& alloc = nullptr, const char* mem = nullptr, size_t mem_size = 0);
-
 struct TextSource;
 // Host-framed ingest of one piece of FASTQ text (a whole file, or a wave of a large one that starts and ends at record
 // starts): only the sequence lines are uploaded (fastq_frame.cpp), then packed on the device.  false = not strict 4-line
-// FASTQ.  The text must be smaller than 8 GB (32-bit offsets into the sequence buffer).
+// FASTQ (the caller uses the host parser); throws on IO errors.  The text must be smaller than 8 GB (32-bit offsets into
+// the sequence buffer).  `alloc` supplies the output buffers (e.g. from the caller's buffer pool); default: cudaMalloc.
 bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
                        const std::function<void*(size_t)>& alloc = nullptr);
 

@@ -278,8 +278,8 @@ class Index:
         return Batch(self, h, len(lens))
 
     def batch_from_fastx(self, path, threads=8):
-        """a reads file as a device-resident batch: strict 4-line FASTQ (plain/gzip) is parsed and packed on the GPU, anything
-        else by the host parser.  Returns (Batch, info)."""
+        """a reads file as a device-resident batch: strict 4-line FASTQ (plain/gzip) is framed on the host and packed on the
+        GPU (info["parsed_on_device"] is True), anything else goes through the host parser.  Returns (Batch, info)."""
         h = C.c_void_p()
         n, tb, nd = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
         fl, dev = C.c_uint32(0), C.c_int(0)

@@ -122,7 +122,8 @@ int drprg_cuda_batch_wrap_device(drprg_index*, const void* d_words, const void* 
                                  const void* d_lens, uint64_t n_reads, uint64_t total_bases, uint32_t read_id_base,
                                  drprg_batch** out);
 /* a reads file (fasta/fastq, plain or gzip: src/predict.rs:166-170) as a device-resident batch.  Strict 4-line FASTQ is
- * sent to the device as raw text and parsed + 2-bit packed there; other inputs use the host parser and an upload. */
+ * framed on the host, and only its sequence lines are sent to the device and 2-bit packed there; other inputs use the
+ * host parser and an upload.  *parsed_on_device = 1 for the first path, 0 for the host parser. */
 int drprg_cuda_batch_from_fastx(drprg_index*, const char* path, uint32_t threads, drprg_batch** out, uint64_t* n_reads,
                                 uint64_t* total_bases, uint64_t* n_dropped, uint32_t* first_read_len, int* parsed_on_device);
 void drprg_cuda_batch_free(drprg_batch*);

@@ -240,22 +240,44 @@ def test_coverage_is_additive_over_shards():
     assert_genotype_equal(gx, ox, mr, oo, refs)
 
 
-def test_drop_in_call_writes_pandora_vcf(tmp_path):
-    """drprg_cuda_map_genotype == Pandora::genotype_with: files in, outdir/pandora_genotyped.vcf out."""
-    d, o = sim.toy_dataset(TOY_PRG, TOY_REFS, depth=40, decoys=2, seed=9)
-    fq = tmp_path / "reads.fq.gz"
-    sim.write_fastq(str(fq), d, o, gz=True)
+def _drop_in_call_matches_oracle(tmp_path, fq, d, o):
+    """maps the reads file fq (the reads d, o) through drprg_cuda_map_genotype into tmp_path and checks the VCF against
+    the oracle's; returns the index and pandora.log"""
     gx, ox = both_indexes(TOY_PRG, 11, 15)
     st = gx.map_genotype(fq, TOY_REFS, tmp_path, lib.make_opts(illumina=True, genome_size=2000))
     assert st["n_reads"] == len(o) - 1 and st["n_records"] == 23
-    assert (tmp_path / "pandora.log").exists()
+    log = (tmp_path / "pandora.log").read_text()
     got = (tmp_path / "pandora_genotyped.vcf").read_text()
     oo = O.make_opts(illumina=True, genome_size=2000)
     og = O.Genotype(ox, O.MapRun(ox, d, o, oo), oo, TOY_REFS)
     strip = lambda t: [l for l in t.splitlines() if not l.startswith("##fileDate")]
     assert strip(got) == strip(og.vcf())
+    return gx, log
+
+
+def test_drop_in_call_writes_pandora_vcf(tmp_path):
+    """drprg_cuda_map_genotype == Pandora::genotype_with: files in, outdir/pandora_genotyped.vcf out."""
+    d, o = sim.toy_dataset(TOY_PRG, TOY_REFS, depth=40, decoys=2, seed=9)
+    fq = tmp_path / "reads.fq.gz"
+    sim.write_fastq(str(fq), d, o, gz=True)
+    gx, log = _drop_in_call_matches_oracle(tmp_path, fq, d, o)
+    assert "ingest=host-framed, " in log, log
     with pytest.raises(lib.DrprgCudaError):
         gx.map_genotype(tmp_path / "missing.fq", TOY_REFS, tmp_path)
+
+
+@pytest.mark.parametrize("fmt", ["wrapped_fastq", "fasta"])
+def test_drop_in_call_host_parser_fallback(tmp_path, fmt):
+    """a wrapped FASTQ (sequence and quality in lines of 60) or a FASTA of the same reads: the framer declines it, the
+    drop-in call maps it through the host parser (pandora.log says so) and writes the oracle's VCF"""
+    d, o = sim.toy_dataset(TOY_PRG, TOY_REFS, depth=40, decoys=2, seed=9)
+    wrap = lambda s: b"".join(s[j:j + 60] + b"\n" for j in range(0, len(s), 60))
+    reads = [d[int(o[i]):int(o[i + 1])].tobytes() for i in range(len(o) - 1)]
+    fq = tmp_path / ("reads.fq" if fmt == "wrapped_fastq" else "reads.fa")
+    fq.write_bytes(b"".join(b"@r%d\n" % i + wrap(r) + b"+\n" + wrap(b"I" * len(r)) if fmt == "wrapped_fastq" else
+                            b">r%d\n" % i + wrap(r) for i, r in enumerate(reads)))
+    _, log = _drop_in_call_matches_oracle(tmp_path, fq, d, o)
+    assert "ingest=host\n" in log, log
 
 
 def test_batch_of_samples_config5(tmp_path):
@@ -438,7 +460,8 @@ def _fastq_bytes(reads, crlf=False, final_newline=True):
 
 
 def _map_file_both_ways(gx, path, opts):
-    """(hits, info) through the device FASTQ parser and through the host parser + upload"""
+    """(hits, info) through batch_from_fastx (framed on the host, packed on the device) and through the host parser +
+    upload"""
     out = []
     b, info = gx.batch_from_fastx(path)
     gx.sample_begin(opts, info["first_read_len"])
@@ -453,8 +476,8 @@ def _map_file_both_ways(gx, path, opts):
 
 @pytest.mark.parametrize("variant", ["plain", "gzip", "crlf", "no_final_newline"])
 def test_device_fastq_ingest_matches_host_parser(tmp_path, variant):
-    """SURVEY 8f rank 2: the reads file goes to the GPU as text and is parsed + 2-bit packed there; the batch must be the
-    one the host parser builds (same reads, lengths, dropped reads, hits and coverage)."""
+    """SURVEY 8f rank 2: the reads file is framed on the host and its sequence lines are 2-bit packed on the GPU; the
+    batch must be the one the host parser builds (same reads, lengths, dropped reads, hits and coverage)."""
     import gzip
     d, o = sim.toy_dataset(TOY_PRG, TOY_REFS, depth=30, decoys=2, seed=4)
     reads = [d[int(o[i]):int(o[i + 1])].tobytes() for i in range(len(o) - 1)]
@@ -482,7 +505,8 @@ def test_device_fastq_ingest_matches_host_parser(tmp_path, variant):
 
 
 def test_device_fastq_ingest_long_reads_and_fallbacks(tmp_path):
-    """ragged layout + segment table for long reads; FASTA, wrapped or blank-line input falls back to the host parser"""
+    """ragged layout + segment table for long reads; FASTA, wrapped or blank-line input falls back to the host parser,
+    which rejects a record whose quality line is not as long as its sequence"""
     p, prg, refs = small_panel()
     d, o, g, pl = long_reads_sample(p, 200)
     reads = [d[int(o[i]):int(o[i + 1])].tobytes() for i in range(len(o) - 1)]
@@ -505,15 +529,20 @@ def test_device_fastq_ingest_long_reads_and_fallbacks(tmp_path):
     blank.write_bytes(_fastq_bytes(reads[:10]) + b"\n")
     b, info = gx.batch_from_fastx(blank)
     assert not info["parsed_on_device"] and info["n_reads"] == 10
+    bad = tmp_path / "bad.fq"  # record 3 of 10: quality one shorter than the sequence
+    bad.write_bytes(b"".join(b"@r%d\n" % i + r + b"\n+\n" + b"I" * (len(r) - (i == 3)) + b"\n" for i, r in enumerate(reads[:10])))
+    with pytest.raises(lib.DrprgCudaError, match="malformed FASTQ record"):
+        gx.batch_from_fastx(bad)
+    with pytest.raises(lib.DrprgCudaError, match="malformed FASTQ record"):
+        gx.map_genotype(bad, refs, tmp_path, opts)
 
 
-@pytest.mark.parametrize("env", [{"DRPRG_INGEST": "device"}, {"DRPRG_FRAME_SLICE": "2048"}, {"DRPRG_WAVE_BYTES": "30000", "DRPRG_FRAME_SLICE": "4096"}])
+@pytest.mark.parametrize("env", [{"DRPRG_FRAME_SLICE": "2048"}, {"DRPRG_WAVE_BYTES": "30000", "DRPRG_FRAME_SLICE": "4096"}])
 def test_file_ingest_variants_keep_parity(env):
-    """the reads file reaches the GPU in two ways: framed on the host (default: only the sequence lines cross PCIe; here
-    also with 2 KB slices so that every test file is cut at many record boundaries) or as raw text parsed by the device
-    kernels (DRPRG_INGEST=device, the second implementation).  Both must build the host parser's batch.  The drop-in call
-    maps a file wave by wave (DRPRG_WAVE_BYTES, default 1 GiB of text per wave): with 30 KB waves every test file takes
-    several and the VCF must not change."""
+    """a strict FASTQ file is framed on the host in slices of 1 MiB of text, which only the sequence lines leave; with
+    2 KB slices every test file is cut at many record boundaries, and the batch must still be the host parser's.  The
+    drop-in call maps a file wave by wave (DRPRG_WAVE_BYTES, default 1 GiB of text per wave): with 30 KB waves every test
+    file takes several and the VCF must not change."""
     import subprocess, sys
     e = dict(os.environ, **env)
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-m", "gpu", "-k",

@@ -1,5 +1,5 @@
-"""Drop-in call from a FASTQ file (drprg_cuda_map_genotype): wall time with the host-framed ingest (default), the device
-FASTQ parser (DRPRG_INGEST=device) and the host parser (DRPRG_HOST_INGEST=1).
+"""Drop-in call from a FASTQ file (drprg_cuda_map_genotype): wall time with the host-framed ingest (default) and the host
+parser (DRPRG_HOST_INGEST=1).
    python tools/e2e_probe.py [n_reads]"""
 import sys, os, subprocess, json, tempfile, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -17,7 +17,7 @@ if len(sys.argv) > 1 and sys.argv[1] == "run":
                          genotype_ms=round(st["ms_genotype"], 2), n_reads=st["n_reads"], records=st["n_records"])
     import hashlib
     res["vcf_sha1"] = hashlib.sha1(b"".join(l for l in open(os.path.join(out, "pandora_genotyped.vcf"), "rb") if not l.startswith(b"##fileDate"))).hexdigest()[:12]
-    print(json.dumps({"host_ingest": os.environ.get("DRPRG_HOST_INGEST", "0"), "ingest": os.environ.get("DRPRG_INGEST", "framed"), **res}))
+    print(json.dumps({"host_ingest": os.environ.get("DRPRG_HOST_INGEST", "0"), **res}))
 else:
     from drprg_b200 import workload, sim
     n = int(sys.argv[1]) if len(sys.argv) > 1 else 1000000
@@ -35,5 +35,5 @@ else:
     rec[:, 12 + L:12 + 2 * L] = ord("I"); rec[:, 12 + 2 * L] = 10
     rec.tofile(fq)
     subprocess.run(f"gzip -1 -c {fq} > {gz}", shell=True, check=True)
-    for extra in ({}, {"DRPRG_INGEST": "device"}, {"DRPRG_HOST_INGEST": "1"}):
+    for extra in ({}, {"DRPRG_HOST_INGEST": "1"}):
         subprocess.run([sys.executable, __file__, "run", fq, gz, wl.prg_path, wl.refs_path], env=dict(os.environ, **extra))
