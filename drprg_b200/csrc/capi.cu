@@ -1,6 +1,6 @@
 // C ABI of include/drprg_cuda.h: the drop-in for Pandora::genotype_with
 // (/root/reference/src/lib.rs:580-642) plus the staged interface used for multi-GPU read sharding,
-// benches and parity tests.  Owns all device memory of an index (plain cudaMalloc; no torch types).
+// benches and parity tests.  Owns all device memory of an index (cuda_owned.hpp; no torch types).
 #include <cuda_runtime.h>
 #include <fcntl.h>
 #include <unistd.h>
@@ -23,6 +23,7 @@
 #include <thread>
 
 #include "../../include/drprg_cuda.h"
+#include "cuda_owned.hpp"
 #include "genotype_host.hpp"
 #include "fastq_frame.hpp"
 #include "ingest.hpp"
@@ -34,97 +35,6 @@ using namespace drprg;
 namespace {
 thread_local std::string g_err;
 
-#define CK(call)                                                                                         \
-    do {                                                                                                 \
-        cudaError_t e__ = (call);                                                                        \
-        if (e__ != cudaSuccess)                                                                          \
-            throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e__) + " at " #call); \
-    } while (0)
-
-template <class T>
-struct DBuf {  // grow-only device buffer
-    T* p = nullptr;
-    size_t cap = 0;
-    void ensure(size_t n) {
-        if (n <= cap) return;
-        if (p) cudaFree(p);
-        p = nullptr;
-        size_t want = n + n / 4 + 1024;
-        CK(cudaMalloc(&p, want * sizeof(T)));
-        cap = want;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
-template <class T>
-struct PinnedBuf {  // grow-only pinned host buffer: async D2H into pageable memory would block the host
-    T* p = nullptr;
-    size_t cap = 0, n = 0;
-    void resize(size_t want) {
-        if (want > cap) {
-            if (p) cudaFreeHost(p);
-            p = nullptr;
-            cap = want + want / 4 + 256;
-            CK(cudaMallocHost(&p, cap * sizeof(T)));
-        }
-        n = want;
-    }
-    T* data() { return p; }
-    size_t size() const { return n; }
-    T* begin() { return p; }
-    T* end() { return p + n; }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = n = 0;
-    }
-};
-
-template <class T>
-T* to_device(const std::vector<T>& v) {
-    T* d = nullptr;
-    CK(cudaMalloc(&d, std::max<size_t>(1, v.size()) * sizeof(T)));
-    if (!v.empty()) CK(cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return d;
-}
-
-// freed batch buffers are parked here and reused by the next upload: cudaFree synchronises the device and
-// cudaMalloc costs ~0.1-1 ms, both of which would sit inside every end-to-end step
-struct DevPool {
-    struct Slot { void* p; size_t bytes; int device; };
-    std::vector<Slot> free_;
-    std::mutex m_;
-    void* get(size_t bytes, int device) {
-        std::lock_guard<std::mutex> g(m_);
-        size_t best = free_.size();
-        for (size_t i = 0; i < free_.size(); ++i)
-            if (free_[i].device == device && free_[i].bytes >= bytes && (best == free_.size() || free_[i].bytes < free_[best].bytes)) best = i;
-        if (best != free_.size() && free_[best].bytes <= bytes * 2 + (1 << 20)) {
-            void* p = free_[best].p;
-            free_.erase(free_.begin() + best);
-            return p;
-        }
-        void* p = nullptr;
-        CK(cudaMalloc(&p, bytes));
-        return p;
-    }
-    void put(void* p, size_t bytes, int device) {
-        std::lock_guard<std::mutex> g(m_);
-        if (free_.size() >= 16) {
-            cudaFree(free_.front().p);
-            free_.erase(free_.begin());
-        }
-        free_.push_back({p, bytes, device});
-    }
-} g_pool;
-
-double now_ms() {
-    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
-}
 }  // namespace
 
 // one persistent host thread per extra GPU of a multi-GPU handle: launches for the devices are issued side by side
@@ -190,20 +100,18 @@ class GpuWorker {
 };
 
 struct drprg_batch {
-    std::vector<drprg_batch*> shards;  // multi-GPU handle: one sub-batch per GPU (this object is then only the container)
+    // multi-GPU handle: one sub-batch per GPU (this object is then only the container)
+    std::vector<std::unique_ptr<drprg_batch>> shards;
     DevReads R{};
-    uint32_t *d_words = nullptr, *d_lens = nullptr, *d_seg_read = nullptr, *d_seg_start = nullptr;
-    uint64_t* d_off = nullptr;
-    bool owned = false;
-    size_t b_words = 0, b_lens = 0, b_off = 0, b_seg = 0;
-    int device = 0;
+    PoolBuf<uint32_t> d_words, d_lens, d_seg_read, d_seg_start;  // empty for a batch wrapping the caller's arrays
+    PoolBuf<uint64_t> d_off;
     uint64_t total_bases = 0;
     uint32_t max_len = UINT32_MAX;  // longest read (bound); selects the short-read kernel
     // host uploads are split into chunks copied on a separate stream; the sketch kernel of chunk c starts as soon
     // as its bytes have landed, so the H2D copy overlaps the sketch of the previous chunks
     int n_chunks = 1;
     uint64_t chunk_lo[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    Event ev[8];
 };
 
 struct drprg_index {
@@ -211,15 +119,16 @@ struct drprg_index {
     int device = 0, sm_count = 148;
     // device-resident index
     DevTable T{};
-    uint2 *d_slots = nullptr, *d_recs = nullptr;
-    uint32_t* d_kfilter = nullptr;
-    uint32_t *d_filter = nullptr, *d_knode_base = nullptr, *d_edge_off = nullptr, *d_edges = nullptr;
-    uint8_t *d_is_terminal = nullptr, *d_needs_mean = nullptr;
-    uint32_t *d_locus_level_off = nullptr, *d_level_start = nullptr, *d_level_nodes = nullptr, *d_level_singles = nullptr;
+    DBuf<uint2> d_slots, d_recs;
+    DBuf<uint32_t> d_kfilter;
+    DBuf<uint32_t> d_filter, d_knode_base, d_edge_off, d_edges;
+    DBuf<uint8_t> d_is_terminal, d_needs_mean;
+    DBuf<uint32_t> d_locus_level_off, d_level_start, d_level_nodes, d_level_singles;
     uint32_t table_slots = 0, filter_words = 0;
     uint64_t n_edges = 0, n_ivs = 0;
-    // accumulators: [2*N coverage | P locus reads | 4 scalars]
-    int32_t* d_accum = nullptr;
+    // accumulators: [2*N coverage | P locus reads | 4 scalars]; one exact allocation, never from g_pool: other processes
+    // open it through cudaIpcGetMemHandle, and the cross-GPU flag words sit behind it
+    DBuf<int32_t> d_accum;
     uint64_t n_accum = 0;
     uint64_t total_bases = 0, n_reads = 0;
     bool scalars_in_buffer = false;
@@ -228,7 +137,7 @@ struct drprg_index {
     SampleOpts opts;
     bool sample_open = false;
     uint32_t first_read_len = 0;
-    uint32_t* d_thresh = nullptr;
+    DBuf<uint32_t> d_thresh;
     uint32_t min_thresh = 0;
     std::vector<uint32_t> thresh_on_device;
     // workspace
@@ -242,8 +151,8 @@ struct drprg_index {
     uint32_t n_partials = 0;
     DBuf<unsigned long long> queue;  // k-mer screen: flagged (read, position) pairs
     DBuf<uint32_t> queue_kmer;       // ... and their k-mers
-    unsigned long long* d_counters = nullptr;  // CTR_* of kernels.cuh
-    unsigned long long* h_counters = nullptr;  // pinned
+    DBuf<unsigned long long> d_counters;  // CTR_* of kernels.cuh
+    PinnedBuf<unsigned long long> h_counters;
     uint64_t last_n_hits = 0, last_n_active = 0;
     uint32_t last_id_base = 0;
     // read-sharded runs: where this GPU's coverage goes (nullptr = its own accumulator; otherwise the root GPU's
@@ -261,7 +170,7 @@ struct drprg_index {
     void* ipc_mapping = nullptr; // non-root: the root's accumulator allocation opened in this process
     uint32_t* flag_ready = nullptr;     // root's "accumulator zeroed for sample e" word
     uint32_t* flag_arrivals = nullptr;  // root's arrival counter (world - 1 per sample)
-    cudaEvent_t ev[6]{};  // batch timeline: start, lookup done, hits grouped, clustered, coverage merged
+    Event ev[6];  // batch timeline: start, lookup done, hits grouped, clustered, coverage merged
     float timings[4] = {0, 0, 0, 0};
     // genotype state
     std::string refs_path;
@@ -280,7 +189,7 @@ struct drprg_index {
     std::vector<const SiteRecord*> records, csr_records;  // csr_records: what the device CSR was built for
     std::deque<std::vector<SiteRecord>> sample_records;    // per-sample merged lists (ML path added records)
     GenotypeArrays GA;
-    uint32_t *d_rec_off = nullptr, *d_allele_off = nullptr, *d_allele_kn = nullptr, *d_knode_locus = nullptr, *d_hist = nullptr;
+    DBuf<uint32_t> d_rec_off, d_allele_off, d_allele_kn, d_knode_locus, d_hist;
     DBuf<uint32_t> d_gt_u32;
     DBuf<double> d_gt_f64;
     DBuf<int32_t> d_gt_i32;
@@ -291,13 +200,13 @@ struct drprg_index {
     std::vector<RetainedHit> retained;
     DiscoverResult discover;
     uint32_t max_locus_knodes = 0, max_locus_edges = 0;
-    cudaEvent_t ev_ml[2] = {nullptr, nullptr};
-    cudaStream_t st_ml = nullptr, st_gt = nullptr, st_copy = nullptr, st_acc = nullptr;
-    cudaEvent_t ev_acc[3] = {nullptr, nullptr, nullptr};  // [2]: node scores + threshold ready on `st`
-    double* d_thresh_f64 = nullptr;
-    int* d_thresh_i32 = nullptr;
+    Event ev_ml[2];
+    Stream st_ml, st_gt, st_copy, st_acc;
+    Event ev_acc[3];  // [2]: node scores + threshold ready on `st`
+    DBuf<double> d_thresh_f64;
+    DBuf<int> d_thresh_i32;
     PinnedBuf<int> h_thresh;
-    uint32_t* d_hist1000 = nullptr;
+    DBuf<uint32_t> d_hist1000;
     PinnedBuf<uint32_t> h_small;  // coverage histogram | locus read counts | scalars  // ML-path kernel / genotype kernels run concurrently
     PinnedBuf<uint32_t> h_path, h_plen, h_u32, h_done;
     PinnedBuf<double> h_f64;
@@ -309,8 +218,8 @@ struct drprg_index {
     PinnedBuf<char> h_vcf;
     size_t vcf_len = 0, vcf_begin = 0;  // the text is h_vcf[vcf_begin, vcf_begin + vcf_len)
     std::string vcf_header, vcf_fallback;
-    char* d_vcf_prefix = nullptr;
-    uint32_t *d_vcf_prefix_off = nullptr, *d_vcf_slot_off = nullptr, *d_vcf_ctl = nullptr;  // ctl: [0] text bytes, [1] flags
+    DBuf<char> d_vcf_prefix;
+    DBuf<uint32_t> d_vcf_prefix_off, d_vcf_slot_off, d_vcf_ctl;  // ctl: [0] text bytes, [1] flags
     DBuf<char> d_vcf_slots;
     DBuf<uint32_t> d_vcf_line_len, d_vcf_out_off;
     PinnedBuf<uint32_t> h_vcf_ctl;
@@ -321,44 +230,13 @@ struct drprg_index {
     DBuf<double> d_prob, d_M;
     DBuf<uint32_t> d_len, d_up, d_path, d_path_len;
 
+    // the members free the rest, on this device; a host-only handle (device -1) owns nothing and makes no CUDA call
     ~drprg_index() {
         workers.clear();
         replicas.clear();
         if (device < 0) return;
         cudaSetDevice(device);
         if (ipc_mapping) cudaIpcCloseMemHandle(ipc_mapping);
-        for (void* p : {(void*)d_slots, (void*)d_recs, (void*)d_filter, (void*)d_knode_base, (void*)d_edge_off, (void*)d_edges,
-                        (void*)d_is_terminal, (void*)d_needs_mean, (void*)d_accum, (void*)d_thresh, (void*)d_counters, (void*)d_rec_off,
-                        (void*)d_allele_off, (void*)d_allele_kn, (void*)d_knode_locus, (void*)d_hist, (void*)d_kfilter, (void*)d_locus_level_off, (void*)d_level_start, (void*)d_level_nodes, (void*)d_level_singles})
-            if (p) cudaFree(p);
-        if (h_counters) cudaFreeHost(h_counters);
-        hi.release(); lo.release(); gkey.release(); gkept.release();
-        act_read.release(); act_base.release(); act_count.release(); act_lk.release(); lk_ovf.release(); big_list.release(); cov_keys.release();
-        for (auto& b : scratch) b.release();
-        read_count.release(); read_base.release();
-        partials.release();
-        queue.release(); queue_kmer.release();
-        d_gt_u32.release(); d_gt_f64.release(); d_gt_i32.release(); d_gt_f32.release();
-        d_prob.release(); d_M.release(); d_len.release(); d_up.release(); d_path.release(); d_path_len.release();
-        for (auto& e : ev)
-            if (e) cudaEventDestroy(e);
-        h_path.release(); h_plen.release(); h_u32.release(); h_done.release(); h_f64.release(); h_gt.release(); h_acc.release();
-        h_vcf.release(); h_vcf_ctl.release(); d_vcf_slots.release(); d_vcf_line_len.release(); d_vcf_out_off.release();
-        for (void* p : {(void*)d_vcf_prefix, (void*)d_vcf_prefix_off, (void*)d_vcf_slot_off, (void*)d_vcf_ctl})
-            if (p) cudaFree(p);
-        for (auto& e : ev_ml)
-            if (e) cudaEventDestroy(e);
-        if (st_copy) cudaStreamDestroy(st_copy);
-        if (st_acc) cudaStreamDestroy(st_acc);
-        for (auto& e : ev_acc)
-            if (e) cudaEventDestroy(e);
-        if (d_hist1000) cudaFree(d_hist1000);
-        if (d_thresh_f64) cudaFree(d_thresh_f64);
-        if (d_thresh_i32) cudaFree(d_thresh_i32);
-        h_thresh.release();
-        h_small.release();
-        if (st_ml) cudaStreamDestroy(st_ml);
-        if (st_gt) cudaStreamDestroy(st_gt);
     }
 };
 
@@ -401,12 +279,12 @@ void upload_index(drprg_index* X) {
         filter[h & ((1u << fb) - 1)] |= (1u << ((h >> fb) & 31)) | (1u << ((h >> (fb + 5)) & 31));
         i = j;
     }
-    X->d_slots = to_device(slots);
-    X->d_recs = to_device(recs);
-    X->d_filter = to_device(filter);
+    X->d_slots.assign(slots);
+    X->d_recs.assign(recs);
+    X->d_filter.assign(filter);
     X->table_slots = 1u << sb;
     X->filter_words = 1u << fb;
-    X->T = DevTable{X->d_slots, sb, X->d_recs, X->d_filter, fb};
+    X->T = DevTable{X->d_slots.p, sb, X->d_recs.p, X->d_filter.p, fb};
     // ---- k-mer screen: the k-mers behind the indexed hashes, both orientations (hash64 is invertible)
     if (H.k >= 8 && H.k <= 15 && distinct > 0) {
         const uint64_t mask = (1ull << (2 * H.k)) - 1;
@@ -436,8 +314,8 @@ void upload_index(drprg_index* X) {
         std::vector<uint32_t> kfilter(nw, 0);
         for (uint32_t x : kmers) screen_filter_insert(kfilter.data(), nw, x, H.k);
         if (screen_pays) {
-            X->d_kfilter = to_device(kfilter);
-            X->T.kfilter = X->d_kfilter;
+            X->d_kfilter.assign(kfilter);
+            X->T.kfilter = X->d_kfilter.p;
             X->T.kfilter_words = nw;
         }
     }
@@ -460,10 +338,10 @@ void upload_index(drprg_index* X) {
     edge_off[N] = (uint32_t)edges.size();
     X->n_edges = edges.size();
     X->n_ivs = n_ivs;
-    X->d_knode_base = to_device(H.knode_base);
-    X->d_edge_off = to_device(edge_off);
-    X->d_edges = to_device(edges);
-    X->d_is_terminal = to_device(term);
+    X->d_knode_base.assign(H.knode_base);
+    X->d_edge_off.assign(edge_off);
+    X->d_edges.assign(edges);
+    X->d_is_terminal.assign(term);
     {   // a node's mean log-prob is only ever compared when one of its predecessors has more than one out-edge
         std::vector<uint8_t> needs(N, 0);
         for (size_t l = 0; l < H.loci.size(); ++l) {
@@ -473,7 +351,7 @@ void upload_index(drprg_index* X) {
                 if (L.kout[r].size() > 1)
                     for (uint32_t o : L.kout[r]) needs[base + o] = 1;
         }
-        X->d_needs_mean = to_device(needs);
+        X->d_needs_mean.assign(needs);
     }
     {   // level order for the level-parallel ML-path kernel: level = 1 + max level of the successors (terminus = 0)
         std::vector<uint32_t> locus_level_off(1, 0), level_start(1, 0), level_nodes, level_singles;
@@ -500,29 +378,30 @@ void upload_index(drprg_index* X) {
             }
             locus_level_off.push_back((uint32_t)level_start.size() - 1);
         }
-        X->d_locus_level_off = to_device(locus_level_off);
-        X->d_level_start = to_device(level_start);
-        X->d_level_nodes = to_device(level_nodes);
-        X->d_level_singles = to_device(level_singles);
+        X->d_locus_level_off.assign(locus_level_off);
+        X->d_level_start.assign(level_start);
+        X->d_level_nodes.assign(level_nodes);
+        X->d_level_singles.assign(level_singles);
     }
     X->n_accum = 2ull * N + H.loci.size() + 4;
     // 16 extra words behind the accumulator hold the cross-GPU flags of a read-sharded run (ready epoch, arrival counter)
-    CK(cudaMalloc(&X->d_accum, (accum_flag_offset(X->n_accum) + 16) * sizeof(int32_t)));
-    CK(cudaMemset(X->d_accum, 0, (accum_flag_offset(X->n_accum) + 16) * sizeof(int32_t)));
-    CK(cudaMalloc(&X->d_thresh, std::max<size_t>(1, H.loci.size()) * sizeof(uint32_t)));
-    CK(cudaMalloc(&X->d_counters, CTR_COUNT * sizeof(unsigned long long)));
-    CK(cudaMallocHost(&X->h_counters, CTR_COUNT * sizeof(unsigned long long)));
+    const size_t accum_words = accum_flag_offset(X->n_accum) + 16;
+    X->d_accum.reserve(accum_words, accum_words);
+    CK(cudaMemset(X->d_accum.p, 0, accum_words * sizeof(int32_t)));
+    X->d_thresh.reserve(std::max<size_t>(1, H.loci.size()), std::max<size_t>(1, H.loci.size()));
+    X->d_counters.reserve(CTR_COUNT, CTR_COUNT);
+    X->h_counters.reserve(CTR_COUNT, CTR_COUNT);
 
-    for (auto& e : X->ev) CK(cudaEventCreate(&e));
+    for (auto& e : X->ev) e = new_event(cudaEventDefault);
     std::vector<uint32_t> knode_locus(N);
     for (size_t l = 0; l < H.loci.size(); ++l) {
         for (uint32_t g = H.knode_base[l]; g < H.knode_base[l + 1]; ++g) knode_locus[g] = (uint32_t)l;
         X->max_locus_knodes = std::max(X->max_locus_knodes, H.knode_base[l + 1] - H.knode_base[l]);
         X->max_locus_edges = std::max(X->max_locus_edges, edge_off[H.knode_base[l + 1]] - edge_off[H.knode_base[l]]);
     }
-    X->d_knode_locus = to_device(knode_locus);
-    CK(cudaMalloc(&X->d_hist, 200 * sizeof(uint32_t)));
-    CK(cudaMalloc(&X->d_hist1000, 1000 * sizeof(uint32_t)));
+    X->d_knode_locus.assign(knode_locus);
+    X->d_hist.reserve(200, 200);
+    X->d_hist1000.reserve(1000, 1000);
     X->sites.assign(H.loci.size(), drprg_index::LocusSites());
     X->loci_by_name.resize(H.loci.size());
     for (uint32_t l = 0; l < H.loci.size(); ++l) X->loci_by_name[l] = l;
@@ -593,13 +472,13 @@ void sample_begin(drprg_index* X, const drprg_map_opts* o, uint32_t first_read_l
     }
     X->min_thresh = thr.empty() ? 0u : *std::min_element(thr.begin(), thr.end());
     if (thr != X->thresh_on_device) {  // unchanged between the samples of a batch: skip the synchronous copy
-        if (!thr.empty()) CK(cudaMemcpy(X->d_thresh, thr.data(), thr.size() * 4, cudaMemcpyHostToDevice));
+        if (!thr.empty()) CK(cudaMemcpy(X->d_thresh.p, thr.data(), thr.size() * 4, cudaMemcpyHostToDevice));
         X->thresh_on_device = thr;
     }
-    CK(cudaMemset(X->d_accum, 0, X->n_accum * sizeof(int32_t)));
+    CK(cudaMemset(X->d_accum.p, 0, X->n_accum * sizeof(int32_t)));
     ++X->epoch;
     if (X->world > 1 && X->accum_shared)  // the other ranks may add to this accumulator from here on
-        launch_flag_publish(reinterpret_cast<uint32_t*>(X->d_accum + accum_flag_offset(X->n_accum)), X->epoch, 0);
+        launch_flag_publish(reinterpret_cast<uint32_t*>(X->d_accum.p + accum_flag_offset(X->n_accum)), X->epoch, 0);
     X->total_bases = X->n_reads = 0;
     X->own_bases = X->own_reads = 0;
     X->retained.clear();
@@ -650,28 +529,28 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     // skip their work, the accumulators are untouched) and the batch is redone with larger buffers.
     for (int attempt = 0;; ++attempt) {
         const uint64_t queue_cap = X->T.kfilter ? std::min(X->queue.cap, X->queue_kmer.cap) : 0;
-        CK(cudaMemsetAsync(X->d_counters, 0, CTR_COUNT * sizeof(unsigned long long), st));
-        CK(cudaEventRecord(X->ev[0], st));
+        CK(cudaMemsetAsync(X->d_counters.p, 0, CTR_COUNT * sizeof(unsigned long long), st));
+        CK(cudaEventRecord(X->ev[0].get(), st));
         for (int c = 0; c < B->n_chunks; ++c) {
             DevReads Rc = B->R;
             Rc.hit_count = X->read_count.p;
             if (B->n_chunks > 1) {
                 const uint64_t lo = B->chunk_lo[c], hi = B->chunk_lo[c + 1];
                 Rc.hit_count = X->read_count.p + lo;
-                if (B->ev[c]) CK(cudaStreamWaitEvent(st, B->ev[c], 0));
+                if (B->ev[c]) CK(cudaStreamWaitEvent(st, B->ev[c].get(), 0));
                 Rc.words = B->R.stride_words ? B->R.words + lo * B->R.stride_words : B->R.words;
                 Rc.word_off = B->R.word_off ? B->R.word_off + lo : nullptr;
                 Rc.lens = B->R.lens + lo;
                 Rc.n_reads = hi - lo;
                 Rc.read_id_base = B->R.read_id_base + (uint32_t)lo;
             }
-            launch_sketch_lookup(Rc, X->T, H.w, H.k, X->hi.p, X->lo.p, X->d_counters + CTR_HITS, X->hi.cap, X->sm_count, B->max_len, st,
-                                 X->queue.p, queue_cap, X->d_counters + CTR_QUEUE, X->queue_kmer.p);
+            launch_sketch_lookup(Rc, X->T, H.w, H.k, X->hi.p, X->lo.p, X->d_counters.p + CTR_HITS, X->hi.cap, X->sm_count, B->max_len, st,
+                                 X->queue.p, queue_cap, X->d_counters.p + CTR_QUEUE, X->queue_kmer.p);
         }
         CK(cudaGetLastError());
-        CK(cudaEventRecord(X->ev[1], st));
+        CK(cudaEventRecord(X->ev[1].get(), st));
         PostBuffers PB{};
-        PB.hi = X->hi.p; PB.lo = X->lo.p; PB.ctr = X->d_counters;
+        PB.hi = X->hi.p; PB.lo = X->lo.p; PB.ctr = X->d_counters.p;
         PB.read_count = X->read_count.p; PB.read_base = X->read_base.p;
         PB.act_read = X->act_read.p; PB.act_base = X->act_base.p; PB.act_count = X->act_count.p;
         PB.act_lk = X->act_lk.p; PB.lk_ovf = X->lk_ovf.p;
@@ -679,26 +558,26 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
         for (int i = 0; i < 10; ++i) PB.scratch[i] = X->scratch[i].p;
         PB.partials = X->partials.p; PB.n_partials = X->n_partials;
         if (X->reduce_dst && X->flag_ready) launch_flag_wait(X->flag_ready, X->epoch, st);  // root has zeroed its accumulator for this sample
-        launch_postprocess(PB, PostCaps{X->hi.cap, queue_cap}, B->R.read_id_base, B->R.n_reads, X->opts.max_diff, X->min_thresh, X->d_thresh,
-                           X->d_knode_base, N, P, X->reduce_dst ? X->reduce_dst : X->d_accum,
+        launch_postprocess(PB, PostCaps{X->hi.cap, queue_cap}, B->R.read_id_base, B->R.n_reads, X->opts.max_diff, X->min_thresh, X->d_thresh.p,
+                           X->d_knode_base.p, N, P, X->reduce_dst ? X->reduce_dst : X->d_accum.p,
                            (X->reduce_dst || X->accum_shared) ? 1 : 0,  // several GPUs add into one accumulator: every writer uses red
                            X->sm_count, st,
-                           X->ev[2], X->ev[3]);
-        CK(cudaEventRecord(X->ev[4], st));
+                           X->ev[2].get(), X->ev[3].get());
+        CK(cudaEventRecord(X->ev[4].get(), st));
         CK(cudaGetLastError());
         if (!X->reduce_dst && !X->accum_shared) {
             // what the genotype step needs first (coverage histogram, locus read counts: 4 KB) rides on this batch's final
             // synchronisation; it stays valid unless the accumulators change before drprg_cuda_genotype (another batch
             // recomputes it, a reduce from other GPUs invalidates it)
-            launch_cov_hist(X->d_accum, N, X->d_is_terminal, X->d_knode_locus, X->d_accum + 2ull * N, X->d_hist1000, st);
+            launch_cov_hist(X->d_accum.p, N, X->d_is_terminal.p, X->d_knode_locus.p, X->d_accum.p + 2ull * N, X->d_hist1000.p, st);
             X->h_small.resize(1000 + (size_t)P + 4);
-            CK(cudaMemcpyAsync(X->h_small.data(), X->d_hist1000, 1000 * 4, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(X->h_small.data() + 1000, X->d_accum + 2ull * N, (size_t)P * 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(X->h_small.data(), X->d_hist1000.p, 1000 * 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(X->h_small.data() + 1000, X->d_accum.p + 2ull * N, (size_t)P * 4, cudaMemcpyDeviceToHost, st));
         }
-        CK(cudaMemcpyAsync(X->h_counters, X->d_counters, CTR_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X->h_counters.p, X->d_counters.p, CTR_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        nh = X->h_counters[CTR_HITS];
-        const uint64_t nq = X->h_counters[CTR_QUEUE_NEED];  // largest screen queue any chunk wanted
+        nh = X->h_counters.p[CTR_HITS];
+        const uint64_t nq = X->h_counters.p[CTR_QUEUE_NEED];  // largest screen queue any chunk wanted
         if (nh <= X->hi.cap && nq <= queue_cap) break;
         if (attempt == 2) throw std::runtime_error("hit buffer overflow");
         // the lookup kernels counted hits per read that were never scattered: the counters must be zero before the redo
@@ -712,14 +591,14 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     static const bool timing = getenv("DRPRG_TIMING") != nullptr;
     if (timing)
         fprintf(stderr, "[drprg-cuda] map batch: %llu reads, %d chunks, screen queue %llu (largest chunk), probe survivors %llu, hits %llu\n",
-                (unsigned long long)B->R.n_reads, B->n_chunks, X->h_counters[CTR_QUEUE_NEED], X->h_counters[CTR_SURVIVORS], (unsigned long long)nh);
+                (unsigned long long)B->R.n_reads, B->n_chunks, X->h_counters.p[CTR_QUEUE_NEED], X->h_counters.p[CTR_SURVIVORS], (unsigned long long)nh);
     X->hist_on_host = !X->reduce_dst && !X->accum_shared;
-    CK(cudaEventElapsedTime(&X->timings[0], X->ev[0], X->ev[1]));
-    CK(cudaEventElapsedTime(&X->timings[1], X->ev[1], X->ev[2]));
-    CK(cudaEventElapsedTime(&X->timings[2], X->ev[2], X->ev[3]));
-    CK(cudaEventElapsedTime(&X->timings[3], X->ev[3], X->ev[4]));
+    CK(cudaEventElapsedTime(&X->timings[0], X->ev[0].get(), X->ev[1].get()));
+    CK(cudaEventElapsedTime(&X->timings[1], X->ev[1].get(), X->ev[2].get()));
+    CK(cudaEventElapsedTime(&X->timings[2], X->ev[2].get(), X->ev[3].get()));
+    CK(cudaEventElapsedTime(&X->timings[3], X->ev[3].get(), X->ev[4].get()));
     X->last_n_hits = nh;
-    X->last_n_active = X->h_counters[CTR_ACTIVE];
+    X->last_n_active = X->h_counters.p[CTR_ACTIVE];
     X->last_id_base = B->R.read_id_base;
     X->total_bases += B->total_bases;
     X->n_reads += B->R.n_reads;
@@ -745,7 +624,7 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
             }
     }
     if (n_hits) *n_hits = nh;
-    if (n_kept) *n_kept = X->h_counters[CTR_KEPT];
+    if (n_kept) *n_kept = X->h_counters.p[CTR_KEPT];
 }
 
 void flush_scalars(drprg_index* X) {
@@ -753,10 +632,10 @@ void flush_scalars(drprg_index* X) {
     int32_t s[4] = {(int32_t)(X->total_bases & 0xffffff), (int32_t)(X->total_bases >> 24), (int32_t)(X->n_reads & 0xffffff),
                     (int32_t)(X->n_reads >> 24)};
     if (X->accum_shared && X->world > 1) {  // the other ranks have added their scalars (shard_done): this rank's join them
-        launch_add_scalars(X->d_accum + X->n_accum - 4, s, 0);
+        launch_add_scalars(X->d_accum.p + X->n_accum - 4, s, 0);
         CK(cudaStreamSynchronize(0));
     } else {
-        CK(cudaMemcpy(X->d_accum + X->n_accum - 4, s, sizeof s, cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(X->d_accum.p + X->n_accum - 4, s, sizeof s, cudaMemcpyHostToDevice));
     }
     X->scalars_in_buffer = true;
 }
@@ -800,7 +679,7 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
     // a previous call that threw after launching the ML-path kernel may have left it running: it writes into the pinned
     // path / flag buffers this call is about to reset
     if (X->ml_in_flight) {
-        cudaStreamSynchronize(X->st_ml);
+        cudaStreamSynchronize(X->st_ml.get());
         X->ml_in_flight = false;
     }
     // --vcf-refs is loaded before anything is launched (a bad path must not leave kernels behind)
@@ -814,34 +693,32 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
         }
     }
     if (X->accum_shared && X->world > 1)  // every other rank has finished adding its shard (shard_done)
-        launch_flag_wait(reinterpret_cast<uint32_t*>(X->d_accum + accum_flag_offset(X->n_accum)) + 1, X->epoch * (uint32_t)(X->world - 1), 0);
+        launch_flag_wait(reinterpret_cast<uint32_t*>(X->d_accum.p + accum_flag_offset(X->n_accum)) + 1, X->epoch * (uint32_t)(X->world - 1), 0);
     const bool reuse_hist = X->hist_on_host;  // downloaded at the end of the last map_batch, accumulators untouched since
     if (!reuse_hist) flush_scalars(X);
     if (!X->st_ml) {
-        CK(cudaStreamCreateWithFlags(&X->st_ml, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&X->st_gt, cudaStreamNonBlocking));
-        CK(cudaStreamCreateWithFlags(&X->st_acc, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&X->ev_acc[0], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&X->ev_acc[1], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&X->ev_acc[2], cudaEventDisableTiming));
-        CK(cudaMalloc(&X->d_thresh_f64, sizeof(double)));
-        CK(cudaMalloc(&X->d_thresh_i32, sizeof(int)));
+        X->st_ml = new_stream();
+        X->st_gt = new_stream();
+        X->st_acc = new_stream();
+        for (auto& e : X->ev_acc) e = new_event(cudaEventDisableTiming);
+        X->d_thresh_f64.reserve(1, 1);
+        X->d_thresh_i32.reserve(1, 1);
     }
     // On the critical path the host only needs the 1000-bin coverage histogram (built on the device), the locus read
     // counts and the scalars: 4 KB.  The full accumulator (0.3 MB, pinned destination) is needed when the ML paths are
     // verified; it comes down on its own stream, ordered after whatever produced the accumulator on `st` (map_batch, or
     // the caller's allreduce).
     X->h_acc.resize(X->n_accum);
-    CK(cudaEventRecord(X->ev_acc[0], st));
-    CK(cudaStreamWaitEvent(X->st_acc, X->ev_acc[0], 0));
-    CK(cudaMemcpyAsync(X->h_acc.data(), X->d_accum, X->n_accum * 4, cudaMemcpyDeviceToHost, X->st_acc));
-    CK(cudaEventRecord(X->ev_acc[1], X->st_acc));
+    CK(cudaEventRecord(X->ev_acc[0].get(), st));
+    CK(cudaStreamWaitEvent(X->st_acc.get(), X->ev_acc[0].get(), 0));
+    CK(cudaMemcpyAsync(X->h_acc.data(), X->d_accum.p, X->n_accum * 4, cudaMemcpyDeviceToHost, X->st_acc.get()));
+    CK(cudaEventRecord(X->ev_acc[1].get(), X->st_acc.get()));
     uint64_t total_bases = X->total_bases;  // this process's batches; after an allreduce the summed scalars are read back
     if (!reuse_hist) {
-        launch_cov_hist(X->d_accum, N, X->d_is_terminal, X->d_knode_locus, X->d_accum + 2ull * N, X->d_hist1000, st);
+        launch_cov_hist(X->d_accum.p, N, X->d_is_terminal.p, X->d_knode_locus.p, X->d_accum.p + 2ull * N, X->d_hist1000.p, st);
         X->h_small.resize(1000 + (size_t)P + 4);
-        CK(cudaMemcpyAsync(X->h_small.data(), X->d_hist1000, 1000 * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(X->h_small.data() + 1000, X->d_accum + 2ull * N, ((size_t)P + 4) * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X->h_small.data(), X->d_hist1000.p, 1000 * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X->h_small.data() + 1000, X->d_accum.p + 2ull * N, ((size_t)P + 4) * 4, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         const int32_t* sc = (const int32_t*)(X->h_small.data() + 1000) + P;
         total_bases = (uint64_t)(uint32_t)sc[0] + ((uint64_t)(uint32_t)sc[1] << 24);
@@ -864,16 +741,16 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
     MP.minor_af = X->minor_af >= 0.0f ? X->minor_af : (X->opts.illumina ? 0.1f : 1.0f);  // src/minor.rs:11-12,26-33
     X->d_prob.ensure(N); X->d_M.ensure(N); X->d_len.ensure(N);
     X->d_up.ensure((size_t)N * LV_MAX); X->d_path.ensure(N); X->d_path_len.ensure(P);
-    launch_node_prob(X->d_accum, N, X->d_is_terminal, MP, X->d_prob.p, st);
-    launch_prob_hist(X->d_prob.p, N, X->d_is_terminal, X->d_knode_locus, X->d_accum + 2ull * N, X->d_hist, st);
+    launch_node_prob(X->d_accum.p, N, X->d_is_terminal.p, MP, X->d_prob.p, st);
+    launch_prob_hist(X->d_prob.p, N, X->d_is_terminal.p, X->d_knode_locus.p, X->d_accum.p + 2ull * N, X->d_hist.p, st);
     bool any_present = false;
     for (uint32_t l = 0; l < P; ++l) any_present = any_present || locus_reads[l] > 0;
     // the threshold (valley of the 200-bin histogram) is found on the device too: the ML-path kernel reads it from
     // device memory and starts without a host round trip; the host picks the value up later
-    launch_prob_thresh(X->d_hist, any_present, X->fit.thresh, X->d_thresh_f64, X->d_thresh_i32, st);
+    launch_prob_thresh(X->d_hist.p, any_present, X->fit.thresh, X->d_thresh_f64.p, X->d_thresh_i32.p, st);
     X->h_thresh.resize(1);
-    CK(cudaMemcpyAsync(X->h_thresh.data(), X->d_thresh_i32, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CK(cudaEventRecord(X->ev_acc[2], st));
+    CK(cudaMemcpyAsync(X->h_thresh.data(), X->d_thresh_i32.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaEventRecord(X->ev_acc[2].get(), st));
     MP.thresh = (double)X->fit.thresh;  // placeholder for kernels that do not read it (S8); S7 uses d_thresh_f64
     lap(1);
     // ---- S7 on the device: the ML-path kernel is a latency chain per locus (~0.4 ms).  It only decides which loci
@@ -881,31 +758,29 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
     // while S8 (per-allele statistics + likelihoods) and the VCF text are produced SPECULATIVELY for the common
     // outcome "every locus with reads is present, no extra records"; the outcome is verified afterwards and
     // anything that deviates is redone on the slow path.
-    if (!X->ev_ml[0]) {
-        CK(cudaEventCreate(&X->ev_ml[0]));
-        CK(cudaEventCreate(&X->ev_ml[1]));
-    }
+    if (!X->ev_ml[0])
+        for (auto& e : X->ev_ml) e = new_event(cudaEventDefault);
     X->h_path.resize(N);
     X->h_plen.resize(P);
     X->h_done.resize(P);
     std::fill(X->h_done.begin(), X->h_done.end(), 0u);
-    CK(cudaStreamWaitEvent(X->st_ml, X->ev_acc[2], 0));  // node scores and threshold are produced on `st`
-    CK(cudaMemsetAsync(X->d_path.p, 0, (size_t)N * 4, X->st_ml));  // absent loci leave their slice unwritten
-    CK(cudaEventRecord(X->ev_ml[0], X->st_ml));
+    CK(cudaStreamWaitEvent(X->st_ml.get(), X->ev_acc[2].get(), 0));  // node scores and threshold are produced on `st`
+    CK(cudaMemsetAsync(X->d_path.p, 0, (size_t)N * 4, X->st_ml.get()));  // absent loci leave their slice unwritten
+    CK(cudaEventRecord(X->ev_ml[0].get(), X->st_ml.get()));
     // The level-parallel kernel writes every locus's path straight into pinned host memory (UVA: the same pointers
     // are valid on the device) and raises a per-locus flag, so the host can verify the small loci while the big ones
     // are still running; the generic kernel leaves the paths in device memory and they are copied back as a whole.
     const bool ml_streamed = launch_mlpath(
-        P, X->d_knode_base, X->d_edge_off, X->d_edges, X->d_prob.p, X->d_accum + 2ull * N, MP, X->d_M.p, X->d_len.p, X->d_up.p, N,
-        X->d_path.p, X->d_path_len.p, X->max_locus_knodes, X->max_locus_edges, X->d_needs_mean, X->st_ml,
-        X->d_locus_level_off, X->d_level_start, X->d_level_nodes, X->d_level_singles,
-        X->h_path.data(), X->h_plen.data(), X->h_done.data(), X->d_thresh_f64);
+        P, X->d_knode_base.p, X->d_edge_off.p, X->d_edges.p, X->d_prob.p, X->d_accum.p + 2ull * N, MP, X->d_M.p, X->d_len.p, X->d_up.p, N,
+        X->d_path.p, X->d_path_len.p, X->max_locus_knodes, X->max_locus_edges, X->d_needs_mean.p, X->st_ml.get(),
+        X->d_locus_level_off.p, X->d_level_start.p, X->d_level_nodes.p, X->d_level_singles.p,
+        X->h_path.data(), X->h_plen.data(), X->h_done.data(), X->d_thresh_f64.p);
     X->ml_in_flight = true;
-    CK(cudaEventRecord(X->ev_ml[1], X->st_ml));
+    CK(cudaEventRecord(X->ev_ml[1].get(), X->st_ml.get()));
     CK(cudaGetLastError());
     if (!ml_streamed) {
-        CK(cudaMemcpyAsync(X->h_path.data(), X->d_path.p, (size_t)N * 4, cudaMemcpyDeviceToHost, X->st_ml));
-        CK(cudaMemcpyAsync(X->h_plen.data(), X->d_path_len.p, (size_t)P * 4, cudaMemcpyDeviceToHost, X->st_ml));
+        CK(cudaMemcpyAsync(X->h_path.data(), X->d_path.p, (size_t)N * 4, cudaMemcpyDeviceToHost, X->st_ml.get()));
+        CK(cudaMemcpyAsync(X->h_plen.data(), X->d_path_len.p, (size_t)P * 4, cudaMemcpyDeviceToHost, X->st_ml.get()));
     }
     // ---- reference paths / site tables (read independent, cached per --vcf-refs file, loaded above)
     auto ensure_sites = [&](uint32_t l) {
@@ -937,11 +812,9 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
                 G.rec_off.push_back((uint32_t)G.allele_off.size() - 1);
             }
             CK(cudaStreamSynchronize(s8));
-            for (void* p : {(void*)X->d_rec_off, (void*)X->d_allele_off, (void*)X->d_allele_kn})
-                if (p) cudaFree(p);
-            X->d_rec_off = to_device(G.rec_off);
-            X->d_allele_off = to_device(G.allele_off);
-            X->d_allele_kn = to_device(G.allele_kn);
+            X->d_rec_off.assign(G.rec_off);
+            X->d_allele_off.assign(G.allele_off);
+            X->d_allele_kn.assign(G.allele_kn);
             {   // the static columns of every record line and the slots of the sample columns (VCF text on the device)
                 std::vector<char> prefix;
                 std::vector<uint32_t> poff(1, 0), soff(1, 0);
@@ -951,14 +824,12 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
                     poff.push_back((uint32_t)prefix.size());
                     soff.push_back(soff.back() + (uint32_t)vcf_sample_column_bound(G.rec_off[i + 1] - G.rec_off[i]));
                 }
-                for (void* p : {(void*)X->d_vcf_prefix, (void*)X->d_vcf_prefix_off, (void*)X->d_vcf_slot_off})
-                    if (p) cudaFree(p);
-                X->d_vcf_prefix = to_device(prefix);
-                X->d_vcf_prefix_off = to_device(poff);
-                X->d_vcf_slot_off = to_device(soff);
+                X->d_vcf_prefix.assign(prefix);
+                X->d_vcf_prefix_off.assign(poff);
+                X->d_vcf_slot_off.assign(soff);
                 X->vcf_prefix_bytes = prefix.size();
                 X->vcf_slot_bytes = soff.back();
-                if (!X->d_vcf_ctl) CK(cudaMalloc(&X->d_vcf_ctl, 2 * sizeof(uint32_t)));
+                X->d_vcf_ctl.reserve(2, 2);
             }
             X->csr_records = X->sample_records.empty() ? X->records : std::vector<const SiteRecord*>();
         }
@@ -979,7 +850,7 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
             X->d_gt_f32.ensure((size_t)nr * 2 + na);
             uint32_t* u = X->d_gt_u32.p;
             double* f = X->d_gt_f64.p;
-            DevGenotype DG{nr, na, X->d_rec_off, X->d_allele_off, X->d_allele_kn, u, u + na, u + 2 * (size_t)na, u + 3 * (size_t)na,
+            DevGenotype DG{nr, na, X->d_rec_off.p, X->d_allele_off.p, X->d_allele_kn.p, u, u + na, u + 2 * (size_t)na, u + 3 * (size_t)na,
                            u + 4 * (size_t)na, u + 5 * (size_t)na, f, f + na, f + 2 * (size_t)na, X->d_gt_i32.p};
             // the statistics drprg's filters derive from the record come out of the same kernel (they stay on the device
             // until drprg_cuda_gt_filter_stats asks for them)
@@ -988,19 +859,19 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
             DG.frs = X->d_gt_f32.p;
             DG.sb_ratio = X->d_gt_f32.p + nr;
             DG.pdp = X->d_gt_f32.p + 2 * (size_t)nr;
-            launch_genotype(X->d_accum, DG, MP, s8);
+            launch_genotype(X->d_accum.p, DG, MP, s8);
             // the record lines: formatted by the device into the host-mapped text buffer, right behind the header
             X->d_vcf_slots.ensure(X->vcf_slot_bytes + 1);
             X->d_vcf_line_len.ensure(nr);
             X->d_vcf_out_off.ensure((size_t)nr + 1);
-            CK(cudaMemsetAsync(X->d_vcf_ctl, 0, 2 * sizeof(uint32_t), s8));
-            DevVcfText VT{X->d_vcf_prefix, X->d_vcf_prefix_off, X->d_vcf_slot_off, X->d_vcf_slots.p, X->d_vcf_line_len.p,
-                          X->d_vcf_out_off.p, X->h_vcf.data() + hl, (uint32_t)(X->vcf_prefix_bytes + X->vcf_slot_bytes), X->d_vcf_ctl,
-                          X->d_vcf_ctl + 1};
+            CK(cudaMemsetAsync(X->d_vcf_ctl.p, 0, 2 * sizeof(uint32_t), s8));
+            DevVcfText VT{X->d_vcf_prefix.p, X->d_vcf_prefix_off.p, X->d_vcf_slot_off.p, X->d_vcf_slots.p, X->d_vcf_line_len.p,
+                          X->d_vcf_out_off.p, X->h_vcf.data() + hl, (uint32_t)(X->vcf_prefix_bytes + X->vcf_slot_bytes), X->d_vcf_ctl.p,
+                          X->d_vcf_ctl.p + 1};
             static const bool host_text = getenv("DRPRG_VCF_TEXT") && std::string(getenv("DRPRG_VCF_TEXT")) == "host";
             if (!host_text) launch_vcf_text(DG, VT, s8);
             CK(cudaGetLastError());
-            CK(cudaMemcpyAsync(X->h_vcf_ctl.data(), X->d_vcf_ctl, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s8));
+            CK(cudaMemcpyAsync(X->h_vcf_ctl.data(), X->d_vcf_ctl.p, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s8));
             // the arrays themselves (getters, drprg_cuda_gt_*): downloaded into pinned buffers, unpacked on first use
             X->h_u32.resize((size_t)na * 6);
             X->h_f64.resize((size_t)na * 2 + nr);
@@ -1047,15 +918,15 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
         for (auto& r : X->sites[l].merged) X->records.push_back(&r);
     }
     lap(2);
-    run_s8_and_format(X->st_gt);
-    CK(cudaEventSynchronize(X->ev_acc[2]));  // long done: the threshold the device chose
+    run_s8_and_format(X->st_gt.get());
+    CK(cudaEventSynchronize(X->ev_acc[2].get()));  // long done: the threshold the device chose
     X->fit.thresh = X->h_thresh.data()[0];
     MP.thresh = (double)X->fit.thresh;
     lap(3);
     // ---- verify the speculation against the ML paths
     const double tw0 = now_ms();
-    if (!ml_streamed) CK(cudaStreamSynchronize(X->st_ml));
-    CK(cudaEventSynchronize(X->ev_acc[1]));  // the full accumulator is on the host from here on
+    if (!ml_streamed) CK(cudaStreamSynchronize(X->st_ml.get()));
+    CK(cudaEventSynchronize(X->ev_acc[1].get()));  // the full accumulator is on the host from here on
     const double tw1 = now_ms();
     const uint32_t* path = X->h_path.data();
     const uint32_t* plen = X->h_plen.data();
@@ -1065,7 +936,7 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
         if (!ml_streamed) return true;
         for (uint64_t spin = 0; done[l] == 0u; ++spin) {
             if (ml_failed.load(std::memory_order_relaxed)) return false;
-            if ((spin & 0xffffu) == 0xffffu && cudaStreamQuery(X->st_ml) != cudaErrorNotReady && done[l] == 0u) {
+            if ((spin & 0xffffu) == 0xffffu && cudaStreamQuery(X->st_ml.get()) != cudaErrorNotReady && done[l] == 0u) {
                 ml_failed = true;  // the stream ended (or failed) without publishing: never spin forever
                 return false;
             }
@@ -1114,7 +985,7 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
         }
     }, 16);
     {
-        const cudaError_t mle = cudaStreamSynchronize(X->st_ml);
+        const cudaError_t mle = cudaStreamSynchronize(X->st_ml.get());
         X->ml_in_flight = false;
         if (mle != cudaSuccess)
             throw std::runtime_error(std::string("ML-path kernel failed: ") + cudaGetErrorString(mle));
@@ -1122,7 +993,7 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
     if (ml_failed.load()) throw std::runtime_error("the ML-path kernel ended without publishing every locus");
     {
         float ms = 0;
-        CK(cudaEventElapsedTime(&ms, X->ev_ml[0], X->ev_ml[1]));
+        CK(cudaEventElapsedTime(&ms, X->ev_ml[0].get(), X->ev_ml[1].get()));
         X->gt_ms[6] = ms;  // device time of the ML-path kernel (overlapped with S8 + VCF text on the host)
     }
     bool speculation_ok = true;
@@ -1152,26 +1023,10 @@ void genotype(drprg_index* X, const char* vcf_refs, const char* sample) {
                 for (auto& r : X->sample_records.back()) X->records.push_back(&r);
             }
         }
-        run_s8_and_format(X->st_gt);
+        run_s8_and_format(X->st_gt.get());
     }
     lap(5);
     X->have_gt = true;
-}
-
-void free_batch(drprg_batch* b) {
-    if (!b) return;
-    for (drprg_batch* sh : b->shards) free_batch(sh);
-    b->shards.clear();
-    for (auto& e : b->ev)
-        if (e) cudaEventDestroy(e);
-    if (b->owned) {
-        if (b->d_words) g_pool.put(b->d_words, b->b_words, b->device);
-        if (b->d_lens) g_pool.put(b->d_lens, b->b_lens, b->device);
-        if (b->d_off) g_pool.put(b->d_off, b->b_off, b->device);
-        if (b->d_seg_read) g_pool.put(b->d_seg_read, b->b_seg, b->device);
-        if (b->d_seg_start) g_pool.put(b->d_seg_start, b->b_seg, b->device);
-    }
-    delete b;
 }
 
 // long reads: cut every read into segments of 40*w k-mer positions so that the thread-per-item kernels get evenly
@@ -1191,64 +1046,57 @@ void build_segments(drprg_index* X, drprg_batch* B, const uint32_t* lens, uint64
         }
     }
     if (sr.empty()) return;
-    B->b_seg = sr.size() * 4;
-    B->d_seg_read = (uint32_t*)g_pool.get(B->b_seg, X->device);
-    B->d_seg_start = (uint32_t*)g_pool.get(B->b_seg, X->device);
-    CK(cudaMemcpyAsync(B->d_seg_read, sr.data(), B->b_seg, cudaMemcpyHostToDevice, cs));
-    CK(cudaMemcpyAsync(B->d_seg_start, ss.data(), B->b_seg, cudaMemcpyHostToDevice, cs));
+    const size_t bytes = sr.size() * 4;
+    B->d_seg_read = pool_get<uint32_t>(bytes, X->device);
+    B->d_seg_start = pool_get<uint32_t>(bytes, X->device);
+    CK(cudaMemcpyAsync(B->d_seg_read.get(), sr.data(), bytes, cudaMemcpyHostToDevice, cs));
+    CK(cudaMemcpyAsync(B->d_seg_start.get(), ss.data(), bytes, cudaMemcpyHostToDevice, cs));
     CK(cudaStreamSynchronize(cs));  // the staging vectors die with this scope
-    B->R.seg_read = B->d_seg_read;
-    B->R.seg_start = B->d_seg_start;
+    B->R.seg_read = B->d_seg_read.get();
+    B->R.seg_start = B->d_seg_start.get();
     B->R.n_segs = sr.size();
     B->R.seg_len = seg_len;
 }
 
-drprg_batch* upload_batch(drprg_index* X, const uint32_t* words, const uint64_t* word_off, uint32_t stride, const uint32_t* lens,
-                          uint64_t n, uint64_t total_bases, uint32_t id_base, cudaStream_t st) {
+std::unique_ptr<drprg_batch> upload_batch(drprg_index* X, const uint32_t* words, const uint64_t* word_off, uint32_t stride,
+                                          const uint32_t* lens, uint64_t n, uint64_t total_bases, uint32_t id_base, cudaStream_t st) {
     need_device(X);
     CK(cudaSetDevice(X->device));
-    std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(new drprg_batch(), free_batch);
-    B->owned = true;
+    std::unique_ptr<drprg_batch> B(new drprg_batch());
     const uint64_t nwords = stride ? n * (uint64_t)stride : (n ? word_off[n] : 0);
-    B->device = X->device;
-    B->b_words = std::max<uint64_t>(1, nwords + 2) * 4;
-    B->b_lens = std::max<uint64_t>(1, n) * 4;
-    B->d_words = (uint32_t*)g_pool.get(B->b_words, X->device);
-    B->d_lens = (uint32_t*)g_pool.get(B->b_lens, X->device);
-    if (!stride) {
-        B->b_off = (n + 1) * 8;
-        B->d_off = (uint64_t*)g_pool.get(B->b_off, X->device);
-    }
+    B->d_words = pool_get<uint32_t>(std::max<uint64_t>(1, nwords + 2) * 4, X->device);
+    B->d_lens = pool_get<uint32_t>(std::max<uint64_t>(1, n) * 4, X->device);
+    if (!stride) B->d_off = pool_get<uint64_t>((n + 1) * 8, X->device);
     const bool chunked = (st == nullptr) && nwords * 4 >= (8u << 20) && stride && stride * 16u <= SHORT_READ_MAX;
     cudaStream_t cs = st;
     if (chunked) {
-        if (!X->st_copy) CK(cudaStreamCreateWithFlags(&X->st_copy, cudaStreamNonBlocking));
-        cs = X->st_copy;
+        if (!X->st_copy) X->st_copy = new_stream();
+        cs = X->st_copy.get();
         B->n_chunks = 4;
     }
-    if (!stride) CK(cudaMemcpyAsync(B->d_off, word_off, (n + 1) * 8, cudaMemcpyHostToDevice, cs));
+    if (!stride) CK(cudaMemcpyAsync(B->d_off.get(), word_off, (n + 1) * 8, cudaMemcpyHostToDevice, cs));
     uint32_t ml = 0;
     for (int c = 0; c < B->n_chunks; ++c) {
         const uint64_t lo = n * (uint64_t)c / B->n_chunks, hi = n * (uint64_t)(c + 1) / B->n_chunks;
         B->chunk_lo[c] = lo;
         B->chunk_lo[c + 1] = hi;
         const uint64_t w0 = stride ? lo * stride : word_off[lo], w1 = stride ? hi * stride : word_off[hi];
-        if (w1 > w0) CK(cudaMemcpyAsync(B->d_words + w0, words + w0, (w1 - w0) * 4, cudaMemcpyHostToDevice, cs));
-        if (hi > lo) CK(cudaMemcpyAsync(B->d_lens + lo, lens + lo, (hi - lo) * 4, cudaMemcpyHostToDevice, cs));
+        if (w1 > w0) CK(cudaMemcpyAsync(B->d_words.get() + w0, words + w0, (w1 - w0) * 4, cudaMemcpyHostToDevice, cs));
+        if (hi > lo) CK(cudaMemcpyAsync(B->d_lens.get() + lo, lens + lo, (hi - lo) * 4, cudaMemcpyHostToDevice, cs));
         if (chunked) {
-            CK(cudaEventCreateWithFlags(&B->ev[c], cudaEventDisableTiming));
-            CK(cudaEventRecord(B->ev[c], cs));
+            B->ev[c] = new_event(cudaEventDisableTiming);
+            CK(cudaEventRecord(B->ev[c].get(), cs));
         }
         // the longest read only selects the kernel: a fixed stride that already bounds it needs no scan
         if (!(stride && stride * 16u <= SHORT_READ_MAX))
             for (uint64_t i = lo; i < hi; ++i) ml = std::max(ml, lens[i]);  // overlaps the copy just enqueued
     }
     if (stride && stride * 16u <= SHORT_READ_MAX) ml = stride * 16u;
-    B->R = DevReads{B->d_words, B->d_off, stride, B->d_lens, n, id_base};
+    B->R = DevReads{B->d_words.get(), B->d_off.get(), stride, B->d_lens.get(), n, id_base};
     B->total_bases = total_bases;
     B->max_len = ml;
     if (ml > SHORT_READ_MAX) build_segments(X, B.get(), lens, n, total_bases, cs);
-    return B.release();
+    return B;
 }
 
 // ============================================================================================
@@ -1325,7 +1173,7 @@ int load_multi(const std::string& text, uint32_t w, uint32_t k, int n_gpus, cons
             if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) CK(pe);
             cudaGetLastError();
         }
-        R->reduce_dst = root->d_accum;  // UVA: the root's pointer is valid on the peer once access is enabled
+        R->reduce_dst = root->d_accum.p;  // UVA: the root's pointer is valid on the peer once access is enabled
         root->replicas.push_back(std::move(R));
         root->workers.emplace_back(new GpuWorker());
     }
@@ -1345,11 +1193,11 @@ void multi_sample_begin(drprg_index* root, const drprg_map_opts* o, uint32_t fir
     });
 }
 
-drprg_batch* multi_upload(drprg_index* root, const uint32_t* words, const uint64_t* word_off, uint32_t stride, const uint32_t* lens,
-                          uint64_t n, uint64_t total_bases, uint32_t id_base) {
+std::unique_ptr<drprg_batch> multi_upload(drprg_index* root, const uint32_t* words, const uint64_t* word_off, uint32_t stride,
+                                          const uint32_t* lens, uint64_t n, uint64_t total_bases, uint32_t id_base) {
     const size_t G = root->gpus.size();
-    std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(new drprg_batch(), free_batch);
-    B->shards.assign(G, nullptr);
+    std::unique_ptr<drprg_batch> B(new drprg_batch());
+    B->shards.resize(G);
     B->R.n_reads = n;
     B->R.read_id_base = id_base;
     B->total_bases = total_bases;
@@ -1370,16 +1218,16 @@ drprg_batch* multi_upload(drprg_index* root, const uint32_t* words, const uint64
     });
     // total_bases counts the bases of dropped reads too (their lens are 0): the difference goes to the last shard
     uint64_t sum = 0;
-    for (auto* sh : B->shards) sum += sh->total_bases;
+    for (auto& sh : B->shards) sum += sh->total_bases;
     if (total_bases > sum) B->shards[G - 1]->total_bases += total_bases - sum;
-    return B.release();
+    return B;
 }
 
 void multi_map_batch(drprg_index* root, drprg_batch* B, uint64_t* n_hits, uint64_t* n_kept) {
     const size_t G = root->gpus.size();
     if (B->shards.size() != G) throw std::runtime_error("the batch was not uploaded through this multi-GPU handle");
     std::vector<uint64_t> nh(G, 0), nk(G, 0);
-    for_each_gpu(root, [&](size_t g, drprg_index* X) { map_batch(X, B->shards[g], 0, &nh[g], &nk[g]); });
+    for_each_gpu(root, [&](size_t g, drprg_index* X) { map_batch(X, B->shards[g].get(), 0, &nh[g], &nk[g]); });
     // every GPU's stream has been synchronised: all remote adds have landed in the root's accumulator
     uint64_t bases = 0, reads = 0, h = 0, kpt = 0;
     for (size_t g = 0; g < G; ++g) {
@@ -1409,7 +1257,7 @@ void map_batch_any(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_
 // device (ingest.cu); FASTA and anything unusual goes through the host parser and an upload.  DRPRG_HOST_INGEST=1 forces
 // the host parser (tests compare the two).
 struct FileBatch {
-    drprg_batch* B = nullptr;
+    std::unique_ptr<drprg_batch> B;
     uint64_t n_dropped = 0;
     uint32_t first_read_len = 0;
     bool on_device = false;  // packed on the device (else: host parser)
@@ -1418,24 +1266,15 @@ bool host_ingest_forced() {
     static const bool on = getenv("DRPRG_HOST_INGEST") != nullptr && atoi(getenv("DRPRG_HOST_INGEST")) != 0;
     return on;
 }
-struct Inflated {  // a gzip reads file inflated ahead of time (batch mode)
-    char* p = nullptr;
+struct Inflated {  // a gzip reads file inflated into host memory (ahead of time in batch mode)
+    std::unique_ptr<char, void (*)(void*)> p{nullptr, free};
     size_t n = 0;
     std::string error;
-    Inflated() = default;
-    Inflated(const Inflated&) = delete;
-    Inflated(Inflated&& o) noexcept : p(o.p), n(o.n), error(std::move(o.error)) { o.p = nullptr; }
-    Inflated& operator=(Inflated&& o) noexcept {
-        if (this != &o) {
-            free(p);
-            p = o.p;
-            n = o.n;
-            error = std::move(o.error);
-            o.p = nullptr;
-        }
-        return *this;
+    void inflate(const std::string& path) {
+        char* q = nullptr;
+        inflate_file(path, &q, &n);
+        p.reset(q);
     }
-    ~Inflated() { free(p); }
 };
 
 // The whole text of a reads file for the framer: a gzip file is inflated into host memory on all host threads
@@ -1445,11 +1284,11 @@ struct ReadsText {
     Inflated local;
     ReadsText(const char* path, const Inflated* pre) {
         if (!pre && file_is_gzip(path)) {
-            inflate_file(path, &local.p, &local.n);
+            local.inflate(path);
             pre = &local;
         }
         if (pre) {
-            src.mem = pre->p;
+            src.mem = pre->p.get();
             src.size = pre->n;
             return;
         }
@@ -1469,26 +1308,21 @@ struct ReadsText {
     }
 };
 
-// the packed reads an ingest left on the device, as a batch of this index
-drprg_batch* batch_from_ingest(drprg_index* X, const IngestResult& I, uint32_t read_id_base) {
-    std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(new drprg_batch(), free_batch);
-    B->owned = true;
-    B->device = X->device;
-    B->d_words = I.d_words;
-    B->d_lens = I.d_lens;
-    B->d_off = I.d_word_off;
-    B->b_words = I.b_words;
-    B->b_lens = I.b_lens;
-    B->b_off = I.b_off;
-    B->R = DevReads{I.d_words, I.d_word_off, I.stride_words, I.d_lens, I.n_reads, read_id_base};
+// the packed reads an ingest left on the device, as a batch of this index: takes over the buffers of I
+std::unique_ptr<drprg_batch> batch_from_ingest(drprg_index* X, IngestResult& I, uint32_t read_id_base) {
+    std::unique_ptr<drprg_batch> B(new drprg_batch());
+    B->d_words = std::move(I.words);
+    B->d_lens = std::move(I.lens);
+    B->d_off = std::move(I.word_off);
+    B->R = DevReads{B->d_words.get(), B->d_off.get(), I.stride_words, B->d_lens.get(), I.n_reads, read_id_base};
     B->total_bases = I.total_bases;
     B->max_len = I.stride_words ? I.stride_words * 16u : I.max_len;
     if (I.max_len > SHORT_READ_MAX) {  // the segment table is built from the lengths on the host
         std::vector<uint32_t> lens(I.n_reads);
-        CK(cudaMemcpy(lens.data(), I.d_lens, I.n_reads * 4, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(lens.data(), B->d_lens.get(), I.n_reads * 4, cudaMemcpyDeviceToHost));
         build_segments(X, B.get(), lens.data(), I.n_reads, I.total_bases, 0);
     }
-    return B.release();
+    return B;
 }
 
 // the host parser's batch; a multi-GPU handle gets one shard of the reads per GPU
@@ -1517,8 +1351,7 @@ FileBatch batch_from_file(drprg_index* X, const char* reads_path, uint32_t threa
         CK(cudaSetDevice(X->device));
         const ReadsText T(reads_path, nullptr);
         IngestResult I;
-        const int dev = X->device;
-        if (T.may_be_fastq() && ingest_fastq_text(T.src, dev, threads, I, 0, [dev](size_t bytes) { return g_pool.get(bytes, dev); })) {
+        if (T.may_be_fastq() && ingest_fastq_text(T.src, X->device, threads, I, 0)) {
             FileBatch F;
             F.B = batch_from_ingest(X, I, 0);
             F.n_dropped = I.n_dropped;
@@ -1555,7 +1388,6 @@ bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_o
     if (!T.may_be_fastq()) return false;
     const TextSource& F = T.src;
     const uint32_t threads = o ? std::max(1u, o->threads) : 1u;
-    const int dev = X->device;
     std::vector<char> scratch;
     size_t lo = 0;
     while (lo < F.size) {
@@ -1569,9 +1401,9 @@ bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_o
         S.origin = lo;
         IngestResult I;
         const double tw0 = now_ms();
-        if (!ingest_fastq_text(S, dev, threads, I, 0, [dev](size_t bytes) { return g_pool.get(bytes, dev); })) return false;
+        if (!ingest_fastq_text(S, X->device, threads, I, 0)) return false;
         if (W.n + I.n_reads > 0xfffffff0ull) throw std::runtime_error("more than 2^32 reads in one sample");
-        std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(batch_from_ingest(X, I, (uint32_t)W.n), free_batch);
+        const std::unique_ptr<drprg_batch> B = batch_from_ingest(X, I, (uint32_t)W.n);
         if (W.waves == 0) {
             W.first_len = I.first_read_len;
             sample_begin_any(X, o, I.first_read_len);
@@ -1619,14 +1451,14 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
     } else {
         // Not strict 4-line FASTQ, or host ingest forced.  Framing the whole file would decline as well: it runs the same
         // framer over the same records as the waves, and it takes at most 8 GB of text where the waves take any size.
-        FileBatch F = host_parsed_batch(X, reads_path, o ? o->threads : 1);
-        std::unique_ptr<drprg_batch, void (*)(drprg_batch*)> B(F.B, free_batch);
+        const FileBatch F = host_parsed_batch(X, reads_path, o ? o->threads : 1);
+        drprg_batch* B = F.B.get();
         pr.n_dropped = F.n_dropped;
         pr.total_bases = B->total_bases;
         t1 = now_ms();
         sample_begin_any(X, o, F.first_read_len);
         n = B->R.n_reads;
-        map_batch_any(X, B.get(), 0, &nh, &nk);
+        map_batch_any(X, B, 0, &nh, &nk);
     }
     const double t2 = now_ms();
     genotype(X, vcf_refs, "sample");
@@ -1698,7 +1530,7 @@ int drprg_cuda_shard_root(drprg_index* X, int world_size, void* handle64) {
     if (is_multi(X)) throw std::runtime_error("a multi-GPU handle shards inside the library already");
     CK(cudaSetDevice(X->device));
     cudaIpcMemHandle_t h;
-    CK(cudaIpcGetMemHandle(&h, X->d_accum));
+    CK(cudaIpcGetMemHandle(&h, X->d_accum.p));
     static_assert(sizeof(h) == 64, "CUDA IPC handles are 64 bytes");
     memcpy(handle64, &h, sizeof h);
     X->world = std::max(1, world_size);
@@ -1761,7 +1593,7 @@ int drprg_cuda_map_genotype_batch(drprg_index* X, size_t n, const char* const* r
         ahead[i] = std::async(std::launch::async, [path]() {
             Inflated r;
             try {
-                inflate_file(path, &r.p, &r.n);
+                r.inflate(path);
             } catch (const std::exception& e) {
                 r.error = e.what();
             }
@@ -1841,8 +1673,8 @@ int drprg_cuda_batch_upload(drprg_index* X, const uint32_t* words, const uint64_
                             const uint32_t* lens, uint64_t n_reads, uint64_t total_bases, uint32_t read_id_base, void* stream,
                             drprg_batch** out) {
     API_BEGIN if (!stride_words && !word_off) throw std::runtime_error("word_off is required without a fixed stride");
-    if (is_multi(X)) *out = multi_upload(X, words, word_off, stride_words, lens, n_reads, total_bases, read_id_base);
-    else *out = upload_batch(X, words, word_off, stride_words, lens, n_reads, total_bases, read_id_base, (cudaStream_t)stream);
+    if (is_multi(X)) *out = multi_upload(X, words, word_off, stride_words, lens, n_reads, total_bases, read_id_base).release();
+    else *out = upload_batch(X, words, word_off, stride_words, lens, n_reads, total_bases, read_id_base, (cudaStream_t)stream).release();
     return 0;
     API_END
 }
@@ -1862,16 +1694,16 @@ int drprg_cuda_batch_wrap_device(drprg_index* X, const void* d_words, const void
 int drprg_cuda_batch_from_fastx(drprg_index* X, const char* path, uint32_t threads, drprg_batch** out, uint64_t* n_reads,
                                 uint64_t* total_bases, uint64_t* n_dropped, uint32_t* first_read_len, int* parsed_on_device) {
     API_BEGIN FileBatch F = batch_from_file(X, path, threads);
-    *out = F.B;
     if (n_reads) *n_reads = F.B->R.n_reads;
     if (total_bases) *total_bases = F.B->total_bases;
     if (n_dropped) *n_dropped = F.n_dropped;
     if (first_read_len) *first_read_len = F.first_read_len;
     if (parsed_on_device) *parsed_on_device = F.on_device ? 1 : 0;
+    *out = F.B.release();
     return 0;
     API_END
 }
-void drprg_cuda_batch_free(drprg_batch* b) { free_batch(b); }
+void drprg_cuda_batch_free(drprg_batch* b) { delete b; }
 
 int drprg_cuda_sample_begin(drprg_index* X, const drprg_map_opts* o, uint32_t first_read_len) {
     API_BEGIN sample_begin_any(X, o, first_read_len);
@@ -1888,7 +1720,7 @@ int drprg_cuda_accum_device_ptr(drprg_index* X, void** d_ptr, uint64_t* n_int32)
     CK(cudaSetDevice(X->device));
     flush_scalars(X);
     X->hist_on_host = false;  // the caller may change the accumulators (allreduce)
-    *d_ptr = X->d_accum;
+    *d_ptr = X->d_accum.p;
     *n_int32 = X->n_accum;
     return 0;
     API_END
@@ -1898,7 +1730,7 @@ int drprg_cuda_accum_download(drprg_index* X, int32_t* out, uint64_t n) {
     if (n != X->n_accum) throw std::runtime_error("accumulator size mismatch");
     CK(cudaSetDevice(X->device));
     flush_scalars(X);
-    CK(cudaMemcpy(out, X->d_accum, n * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(out, X->d_accum.p, n * 4, cudaMemcpyDeviceToHost));
     return 0;
     API_END
 }
@@ -1906,7 +1738,7 @@ int drprg_cuda_accum_upload(drprg_index* X, const int32_t* in, uint64_t n) {
     API_BEGIN need_device(X);
     if (n != X->n_accum) throw std::runtime_error("accumulator size mismatch");
     CK(cudaSetDevice(X->device));
-    CK(cudaMemcpy(X->d_accum, in, n * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(X->d_accum.p, in, n * 4, cudaMemcpyHostToDevice));
     X->hist_on_host = false;
     X->scalars_in_buffer = true;
     return 0;
@@ -2008,25 +1840,21 @@ int64_t drprg_cuda_sketch_batch(drprg_index* X, drprg_batch* B, void* stream, ui
         DBuf<unsigned long long> key, val;
         key.ensure(cap);
         val.ensure(cap);
-        CK(cudaMemsetAsync(X->d_counters, 0, 16, st));
+        CK(cudaMemsetAsync(X->d_counters.p, 0, 16, st));
         for (auto& e : B->ev)
-            if (e) CK(cudaStreamWaitEvent(st, e, 0));
-        launch_sketch_only(B->R, X->H.w, X->H.k, key.p, val.p, X->d_counters, cap, X->sm_count, B->max_len, st);
+            if (e) CK(cudaStreamWaitEvent(st, e.get(), 0));
+        launch_sketch_only(B->R, X->H.w, X->H.k, key.p, val.p, X->d_counters.p, cap, X->sm_count, B->max_len, st);
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(X->h_counters, X->d_counters, 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X->h_counters.p, X->d_counters.p, 8, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        uint64_t n = X->h_counters[0];
+        uint64_t n = X->h_counters.p[0];
         if (n > cap) {
-            key.release();
-            val.release();
             g_err = "sketch output capacity too small";
             return -(int64_t)n;
         }
         std::vector<unsigned long long> hk(n), hv(n);
         CK(cudaMemcpy(hk.data(), key.p, n * 8, cudaMemcpyDeviceToHost));
         CK(cudaMemcpy(hv.data(), val.p, n * 8, cudaMemcpyDeviceToHost));
-        key.release();
-        val.release();
         std::vector<uint64_t> ord(n);
         for (uint64_t i = 0; i < n; ++i) ord[i] = i;
         std::sort(ord.begin(), ord.end(), [&](uint64_t a, uint64_t b) { return hk[a] < hk[b]; });
@@ -2169,10 +1997,6 @@ int drprg_cuda_genotype_rows(int device, uint32_t n_records, const uint32_t* rec
     d_f32.ensure((size_t)n_records * 2 + na);
     uint32_t *d_off = d_u32.p, *d_mf = d_off + n_records + 1, *d_mr = d_mf + na;
     double *d_gaps = d_f64.p, *d_lik = d_gaps + na, *d_conf = d_lik + na;
-    struct Guard {
-        DBuf<uint32_t>& a; DBuf<double>& b; DBuf<int32_t>& c; DBuf<float>& d;
-        ~Guard() { a.release(); b.release(); c.release(); d.release(); }
-    } guard{d_u32, d_f64, d_i32, d_f32};
     CK(cudaMemcpy(d_off, rec_off, ((size_t)n_records + 1) * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_mf, mean_fwd, (size_t)na * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_mr, mean_rev, (size_t)na * 4, cudaMemcpyHostToDevice));
@@ -2321,7 +2145,6 @@ int drprg_cuda_format_g6_device(int device, const double* v, uint32_t n, char* o
     CK(cudaMemcpy(out, dout.p, 48ull * n, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(len, dl.p, n, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(refused, dr.p, n, cudaMemcpyDeviceToHost));
-    dv.release(); dout.release(); dl.release(); dr.release();
     return 0;
     API_END
 }

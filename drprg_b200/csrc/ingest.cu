@@ -10,10 +10,8 @@
 
 #include <algorithm>
 #include <atomic>
-#include <chrono>
 #include <cstdio>
 #include <cstring>
-#include <functional>
 #include <mutex>
 #include <stdexcept>
 #include <string>
@@ -27,71 +25,18 @@
 namespace drprg {
 namespace {
 
-#define ICK(call)                                                                                         \
-    do {                                                                                                  \
-        cudaError_t e__ = (call);                                                                         \
-        if (e__ != cudaSuccess)                                                                           \
-            throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e__) + " at " #call); \
-    } while (0)
-
-double now_ms_i() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-
 struct Staging {  // process-wide grow-only pinned and device buffers (one ingest at a time)
     std::mutex m;
     int device = -1;
-    char* d_text = nullptr;  // the sequence lines
-    size_t text_cap = 0;
-    uint32_t* d_rec = nullptr;  // per record: sequence start | raw length | bad flag (3 x rec_cap)
-    size_t rec_cap = 0;
-    unsigned long long* d_scalars = nullptr;  // [4] dropped reads (finish_lens_kernel)
-    unsigned long long* h_scalars = nullptr;
-    char* pinned_seq = nullptr;  // the sequence lines, framed on the host
-    size_t seq_cap = 0;
-    uint32_t* h_rec = nullptr;   // sequence start | length per read (2 x hrec_cap)
-    size_t hrec_cap = 0;
-    void ensure_seq(size_t bytes) {
-        if (bytes <= seq_cap) return;
-        if (pinned_seq) cudaFreeHost(pinned_seq);
-        pinned_seq = nullptr;
-        seq_cap = 0;
-        const size_t want = bytes + bytes / 8 + (1u << 20);
-        ICK(cudaMallocHost(&pinned_seq, want));
-        seq_cap = want;
-    }
-    void ensure_hrec(size_t reads) {
-        if (reads <= hrec_cap) return;
-        if (h_rec) cudaFreeHost(h_rec);
-        h_rec = nullptr;
-        hrec_cap = 0;
-        const size_t want = reads + reads / 8 + 1024;
-        ICK(cudaMallocHost(&h_rec, want * 2 * sizeof(uint32_t)));
-        hrec_cap = want;
-    }
-    void ensure_device(int dev, size_t text_bytes) {
-        if (dev != device) {  // buffers belong to one device; switching devices starts over
-            release_device();
-            device = dev;
-        }
-        if (!d_scalars) ICK(cudaMalloc(&d_scalars, 8 * sizeof(unsigned long long)));
-        if (!h_scalars) ICK(cudaMallocHost(&h_scalars, 8 * sizeof(unsigned long long)));
-        if (text_bytes > text_cap) {  // every ingest writes the buffer afresh: nothing to carry over
-            if (d_text) cudaFree(d_text);
-            d_text = nullptr;
-            text_cap = 0;
-            const size_t want = text_bytes + text_bytes / 8 + (1u << 20);
-            ICK(cudaMalloc(&d_text, want));
-            text_cap = want;
-        }
-    }
-    void release_device() {
-        for (void* p : {(void*)d_text, (void*)d_scalars, (void*)d_rec})
-            if (p) cudaFree(p);
-        d_text = nullptr;
-        d_scalars = nullptr;
-        d_rec = nullptr;
-        text_cap = rec_cap = 0;
-    }
-} g_stage;
+    DBuf<char> d_text;      // the sequence lines
+    DBuf<uint32_t> d_rec;   // per record: sequence start | raw length | bad flag (3 columns of d_rec.cap / 3)
+    DBuf<unsigned long long> d_scalars;  // [4] dropped reads (finish_lens_kernel)
+    PinnedBuf<unsigned long long> h_scalars;
+    PinnedBuf<char> pinned_seq;  // the sequence lines, framed on the host
+    PinnedBuf<uint32_t> h_rec;   // sequence start | length per read (2 columns of h_rec.cap / 2)
+};
+// never destroyed: static teardown may run after the CUDA runtime has been unloaded
+Staging& g_stage = *new Staging;
 
 __device__ __forceinline__ uint32_t code4_dev(uint32_t c) {
     c &= 0xdfu;  // fold case (only letters matter)
@@ -155,70 +100,44 @@ __global__ void finish_lens_kernel(const uint32_t* __restrict__ raw_len, const u
 // records (sequence start, raw length in g_stage.d_rec) -> 2-bit words, lengths (0 = dropped), dropped-read count
 // h_lens: the same raw lengths on the host, from which the ragged layout's word offsets are summed
 void pack_records(const char* text, uint64_t n, uint32_t max_len, uint64_t total_bases, uint32_t first_len, IngestResult& out,
-                  cudaStream_t st, const std::function<void*(size_t)>& alloc, const uint32_t* h_lens) {
-    uint32_t *d_start = g_stage.d_rec, *d_rawlen = g_stage.d_rec + g_stage.rec_cap, *d_bad = g_stage.d_rec + 2 * g_stage.rec_cap;
-    auto dev_alloc = [&](size_t bytes) -> void* {
-        if (alloc) return alloc(bytes);
-        void* p = nullptr;
-        ICK(cudaMalloc(&p, bytes));
-        return p;
-    };
-    try {
-        const unsigned rb = (unsigned)((n + 255) / 256);
-        ICK(cudaMemsetAsync(d_bad, 0, n * 4, st));
-        ICK(cudaMemsetAsync(g_stage.d_scalars + 4, 0, sizeof(unsigned long long), st));
-        out.max_len = max_len;
-        out.total_bases = total_bases;
-        out.first_read_len = first_len;
-        out.n_reads = n;
-        out.b_lens = std::max<uint64_t>(1, n) * 4;
-        out.d_lens = (uint32_t*)dev_alloc(out.b_lens);
-        if (out.max_len <= SHORT_READ_MAX) {
-            uint32_t stride = std::max(1u, (out.max_len + 15) / 16);
-            stride += stride & 1u;  // even: every read starts 8-byte aligned (wide loads in the screen kernel)
-            out.stride_words = stride;
-            out.b_words = (n * (uint64_t)stride + 2) * 4;
-            out.d_words = (uint32_t*)dev_alloc(out.b_words);
-            const uint64_t items = n * (uint64_t)stride;
-            pack_stride_kernel<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(text, d_start, d_rawlen, n, stride, out.d_words, d_bad);
-        } else {
-            out.b_off = (n + 1) * 8;
-            out.d_word_off = (uint64_t*)dev_alloc(out.b_off);
-            unsigned long long total_words = 0;
-            std::vector<uint64_t> off(n + 1);
-            for (uint64_t r = 0; r < n; ++r) {
-                off[r] = total_words;
-                total_words += (h_lens[r] + 15u) >> 4;
-            }
-            off[n] = total_words;
-            ICK(cudaMemcpyAsync(out.d_word_off, off.data(), (n + 1) * 8, cudaMemcpyHostToDevice, st));
-            ICK(cudaStreamSynchronize(st));  // `off` dies with this scope
-            out.b_words = (total_words + 2) * 4;
-            out.d_words = (uint32_t*)dev_alloc(out.b_words);
-            pack_ragged_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(text, d_start, d_rawlen, n,
-                                                                                (const unsigned long long*)out.d_word_off, out.d_words, d_bad);
+                  cudaStream_t st, int device, const uint32_t* h_lens) {
+    const size_t rec_cap = g_stage.d_rec.cap / 3;
+    uint32_t *d_start = g_stage.d_rec.p, *d_rawlen = d_start + rec_cap, *d_bad = d_start + 2 * rec_cap;
+    const unsigned rb = (unsigned)((n + 255) / 256);
+    CK(cudaMemsetAsync(d_bad, 0, n * 4, st));
+    CK(cudaMemsetAsync(g_stage.d_scalars.p + 4, 0, sizeof(unsigned long long), st));
+    out.max_len = max_len;
+    out.total_bases = total_bases;
+    out.first_read_len = first_len;
+    out.n_reads = n;
+    out.lens = pool_get<uint32_t>(std::max<uint64_t>(1, n) * 4, device);
+    if (out.max_len <= SHORT_READ_MAX) {
+        uint32_t stride = std::max(1u, (out.max_len + 15) / 16);
+        stride += stride & 1u;  // even: every read starts 8-byte aligned (wide loads in the screen kernel)
+        out.stride_words = stride;
+        out.words = pool_get<uint32_t>((n * (uint64_t)stride + 2) * 4, device);
+        const uint64_t items = n * (uint64_t)stride;
+        pack_stride_kernel<<<(unsigned)((items + 255) / 256), 256, 0, st>>>(text, d_start, d_rawlen, n, stride, out.words.get(), d_bad);
+    } else {
+        out.word_off = pool_get<uint64_t>((n + 1) * 8, device);
+        unsigned long long total_words = 0;
+        std::vector<uint64_t> off(n + 1);
+        for (uint64_t r = 0; r < n; ++r) {
+            off[r] = total_words;
+            total_words += (h_lens[r] + 15u) >> 4;
         }
-        finish_lens_kernel<<<rb, 256, 0, st>>>(d_rawlen, d_bad, n, out.d_lens, g_stage.d_scalars);
-        ICK(cudaGetLastError());
-        ICK(cudaMemcpyAsync(g_stage.h_scalars, g_stage.d_scalars, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        ICK(cudaStreamSynchronize(st));
-        out.n_dropped = g_stage.h_scalars[4];
-    } catch (...) {
-        for (void* p : {(void*)out.d_words, (void*)out.d_word_off, (void*)out.d_lens})
-            if (p) cudaFree(p);
-        out = IngestResult();
-        throw;
+        off[n] = total_words;
+        CK(cudaMemcpyAsync(out.word_off.get(), off.data(), (n + 1) * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaStreamSynchronize(st));  // `off` dies with this scope
+        out.words = pool_get<uint32_t>((total_words + 2) * 4, device);
+        pack_ragged_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(text, d_start, d_rawlen, n,
+                                                                            (const unsigned long long*)out.word_off.get(), out.words.get(), d_bad);
     }
-}
-
-void ensure_records(uint64_t n) {  // grow-only scratch: cudaMalloc / cudaFree per sample cost more than the kernels
-    if (n <= g_stage.rec_cap) return;
-    if (g_stage.d_rec) cudaFree(g_stage.d_rec);
-    g_stage.d_rec = nullptr;
-    g_stage.rec_cap = 0;
-    const size_t want = n + n / 8 + 1024;
-    ICK(cudaMalloc(&g_stage.d_rec, want * 3 * sizeof(uint32_t)));
-    g_stage.rec_cap = want;
+    finish_lens_kernel<<<rb, 256, 0, st>>>(d_rawlen, d_bad, n, out.lens.get(), g_stage.d_scalars.p);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(g_stage.h_scalars.p, g_stage.d_scalars.p, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    out.n_dropped = g_stage.h_scalars.p[4];
 }
 
 }  // namespace
@@ -229,18 +148,27 @@ void ensure_records(uint64_t n) {  // grow-only scratch: cudaMalloc / cudaFree p
 // a record's sequence is less than half of its bytes — and the thread that framed a slice also queues its H2D copy, so
 // the copies overlap the framing of the other slices.  Then (start, length) of every read is uploaded and the pack
 // kernels run.  false = not strict 4-line FASTQ (nothing is left behind; the caller goes on with the host parser).
-bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st,
-                       const std::function<void*(size_t)>& alloc) {
+bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, IngestResult& out, cudaStream_t st) {
     out = IngestResult();
     std::lock_guard<std::mutex> lock(g_stage.m);
     static const bool timing = getenv("DRPRG_TIMING") != nullptr;
-    const double t0 = now_ms_i();
+    const double t0 = now_ms();
     if (src.size < 8 || src.size / 2 + 64 >= 0xfff00000ull) return false;  // 32-bit sequence offsets
-    ICK(cudaSetDevice(device));
-    g_stage.ensure_seq(src.size / 2 + 64);
-    g_stage.ensure_device(device, src.size / 2 + 64);
-    char* const pinned = g_stage.pinned_seq;
-    char* const d_text = g_stage.d_text;
+    CK(cudaSetDevice(device));
+    const size_t seq_bytes = src.size / 2 + 64;
+    g_stage.pinned_seq.reserve(seq_bytes, seq_bytes + seq_bytes / 8 + (1u << 20));
+    if (device != g_stage.device) {  // device buffers belong to one device; switching devices starts over
+        g_stage.d_text.release();
+        g_stage.d_scalars.release();
+        g_stage.d_rec.release();
+        g_stage.device = device;
+    }
+    g_stage.d_scalars.reserve(8, 8);
+    g_stage.h_scalars.reserve(8, 8);
+    // every ingest writes the text buffer afresh: nothing to carry over
+    g_stage.d_text.reserve(seq_bytes, seq_bytes + seq_bytes / 8 + (1u << 20));
+    char* const pinned = g_stage.pinned_seq.p;
+    char* const d_text = g_stage.d_text.p;
     std::vector<FramedSlice> sl;
     std::atomic<bool> cuda_failed{false};
     bool is_fastq = false;
@@ -264,7 +192,7 @@ bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, Inge
         return false;
     }
     const size_t S = sl.size();
-    const double t1 = now_ms_i();
+    const double t1 = now_ms();
     // ---- totals, then (start, length) of every read to the device
     FrameStats T;
     std::vector<size_t> first(S + 1, 0);
@@ -285,23 +213,24 @@ bool ingest_fastq_text(const TextSource& src, int device, uint32_t threads, Inge
         return false;
     }
     if (n > 0xfffffff0ull) throw std::runtime_error("more than 2^32 reads in one sample");
-    g_stage.ensure_hrec(n);
-    ensure_records(n);
-    uint32_t* h_start = g_stage.h_rec;
-    uint32_t* h_len = g_stage.h_rec + g_stage.hrec_cap;
+    // grow-only record tables: cudaMalloc / cudaFree per sample cost more than the kernels
+    g_stage.h_rec.reserve(2 * n, 2 * (n + n / 8 + 1024));
+    g_stage.d_rec.reserve(3 * n, 3 * (n + n / 8 + 1024));
+    uint32_t* h_start = g_stage.h_rec.p;
+    uint32_t* h_len = h_start + g_stage.h_rec.cap / 2;
     parallel_for(S, [&](size_t s) {
         const size_t k = sl[s].lens.size();
         if (!k) return;
         memcpy(h_start + first[s], sl[s].starts.data(), k * 4);
         memcpy(h_len + first[s], sl[s].lens.data(), k * 4);
     }, std::max<size_t>(1, std::min<size_t>(threads, 8)));
-    ICK(cudaMemcpyAsync(g_stage.d_rec, h_start, n * 4, cudaMemcpyHostToDevice, st));
-    ICK(cudaMemcpyAsync(g_stage.d_rec + g_stage.rec_cap, h_len, n * 4, cudaMemcpyHostToDevice, st));
-    const double t2 = now_ms_i();
-    pack_records(d_text, n, T.max_len, T.total_bases, T.first_len, out, st, alloc, h_len);
+    CK(cudaMemcpyAsync(g_stage.d_rec.p, h_start, n * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(g_stage.d_rec.p + g_stage.d_rec.cap / 3, h_len, n * 4, cudaMemcpyHostToDevice, st));
+    const double t2 = now_ms();
+    pack_records(d_text, n, T.max_len, T.total_bases, T.first_len, out, st, device, h_len);
     if (timing)
         fprintf(stderr, "[drprg-cuda] ingest (host-framed): %.1f MB text in %zu slices, frame + queue H2D %.2f ms, record table %.2f ms, "
-                        "upload tail + pack %.2f ms\n", src.size / 1e6, S, t1 - t0, t2 - t1, now_ms_i() - t2);
+                        "upload tail + pack %.2f ms\n", src.size / 1e6, S, t1 - t0, t2 - t1, now_ms() - t2);
     return true;
 }
 
