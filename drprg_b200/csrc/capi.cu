@@ -590,8 +590,9 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     }
     static const bool timing = getenv("DRPRG_TIMING") != nullptr;
     if (timing)
-        fprintf(stderr, "[drprg-cuda] map batch: %llu reads, %d chunks, screen queue %llu (largest chunk), probe survivors %llu, hits %llu\n",
-                (unsigned long long)B->R.n_reads, B->n_chunks, X->h_counters.p[CTR_QUEUE_NEED], X->h_counters.p[CTR_SURVIVORS], (unsigned long long)nh);
+        fprintf(stderr, "[drprg-cuda] map batch: %llu reads, %d chunks, screen queue %llu (largest chunk), probe survivors %llu, hits %llu, active reads %llu\n",
+                (unsigned long long)B->R.n_reads, B->n_chunks, X->h_counters.p[CTR_QUEUE_NEED], X->h_counters.p[CTR_SURVIVORS], (unsigned long long)nh,
+                X->h_counters.p[CTR_ACTIVE]);
     X->hist_on_host = !X->reduce_dst && !X->accum_shared;
     CK(cudaEventElapsedTime(&X->timings[0], X->ev[0].get(), X->ev[1].get()));
     CK(cudaEventElapsedTime(&X->timings[1], X->ev[1].get(), X->ev[2].get()));

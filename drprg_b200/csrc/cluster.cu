@@ -21,10 +21,9 @@
 //                         bitonic sort and a block scan for the cluster boundaries
 //   both write, next to every grouped hit, its coverage key 2 * k-mer node + strand (or "none" when the hit is dropped),
 //   and per read the keys 2N + locus of its kept clusters: no allocation, no atomics
-//   cov_count_kernel      S5 without atomics: a job = (range of 6 k counters, stretch of 32 k key slots); its CTA keeps a
-//                         PRIVATE copy of the range's counters per warp in shared memory, every warp compacts the keys
-//                         of its share of the stretch that fall into the range and counts them, equal keys of one step
-//                         combined by match.any: every increment is a plain read-modify-write with a single writer
+//   cov_count_kernel      S5: a job = (range of 56 k counters, stretch of key slots); its CTA counts the keys of the
+//                         stretch that fall into the range in ONE copy of the range's 32-bit counters in shared memory,
+//                         with shared-memory atomic adds, and stores the copy as the job's partial
 //   cov_merge_kernel      column sum of the partials into the sample's accumulator — or, on a read-sharded run, straight
 //                         into the ROOT GPU's accumulator over NVLink with red.global.add (integers: bit-exact for any
 //                         number of GPUs), which is the whole "allreduce" of the path; also counts the kept hits
@@ -128,18 +127,40 @@ __global__ void __launch_bounds__(AS_THREADS) assign_kernel(unsigned long long* 
     }
 }
 
+// The lookup kernels emit a read's hits next to each other, so the lanes of a warp mostly share a read: its lanes are
+// grouped by read and one atomic per group takes the group's slots (their order within the slice does not matter, the
+// cluster kernels sort it)
+constexpr int SC_UNROLL = 4;  // warp chunks of 32 hits in flight per warp: their loads, then their atomics, are issued together
 __global__ void scatter_kernel(const unsigned long long* __restrict__ hi, const unsigned long long* __restrict__ lo,
                                const unsigned long long* __restrict__ ctr, PostCaps C, uint32_t read_id_base,
                                int32_t* __restrict__ read_count, const uint32_t* __restrict__ read_base,
                                unsigned long long* __restrict__ gkey) {
     if (batch_overflowed(ctr, C)) return;
     const unsigned long long n = ctr[CTR_HITS];
-    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (unsigned long long)gridDim.x * blockDim.x) {
-        const unsigned long long h = hi[i];
-        const uint32_t r = (uint32_t)(h >> 32) - read_id_base;
-        const uint32_t slot = read_base[r] + (uint32_t)(atomicSub(read_count + r, 1) - 1);  // the counter ends at 0 again
-        gkey[slot] = group_key(h, lo[i]);
+    const int lane = threadIdx.x & 31;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x * SC_UNROLL;
+    for (unsigned long long i0 = ((unsigned long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31u)) * SC_UNROLL; i0 < n; i0 += stride) {  // warp-uniform
+        unsigned long long h[SC_UNROLL];
+        uint32_t r[SC_UNROLL], peers[SC_UNROLL];
+        int32_t old[SC_UNROLL];
+#pragma unroll
+        for (int u = 0; u < SC_UNROLL; ++u) {
+            const unsigned long long i = i0 + 32 * u + lane;
+            h[u] = i < n ? hi[i] : 0ull;
+            r[u] = i < n ? (uint32_t)(h[u] >> 32) - read_id_base : 0xffffffffu;  // a read index is below 2^32 - 1
+        }
+#pragma unroll
+        for (int u = 0; u < SC_UNROLL; ++u) {
+            peers[u] = __match_any_sync(FULL, r[u]);
+            old[u] = 0;
+            if (r[u] != 0xffffffffu && lane == __ffs(peers[u]) - 1) old[u] = atomicSub(read_count + r[u], __popc(peers[u]));  // ends at 0 again
+        }
+#pragma unroll
+        for (int u = 0; u < SC_UNROLL; ++u) {
+            old[u] = __shfl_sync(FULL, old[u], __ffs(peers[u]) - 1);
+            const unsigned long long i = i0 + 32 * u + lane;
+            if (i < n) gkey[read_base[r[u]] + (uint32_t)(old[u] - 1) - (uint32_t)__popc(peers[u] & ((1u << lane) - 1u))] = group_key(h[u], lo[i]);
+        }
     }
 }
 
@@ -276,6 +297,130 @@ __device__ __forceinline__ void warp_sort64(unsigned long long& x0, unsigned lon
     }
 }
 
+// the keys of read slice [base, base + c) a warp sorts (element i in lane i & 31, register i >> 5; padding sorts to the
+// end), loaded only for a read this kernel clusters
+struct WarpRead {
+    uint32_t c, base;
+    unsigned long long x0, x1;
+};
+__device__ __forceinline__ void load_warp_read_keys(WarpRead& R, const unsigned long long* __restrict__ gkey, uint32_t min_thresh, int lane) {
+    const bool mine = R.c > min_thresh && R.c <= CLUSTER_WARP_MAX;
+    R.x0 = mine && (uint32_t)lane < R.c ? gkey[R.base + lane] : ~0ull;
+    R.x1 = mine && (uint32_t)lane + 32u < R.c ? gkey[R.base + 32 + lane] : ~0ull;
+}
+
+__device__ __forceinline__ void cluster_warp_read(
+    unsigned long long a, WarpRead R, unsigned long long* __restrict__ ctr, unsigned long long* __restrict__ gkey, uint8_t* __restrict__ gkept,
+    uint32_t max_diff, uint32_t min_thresh, const uint32_t* __restrict__ thresh, const uint32_t* __restrict__ knode_base, uint32_t locus_key_base,
+    uint32_t* __restrict__ cov_keys, uint32_t* __restrict__ act_lk, uint32_t* __restrict__ lk_ovf, uint32_t (*s_u32)[64], uint32_t* s_alive, int lane) {
+    const uint32_t c = R.c, base = R.base;
+    if (c > CLUSTER_WARP_MAX) return;  // the CTA kernel's read
+    if (c <= min_thresh) {  // no cluster of this read can exceed any locus's size threshold (stray hits): nothing is kept
+        if ((uint32_t)lane < c) {
+            gkept[base + lane] = 0;
+            cov_keys[base + lane] = COV_KEY_NONE;
+        }
+        if ((uint32_t)lane + 32u < c) {
+            gkept[base + 32 + lane] = 0;
+            cov_keys[base + 32 + lane] = COV_KEY_NONE;
+        }
+        if (lane < 2) act_lk[2 * a + lane] = COV_KEY_NONE;
+        return;
+    }
+    unsigned long long x0 = R.x0, x1 = R.x1;
+    if (c > 32u) warp_sort64<2>(x0, x1, lane);  // warp-uniform
+    else warp_sort64<1>(x0, x1, lane);
+    if ((uint32_t)lane < c) gkey[base + lane] = x0;  // the slice stays sorted for the hooks / later consumers
+    if ((uint32_t)lane + 32u < c) gkey[base + 32 + lane] = x1;
+    // ---- define_clusters: a hit opens a cluster when prg or strand change or the gap exceeds max_diff
+    const unsigned long long p0 = shfl_up64(x0, 1), x0_31 = shfl64(x0, 31);
+    unsigned long long p1 = shfl_up64(x1, 1);
+    if (lane == 0) p1 = x0_31;
+    auto opens = [&](unsigned long long cur, unsigned long long prev, uint32_t i) {
+        if (i == 0u || i == c) return true;  // i == c: the first padding element closes the last cluster
+        if (i > c) return false;
+        return gk_pf(cur) != gk_pf(prev) || gk_start(cur) - gk_start(prev) > max_diff;
+    };
+    const uint32_t m0 = __ballot_sync(FULL, opens(x0, p0, (uint32_t)lane));
+    const uint32_t m1 = __ballot_sync(FULL, opens(x1, p1, (uint32_t)lane + 32u));
+    const unsigned long long S = (unsigned long long)m0 | ((unsigned long long)m1 << 32);
+    uint32_t cb[2], ce[2];
+    bool pass[2], begin_pass[2];
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+        const uint32_t i = (uint32_t)lane + 32u * r;
+        const unsigned long long le = i == 63u ? ~0ull : ((2ull << i) - 1ull);
+        cb[r] = 63u - (uint32_t)__clzll((long long)(S & le));
+        const unsigned long long gt = S & ~le;
+        ce[r] = gt ? (uint32_t)__ffsll((long long)gt) - 1u : c;
+        const unsigned long long xr = r ? x1 : x0;
+        pass[r] = i < c && (ce[r] - cb[r]) > thresh[gk_prg(xr)];
+        begin_pass[r] = pass[r] && cb[r] == i;
+    }
+    const uint32_t b0 = __ballot_sync(FULL, begin_pass[0]), b1 = __ballot_sync(FULL, begin_pass[1]);
+    const unsigned long long BP = (unsigned long long)b0 | ((unsigned long long)b1 << 32);
+    const uint32_t ncl = (uint32_t)__popcll(BP);
+    if (ncl == 0u) {
+        if ((uint32_t)lane < c) {
+            gkept[base + lane] = 0;
+            cov_keys[base + lane] = COV_KEY_NONE;
+        }
+        if ((uint32_t)lane + 32u < c) {
+            gkept[base + 32 + lane] = 0;
+            cov_keys[base + 32 + lane] = COV_KEY_NONE;
+        }
+        if (lane < 2) act_lk[2 * a + lane] = COV_KEY_NONE;
+        return;
+    }
+    bool alive[2] = {pass[0], pass[1]};
+    if (ncl > 1u) {
+        uint32_t* first = s_u32[0];
+        uint32_t* last = s_u32[1];
+        uint32_t* size = s_u32[2];
+        uint32_t* pf = s_u32[3];
+        __syncwarp();
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+            const unsigned long long xr = r ? x1 : x0;
+            const uint32_t i = (uint32_t)lane + 32u * r;
+            if (begin_pass[r]) {
+                const uint32_t t = (uint32_t)__popcll(BP & ((1ull << i) - 1ull));
+                first[t] = gk_start(xr);
+                size[t] = ce[r] - cb[r];
+                pf[t] = gk_pf(xr);
+                s_alive[t] = 1u;
+            }
+            if (pass[r] && i + 1u == ce[r]) last[(uint32_t)__popcll(BP & ((1ull << cb[r]) - 1ull))] = gk_start(xr);
+        }
+        __syncwarp();
+        ClusterArrays A{first, last, size, pf, s_u32[4], s_u32[5], s_alive};
+        filter_clusters_warp(ncl, A, lane);
+        __syncwarp();
+#pragma unroll
+        for (int r = 0; r < 2; ++r)
+            if (pass[r]) alive[r] = s_alive[(uint32_t)__popcll(BP & ((1ull << cb[r]) - 1ull))] != 0u;
+    }
+    // ---- add_clusters_to_pangraph: kept flags, one coverage key per kept hit, one locus key per kept cluster
+    const uint32_t k0m = __ballot_sync(FULL, alive[0] && begin_pass[0]), k1m = __ballot_sync(FULL, alive[1] && begin_pass[1]);
+    const unsigned long long KB = (unsigned long long)k0m | ((unsigned long long)k1m << 32);  // begins of the kept clusters
+    if (lane < 2 && (uint32_t)__popcll(KB) <= (uint32_t)lane) act_lk[2 * a + lane] = COV_KEY_NONE;
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+        const uint32_t i = (uint32_t)lane + 32u * r;
+        if (i >= c) continue;
+        const unsigned long long xr = r ? x1 : x0;
+        gkept[base + i] = alive[r] ? 1 : 0;
+        cov_keys[base + i] = alive[r] ? 2u * (knode_base[gk_prg(xr)] + gk_knode(xr)) + gk_rev(xr) : COV_KEY_NONE;
+        if (alive[r] && begin_pass[r]) {
+            const uint32_t t = (uint32_t)__popcll(KB & ((1ull << i) - 1ull));
+            if (t < 2u) act_lk[2 * a + t] = locus_key_base + gk_prg(xr);
+            else lk_ovf[atomicAdd(ctr + CTR_LKOVF, 1ull)] = locus_key_base + gk_prg(xr);  // a third kept cluster on one short read: rare
+        }
+    }
+}
+
+// One warp per read, the next read's keys and the one after's count and slice base in flight while the current read is
+// clustered: each read is a chain of dependent loads (count, base -> keys -> thresholds), which the pipeline overlaps
 __global__ void __launch_bounds__(CW_WARPS * 32) cluster_warp_kernel(
     unsigned long long* __restrict__ ctr, PostCaps C, const uint32_t* __restrict__ act_base, const uint32_t* __restrict__ act_count,
     unsigned long long* __restrict__ gkey, uint8_t* __restrict__ gkept, uint32_t max_diff, uint32_t min_thresh, const uint32_t* __restrict__ thresh,
@@ -286,114 +431,26 @@ __global__ void __launch_bounds__(CW_WARPS * 32) cluster_warp_kernel(
     if (batch_overflowed(ctr, C)) return;
     const unsigned long long n_active = ctr[CTR_ACTIVE];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (unsigned long long a = (unsigned long long)blockIdx.x * CW_WARPS + wid; a < n_active; a += (unsigned long long)gridDim.x * CW_WARPS) {
-        const uint32_t c = act_count[a];
-        if (c > CLUSTER_WARP_MAX) continue;  // the CTA kernel's read
-        const uint32_t base = act_base[a];
-        if (c <= min_thresh) {  // no cluster of this read can exceed any locus's size threshold (stray hits): nothing is kept
-            if ((uint32_t)lane < c) {
-                gkept[base + lane] = 0;
-                cov_keys[base + lane] = COV_KEY_NONE;
-            }
-            if ((uint32_t)lane + 32u < c) {
-                gkept[base + 32 + lane] = 0;
-                cov_keys[base + 32 + lane] = COV_KEY_NONE;
-            }
-            if (lane < 2) act_lk[2 * a + lane] = COV_KEY_NONE;
-            continue;
+    const unsigned long long stride = (unsigned long long)gridDim.x * CW_WARPS;
+    auto head = [&](unsigned long long a) {
+        WarpRead R{0u, 0u, ~0ull, ~0ull};
+        if (a < n_active) {
+            R.c = act_count[a];
+            R.base = act_base[a];
         }
-        // element i lives in lane i & 31, register i >> 5; padding sorts to the end
-        unsigned long long x0 = (uint32_t)lane < c ? gkey[base + lane] : ~0ull;
-        unsigned long long x1 = (uint32_t)lane + 32u < c ? gkey[base + 32 + lane] : ~0ull;
-        if (c > 32u) warp_sort64<2>(x0, x1, lane);  // warp-uniform
-        else warp_sort64<1>(x0, x1, lane);
-        if ((uint32_t)lane < c) gkey[base + lane] = x0;  // the slice stays sorted for the hooks / later consumers
-        if ((uint32_t)lane + 32u < c) gkey[base + 32 + lane] = x1;
-        // ---- define_clusters: a hit opens a cluster when prg or strand change or the gap exceeds max_diff
-        const unsigned long long p0 = shfl_up64(x0, 1), x0_31 = shfl64(x0, 31);
-        unsigned long long p1 = shfl_up64(x1, 1);
-        if (lane == 0) p1 = x0_31;
-        auto opens = [&](unsigned long long cur, unsigned long long prev, uint32_t i) {
-            if (i == 0u || i == c) return true;  // i == c: the first padding element closes the last cluster
-            if (i > c) return false;
-            return gk_pf(cur) != gk_pf(prev) || gk_start(cur) - gk_start(prev) > max_diff;
-        };
-        const uint32_t m0 = __ballot_sync(FULL, opens(x0, p0, (uint32_t)lane));
-        const uint32_t m1 = __ballot_sync(FULL, opens(x1, p1, (uint32_t)lane + 32u));
-        const unsigned long long S = (unsigned long long)m0 | ((unsigned long long)m1 << 32);
-        uint32_t cb[2], ce[2];
-        bool pass[2], begin_pass[2];
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            const uint32_t i = (uint32_t)lane + 32u * r;
-            const unsigned long long le = i == 63u ? ~0ull : ((2ull << i) - 1ull);
-            cb[r] = 63u - (uint32_t)__clzll((long long)(S & le));
-            const unsigned long long gt = S & ~le;
-            ce[r] = gt ? (uint32_t)__ffsll((long long)gt) - 1u : c;
-            const unsigned long long xr = r ? x1 : x0;
-            pass[r] = i < c && (ce[r] - cb[r]) > thresh[gk_prg(xr)];
-            begin_pass[r] = pass[r] && cb[r] == i;
-        }
-        const uint32_t b0 = __ballot_sync(FULL, begin_pass[0]), b1 = __ballot_sync(FULL, begin_pass[1]);
-        const unsigned long long BP = (unsigned long long)b0 | ((unsigned long long)b1 << 32);
-        const uint32_t ncl = (uint32_t)__popcll(BP);
-        if (ncl == 0u) {
-            if ((uint32_t)lane < c) {
-                gkept[base + lane] = 0;
-                cov_keys[base + lane] = COV_KEY_NONE;
-            }
-            if ((uint32_t)lane + 32u < c) {
-                gkept[base + 32 + lane] = 0;
-                cov_keys[base + 32 + lane] = COV_KEY_NONE;
-            }
-            if (lane < 2) act_lk[2 * a + lane] = COV_KEY_NONE;
-            continue;
-        }
-        bool alive[2] = {pass[0], pass[1]};
-        if (ncl > 1u) {
-            uint32_t* first = s_u32[wid][0];
-            uint32_t* last = s_u32[wid][1];
-            uint32_t* size = s_u32[wid][2];
-            uint32_t* pf = s_u32[wid][3];
-            __syncwarp();
-#pragma unroll
-            for (int r = 0; r < 2; ++r) {
-                const unsigned long long xr = r ? x1 : x0;
-                const uint32_t i = (uint32_t)lane + 32u * r;
-                if (begin_pass[r]) {
-                    const uint32_t t = (uint32_t)__popcll(BP & ((1ull << i) - 1ull));
-                    first[t] = gk_start(xr);
-                    size[t] = ce[r] - cb[r];
-                    pf[t] = gk_pf(xr);
-                    s_alive[wid][t] = 1u;
-                }
-                if (pass[r] && i + 1u == ce[r]) last[(uint32_t)__popcll(BP & ((1ull << cb[r]) - 1ull))] = gk_start(xr);
-            }
-            __syncwarp();
-            ClusterArrays A{first, last, size, pf, s_u32[wid][4], s_u32[wid][5], s_alive[wid]};
-            filter_clusters_warp(ncl, A, lane);
-            __syncwarp();
-#pragma unroll
-            for (int r = 0; r < 2; ++r)
-                if (pass[r]) alive[r] = s_alive[wid][(uint32_t)__popcll(BP & ((1ull << cb[r]) - 1ull))] != 0u;
-        }
-        // ---- add_clusters_to_pangraph: kept flags, one coverage key per kept hit, one locus key per kept cluster
-        const uint32_t k0m = __ballot_sync(FULL, alive[0] && begin_pass[0]), k1m = __ballot_sync(FULL, alive[1] && begin_pass[1]);
-        const unsigned long long KB = (unsigned long long)k0m | ((unsigned long long)k1m << 32);  // begins of the kept clusters
-        if (lane < 2 && (uint32_t)__popcll(KB) <= (uint32_t)lane) act_lk[2 * a + lane] = COV_KEY_NONE;
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            const uint32_t i = (uint32_t)lane + 32u * r;
-            if (i >= c) continue;
-            const unsigned long long xr = r ? x1 : x0;
-            gkept[base + i] = alive[r] ? 1 : 0;
-            cov_keys[base + i] = alive[r] ? 2u * (knode_base[gk_prg(xr)] + gk_knode(xr)) + gk_rev(xr) : COV_KEY_NONE;
-            if (alive[r] && begin_pass[r]) {
-                const uint32_t t = (uint32_t)__popcll(KB & ((1ull << i) - 1ull));
-                if (t < 2u) act_lk[2 * a + t] = locus_key_base + gk_prg(xr);
-                else lk_ovf[atomicAdd(ctr + CTR_LKOVF, 1ull)] = locus_key_base + gk_prg(xr);  // a third kept cluster on one short read: rare
-            }
-        }
+        return R;
+    };
+    unsigned long long a = (unsigned long long)blockIdx.x * CW_WARPS + wid;
+    WarpRead cur = head(a);
+    load_warp_read_keys(cur, gkey, min_thresh, lane);
+    WarpRead nxt = head(a + stride);
+    for (; a < n_active; a += stride) {
+        load_warp_read_keys(nxt, gkey, min_thresh, lane);
+        const WarpRead after = head(a + 2 * stride);
+        cluster_warp_read(a, cur, ctr, gkey, gkept, max_diff, min_thresh, thresh, knode_base, locus_key_base, cov_keys, act_lk, lk_ovf,
+                          s_u32[wid], s_alive[wid], lane);
+        cur = nxt;
+        nxt = after;
     }
 }
 
@@ -533,107 +590,95 @@ __global__ void __launch_bounds__(CC_THREADS) cluster_cta_kernel(
 }
 
 // ============================================================================================
-// S5 : coverage without atomics.
+// S5 : coverage counted in shared memory.
 // The key slots of a batch ([one per grouped hit | two per active read | overflow list], "none" where nothing is
-// counted) are cut into STRETCHES of 64 k slots and the key space into RANGES of 6 k counters.  A job = (range, stretch):
-// its CTA keeps one PRIVATE copy of the range's counters per warp in shared memory (16 warps x 6144 x 16 bit = 192 KB);
-// every warp walks its own sixteenth of the stretch, ignores keys outside the range, and combines equal keys of one step
-// with match.any, so every increment is a plain read-modify-write with a single writer.  The sixteen copies are then
-// summed and STORED (not added) to the job's own piece of partial[stretch][range]; cov_merge_kernel sums over the
-// stretches.  A slot is read once per range (13 times for the Mtb-scale panel, from L2).
+// counted) are cut into STRETCHES and the key space into RANGES of 56 k counters, as many 32-bit counters as one CTA's
+// shared memory holds (224 KB: the Mtb-scale panel's 76 k keys are two ranges).  A job = (range, stretch): its CTA zeroes
+// one copy of the range's counters, every thread counts the keys of its share of the stretch that fall into the range
+// with shared-memory atomic adds (integers: the order of the adds does not matter), and the copy is STORED (not added) to
+// the job's own piece of partial[stretch][range]; cov_merge_kernel sums over the stretches.  A slot is read once per range.
 // ============================================================================================
-constexpr int CV_THREADS = 512, CV_WARPS = CV_THREADS / 32;
-constexpr uint32_t CV_RANGE = 6144;            // counters per range
-constexpr uint32_t CV_STRETCH_MIN = 8192;      // a stretch is sized so that (ranges x stretches) fills the grid once, within these
-constexpr uint32_t CV_STRETCH_MAX = 983040;    // bounds: a warp sees a sixteenth of it and its counters are 16 bit (61 440 < 65 536)
-constexpr uint32_t CV_UNROLL = 8;              // independent slot loads in flight per lane; 8 x 32 slots are compacted, then counted
+constexpr int CV_THREADS = 1024;
+constexpr uint32_t CV_RANGE = 56 * 1024;                 // counters per range: 224 KB of shared memory
+constexpr uint32_t CV_STRETCH_MIN = 32768;               // a job's fixed cost is zeroing and storing 224 KB: a small batch
+                                                         // gets fewer, longer stretches rather than more jobs
+constexpr unsigned long long CV_STRETCH_MAX = 1ull << 28;  // the per-stretch partials are int32: far below 2^31 slots
+constexpr int CV_UNROLL = 4;                             // 16-byte slot loads in flight per thread
 
 // slots per stretch for n slots on a grid of `grid` CTAs and n_range key ranges: the (range, stretch) jobs fill the grid in
-// whole waves (one wave while a stretch stays below CV_STRETCH_MAX); a multiple of 512 (16 warps x 32 lanes)
+// whole waves (one wave while a stretch stays below CV_STRETCH_MAX); a multiple of 1024
 __host__ __device__ __forceinline__ unsigned long long cov_stretch_len(unsigned long long n, uint32_t grid, uint32_t n_range) {
     const unsigned long long min_stretches = (n + CV_STRETCH_MAX - 1) / CV_STRETCH_MAX;
     const unsigned long long waves = (min_stretches * n_range + grid - 1) / grid;          // at least this many waves
     unsigned long long stretches = (waves < 1 ? 1 : waves) * grid / n_range;               // stretches that fill them
     if (stretches < 1) stretches = 1;
     unsigned long long len = (n + stretches - 1) / stretches;
-    len = (len + 511ull) & ~511ull;
+    len = (len + 1023ull) & ~1023ull;
     return len < CV_STRETCH_MIN ? CV_STRETCH_MIN : (len > CV_STRETCH_MAX ? CV_STRETCH_MAX : len);
 }
 
-// key slots of a batch, concatenated: [per grouped hit | two per active read | overflow list]
-struct CovSlots {
-    const uint32_t *cov_keys, *act_lk, *lk_ovf;
-    unsigned long long n0, n1, n2;
-    __device__ __forceinline__ uint32_t at(unsigned long long i, unsigned long long end) const {  // slots from `end` on read as "none"
-        if (i >= end) return COV_KEY_NONE;
-        if (i < n0) return __ldg(cov_keys + i);
-        i -= n0;
-        if (i < n1) return __ldg(act_lk + i);
-        return __ldg(lk_ovf + (i - n1));
+// counts the keys of p[lo, hi) that fall into [k_lo, k_lo + k_n): whole 16-byte groups by vector loads, the ends singly
+__device__ __forceinline__ void cov_count_segment(const uint32_t* __restrict__ p, unsigned long long lo, unsigned long long hi,
+                                                  uint32_t k_lo, uint32_t k_n, uint32_t* cnt, int tid) {
+    if (lo >= hi) return;
+    auto count = [&](uint32_t key) {
+        const uint32_t rel = key - k_lo;  // "none" is far above every range
+        if (rel < k_n) atomicAdd(cnt + rel, 1u);
+    };
+    const unsigned long long v_lo = (lo + 3) & ~3ull, v_hi = hi & ~3ull;
+    if (v_lo >= v_hi) {
+        for (unsigned long long i = lo + tid; i < hi; i += CV_THREADS) count(__ldg(p + i));
+        return;
     }
-};
+    if (lo + tid < v_lo) count(__ldg(p + lo + tid));
+    if (v_hi + tid < hi) count(__ldg(p + v_hi + tid));
+    const uint4* v = reinterpret_cast<const uint4*>(p);  // the slot arrays come from cudaMalloc: 16-byte aligned
+    const unsigned long long g_lo = v_lo / 4, g_hi = v_hi / 4;
+    for (unsigned long long g0 = g_lo + tid; g0 < g_hi; g0 += (unsigned long long)CV_UNROLL * CV_THREADS) {
+        uint4 x[CV_UNROLL];
+#pragma unroll
+        for (int u = 0; u < CV_UNROLL; ++u) {
+            const unsigned long long g = g0 + (unsigned long long)u * CV_THREADS;
+            x[u] = g < g_hi ? __ldg(v + g) : make_uint4(COV_KEY_NONE, COV_KEY_NONE, COV_KEY_NONE, COV_KEY_NONE);
+        }
+#pragma unroll
+        for (int u = 0; u < CV_UNROLL; ++u) {
+            count(x[u].x);
+            count(x[u].y);
+            count(x[u].z);
+            count(x[u].w);
+        }
+    }
+}
 
-__global__ void __launch_bounds__(CV_THREADS, 1) cov_count_kernel(const unsigned long long* __restrict__ ctr, PostCaps C, CovSlots S,
-                                                                 int32_t* __restrict__ partials, uint32_t max_stretches,
-                                                                 uint32_t n_accum, uint32_t n_keys) {
-    extern __shared__ unsigned short s_cnt[];  // [CV_WARPS][CV_RANGE] counters, then [CV_WARPS][CV_UNROLL * 32] compacted keys
+__global__ void __launch_bounds__(CV_THREADS, 1) cov_count_kernel(const unsigned long long* __restrict__ ctr, PostCaps C,
+                                                                 const uint32_t* __restrict__ cov_keys, const uint32_t* __restrict__ act_lk,
+                                                                 const uint32_t* __restrict__ lk_ovf, int32_t* __restrict__ partials,
+                                                                 uint32_t max_stretches, uint32_t n_accum, uint32_t n_keys) {
+    extern __shared__ uint32_t s_cnt[];  // [CV_RANGE] counters
     if (batch_overflowed(ctr, C)) return;
-    S.n0 = ctr[CTR_HITS];
-    S.n1 = 2ull * ctr[CTR_ACTIVE];
-    S.n2 = ctr[CTR_LKOVF];
-    const unsigned long long n = S.n0 + S.n1 + S.n2;
+    // the slots, concatenated: [per grouped hit | two per active read | overflow list]
+    const unsigned long long n0 = ctr[CTR_HITS], n1 = 2ull * ctr[CTR_ACTIVE], n = n0 + n1 + ctr[CTR_LKOVF];
     const uint32_t n_range = (n_keys + CV_RANGE - 1) / CV_RANGE;
     const unsigned long long stretch_len = cov_stretch_len(n, gridDim.x, n_range);
     const uint32_t n_stretch = (uint32_t)min((unsigned long long)max_stretches, (n + stretch_len - 1) / stretch_len);
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    unsigned short* mine = s_cnt + (size_t)wid * CV_RANGE;
-    unsigned short* list = s_cnt + (size_t)CV_WARPS * CV_RANGE + (size_t)wid * (CV_UNROLL * 32);
-    const uint32_t lt = (1u << lane) - 1u;
+    const int tid = threadIdx.x;
     for (uint32_t job = blockIdx.x; job < n_stretch * n_range; job += gridDim.x) {
         const uint32_t stretch = job / n_range, k_lo = (job % n_range) * CV_RANGE;
         const uint32_t k_n = min(CV_RANGE, n_keys - k_lo);
-        for (uint32_t i = tid; i < CV_WARPS * CV_RANGE / 8; i += CV_THREADS) reinterpret_cast<uint4*>(s_cnt)[i] = make_uint4(0u, 0u, 0u, 0u);
+        for (uint32_t i = tid; i < CV_RANGE / 4; i += CV_THREADS) reinterpret_cast<uint4*>(s_cnt)[i] = make_uint4(0u, 0u, 0u, 0u);
         __syncthreads();
-        // this warp's share of the stretch, CV_UNROLL x 32 slots at a time (the loads of the next group are issued first)
-        const unsigned long long s_lo = (unsigned long long)stretch * stretch_len + (unsigned long long)wid * (stretch_len / CV_WARPS);
-        const unsigned long long s_hi = min(n, s_lo + stretch_len / CV_WARPS);
-        uint32_t cur[CV_UNROLL], nxt[CV_UNROLL];
-#pragma unroll
-        for (uint32_t u = 0; u < CV_UNROLL; ++u) cur[u] = S.at(s_lo + u * 32 + lane, s_hi);
-        for (unsigned long long g0 = s_lo; g0 < s_hi; g0 += CV_UNROLL * 32) {
-#pragma unroll
-            for (uint32_t u = 0; u < CV_UNROLL; ++u) nxt[u] = S.at(g0 + (CV_UNROLL + u) * 32 + lane, s_hi);
-            // compact the keys of this group that fall into the range ("none" is far above every range)
-            uint32_t cnt = 0;
-#pragma unroll
-            for (uint32_t u = 0; u < CV_UNROLL; ++u) {
-                const uint32_t rel = cur[u] - k_lo;
-                const bool own = rel < k_n;
-                const uint32_t m = __ballot_sync(FULL, own);
-                if (own) list[cnt + __popc(m & lt)] = (unsigned short)rel;
-                cnt += __popc(m);
-            }
-            __syncwarp();
-            // count them: equal keys of one step are combined, the lowest lane of each group adds
-            for (uint32_t e0 = 0; e0 < cnt; e0 += 32) {
-                const bool have = e0 + lane < cnt;
-                const uint32_t rel = have ? list[e0 + lane] : 0xffffffffu;
-                const uint32_t peers = __match_any_sync(FULL, rel);
-                if (have && lane == __ffs(peers) - 1) mine[rel] = (unsigned short)(mine[rel] + __popc(peers));
-                __syncwarp();
-            }
-#pragma unroll
-            for (uint32_t u = 0; u < CV_UNROLL; ++u) cur[u] = nxt[u];
-        }
+        const unsigned long long s_lo = (unsigned long long)stretch * stretch_len, s_hi = min(n, s_lo + stretch_len);
+        auto segment = [&](const uint32_t* p, unsigned long long b, unsigned long long e) {  // the stretch's part of slots [b, e)
+            cov_count_segment(p, min(max(s_lo, b), e) - b, min(max(s_hi, b), e) - b, k_lo, k_n, s_cnt, tid);
+        };
+        segment(cov_keys, 0, n0);
+        segment(act_lk, n0, n0 + n1);
+        segment(lk_ovf, n0 + n1, n);
         __syncthreads();
-        // sum the sixteen copies and store the job's piece of the partial (it is this job's alone: a store, not an add)
+        // the job's piece of the partial is this job's alone: a store, not an add
         int32_t* out = partials + (size_t)stretch * n_accum + k_lo;
-        for (uint32_t k = tid; k < k_n; k += CV_THREADS) {
-            uint32_t v = 0;
-#pragma unroll
-            for (int w = 0; w < CV_WARPS; ++w) v += s_cnt[(size_t)w * CV_RANGE + k];
-            out[k] = (int32_t)v;
-        }
+        for (uint32_t k = tid; k < k_n; k += CV_THREADS) out[k] = (int32_t)s_cnt[k];
         __syncthreads();
     }
 }
@@ -651,7 +696,8 @@ __global__ void cov_merge_kernel(unsigned long long* __restrict__ ctr, PostCaps 
     unsigned long long kept = 0;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n_keys; k += gridDim.x * blockDim.x) {
         int32_t sum = 0;
-        for (uint32_t g = 0; g < used; ++g) sum += partials[(size_t)g * n_accum + k];
+#pragma unroll 8
+        for (uint32_t g = 0; g < used; ++g) sum += partials[(size_t)g * n_accum + k];  // a row per stretch: eight loads in flight
         if (!sum) continue;
         if (k < n_cov_keys) kept += (unsigned long long)sum;
         if (remote) asm volatile("red.relaxed.sys.global.add.s32 [%0], %1;" ::"l"(dst + k), "r"(sum) : "memory");
@@ -722,8 +768,13 @@ void launch_postprocess(const PostBuffers& P, PostCaps C, uint32_t read_id_base,
     scatter_kernel<<<sm * 16, 256, 0, st>>>(P.hi, P.lo, P.ctr, C, read_id_base, P.read_count, P.read_base, P.gkey);
     if (ev_grouped) cudaEventRecord(ev_grouped, st);
     const uint32_t locus_key_base = 2u * total_knodes;
-    cluster_warp_kernel<<<sm * 4, CW_WARPS * 32, 0, st>>>(P.ctr, C, P.act_base, P.act_count, P.gkey, P.gkept, max_diff, min_thresh, d_thresh_per_prg,
-                                                         d_knode_base, locus_key_base, P.cov_keys, P.act_lk, P.lk_ovf);
+    static const int cw_per_sm = [] {
+        int n = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, cluster_warp_kernel, CW_WARPS * 32, 0);
+        return std::max(n, 1);
+    }();
+    cluster_warp_kernel<<<sm * cw_per_sm, CW_WARPS * 32, 0, st>>>(P.ctr, C, P.act_base, P.act_count, P.gkey, P.gkept, max_diff, min_thresh, d_thresh_per_prg,
+                                                                  d_knode_base, locus_key_base, P.cov_keys, P.act_lk, P.lk_ovf);
     ensure_dyn_smem(cluster_cta_kernel, (size_t)CC_SMEM_KEYS * 8);
     BigScratch B{P.scratch[0], P.scratch[1], P.scratch[2], P.scratch[3], P.scratch[4], P.scratch[5], P.scratch[6], P.scratch[7],
                  P.scratch[8], P.scratch[9]};
@@ -732,10 +783,9 @@ void launch_postprocess(const PostBuffers& P, PostCaps C, uint32_t read_id_base,
                                                                             locus_key_base, P.cov_keys, P.act_lk, P.lk_ovf, B);
     if (ev_clustered) cudaEventRecord(ev_clustered, st);
     const uint32_t n_accum = 2u * total_knodes + n_loci + 4u, n_keys = 2u * total_knodes + n_loci;
-    const size_t cv_smem = (size_t)CV_WARPS * (CV_RANGE + CV_UNROLL * 32) * sizeof(unsigned short);
+    const size_t cv_smem = (size_t)CV_RANGE * sizeof(uint32_t);
     ensure_dyn_smem(cov_count_kernel, cv_smem);
-    CovSlots S{P.cov_keys, P.act_lk, P.lk_ovf, 0, 0, 0};
-    cov_count_kernel<<<sm, CV_THREADS, cv_smem, st>>>(P.ctr, C, S, P.partials, P.n_partials, n_accum, n_keys);
+    cov_count_kernel<<<sm, CV_THREADS, cv_smem, st>>>(P.ctr, C, P.cov_keys, P.act_lk, P.lk_ovf, P.partials, P.n_partials, n_accum, n_keys);
     cov_merge_kernel<<<(n_keys + 255) / 256, 256, 0, st>>>(P.ctr, C, P.partials, P.n_partials, sm, n_accum, n_keys, 2u * total_knodes, d_accum_dst,
                                                           remote_dst);
     g_launches += 6;
