@@ -68,6 +68,43 @@ pub struct CandidateRegion {
     pub read_off: u64,
 }
 
+/// Options of the local assembler (`drprg_assemble_opts`); 0 = pandora's default (min DBG depth 2, 25 candidate paths),
+/// max_insertion u32::MAX = 15.  max_candidate_paths is at most 64.
+#[repr(C)]
+#[derive(Debug, Default, Clone, Copy)]
+pub struct AssembleOpts {
+    pub min_dbg_dp: u32,
+    pub max_insertion: u32,
+    pub max_candidate_paths: u32,
+}
+
+/// One de-novo allele as the C ABI lists it (`drprg_denovo_path`): it replaces `[a, b)` of its region's locus consensus;
+/// its bases are `length` bytes at `offset` of the bases buffer.
+#[repr(C)]
+#[derive(Debug, Default, Clone, Copy)]
+pub struct DenovoPath {
+    pub region: u32,
+    pub a: u32,
+    pub b: u32,
+    pub length: u32,
+    pub offset: u64,
+}
+
+/// Region status of the local assembler (`DRPRG_DENOVO_*`).
+pub const DENOVO_ASSEMBLED: u8 = 0;
+pub const DENOVO_NO_ANCHOR: u8 = 1;
+pub const DENOVO_TOO_MANY_PATHS: u8 = 2;
+pub const DENOVO_NO_PATH: u8 = 3;
+
+/// A de-novo allele: region index, the consensus interval `[a, b)` it replaces, its sequence.
+#[derive(Debug, Default, Clone)]
+pub struct DenovoAllele {
+    pub region: u32,
+    pub a: u32,
+    pub b: u32,
+    pub seq: Vec<u8>,
+}
+
 /// Reads overlapping the candidate regions: read id, span on the read, strand (parallel arrays).
 #[derive(Debug, Default, Clone)]
 pub struct CandidateReads {
@@ -119,6 +156,14 @@ extern "C" {
     fn drprg_cuda_discover_regions(idx: *mut RawIndex, out: *mut CandidateRegion) -> c_int;
     fn drprg_cuda_discover_region_reads(idx: *mut RawIndex, read: *mut u32, start: *mut u32, end: *mut u32, fwd: *mut u8) -> c_int;
     fn drprg_cuda_discover_consensus(idx: *mut RawIndex, locus: u32, len: *mut u64) -> *const c_char;
+    fn drprg_cuda_discover_assemble(
+        idx: *mut RawIndex,
+        opts: *const AssembleOpts,
+        n_paths: *mut u32,
+        n_path_bases: *mut u64,
+    ) -> c_int;
+    fn drprg_cuda_discover_paths(idx: *mut RawIndex, out: *mut DenovoPath, bases: *mut c_char) -> c_int;
+    fn drprg_cuda_discover_region_status(idx: *mut RawIndex, status: *mut u8) -> c_int;
     fn drprg_cuda_gt_counts(idx: *mut RawIndex, n_records: *mut u32, n_alleles: *mut u32, n_allele_knodes: *mut u64) -> c_int;
     fn drprg_cuda_gt_filter_stats(
         idx: *mut RawIndex,
@@ -245,6 +290,37 @@ impl Index {
             return Err(CudaError::ProcessError(last_error()));
         }
         Ok((regions, reads))
+    }
+
+    /// pandora discover's local assembly of every candidate region, on the GPU, from the bases the map pass retained.  Call
+    /// after `discover_candidates` (`n_regions` = its region count).  Returns the status of every region and the de-novo
+    /// alleles, sorted within a region.
+    pub fn discover_assemble(&mut self, opts: Option<&AssembleOpts>, n_regions: usize) -> Result<(Vec<u8>, Vec<DenovoAllele>), CudaError> {
+        let (mut n_paths, mut n_bases) = (0u32, 0u64);
+        let o = opts.map_or(std::ptr::null(), |o| o as *const AssembleOpts);
+        if unsafe { drprg_cuda_discover_assemble(self.raw, o, &mut n_paths, &mut n_bases) } != 0 {
+            return Err(CudaError::ProcessError(last_error()));
+        }
+        let mut paths = vec![DenovoPath::default(); n_paths as usize];
+        let mut bases = vec![0u8; n_bases as usize];
+        let mut status = vec![0u8; n_regions];
+        let rc = unsafe {
+            drprg_cuda_discover_paths(self.raw, paths.as_mut_ptr(), bases.as_mut_ptr() as *mut c_char)
+                | drprg_cuda_discover_region_status(self.raw, status.as_mut_ptr())
+        };
+        if rc != 0 {
+            return Err(CudaError::ProcessError(last_error()));
+        }
+        let alleles = paths
+            .iter()
+            .map(|p| DenovoAllele {
+                region: p.region,
+                a: p.a,
+                b: p.b,
+                seq: bases[p.offset as usize..(p.offset + p.length as u64) as usize].to_vec(),
+            })
+            .collect();
+        Ok((status, alleles))
     }
 
     /// The maximum-likelihood sequence of a locus in this sample (`None`: the locus is absent).

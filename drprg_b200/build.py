@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 SO = os.path.join(HERE, "libdrprg_cuda.so")
 SOURCES = ["sketch.cu", "cluster.cu", "mlpath.cu", "genotype.cu", "capi.cu", "ingest.cu", "gzip_inflate.cpp",
-           "prg_graph.cpp", "genotype_host.cpp", "discover.cpp", "fastq_frame.cpp"]
+           "prg_graph.cpp", "genotype_host.cpp", "discover.cpp", "assemble.cu", "fastq_frame.cpp"]
 EXTRA = ["pandora_cuda_main.cpp"]
 HEADERS = ["kernels.cuh", "kernels_common.cuh", "prg_graph.hpp", "genotype_host.hpp", "ingest.hpp", "cuda_owned.hpp",
            "gzip_inflate.hpp", "fastq_frame.hpp", "../../include/drprg_cuda.h"]

@@ -21,6 +21,7 @@
 #include <mutex>
 #include <stdexcept>
 #include <thread>
+#include <unordered_map>
 
 #include "../../include/drprg_cuda.h"
 #include "cuda_owned.hpp"
@@ -198,7 +199,22 @@ struct drprg_index {
     // discover's front half from the map pass (SURVEY 8f rank 1): kept hits of the sample, retained on request
     bool retain_hits = false;
     std::vector<RetainedHit> retained;
+    // ... and the 2-bit words of every read with a kept hit (per global read id: word offset and length in bases)
+    struct RetainedReads {
+        std::vector<uint32_t> read, len;
+        std::vector<uint64_t> off;
+        std::vector<uint32_t> words;
+    } retained_reads;
+    DBuf<uint2> d_rt_table;
+    DBuf<uint32_t> d_rt_words;
+    DBuf<unsigned long long> d_rt_cursor;
     DiscoverResult discover;
+    bool discover_ready = false;  // drprg_cuda_discover_candidates ran for the current sample
+    // the local assembler's results (drprg_cuda_discover_assemble)
+    std::vector<uint8_t> asm_status;
+    std::vector<drprg_denovo_path> asm_paths;
+    std::string asm_bases;
+    double asm_stats[4] = {0, 0, 0, 0};
     uint32_t max_locus_knodes = 0, max_locus_edges = 0;
     Event ev_ml[2];
     Stream st_ml, st_gt, st_copy, st_acc;
@@ -482,6 +498,8 @@ void sample_begin(drprg_index* X, const drprg_map_opts* o, uint32_t first_read_l
     X->total_bases = X->n_reads = 0;
     X->own_bases = X->own_reads = 0;
     X->retained.clear();
+    X->retained_reads = drprg_index::RetainedReads();
+    X->discover_ready = false;
     X->scalars_in_buffer = false;
     X->hist_on_host = false;
     X->sample_open = true;
@@ -508,6 +526,41 @@ void ensure_read_capacity(drprg_index* X, uint64_t n_reads) {
     X->read_count.ensure(n_reads);
     X->read_base.ensure(X->read_count.cap);
     CK(cudaMemset(X->read_count.p, 0, X->read_count.cap * sizeof(int32_t)));  // the kernels leave it zero after every batch
+}
+
+// The words of the batch's reads that kept a hit, into the sample's host-side store: the assembler needs their bases after
+// the batch (a file's wave) is gone.  ar = the active reads of the batch (act_read, downloaded).
+void retain_read_bases(drprg_index* X, drprg_batch* B, cudaStream_t st, const std::vector<uint32_t>& ar) {
+    const uint64_t na = ar.size();
+    if (!na) return;
+    X->d_rt_table.ensure(na);
+    X->d_rt_cursor.ensure(1);
+    if (!X->d_rt_words.cap) X->d_rt_words.ensure(na * 16);
+    unsigned long long used = 0;
+    for (;;) {  // the words wanted are counted past the capacity: regrow once to the exact need
+        CK(cudaMemsetAsync(X->d_rt_cursor.p, 0, sizeof(unsigned long long), st));
+        launch_retain_gather(B->R, X->act_read.p, X->act_base.p, X->act_count.p, X->gkept.p, (uint32_t)na, X->d_rt_table.p,
+                             X->d_rt_words.p, X->d_rt_words.cap, X->d_rt_cursor.p, st);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&used, X->d_rt_cursor.p, sizeof used, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (used <= X->d_rt_words.cap) break;
+        if (used >= 0xffffffffull) throw std::runtime_error("the reads of one batch that kept a hit exceed 2^32 words: split the batch");
+        X->d_rt_words.ensure(used);
+    }
+    std::vector<uint2> table(na);
+    drprg_index::RetainedReads& S = X->retained_reads;
+    const uint64_t base = S.words.size();
+    S.words.resize(base + used);
+    CK(cudaMemcpyAsync(table.data(), X->d_rt_table.p, na * sizeof(uint2), cudaMemcpyDeviceToHost, st));
+    if (used) CK(cudaMemcpyAsync(S.words.data() + base, X->d_rt_words.p, used * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (uint64_t a = 0; a < na; ++a) {
+        if (table[a].x == 0xffffffffu) continue;
+        S.read.push_back(B->R.read_id_base + ar[a]);
+        S.off.push_back(base + table[a].x);
+        S.len.push_back(table[a].y);
+    }
 }
 
 void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits, uint64_t* n_kept) {
@@ -623,6 +676,7 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
                                                   (uint32_t)k & ((1u << GKEY_KNODE_BITS) - 1u), (uint16_t)(k >> 48),
                                                   (uint8_t)(((k >> 47) & 1ull) ^ 1ull)});
             }
+        retain_read_bases(X, B, st, ar);
     }
     if (n_hits) *n_hits = nh;
     if (n_kept) *n_kept = X->h_counters.p[CTR_KEPT];
@@ -1425,6 +1479,168 @@ bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_o
     return W.waves > 0;
 }
 
+// ============================================================================================
+// discover's local assembler (assemble.cu): the pileups of all candidate regions of the sample are uploaded once, one
+// CTA per region counts and walks them, and the host reads back the statuses, the walk lengths and the walks' bases.
+// The consensus walk is dropped and the rest sorted here.
+// ============================================================================================
+uint32_t consensus_kmer(const std::string& c, size_t at) {  // UINT32_MAX when a base is not ACGT: never solid
+    static const char acgt[] = "ACGT";
+    uint32_t x = 0;
+    for (size_t i = at; i < at + DISCOVER_K; ++i) {
+        const char* q = c[i] ? strchr(acgt, c[i]) : nullptr;
+        if (!q) return UINT32_MAX;
+        x = (x << 2) | (uint32_t)(q - acgt);
+    }
+    return x;
+}
+
+void assemble_regions(drprg_index* X, const drprg_assemble_opts* o) {
+    AsmParams P{2, 15, 25};  // pandora discover: --min-dbg-dp 2, --max-ins 15, --max-num-candidate-paths 25
+    if (o && o->min_dbg_dp) P.min_dp = o->min_dbg_dp;
+    if (o && o->max_insertion != 0xffffffffu) P.max_insertion = o->max_insertion;
+    if (o && o->max_candidate_paths) P.max_paths = o->max_candidate_paths;
+    if (P.max_paths > ASM_MAX_PATHS_LIMIT) throw std::runtime_error("max_candidate_paths above " + std::to_string(ASM_MAX_PATHS_LIMIT));
+    const DiscoverResult& D = X->discover;
+    const size_t nR = D.regions.size();
+    // every retained read of the sample, over the GPUs of a multi-GPU handle
+    std::unordered_map<uint32_t, std::pair<const drprg_index::RetainedReads*, size_t>> where;
+    for (drprg_index* g : (X->gpus.empty() ? std::vector<drprg_index*>{X} : X->gpus))
+        for (size_t i = 0; i < g->retained_reads.read.size(); ++i) where[g->retained_reads.read[i]] = {&g->retained_reads, i};
+    std::unordered_map<uint32_t, uint32_t> uploaded;  // read -> its words in `words`
+    std::vector<uint32_t> words, list;
+    std::vector<uint4> entries;
+    std::vector<AsmRegion> regs(nR);
+    std::vector<uint32_t> global_list;
+    uint64_t global_slots = 0, out_cap = 0;
+    uint32_t max_walk = DISCOVER_K, smem_slots = 64;
+    for (size_t r = 0; r < nR; ++r) {
+        const CandidateRegion& c = D.regions[r];
+        const std::string& cons = D.consensus[c.locus];
+        AsmRegion& A = regs[r];
+        memset(&A, 0, sizeof A);
+        A.entry_off = (uint32_t)entries.size();
+        uint64_t n_pos = 0;
+        for (uint64_t q = c.read_off; q < c.read_off + c.n_reads; ++q) {
+            const ReadCoordinate& rc = D.reads[q];
+            const auto it = where.find(rc.read);
+            if (it == where.end()) throw std::runtime_error("the bases of read " + std::to_string(rc.read) + " were not retained");
+            const drprg_index::RetainedReads& S = *it->second.first;
+            const size_t i = it->second.second;
+            if (rc.start > rc.end || rc.end > S.len[i]) throw std::runtime_error("region read span outside its read");
+            auto up = uploaded.find(rc.read);
+            if (up == uploaded.end()) {
+                up = uploaded.emplace(rc.read, (uint32_t)words.size()).first;
+                words.insert(words.end(), S.words.begin() + S.off[i], S.words.begin() + S.off[i] + (S.len[i] + 15) / 16);
+                if (words.size() >= 0xffffffffull) throw std::runtime_error("region reads exceed 2^32 words");
+            }
+            entries.push_back(make_uint4(up->second, rc.start, rc.end, rc.fwd));
+            if (rc.end - rc.start >= DISCOVER_K) n_pos += rc.end - rc.start - DISCOVER_K + 1;
+        }
+        if (entries.size() >= 0xffffffffull) throw std::runtime_error("too many region reads");
+        A.n_entries = (uint32_t)(entries.size() - A.entry_off);
+        uint64_t slots = 64;
+        while (slots < 2 * n_pos) slots <<= 1;
+        A.slots = (uint32_t)slots;
+        A.span = c.pad_end - c.pad_start;
+        for (uint32_t i = 0; i < KMER_ATTEMPTS && c.pad_start + i + DISCOVER_K <= c.start; ++i)
+            A.start_kmer[A.n_start++] = consensus_kmer(cons, c.pad_start + i);
+        for (uint32_t j = 0; j < KMER_ATTEMPTS && c.pad_end >= c.end + DISCOVER_K + j; ++j)
+            A.end_kmer[A.n_end++] = consensus_kmer(cons, c.pad_end - DISCOVER_K - j);
+        const uint32_t walk = A.span + P.max_insertion;
+        if (walk > ASM_MAX_WALK) throw std::runtime_error("a candidate region is wider than the assembler takes (" + std::to_string(ASM_MAX_WALK) + " bases with the insertion)");
+        max_walk = std::max(max_walk, walk);
+        out_cap += (uint64_t)P.max_paths * walk;
+        if (slots <= ASM_SMEM_SLOTS) {
+            list.push_back((uint32_t)r);
+            smem_slots = std::max(smem_slots, (uint32_t)slots);
+        } else {
+            A.table_off = global_slots;
+            global_slots += slots;
+            global_list.push_back((uint32_t)r);
+        }
+    }
+    const uint32_t n_smem = (uint32_t)list.size(), n_global = (uint32_t)global_list.size();
+    list.insert(list.end(), global_list.begin(), global_list.end());
+    X->asm_status.assign(nR, 0);
+    X->asm_paths.clear();
+    X->asm_bases.clear();
+    X->asm_stats[0] = n_smem;
+    X->asm_stats[1] = n_global;
+    X->asm_stats[2] = X->asm_stats[3] = 0;
+    if (!nR) return;
+    CK(cudaSetDevice(X->device));
+    Stream st = new_stream();
+    Event ev[3] = {new_event(cudaEventDefault), new_event(cudaEventDefault), new_event(cudaEventDefault)};
+    DBuf<uint32_t> d_words, d_list, d_keys, d_counts, d_wlen;
+    DBuf<uint4> d_entries;
+    DBuf<AsmRegion> d_regs;
+    DBuf<AsmResult> d_res;
+    DBuf<char> d_out;
+    DBuf<unsigned long long> d_cursor;
+    d_words.ensure(std::max<size_t>(1, words.size()));
+    d_entries.ensure(std::max<size_t>(1, entries.size()));
+    d_regs.ensure(nR);
+    d_list.ensure(nR);
+    d_keys.ensure(std::max<uint64_t>(1, global_slots));
+    d_counts.ensure(std::max<uint64_t>(1, global_slots));
+    d_res.ensure(nR);
+    d_wlen.ensure(nR * P.max_paths);
+    d_out.ensure(std::max<uint64_t>(1, out_cap));
+    d_cursor.ensure(1);
+    if (!words.empty()) CK(cudaMemcpyAsync(d_words.p, words.data(), words.size() * 4, cudaMemcpyHostToDevice, st.get()));
+    if (!entries.empty()) CK(cudaMemcpyAsync(d_entries.p, entries.data(), entries.size() * sizeof(uint4), cudaMemcpyHostToDevice, st.get()));
+    CK(cudaMemcpyAsync(d_regs.p, regs.data(), nR * sizeof(AsmRegion), cudaMemcpyHostToDevice, st.get()));
+    CK(cudaMemcpyAsync(d_list.p, list.data(), nR * 4, cudaMemcpyHostToDevice, st.get()));
+    CK(cudaMemsetAsync(d_cursor.p, 0, sizeof(unsigned long long), st.get()));
+    CK(cudaEventRecord(ev[0].get(), st.get()));
+    launch_assemble(d_regs.p, d_list.p, n_smem, d_entries.p, d_words.p, smem_slots, nullptr, nullptr, max_walk, P, d_res.p,
+                    d_wlen.p, d_out.p, d_cursor.p, st.get());
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[1].get(), st.get()));
+    launch_assemble(d_regs.p, d_list.p + n_smem, n_global, d_entries.p, d_words.p, 0, d_keys.p, d_counts.p, max_walk, P, d_res.p,
+                    d_wlen.p, d_out.p, d_cursor.p, st.get());
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[2].get(), st.get()));
+    std::vector<AsmResult> res(nR);
+    std::vector<uint32_t> wlen(nR * P.max_paths);
+    unsigned long long used = 0;
+    CK(cudaMemcpyAsync(res.data(), d_res.p, nR * sizeof(AsmResult), cudaMemcpyDeviceToHost, st.get()));
+    CK(cudaMemcpyAsync(wlen.data(), d_wlen.p, wlen.size() * 4, cudaMemcpyDeviceToHost, st.get()));
+    CK(cudaMemcpyAsync(&used, d_cursor.p, sizeof used, cudaMemcpyDeviceToHost, st.get()));
+    CK(cudaStreamSynchronize(st.get()));
+    std::string out(used, '\0');
+    if (used) CK(cudaMemcpyAsync(&out[0], d_out.p, used, cudaMemcpyDeviceToHost, st.get()));
+    CK(cudaStreamSynchronize(st.get()));
+    float ms[2] = {0, 0};
+    CK(cudaEventElapsedTime(&ms[0], ev[0].get(), ev[1].get()));
+    CK(cudaEventElapsedTime(&ms[1], ev[1].get(), ev[2].get()));
+    X->asm_stats[2] = ms[0];
+    X->asm_stats[3] = ms[1];
+    for (size_t r = 0; r < nR; ++r) {
+        const AsmResult& R = res[r];
+        X->asm_status[r] = (uint8_t)R.status;
+        if (R.status != ASM_ASSEMBLED) continue;
+        const CandidateRegion& c = D.regions[r];
+        const uint32_t a = c.pad_start + R.anchor_i, b = c.pad_end - R.anchor_j;
+        const std::string& cons = D.consensus[c.locus];
+        std::vector<std::string> alleles;
+        uint64_t off = R.byte_off;
+        for (uint32_t w = 0; w < R.n_walks; ++w) {
+            const uint32_t L = wlen[r * P.max_paths + w];
+            if (off + L > used) throw std::runtime_error("assembled walks outside the output buffer");
+            std::string s = out.substr(off, L);
+            off += L;
+            if (s.compare(0, std::string::npos, cons, a, b - a) != 0) alleles.push_back(std::move(s));
+        }
+        std::sort(alleles.begin(), alleles.end());
+        for (const std::string& s : alleles) {
+            X->asm_paths.push_back(drprg_denovo_path{(uint32_t)r, a, b, (uint32_t)s.size(), (uint64_t)X->asm_bases.size()});
+            X->asm_bases += s;
+        }
+    }
+}
+
 int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, const char* outdir, const drprg_map_opts* o,
                drprg_map_stats* stats, const Inflated* pre = nullptr) {
     need_device(X);
@@ -2065,6 +2281,10 @@ int drprg_cuda_discover_candidates(drprg_index* X, const drprg_discover_opts* o,
         hits = &all;
     }
     discover_candidates(X->H, X->present, X->mlpaths, X->h_acc.data(), *hits, D, X->discover);
+    X->discover_ready = true;
+    X->asm_status.clear();
+    X->asm_paths.clear();
+    X->asm_bases.clear();
     if (n_regions) *n_regions = (uint32_t)X->discover.regions.size();
     if (n_region_reads) *n_region_reads = X->discover.reads.size();
     return 0;
@@ -2098,6 +2318,33 @@ const char* drprg_cuda_discover_consensus(drprg_index* X, uint32_t locus, uint64
 int drprg_cuda_discover_coverage(drprg_index* X, uint32_t locus, uint32_t* covg) {
     if (locus >= X->discover.coverage.size()) return 1;
     memcpy(covg, X->discover.coverage[locus].data(), X->discover.coverage[locus].size() * 4);
+    return 0;
+}
+int drprg_cuda_discover_assemble(drprg_index* X, const drprg_assemble_opts* o, uint32_t* n_paths, uint64_t* n_path_bases) {
+    API_BEGIN need_device(X);
+    if (X->world > 1 || X->ipc_mapping)
+        throw std::runtime_error("one-process-per-GPU handles (drprg_cuda_shard_root / drprg_cuda_shard_attach) keep no read bases: "
+                                 "assemble on a single-GPU or drprg_cuda_index_load_multi handle");
+    if (!X->have_gt) throw std::runtime_error("drprg_cuda_genotype has not run for this sample");
+    if (!X->retain_hits) throw std::runtime_error("drprg_cuda_retain_hits(idx, 1) must be set before the sample is mapped");
+    if (!X->discover_ready) throw std::runtime_error("drprg_cuda_discover_candidates has not run for this sample");
+    assemble_regions(X, o);
+    if (n_paths) *n_paths = (uint32_t)X->asm_paths.size();
+    if (n_path_bases) *n_path_bases = X->asm_bases.size();
+    return 0;
+    API_END
+}
+int drprg_cuda_discover_paths(drprg_index* X, drprg_denovo_path* out, char* bases) {
+    if (!X->asm_paths.empty()) memcpy(out, X->asm_paths.data(), X->asm_paths.size() * sizeof(drprg_denovo_path));
+    if (!X->asm_bases.empty()) memcpy(bases, X->asm_bases.data(), X->asm_bases.size());
+    return 0;
+}
+int drprg_cuda_discover_region_status(drprg_index* X, uint8_t* status) {
+    if (!X->asm_status.empty()) memcpy(status, X->asm_status.data(), X->asm_status.size());
+    return 0;
+}
+int drprg_cuda_last_assemble_stats(drprg_index* X, double* out4) {
+    memcpy(out4, X->asm_stats, sizeof X->asm_stats);
     return 0;
 }
 int drprg_cuda_set_minor_af(drprg_index* X, float minor_af) {

@@ -10,7 +10,7 @@
 //   region reads        for every read with kept hits on the locus: its hits whose k-mer lies on the ML path inside the
 //                       padded region; reads with at least two such hits contribute the span [min start, max start + k) and
 //                       the strand of the first hit (get_read_overlap_coordinates / find_hits_inside_path)
-// The de-novo assembly itself (pandora's de Bruijn graph walk) stays where it is; this file only produces its inputs.
+// The de-novo assembly itself (pandora's de Bruijn graph walk) runs on the GPU (assemble.cu); this file produces its inputs.
 // Option names and defaults are upstream pandora's `discover` (drprg passes none of them, src/predict.rs:236-245).
 #include <algorithm>
 #include <stdexcept>

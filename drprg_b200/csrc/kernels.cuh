@@ -190,4 +190,40 @@ void launch_format_g6_batch(const double* d_v, uint32_t n, char* d_out, uint8_t*
 // the likelihood / GT / GT_CONF kernel alone, on per-allele rows already in G.mean_fwd / G.mean_rev / G.gaps
 void launch_genotype_rows(const DevGenotype& G, ModelParams P, cudaStream_t st);
 
+// ---- discover: the bases of retained reads and the local assembler (assemble.cu) ------------------------------------
+// per active read of the last batch (n_active, lists of PostBuffers): a read with at least one kept hit gets its 2-bit words
+// copied to out_words[table[a].x ...] (table[a].y = its length in bases); table[a].x = UINT32_MAX for the other reads.  The
+// words wanted are counted in *d_cursor (zeroed by the caller) even past word_cap: the caller regrows and launches again.
+void launch_retain_gather(const DevReads& R, const uint32_t* act_read, const uint32_t* act_base, const uint32_t* act_count,
+                          const uint8_t* gkept, uint32_t n_active, uint2* table, uint32_t* out_words, uint64_t word_cap,
+                          unsigned long long* d_cursor, cudaStream_t st);
+constexpr uint32_t DISCOVER_K = 11;             // de Bruijn k-mer size: 22-bit k-mers
+constexpr uint32_t KMER_ATTEMPTS = 10;          // anchor k-mers tried per flank
+constexpr uint32_t ASM_MAX_PATHS_LIMIT = 64;    // largest max_candidate_paths the walk's shared-memory store takes
+constexpr uint32_t ASM_SMEM_SLOTS = 16384;      // k-mer table slots one CTA keeps in shared memory (128 KB)
+constexpr uint32_t ASM_MAX_WALK = 1024;         // longest walk (consensus span + max insertion) the kernel takes
+enum : uint32_t { ASM_ASSEMBLED = 0, ASM_NO_ANCHOR = 1, ASM_TOO_MANY_PATHS = 2, ASM_NO_PATH = 3 };
+struct AsmRegion {
+    uint32_t entry_off, n_entries;  // pileup reads: entries[entry_off, + n_entries)
+    uint32_t slots;                 // k-mer table slots, a power of two >= 2 x the pileup's k-mer positions
+    uint32_t span;                  // padded interval length pe - ps
+    unsigned long long table_off;   // global-table launch: first slot of the region's table in the scratch
+    uint32_t n_start, n_end;        // anchor candidates: C[ps + i, + K) and C[pe - K - j, pe - j), UINT32_MAX if not ACGT
+    uint32_t start_kmer[KMER_ATTEMPTS], end_kmer[KMER_ATTEMPTS];
+};
+struct AsmResult {
+    uint32_t status, anchor_i, anchor_j, n_walks;  // n_walks complete walks (the consensus one included) when assembled
+    unsigned long long byte_off;                     // their bases, back to back in out_bases
+};
+struct AsmParams {
+    uint32_t min_dp, max_insertion, max_paths;
+};
+// one CTA per listed region: count the pileup's k-mers (entries: {word offset into words, start, end, fwd}) into an
+// open-addressed table, in shared memory (g_keys == nullptr; every region's slots <= smem_slots) or in the global scratch
+// g_keys / g_counts at the region's table_off; then one warp picks the anchors and enumerates the walks.  Complete walks of
+// an assembled region go to out_bases at an offset taken from *d_cursor, their lengths to walk_len[region * max_paths + w].
+void launch_assemble(const AsmRegion* regions, const uint32_t* list, uint32_t n_list, const uint4* entries, const uint32_t* words,
+                     uint32_t smem_slots, uint32_t* g_keys, uint32_t* g_counts, uint32_t max_walk, AsmParams P,
+                     AsmResult* res, uint32_t* walk_len, char* out_bases, unsigned long long* d_cursor, cudaStream_t st);
+
 }  // namespace drprg

@@ -46,6 +46,18 @@ class CandidateRegion(C.Structure):
                 ("n_reads", C.c_uint32), ("read_off", C.c_uint64)]
 
 
+class AssembleOpts(C.Structure):
+    _fields_ = [("min_dbg_dp", C.c_uint32), ("max_insertion", C.c_uint32), ("max_candidate_paths", C.c_uint32)]
+
+
+class DenovoPath(C.Structure):
+    _fields_ = [("region", C.c_uint32), ("a", C.c_uint32), ("b", C.c_uint32), ("length", C.c_uint32), ("offset", C.c_uint64)]
+
+
+# region status of discover_assemble (DRPRG_DENOVO_* of the header)
+ASSEMBLED, NO_ANCHOR, TOO_MANY_PATHS, NO_PATH = 0, 1, 2, 3
+
+
 class IndexInfo(C.Structure):
     _fields_ = [
         ("w", C.c_uint32), ("k", C.c_uint32), ("n_loci", C.c_uint32), ("total_knodes", C.c_uint32),
@@ -73,7 +85,8 @@ SYMBOLS = [
     "drprg_cuda_index_records", "drprg_cuda_index_min_path_length", "drprg_cuda_sketch_batch", "drprg_cuda_last_hits",
     "drprg_cuda_gt_params", "drprg_cuda_gt_mlpath", "drprg_cuda_gt_counts", "drprg_cuda_gt_records",
     "drprg_cuda_gt_alleles", "drprg_cuda_gt_allele_knodes", "drprg_cuda_genotype_rows", "drprg_cuda_gt_filter_stats", "drprg_cuda_set_minor_af", "drprg_cuda_retain_hits", "drprg_cuda_discover_candidates",
-    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_last_timings", "drprg_cuda_last_genotype_timings", "drprg_cuda_format_g6", "drprg_cuda_format_g6_device", "drprg_cuda_launch_count", "drprg_cuda_hash64", "drprg_cuda_hash64_inverse", "drprg_cuda_issue_peak",
+    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover_paths",
+    "drprg_cuda_discover_region_status", "drprg_cuda_last_assemble_stats", "drprg_cuda_last_timings", "drprg_cuda_last_genotype_timings", "drprg_cuda_format_g6", "drprg_cuda_format_g6_device", "drprg_cuda_launch_count", "drprg_cuda_hash64", "drprg_cuda_hash64_inverse", "drprg_cuda_issue_peak",
 ]
 
 
@@ -451,6 +464,29 @@ class Index:
             regions.append((r.locus, r.start, r.end, r.pad_start, r.pad_end,
                             list(zip(rd[a:b].tolist(), st[a:b].tolist(), en[a:b].tolist(), fw[a:b].tolist()))))
         return loci, regions
+
+    def discover_assemble(self, min_dbg_dp=0, max_insertion=0xFFFFFFFF, max_candidate_paths=0):
+        """after discover_candidates(): the local assembler on the GPU -> (status uint8[n_regions], paths) with paths =
+        [(region, a, b, sequence)]: the de-novo alleles replacing consensus[a:b] of the region's locus, sorted per region"""
+        L = lib()
+        o = AssembleOpts(min_dbg_dp, max_insertion, max_candidate_paths)
+        n, nb = C.c_uint32(), C.c_uint64()
+        _check(L.drprg_cuda_discover_assemble(self.h, C.byref(o), C.byref(n), C.byref(nb)), "drprg_cuda_discover_assemble")
+        out = (DenovoPath * max(1, n.value))()
+        bases = C.create_string_buffer(max(1, nb.value))
+        _check(L.drprg_cuda_discover_paths(self.h, out, bases), "drprg_cuda_discover_paths")
+        st = self.last_assemble_stats()
+        status = np.zeros(st["regions_shared"] + st["regions_global"], np.uint8)
+        _check(L.drprg_cuda_discover_region_status(self.h, _p(status)), "drprg_cuda_discover_region_status")
+        raw = bases.raw
+        paths = [(p.region, p.a, p.b, raw[p.offset:p.offset + p.length].decode()) for p in out[:n.value]]
+        return status, paths
+
+    def last_assemble_stats(self):
+        """regions counted in a shared-memory table / in a global one, and the device ms of the two kernel launches"""
+        o = np.zeros(4, np.float64)
+        lib().drprg_cuda_last_assemble_stats(self.h, _p(o))
+        return dict(regions_shared=int(o[0]), regions_global=int(o[1]), ms_shared=float(o[2]), ms_global=float(o[3]))
 
     def set_minor_af(self, maf):
         lib().drprg_cuda_set_minor_af(self.h, C.c_float(maf))

@@ -1,7 +1,8 @@
 """Host-side mirror of the reference's adapter for this path: `Pandora::genotype_with`
 (/root/reference/src/lib.rs:580-642), `Pandora::vcf_filename` (:644-646) and `Pandora::index_with` (:479-510), same
 names, argument meaning and error behaviour, but backed by the CUDA library instead of a pandora subprocess.
-`discover_candidates` is the mapping front half of `Pandora::discover_with` (:513-578) taken from the map pass.
+`discover_candidates` is the mapping front half of `Pandora::discover_with` (:513-578) taken from the map pass, and
+`discover_paths` its local assembly, on the GPU.
 
 The reference builds the argv  -t T -w W -k K -c C [-I] [-K]  (src/predict.rs:288-294) after the fixed
 `map --genotype --local --gt-conf 0 -v -o OUT -g 4411532 --max-covg 4294967295 --vcf-refs REF`
@@ -115,3 +116,20 @@ class Pandora:
             return self._index.discover_candidates(**opts)
         except lib.DrprgCudaError as e:
             raise DependencyError(str(e)) from e
+
+    def discover_paths(self, **opts):
+        """After genotype_with(..., retain_hits=True): pandora discover's de-novo alleles from the same pass, with pandora's
+        defaults for the candidate regions -> {locus name: [(a, b, sequence), ...]}, each replacing [a, b) of the locus's
+        maximum-likelihood sequence; opts go to lib.Index.discover_assemble."""
+        if self._index is None:
+            raise DependencyError("genotype_with(..., retain_hits=True) has not been run")
+        try:
+            ix = self._index
+            _, regions = ix.discover_candidates()
+            _, paths = ix.discover_assemble(**opts)
+        except lib.DrprgCudaError as e:
+            raise DependencyError(str(e)) from e
+        out = {}
+        for r, a, b, seq in paths:
+            out.setdefault(ix.names[regions[r][0]], []).append((a, b, seq))
+        return out

@@ -206,6 +206,35 @@ def sample_haplotype(panel, seed, alt_frac=0.10):
     return out
 
 
+def insert_novel_variants(panel, hap, kinds, seed=0):
+    """Variants the PRG does not know, in the sample's locus sequences: kinds[i] in ("snp", "del3", "ins6") goes into locus i,
+    in the middle of its longest stretch between sites.  hap = sample_haplotype(panel, ...).  Returns (sequences,
+    [(locus, offset, ref_len, alt, sequence without the variant)])."""
+    rng = np.random.default_rng(seed)
+
+    def spell(parts, it):  # replays the site choices of sample_haplotype, depth first like Locus.spell
+        out = bytearray()
+        for q in parts:
+            out += q if isinstance(q, (bytes, bytearray)) else spell(q.alleles[next(it)], it)
+        return bytes(out)
+
+    seqs, variants = [h[0] for h in hap], []
+    for li, kind in enumerate(kinds):
+        L = panel.loci[li]
+        i = max((j for j, q in enumerate(L.parts) if isinstance(q, (bytes, bytearray))), key=lambda j: len(L.parts[j]))
+        v = len(spell(L.parts[:i], iter(hap[li][1]))) + len(L.parts[i]) // 2
+        old = seqs[li]
+        if kind == "snp":
+            ref_len, alt = 1, BASES[(int(_CODE[old[v]]) + int(rng.integers(1, 4))) % 4:][:1].tobytes()
+        elif kind == "del3":
+            ref_len, alt = 3, b""
+        else:
+            ref_len, alt = 0, random_dna(rng, 6).tobytes()
+        seqs[li] = old[:v] + alt + old[v + ref_len:]
+        variants.append((li, v, ref_len, alt.decode(), old.decode()))
+    return seqs, variants
+
+
 def make_genome(panel, hap_seqs, size=4_411_532, seed=1, gc=0.65, min_sep=5000):
     """Random genome with the sample's locus sequences embedded (random strand, >= min_sep apart)."""
     rng = np.random.default_rng(seed)

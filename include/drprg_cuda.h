@@ -168,6 +168,37 @@ int drprg_cuda_discover_region_reads(drprg_index*, uint32_t* read, uint32_t* sta
 const char* drprg_cuda_discover_consensus(drprg_index*, uint32_t locus, uint64_t* len); /* NULL: locus absent from the sample */
 int drprg_cuda_discover_coverage(drprg_index*, uint32_t locus, uint32_t* covg /* consensus length */);
 
+/* The second half of `pandora discover`: local assembly of every candidate region into de-novo alleles, on the GPU, from the
+ * bases of the reads the map pass retained (hit retention keeps the 2-bit words of every read with a kept hit).  Call after
+ * drprg_cuda_discover_candidates; refused without retention, before genotyping, and on one-process-per-GPU handles
+ * (drprg_cuda_shard_root / _attach).  Per region (padded interval [ps, pe), core [s, e) on the ML sequence C): the
+ * region reads' spans, reverse-complemented where fwd = 0, give the oriented 11-mers of a de Bruijn graph whose k-mers seen
+ * at least min_dbg_dp times are solid; the anchors are the first solid pair (i, j), i outer, of C[ps+i, +11) inside the
+ * left flank and C[pe-11-j, pe-j) inside the right flank, up to 10 each; every walk through solid k-mers from the start to
+ * the end anchor (A, C, G, T order, cycles allowed, at most (pe-j) - (ps+i) + max_insertion bases) is enumerated, and more
+ * than max_candidate_paths walks abandon the region.  The walks other than C[ps+i, pe-j) are the region's de-novo alleles,
+ * sorted.  Fields left 0 take pandora's defaults (2, 25); max_insertion 0xffffffff = default 15; max_candidate_paths <= 64. */
+typedef struct {
+    uint32_t min_dbg_dp, max_insertion, max_candidate_paths;
+} drprg_assemble_opts;
+typedef struct {
+    uint32_t region;  /* index into drprg_cuda_discover_regions */
+    uint32_t a, b;    /* the consensus interval [a, b) the allele replaces */
+    uint32_t length;  /* bases at `offset` in the bases buffer of drprg_cuda_discover_paths */
+    uint64_t offset;
+} drprg_denovo_path;
+#define DRPRG_DENOVO_ASSEMBLED 0      /* walks found; none besides the consensus = the reads agree with it */
+#define DRPRG_DENOVO_NO_ANCHOR 1      /* no solid anchor pair */
+#define DRPRG_DENOVO_TOO_MANY_PATHS 2 /* more than max_candidate_paths walks: abandoned */
+#define DRPRG_DENOVO_NO_PATH 3        /* anchors, but no walk between them */
+int drprg_cuda_discover_assemble(drprg_index*, const drprg_assemble_opts* /* NULL = defaults */, uint32_t* n_paths,
+                                 uint64_t* n_path_bases);
+int drprg_cuda_discover_paths(drprg_index*, drprg_denovo_path* out /* n_paths */, char* bases /* n_path_bases */);
+int drprg_cuda_discover_region_status(drprg_index*, uint8_t* status /* n_regions, DRPRG_DENOVO_* */);
+/* the last assembly's shape: regions counted in a shared-memory k-mer table, regions whose pileup needed a table in global
+ * memory, and the device time in ms of the two kernel launches (CUDA events) — 4 doubles */
+int drprg_cuda_last_assemble_stats(drprg_index*, double* out4);
+
 /* ---- introspection / parity hooks (same .so, used by tests and bench) --------------------------- */
 /* pandora's hash64 on a 2k-bit k-mer and its inverse (the k-mer screen is built from the inverse): host functions */
 uint64_t drprg_cuda_hash64(uint64_t kmer, uint32_t k);
