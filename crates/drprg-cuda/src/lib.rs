@@ -68,6 +68,27 @@ pub struct CandidateRegion {
     pub read_off: u64,
 }
 
+/// What one `discover` call did (`drprg_discover_stats`): region statuses are `DRPRG_DENOVO_*` counts, times are wall ms.
+#[repr(C)]
+#[derive(Debug, Default, Clone, Copy)]
+pub struct DiscoverStats {
+    pub n_reads: u64,
+    pub n_hits_kept: u64,
+    pub n_region_reads: u64,
+    pub n_regions: u32,
+    pub n_assembled: u32,
+    pub n_no_anchor: u32,
+    pub n_too_many_paths: u32,
+    pub n_no_path: u32,
+    pub n_loci_with_variants: u32,
+    pub n_variants: u32,
+    pub ms_ingest: f64,
+    pub ms_map: f64,
+    pub ms_ml_path: f64,
+    pub ms_discover: f64,
+    pub ms_total: f64,
+}
+
 /// Options of the local assembler (`drprg_assemble_opts`); 0 = pandora's default (min DBG depth 2, 25 candidate paths),
 /// max_insertion u32::MAX = 15.  max_candidate_paths is at most 64.
 #[repr(C)]
@@ -161,6 +182,16 @@ extern "C" {
         opts: *const AssembleOpts,
         n_paths: *mut u32,
         n_path_bases: *mut u64,
+    ) -> c_int;
+    fn drprg_cuda_discover(
+        idx: *mut RawIndex,
+        sample: *const c_char,
+        reads_path: *const c_char,
+        outdir: *const c_char,
+        map_opts: *const MapOpts,
+        discover_opts: *const DiscoverOpts,
+        assemble_opts: *const AssembleOpts,
+        stats: *mut DiscoverStats,
     ) -> c_int;
     fn drprg_cuda_discover_paths(idx: *mut RawIndex, out: *mut DenovoPath, bases: *mut c_char) -> c_int;
     fn drprg_cuda_discover_region_status(idx: *mut RawIndex, status: *mut u8) -> c_int;
@@ -321,6 +352,21 @@ impl Index {
             })
             .collect();
         Ok((status, alleles))
+    }
+
+    /// Drop-in for `Pandora::discover_with` (drprg src/lib.rs:513-578) for one sample: maps `reads` (hit retention on for
+    /// this call only), assembles the candidate regions on the GPU and writes `<outdir>/denovo_paths.txt`.  Blocking.
+    pub fn discover(&mut self, sample: &str, reads: &Path, outdir: &Path, opts: &MapOpts) -> Result<DiscoverStats, CudaError> {
+        let s = CString::new(sample).map_err(|_| CudaError::ProcessError("sample name contains a NUL byte".into()))?;
+        let (r, o) = (cpath(reads)?, cpath(outdir)?);
+        let mut stats = DiscoverStats::default();
+        let rc = unsafe {
+            drprg_cuda_discover(self.raw, s.as_ptr(), r.as_ptr(), o.as_ptr(), opts, std::ptr::null(), std::ptr::null(), &mut stats)
+        };
+        if rc != 0 {
+            return Err(CudaError::ProcessError(last_error()));
+        }
+        Ok(stats)
     }
 
     /// The maximum-likelihood sequence of a locus in this sample (`None`: the locus is absent).

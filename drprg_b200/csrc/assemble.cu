@@ -2,8 +2,11 @@
 // the local assembly of the reads over each candidate region into de-novo alleles.  discover.cpp finds the regions and
 // their reads from the map pass; the semantics restated here are tests/denovo_oracle.py's (assemble_region), which pins
 // every choice that upstream's GATB-based assembler leaves unpinned.
-//   retain_gather_kernel  at the end of a mapped batch (hit retention on): one warp per active read copies the 2-bit words
-//                         of every read with a kept hit into one buffer, so the bases outlive the batch
+//   retain_gather_kernel  at the end of a mapped batch (hit retention on): one warp per active read appends the kept hits
+//                         of every read that has one to the GPU's retained-hit store (slice order, one cursor atomic per
+//                         read) and copies the read's 2-bit words into one buffer, so the bases outlive the batch
+//   region_reads_kernel   one warp per retained read: its hits inside each padded candidate region of their locus give
+//                         the read's span and strand over the region (discover.cpp's host half finds the regions)
 //   assemble_kernel       one CTA per region.  Counting: the warps take the pileup reads in turn, their lanes stride over
 //                         the k-mer positions, read each 22-bit k-mer with a funnel shift of two words (reverse complement
 //                         for reads on the reverse strand) and count it in an open-addressed table (atomicCAS on the key,
@@ -25,27 +28,105 @@ constexpr uint32_t KMASK = (1u << (2 * DISCOVER_K)) - 1u;
 __global__ void __launch_bounds__(256) retain_gather_kernel(DevReads R, const uint32_t* __restrict__ act_read,
                                                             const uint32_t* __restrict__ act_base,
                                                             const uint32_t* __restrict__ act_count,
+                                                            const unsigned long long* __restrict__ gkey,
                                                             const uint8_t* __restrict__ gkept, uint32_t n_active,
-                                                            uint2* __restrict__ table, uint32_t* __restrict__ out_words,
-                                                            uint64_t word_cap, unsigned long long* __restrict__ cursor) {
+                                                            RetainStore S, uint64_t row_base, uint4* __restrict__ table,
+                                                            uint32_t* __restrict__ out_words, uint64_t word_cap,
+                                                            unsigned long long* __restrict__ cursor) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t a = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; a < n_active; a += warps) {
         const uint32_t b = act_base[a], n = act_count[a];
-        bool any = false;
-        for (uint32_t j = lane; j < n && !any; j += 32) any = gkept[b + j] != 0;
-        const bool keep = __any_sync(FULL, any);
-        const uint32_t r = act_read[a];
-        const uint32_t len = keep ? R.lens[r] : 0u;
+        uint32_t n_kept = 0;
+        for (uint32_t j0 = 0; j0 < n; j0 += 32) n_kept += __popc(__ballot_sync(FULL, j0 + lane < n && gkept[b + j0 + lane]));
+        if (n_kept == 0) continue;
+        const uint32_t r = act_read[a], read = R.read_id_base + r;
+        const uint32_t len = R.lens[r];
         const uint32_t nw = (len + 15) / 16;
-        unsigned long long off = 0;
-        if (lane == 0 && keep) off = atomicAdd(cursor, (unsigned long long)nw);
-        off = __shfl_sync(FULL, off, 0);
-        const bool fits = keep && off + nw <= word_cap;
-        if (lane == 0) table[a] = make_uint2(fits ? (uint32_t)off : 0xffffffffu, len);
-        if (!fits) continue;
+        // lanes 0-2 take the read's three cursor slots side by side: its words, its hits, its row
+        unsigned long long got = 0;
+        if (lane < RT_COUNT) got = atomicAdd(cursor + lane, lane == RT_WORDS ? (unsigned long long)nw : lane == RT_HITS ? n_kept : 1ull);
+        const unsigned long long woff = __shfl_sync(FULL, got, RT_WORDS), hoff = __shfl_sync(FULL, got, RT_HITS),
+                                 row = __shfl_sync(FULL, got, RT_ROWS);
+        const bool words_fit = woff + nw <= word_cap;
+        if (lane == 0) table[row - row_base] = make_uint4(words_fit ? (uint32_t)woff : 0xffffffffu, len, read, 0u);
+        if (lane == 0 && row < S.row_cap) S.rows[row] = make_uint2((uint32_t)hoff, n_kept);
+        if (hoff + n_kept <= S.hit_cap) {  // slice order: a kept hit's place is the kept hits before it
+            uint32_t before = 0;
+            for (uint32_t j0 = 0; j0 < n; j0 += 32) {
+                const bool kept = j0 + lane < n && gkept[b + j0 + lane];
+                const uint32_t m = __ballot_sync(FULL, kept);
+                if (kept) {
+                    const uint64_t q = hoff + before + __popc(m & ((1u << lane) - 1u));
+                    S.hit_read[q] = read;
+                    S.hit_key[q] = gkey[b + j0 + lane];
+                }
+                before += __popc(m);
+            }
+        }
+        if (!words_fit) continue;
         const uint32_t* src = R.stride_words ? R.words + (uint64_t)r * R.stride_words : R.words + R.word_off[r];
-        for (uint32_t w = lane; w < nw; w += 32) out_words[off + w] = src[w];
+        for (uint32_t w = lane; w < nw; w += 32) out_words[woff + w] = src[w];
+    }
+}
+
+__global__ void __launch_bounds__(256) region_reads_kernel(RetainStore S, uint32_t n_rows, const uint32_t* __restrict__ knode_base,
+                                                           const uint32_t* __restrict__ cons_start,
+                                                           const uint32_t* __restrict__ locus_region_off, uint32_t n_loci,
+                                                           const uint2* __restrict__ pad, uint32_t k, uint32_t min_hits,
+                                                           RegionRead* __restrict__ out, uint64_t out_cap,
+                                                           unsigned long long* __restrict__ cursor) {
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    for (uint32_t row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < n_rows; row += warps) {
+        const uint2 rw = S.rows[row];
+        const unsigned long long* key = S.hit_key + rw.x;
+        const uint32_t n = rw.y, read = S.hit_read[rw.x];
+        for (uint32_t i = 0; i < n;) {
+            // a (read, locus) group: the hits are sorted by locus within a read
+            const uint32_t l = (uint32_t)(key[i] >> 48);
+            uint32_t j = i;
+            for (;; j += 32) {
+                const uint32_t m = __ballot_sync(FULL, j + lane >= n || (uint32_t)(key[j + lane] >> 48) != l);
+                if (m) {
+                    j += __ffs(m) - 1;
+                    break;
+                }
+            }
+            const uint32_t r0 = l < n_loci ? locus_region_off[l] : 0u, r1 = l < n_loci ? locus_region_off[l + 1] : 0u;
+            for (uint32_t rg = r0; rg < r1; ++rg) {
+                const uint2 P = pad[rg];
+                uint32_t cnt = 0, lo = 0xffffffffu, hi = 0, fwd = 2;
+                for (uint32_t c = i; c < j; c += 32) {
+                    bool in = false;
+                    uint32_t st = 0, f = 0;
+                    if (c + lane < j) {
+                        const unsigned long long x = key[c + lane];
+                        const uint32_t cs = cons_start[knode_base[l] + ((uint32_t)x & ((1u << GKEY_KNODE_BITS) - 1u))];
+                        in = cs != 0xffffffffu && cs >= P.x && cs + k <= P.y;
+                        st = (uint32_t)(x >> GKEY_KNODE_BITS) & ((1u << GKEY_START_BITS) - 1u);
+                        f = (uint32_t)((x >> 47) & 1ull) ^ 1u;
+                    }
+                    const uint32_t m = __ballot_sync(FULL, in);
+                    if (m && fwd == 2) fwd = __shfl_sync(FULL, f, __ffs(m) - 1);
+                    cnt += __popc(m);
+                    if (in) {
+                        lo = min(lo, st);
+                        hi = max(hi, st + k);
+                    }
+                }
+                if (cnt < min_hits) continue;
+                for (int o = 16; o; o >>= 1) {
+                    lo = min(lo, __shfl_xor_sync(FULL, lo, o));
+                    hi = max(hi, __shfl_xor_sync(FULL, hi, o));
+                }
+                if (lane == 0) {
+                    const unsigned long long q = atomicAdd(cursor, 1ull);
+                    if (q < out_cap) out[q] = RegionRead{rg, read, lo, hi, fwd};
+                }
+            }
+            i = j;
+        }
     }
 }
 
@@ -204,11 +285,23 @@ __global__ void __launch_bounds__(128) assemble_kernel(const AsmRegion* __restri
 }  // namespace
 
 void launch_retain_gather(const DevReads& R, const uint32_t* act_read, const uint32_t* act_base, const uint32_t* act_count,
-                          const uint8_t* gkept, uint32_t n_active, uint2* table, uint32_t* out_words, uint64_t word_cap,
-                          unsigned long long* d_cursor, cudaStream_t st) {
+                          const unsigned long long* gkey, const uint8_t* gkept, uint32_t n_active, RetainStore S,
+                          uint64_t row_base, uint4* table, uint32_t* out_words, uint64_t word_cap, unsigned long long* d_cursor,
+                          cudaStream_t st) {
     if (!n_active) return;
     const uint32_t blocks = (uint32_t)std::min<uint64_t>(4096, ((uint64_t)n_active + 7) / 8);
-    retain_gather_kernel<<<blocks, 256, 0, st>>>(R, act_read, act_base, act_count, gkept, n_active, table, out_words, word_cap, d_cursor);
+    retain_gather_kernel<<<blocks, 256, 0, st>>>(R, act_read, act_base, act_count, gkey, gkept, n_active, S, row_base, table,
+                                                 out_words, word_cap, d_cursor);
+    ++g_launches;
+}
+
+void launch_region_reads(RetainStore S, uint32_t n_rows, const uint32_t* knode_base, const uint32_t* cons_start,
+                         const uint32_t* locus_region_off, uint32_t n_loci, const uint2* pad, uint32_t k, uint32_t min_hits,
+                         RegionRead* out, uint64_t out_cap, unsigned long long* d_cursor, cudaStream_t st) {
+    if (!n_rows) return;
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>(4096, ((uint64_t)n_rows + 7) / 8);
+    region_reads_kernel<<<blocks, 256, 0, st>>>(S, n_rows, knode_base, cons_start, locus_region_off, n_loci, pad, k, min_hits,
+                                                out, out_cap, d_cursor);
     ++g_launches;
 }
 

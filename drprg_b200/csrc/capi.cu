@@ -7,6 +7,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <chrono>
 #include <condition_variable>
 #include <functional>
@@ -198,16 +199,22 @@ struct drprg_index {
     float minor_af = -1.0f;  // < 0: drprg's default (1.0, or 0.1 with --illumina)
     // discover's front half from the map pass (SURVEY 8f rank 1): kept hits of the sample, retained on request
     bool retain_hits = false;
-    std::vector<RetainedHit> retained;
+    DBuf<uint32_t> d_rt_hit_read;        // the RetainStore of this GPU, filled to rt_hits hits and rt_rows rows
+    DBuf<unsigned long long> d_rt_hit_key;
+    DBuf<uint2> d_rt_rows;
+    uint64_t rt_hits = 0, rt_rows = 0;
     // ... and the 2-bit words of every read with a kept hit (per global read id: word offset and length in bases)
     struct RetainedReads {
         std::vector<uint32_t> read, len;
         std::vector<uint64_t> off;
         std::vector<uint32_t> words;
     } retained_reads;
-    DBuf<uint2> d_rt_table;
+    DBuf<uint4> d_rt_table;
     DBuf<uint32_t> d_rt_words;
-    DBuf<unsigned long long> d_rt_cursor;
+    DBuf<unsigned long long> d_rt_cursor;  // RT_COUNT: the hit and row cursors carry over from batch to batch
+    PinnedBuf<uint4> h_rt_table;
+    PinnedBuf<uint32_t> h_rt_words;
+    PinnedBuf<unsigned long long> h_rt_cursor;
     DiscoverResult discover;
     bool discover_ready = false;  // drprg_cuda_discover_candidates ran for the current sample
     // the local assembler's results (drprg_cuda_discover_assemble)
@@ -497,7 +504,7 @@ void sample_begin(drprg_index* X, const drprg_map_opts* o, uint32_t first_read_l
         launch_flag_publish(reinterpret_cast<uint32_t*>(X->d_accum.p + accum_flag_offset(X->n_accum)), X->epoch, 0);
     X->total_bases = X->n_reads = 0;
     X->own_bases = X->own_reads = 0;
-    X->retained.clear();
+    X->rt_hits = X->rt_rows = 0;
     X->retained_reads = drprg_index::RetainedReads();
     X->discover_ready = false;
     X->scalars_in_buffer = false;
@@ -528,38 +535,70 @@ void ensure_read_capacity(drprg_index* X, uint64_t n_reads) {
     CK(cudaMemset(X->read_count.p, 0, X->read_count.cap * sizeof(int32_t)));  // the kernels leave it zero after every batch
 }
 
-// The words of the batch's reads that kept a hit, into the sample's host-side store: the assembler needs their bases after
-// the batch (a file's wave) is gone.  ar = the active reads of the batch (act_read, downloaded).
-void retain_read_bases(drprg_index* X, drprg_batch* B, cudaStream_t st, const std::vector<uint32_t>& ar) {
-    const uint64_t na = ar.size();
+RetainStore retain_store(drprg_index* X) {
+    return RetainStore{X->d_rt_hit_read.p, X->d_rt_hit_key.p, std::min(X->d_rt_hit_read.cap, X->d_rt_hit_key.cap), X->d_rt_rows.p,
+                       X->d_rt_rows.cap};
+}
+
+// grow-only like DBuf::ensure, but the first `used` elements survive the move to the larger buffer
+template <class T>
+void grow_keep(DBuf<T>& b, size_t used, size_t need, cudaStream_t st) {
+    if (need <= b.cap) return;
+    DBuf<T> g;
+    g.ensure(need);
+    if (used) CK(cudaMemcpyAsync(g.p, b.p, used * sizeof(T), cudaMemcpyDeviceToDevice, st));
+    CK(cudaStreamSynchronize(st));
+    b = std::move(g);
+}
+
+// The kept hits of the batch into the GPU's retained-hit store, and the words of the reads that kept a hit into the
+// sample's host-side store: the assembler needs their bases after the batch (a file's wave) is gone.  What a store lacked
+// is counted past its capacity: it regrows, keeping what earlier batches appended, and the append is redone.
+void retain_batch(drprg_index* X, drprg_batch* B, cudaStream_t st) {
+    const uint64_t na = X->last_n_active;
     if (!na) return;
     X->d_rt_table.ensure(na);
-    X->d_rt_cursor.ensure(1);
+    X->d_rt_cursor.ensure(RT_COUNT);
     if (!X->d_rt_words.cap) X->d_rt_words.ensure(na * 16);
-    unsigned long long used = 0;
-    for (;;) {  // the words wanted are counted past the capacity: regrow once to the exact need
-        CK(cudaMemsetAsync(X->d_rt_cursor.p, 0, sizeof(unsigned long long), st));
-        launch_retain_gather(B->R, X->act_read.p, X->act_base.p, X->act_count.p, X->gkept.p, (uint32_t)na, X->d_rt_table.p,
-                             X->d_rt_words.p, X->d_rt_words.cap, X->d_rt_cursor.p, st);
+    grow_keep(X->d_rt_rows, X->rt_rows, X->rt_rows + na, st);  // at most one row per active read: never short
+    grow_keep(X->d_rt_hit_read, X->rt_hits, X->rt_hits + na, st);  // first guess: one kept hit per active read
+    grow_keep(X->d_rt_hit_key, X->rt_hits, X->rt_hits + na, st);
+    // a new sample starts its store empty; later batches only restart the per-batch words cursor
+    CK(cudaMemsetAsync(X->d_rt_cursor.p, 0, (X->rt_hits || X->rt_rows ? 1 : RT_COUNT) * sizeof(unsigned long long), st));
+    X->h_rt_cursor.resize(RT_COUNT);
+    const unsigned long long* c = X->h_rt_cursor.data();
+    for (;;) {
+        const RetainStore S = retain_store(X);
+        launch_retain_gather(B->R, X->act_read.p, X->act_base.p, X->act_count.p, X->gkey.p, X->gkept.p, (uint32_t)na, S, X->rt_rows,
+                             X->d_rt_table.p, X->d_rt_words.p, X->d_rt_words.cap, X->d_rt_cursor.p, st);
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(&used, X->d_rt_cursor.p, sizeof used, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(X->h_rt_cursor.data(), X->d_rt_cursor.p, RT_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        if (used <= X->d_rt_words.cap) break;
-        if (used >= 0xffffffffull) throw std::runtime_error("the reads of one batch that kept a hit exceed 2^32 words: split the batch");
-        X->d_rt_words.ensure(used);
+        if (c[RT_WORDS] <= X->d_rt_words.cap && c[RT_HITS] <= S.hit_cap && c[RT_ROWS] <= S.row_cap) break;
+        if (c[RT_WORDS] >= 0xffffffffull) throw std::runtime_error("the reads of one batch that kept a hit exceed 2^32 words: split the batch");
+        if (c[RT_HITS] >= 0xffffffffull) throw std::runtime_error("the kept hits of one sample exceed 2^32 on one GPU");
+        X->d_rt_words.ensure(c[RT_WORDS]);
+        grow_keep(X->d_rt_hit_read, X->rt_hits, c[RT_HITS], st);
+        grow_keep(X->d_rt_hit_key, X->rt_hits, c[RT_HITS], st);
+        grow_keep(X->d_rt_rows, X->rt_rows, c[RT_ROWS], st);
+        const unsigned long long again[RT_COUNT] = {0, X->rt_hits, X->rt_rows};  // the batch's append is redone
+        CK(cudaMemcpyAsync(X->d_rt_cursor.p, again, sizeof again, cudaMemcpyHostToDevice, st));
     }
-    std::vector<uint2> table(na);
-    drprg_index::RetainedReads& S = X->retained_reads;
-    const uint64_t base = S.words.size();
-    S.words.resize(base + used);
-    CK(cudaMemcpyAsync(table.data(), X->d_rt_table.p, na * sizeof(uint2), cudaMemcpyDeviceToHost, st));
-    if (used) CK(cudaMemcpyAsync(S.words.data() + base, X->d_rt_words.p, used * 4, cudaMemcpyDeviceToHost, st));
+    const uint64_t n_rows = c[RT_ROWS] - X->rt_rows, used = c[RT_WORDS];
+    X->rt_hits = c[RT_HITS];
+    X->rt_rows = c[RT_ROWS];
+    X->h_rt_table.resize(n_rows);
+    X->h_rt_words.resize(used);
+    if (n_rows) CK(cudaMemcpyAsync(X->h_rt_table.data(), X->d_rt_table.p, n_rows * sizeof(uint4), cudaMemcpyDeviceToHost, st));
+    if (used) CK(cudaMemcpyAsync(X->h_rt_words.data(), X->d_rt_words.p, used * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    for (uint64_t a = 0; a < na; ++a) {
-        if (table[a].x == 0xffffffffu) continue;
-        S.read.push_back(B->R.read_id_base + ar[a]);
-        S.off.push_back(base + table[a].x);
-        S.len.push_back(table[a].y);
+    drprg_index::RetainedReads& R = X->retained_reads;
+    const uint64_t base = R.words.size();
+    R.words.insert(R.words.end(), X->h_rt_words.begin(), X->h_rt_words.end());
+    for (const uint4& t : X->h_rt_table) {
+        R.read.push_back(t.z);
+        R.off.push_back(base + t.x);
+        R.len.push_back(t.y);
     }
 }
 
@@ -658,26 +697,7 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     X->n_reads += B->R.n_reads;
     X->own_bases += B->total_bases;
     X->own_reads += B->R.n_reads;
-    if (X->retain_hits && nh) {  // the kept hits of this batch, grouped by read, pandora order within a read
-        const uint64_t na = X->last_n_active;
-        std::vector<unsigned long long> key(nh);
-        std::vector<uint8_t> kp(nh);
-        std::vector<uint32_t> ar(na), ab(na), ac(na);
-        CK(cudaMemcpy(key.data(), X->gkey.p, nh * 8, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(kp.data(), X->gkept.p, nh, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(ar.data(), X->act_read.p, na * 4, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(ab.data(), X->act_base.p, na * 4, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(ac.data(), X->act_count.p, na * 4, cudaMemcpyDeviceToHost));
-        for (uint64_t a = 0; a < na; ++a)
-            for (uint32_t j = ab[a]; j < ab[a] + ac[a]; ++j) {
-                if (!kp[j]) continue;  // kept hits sit in slices the cluster kernels sorted
-                const unsigned long long k = key[j];
-                X->retained.push_back(RetainedHit{B->R.read_id_base + ar[a], (uint32_t)(k >> GKEY_KNODE_BITS) & ((1u << GKEY_START_BITS) - 1u),
-                                                  (uint32_t)k & ((1u << GKEY_KNODE_BITS) - 1u), (uint16_t)(k >> 48),
-                                                  (uint8_t)(((k >> 47) & 1ull) ^ 1ull)});
-            }
-        retain_read_bases(X, B, st, ar);
-    }
+    if (X->retain_hits && nh) retain_batch(X, B, st);
     if (n_hits) *n_hits = nh;
     if (n_kept) *n_kept = X->h_counters.p[CTR_KEPT];
 }
@@ -1479,6 +1499,76 @@ bool map_file_in_waves(drprg_index* X, const char* reads_path, const drprg_map_o
     return W.waves > 0;
 }
 
+// discover's candidate regions and the reads over them: the per-locus half on the host (discover.cpp), the reads on every
+// GPU from its retained-hit store (region_reads_kernel), sorted by (region, read) here
+void find_candidates(drprg_index* X, const DiscoverOpts& o) {
+    std::vector<uint32_t> cons_start;
+    discover_regions(X->H, X->present, X->mlpaths, X->h_acc.data(), o, X->discover, cons_start);
+    DiscoverResult& D = X->discover;
+    X->discover_ready = true;
+    X->asm_status.clear();
+    X->asm_paths.clear();
+    X->asm_bases.clear();
+    const size_t nR = D.regions.size();
+    if (nR >= 0xffffffffull) throw std::runtime_error("more than 2^32 candidate regions");
+    const uint32_t P = (uint32_t)X->H.loci.size();
+    std::vector<uint32_t> region_off(P + 1, 0);
+    std::vector<uint2> pad(nR);
+    for (size_t r = 0; r < nR; ++r) {
+        ++region_off[D.regions[r].locus + 1];
+        pad[r] = make_uint2(D.regions[r].pad_start, D.regions[r].pad_end);
+    }
+    for (uint32_t l = 0; l < P; ++l) region_off[l + 1] += region_off[l];
+    const std::vector<drprg_index*> gpus = X->gpus.empty() ? std::vector<drprg_index*>{X} : X->gpus;
+    std::vector<std::vector<RegionRead>> found(gpus.size());
+    auto run = [&](size_t g, drprg_index* G) {
+        if (!nR || !G->rt_rows) return;
+        Stream st = new_stream();
+        DBuf<uint32_t> d_cons_start, d_region_off;
+        DBuf<uint2> d_pad;
+        DBuf<RegionRead> d_out;
+        DBuf<unsigned long long> d_cursor;
+        d_cons_start.assign(cons_start);
+        d_region_off.assign(region_off);
+        d_pad.assign(pad);
+        d_cursor.ensure(1);
+        d_out.ensure(std::max<uint64_t>(1024, G->rt_rows / 8));
+        unsigned long long n = 0;
+        for (;;) {  // the entries wanted are counted past the capacity: regrow once to the exact need
+            CK(cudaMemsetAsync(d_cursor.p, 0, sizeof(unsigned long long), st.get()));
+            launch_region_reads(retain_store(G), (uint32_t)G->rt_rows, G->d_knode_base.p, d_cons_start.p, d_region_off.p, P, d_pad.p,
+                                G->H.k, o.min_hits, d_out.p, d_out.cap, d_cursor.p, st.get());
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(&n, d_cursor.p, sizeof n, cudaMemcpyDeviceToHost, st.get()));
+            CK(cudaStreamSynchronize(st.get()));
+            if (n <= d_out.cap) break;
+            d_out.ensure(n);
+        }
+        found[g].resize(n);
+        if (n) CK(cudaMemcpyAsync(found[g].data(), d_out.p, n * sizeof(RegionRead), cudaMemcpyDeviceToHost, st.get()));
+        CK(cudaStreamSynchronize(st.get()));
+    };
+    if (is_multi(X)) {
+        for_each_gpu(X, run);
+    } else {
+        CK(cudaSetDevice(X->device));
+        run(0, X);
+    }
+    std::vector<RegionRead> all;
+    for (auto& f : found) all.insert(all.end(), f.begin(), f.end());
+    std::sort(all.begin(), all.end(), [](const RegionRead& a, const RegionRead& b) {
+        return a.region != b.region ? a.region < b.region : a.read < b.read;
+    });
+    D.reads.resize(all.size());
+    for (size_t i = 0; i < all.size(); ++i) D.reads[i] = ReadCoordinate{all[i].read, all[i].start, all[i].end, (uint8_t)all[i].fwd};
+    for (size_t r = 0, i = 0; r < nR; ++r) {
+        CandidateRegion& c = D.regions[r];
+        c.read_off = i;
+        while (i < all.size() && all[i].region == r) ++i;
+        c.n_reads = (uint32_t)(i - c.read_off);
+    }
+}
+
 // ============================================================================================
 // discover's local assembler (assemble.cu): the pileups of all candidate regions of the sample are uploaded once, one
 // CTA per region counts and walks them, and the host reads back the statuses, the walk lengths and the walks' bases.
@@ -1641,6 +1731,43 @@ void assemble_regions(drprg_index* X, const drprg_assemble_opts* o) {
     }
 }
 
+// The map half of a sample from a reads file: strict FASTQ (plain or gzip) in waves of host-framed text, anything else
+// through the host parser as one batch
+struct FileMapped {
+    uint64_t n = 0, dropped = 0, bases = 0, hits = 0, kept = 0;
+    size_t waves = 0;
+    double ms_ingest = 0, ms_map = 0;
+};
+FileMapped map_reads_file(drprg_index* X, const char* reads_path, const drprg_map_opts* o, const Inflated* pre) {
+    const double t0 = now_ms();
+    FileMapped M;
+    WaveTotals W;
+    if (map_file_in_waves(X, reads_path, o, pre, W)) {
+        M.dropped = W.dropped;
+        M.bases = W.bases;
+        M.hits = W.hits;
+        M.kept = W.kept;
+        M.n = W.n;
+        M.waves = W.waves;
+        M.ms_ingest = W.ms_ingest;  // ingest and map alternate wave by wave
+        M.ms_map = W.ms_map;
+        return M;
+    }
+    // Not strict 4-line FASTQ, or host ingest forced.  Framing the whole file would decline as well: it runs the same
+    // framer over the same records as the waves, and it takes at most 8 GB of text where the waves take any size.
+    const FileBatch F = host_parsed_batch(X, reads_path, o ? o->threads : 1);
+    drprg_batch* B = F.B.get();
+    M.dropped = F.n_dropped;
+    M.bases = B->total_bases;
+    const double t1 = now_ms();
+    sample_begin_any(X, o, F.first_read_len);
+    M.n = B->R.n_reads;
+    map_batch_any(X, B, 0, &M.hits, &M.kept);
+    M.ms_ingest = t1 - t0;
+    M.ms_map = now_ms() - t1;
+    return M;
+}
+
 int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, const char* outdir, const drprg_map_opts* o,
                drprg_map_stats* stats, const Inflated* pre = nullptr) {
     need_device(X);
@@ -1649,34 +1776,7 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
     // any GPU work is done
     std::ofstream log(std::string(outdir) + "/pandora.log");
     if (!log) throw std::runtime_error(std::string("cannot write ") + outdir + "/pandora.log");
-    struct {
-        uint64_t n_dropped, total_bases;
-    } pr{0, 0};
-    uint64_t nh = 0, nk = 0, n = 0;
-    size_t waves = 0;
-    double t1 = t0, wave_ingest_ms = -1, wave_map_ms = 0;
-    WaveTotals W;
-    if (map_file_in_waves(X, reads_path, o, pre, W)) {
-        pr.n_dropped = W.dropped;
-        pr.total_bases = W.bases;
-        nh = W.hits;
-        nk = W.kept;
-        n = W.n;
-        waves = W.waves;
-        wave_ingest_ms = W.ms_ingest;  // ingest and map alternate wave by wave
-        wave_map_ms = W.ms_map;
-    } else {
-        // Not strict 4-line FASTQ, or host ingest forced.  Framing the whole file would decline as well: it runs the same
-        // framer over the same records as the waves, and it takes at most 8 GB of text where the waves take any size.
-        const FileBatch F = host_parsed_batch(X, reads_path, o ? o->threads : 1);
-        drprg_batch* B = F.B.get();
-        pr.n_dropped = F.n_dropped;
-        pr.total_bases = B->total_bases;
-        t1 = now_ms();
-        sample_begin_any(X, o, F.first_read_len);
-        n = B->R.n_reads;
-        map_batch_any(X, B, 0, &nh, &nk);
-    }
+    const FileMapped M = map_reads_file(X, reads_path, o, pre);
     const double t2 = now_ms();
     genotype(X, vcf_refs, "sample");
     std::ofstream vcf(std::string(outdir) + "/pandora_genotyped.vcf");
@@ -1684,25 +1784,106 @@ int run_sample(drprg_index* X, const char* reads_path, const char* vcf_refs, con
     vcf.write(X->h_vcf.data() + X->vcf_begin, (std::streamsize)X->vcf_len);
     const double t3 = now_ms();
     drprg_map_stats s{};
-    s.n_reads = n;
-    s.n_reads_dropped = pr.n_dropped;
-    s.total_bases = pr.total_bases;
-    s.n_hits = nh;
-    s.n_hits_kept = nk;
+    s.n_reads = M.n;
+    s.n_reads_dropped = M.dropped;
+    s.total_bases = M.bases;
+    s.n_hits = M.hits;
+    s.n_hits_kept = M.kept;
     s.n_loci_present = (uint32_t)X->contigs.size();
     s.n_records = (uint32_t)X->records.size();
     s.exp_depth_covg = X->fit.E;
-    s.ms_ingest = wave_ingest_ms >= 0 ? wave_ingest_ms : t1 - t0;
-    s.ms_map = wave_ingest_ms >= 0 ? wave_map_ms : t2 - t1;
+    s.ms_ingest = M.ms_ingest;
+    s.ms_map = M.ms_map;
     s.ms_genotype = t3 - t2;
     s.ms_total = t3 - t0;
     if (stats) *stats = s;
-    log << "drprg-cuda map: reads=" << n << " dropped=" << pr.n_dropped << " bases=" << pr.total_bases << " hits=" << nh
-        << " kept=" << nk << " loci=" << s.n_loci_present << " records=" << s.n_records << " E=" << s.exp_depth_covg
-        << " ingest=" << (waves ? "host-framed, " + std::to_string(waves) + " wave(s)" : "host") << "\nkernel ms: sketch_lookup=" << X->timings[0] << " sort=" << X->timings[1] << " cluster=" << X->timings[2]
+    log << "drprg-cuda map: reads=" << M.n << " dropped=" << M.dropped << " bases=" << M.bases << " hits=" << M.hits
+        << " kept=" << M.kept << " loci=" << s.n_loci_present << " records=" << s.n_records << " E=" << s.exp_depth_covg
+        << " ingest=" << (M.waves ? "host-framed, " + std::to_string(M.waves) + " wave(s)" : "host") << "\nkernel ms: sketch_lookup=" << X->timings[0] << " sort=" << X->timings[1] << " cluster=" << X->timings[2]
         << " coverage=" << X->timings[3] << "\nwall ms: ingest=" << s.ms_ingest << " map=" << s.ms_map
         << " genotype=" << s.ms_genotype << " total=" << s.ms_total << "\n";
     return 0;
+}
+
+DiscoverOpts discover_opts_from(const drprg_discover_opts* o) {
+    DiscoverOpts D;
+    if (o) {
+        if (o->covg_threshold) D.covg_threshold = o->covg_threshold;
+        if (o->min_len) D.min_len = o->min_len;
+        if (o->max_len) D.max_len = o->max_len;
+        if (o->padding != 0xffffffffu) D.padding = o->padding;
+        if (o->min_hits) D.min_hits = o->min_hits;
+    }
+    return D;
+}
+
+void refuse_shard_handles(const drprg_index* X) {
+    if (X->world > 1 || X->ipc_mapping)
+        throw std::runtime_error("one-process-per-GPU handles (drprg_cuda_shard_root / drprg_cuda_shard_attach) keep no read bases: "
+                                 "assemble on a single-GPU or drprg_cuda_index_load_multi handle");
+}
+
+// `pandora discover` for one sample from the one map pass: map (hit retention on), ML path, candidate regions, local
+// assembly, and <outdir>/denovo_paths.txt from the de-novo alleles
+void run_discover(drprg_index* X, const char* sample_name, const char* reads_path, const char* outdir, const drprg_map_opts* o,
+                  const drprg_discover_opts* d, const drprg_assemble_opts* a, drprg_discover_stats* stats) {
+    need_device(X);
+    refuse_shard_handles(X);
+    const char* sample = sample_name ? sample_name : "sample";
+    const double t0 = now_ms();
+    const std::string path = std::string(outdir) + "/denovo_paths.txt";
+    // an unusable outdir fails before any GPU work is done; the file itself is only created once its text is known
+    if (access(outdir, W_OK | X_OK) != 0) throw std::runtime_error("cannot write " + path + ": " + strerror(errno));
+    struct RetainGuard {  // the caller's retention setting comes back whatever happens
+        drprg_index* X;
+        bool was;
+        ~RetainGuard() {
+            for (drprg_index* g : (X->gpus.empty() ? std::vector<drprg_index*>{X} : X->gpus)) g->retain_hits = was;
+        }
+    } guard{X, X->retain_hits};
+    for (drprg_index* g : (X->gpus.empty() ? std::vector<drprg_index*>{X} : X->gpus)) g->retain_hits = true;
+    const FileMapped M = map_reads_file(X, reads_path, o, nullptr);
+    const double t1 = now_ms();
+    genotype(X, nullptr, sample);  // pandora discover takes no --vcf-refs: the ML path does not depend on them
+    const double t2 = now_ms();
+    find_candidates(X, discover_opts_from(d));
+    assemble_regions(X, a);
+    const DiscoverResult& D = X->discover;
+    std::vector<std::vector<DenovoVariant>> variants(X->H.loci.size());
+    for (const drprg_denovo_path& p : X->asm_paths) {
+        const uint32_t l = D.regions[p.region].locus;
+        allele_variants(D.consensus[l], p.a, p.b, X->asm_bases.substr(p.offset, p.length), variants[l]);
+    }
+    drprg_discover_stats s{};
+    for (auto& v : variants) {
+        std::sort(v.begin(), v.end());
+        v.erase(std::unique(v.begin(), v.end()), v.end());
+        s.n_loci_with_variants += !v.empty();
+        s.n_variants += (uint32_t)v.size();
+    }
+    const std::string text = denovo_paths_text(X->H, sample, D, variants);
+    std::ofstream out(path);
+    if (!out) throw std::runtime_error("cannot write " + path);
+    out.write(text.data(), (std::streamsize)text.size());
+    out.close();
+    if (!out) throw std::runtime_error("write error on " + path);
+    const double t3 = now_ms();
+    s.n_reads = M.n;
+    s.n_hits_kept = M.kept;
+    s.n_region_reads = D.reads.size();
+    s.n_regions = (uint32_t)D.regions.size();
+    for (uint8_t st : X->asm_status) {
+        s.n_assembled += st == ASM_ASSEMBLED;
+        s.n_no_anchor += st == ASM_NO_ANCHOR;
+        s.n_too_many_paths += st == ASM_TOO_MANY_PATHS;
+        s.n_no_path += st == ASM_NO_PATH;
+    }
+    s.ms_ingest = M.ms_ingest;
+    s.ms_map = M.ms_map;
+    s.ms_ml_path = t2 - t1;
+    s.ms_discover = t3 - t2;
+    s.ms_total = t3 - t0;
+    if (stats) *stats = s;
 }
 }  // namespace
 
@@ -2266,25 +2447,7 @@ int drprg_cuda_discover_candidates(drprg_index* X, const drprg_discover_opts* o,
     API_BEGIN need_device(X);
     if (!X->have_gt) throw std::runtime_error("drprg_cuda_genotype has not run for this sample");
     if (!X->retain_hits) throw std::runtime_error("drprg_cuda_retain_hits(idx, 1) must be set before the sample is mapped");
-    DiscoverOpts D;
-    if (o) {
-        if (o->covg_threshold) D.covg_threshold = o->covg_threshold;
-        if (o->min_len) D.min_len = o->min_len;
-        if (o->max_len) D.max_len = o->max_len;
-        if (o->padding != 0xffffffffu) D.padding = o->padding;
-        if (o->min_hits) D.min_hits = o->min_hits;
-    }
-    const std::vector<RetainedHit>* hits = &X->retained;
-    std::vector<RetainedHit> all;
-    if (X->gpus.size() > 1) {  // shards are contiguous read ranges: concatenation keeps the hits grouped by read
-        for (drprg_index* g : X->gpus) all.insert(all.end(), g->retained.begin(), g->retained.end());
-        hits = &all;
-    }
-    discover_candidates(X->H, X->present, X->mlpaths, X->h_acc.data(), *hits, D, X->discover);
-    X->discover_ready = true;
-    X->asm_status.clear();
-    X->asm_paths.clear();
-    X->asm_bases.clear();
+    find_candidates(X, discover_opts_from(o));
     if (n_regions) *n_regions = (uint32_t)X->discover.regions.size();
     if (n_region_reads) *n_region_reads = X->discover.reads.size();
     return 0;
@@ -2322,15 +2485,19 @@ int drprg_cuda_discover_coverage(drprg_index* X, uint32_t locus, uint32_t* covg)
 }
 int drprg_cuda_discover_assemble(drprg_index* X, const drprg_assemble_opts* o, uint32_t* n_paths, uint64_t* n_path_bases) {
     API_BEGIN need_device(X);
-    if (X->world > 1 || X->ipc_mapping)
-        throw std::runtime_error("one-process-per-GPU handles (drprg_cuda_shard_root / drprg_cuda_shard_attach) keep no read bases: "
-                                 "assemble on a single-GPU or drprg_cuda_index_load_multi handle");
+    refuse_shard_handles(X);
     if (!X->have_gt) throw std::runtime_error("drprg_cuda_genotype has not run for this sample");
     if (!X->retain_hits) throw std::runtime_error("drprg_cuda_retain_hits(idx, 1) must be set before the sample is mapped");
     if (!X->discover_ready) throw std::runtime_error("drprg_cuda_discover_candidates has not run for this sample");
     assemble_regions(X, o);
     if (n_paths) *n_paths = (uint32_t)X->asm_paths.size();
     if (n_path_bases) *n_path_bases = X->asm_bases.size();
+    return 0;
+    API_END
+}
+int drprg_cuda_discover(drprg_index* X, const char* sample, const char* reads_path, const char* outdir, const drprg_map_opts* o,
+                        const drprg_discover_opts* d, const drprg_assemble_opts* a, drprg_discover_stats* stats) {
+    API_BEGIN run_discover(X, sample, reads_path, outdir, o, d, a, stats);
     return 0;
     API_END
 }

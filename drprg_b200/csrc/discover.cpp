@@ -9,8 +9,10 @@
 //                       = [1, 30] (identify_low_coverage_intervals), padded by -P 22 either side
 //   region reads        for every read with kept hits on the locus: its hits whose k-mer lies on the ML path inside the
 //                       padded region; reads with at least two such hits contribute the span [min start, max start + k) and
-//                       the strand of the first hit (get_read_overlap_coordinates / find_hits_inside_path)
-// The de-novo assembly itself (pandora's de Bruijn graph walk) runs on the GPU (assemble.cu); this file produces its inputs.
+//                       the strand of the first hit (get_read_overlap_coordinates / find_hits_inside_path).  These are
+//                       found on the GPU from the retained hits (assemble.cu, region_reads_kernel) with the tables made here.
+// The de-novo assembly itself (pandora's de Bruijn graph walk) runs on the GPU (assemble.cu); this file produces its inputs
+// and writes its result, discover/denovo_paths.txt.
 // Option names and defaults are upstream pandora's `discover` (drprg passes none of them, src/predict.rs:236-245).
 #include <algorithm>
 #include <stdexcept>
@@ -90,24 +92,25 @@ std::vector<uint32_t> knode_consensus_start(const Locus& L, const std::vector<ui
     return out;
 }
 
-void discover_candidates(const HostIndex& H, const std::vector<char>& present, const std::vector<std::vector<uint32_t>>& mlpaths,
-                         const int32_t* cov, const std::vector<RetainedHit>& hits, const DiscoverOpts& o, DiscoverResult& R) {
+void discover_regions(const HostIndex& H, const std::vector<char>& present, const std::vector<std::vector<uint32_t>>& mlpaths,
+                      const int32_t* cov, const DiscoverOpts& o, DiscoverResult& R, std::vector<uint32_t>& cons_start) {
     R = DiscoverResult();
     const uint32_t P = (uint32_t)H.loci.size();
     R.consensus.assign(P, std::string());
     R.coverage.assign(P, {});
-    std::vector<std::vector<uint32_t>> cons_start(P);
-    std::vector<std::pair<size_t, size_t>> locus_regions(P, {0, 0});
+    R.local_path.assign(P, {});
+    cons_start.assign(H.total_knodes(), UINT32_MAX);
     for (uint32_t l = 0; l < P; ++l) {
         if (l >= present.size() || !present[l]) continue;
         const Locus& L = H.loci[l];
-        const std::vector<uint32_t> lp = local_path_of(L, mlpaths[l]);
+        const std::vector<uint32_t>& lp = R.local_path[l] = local_path_of(L, mlpaths[l]);
         R.consensus[l] = spell_local_path(L, lp);
         R.coverage[l] = ml_path_base_coverage(H, l, mlpaths[l], lp, cov);
-        cons_start[l] = knode_consensus_start(L, lp);
         std::vector<std::pair<uint32_t, uint32_t>> iv;
         low_coverage_intervals(R.coverage[l], o.covg_threshold, o.min_len, o.max_len, iv);
-        locus_regions[l].first = R.regions.size();
+        if (iv.empty()) continue;
+        const std::vector<uint32_t> cs = knode_consensus_start(L, lp);
+        std::copy(cs.begin(), cs.end(), cons_start.begin() + H.knode_base[l]);
         const uint32_t n = (uint32_t)R.coverage[l].size();
         for (auto& p : iv) {
             CandidateRegion c;
@@ -118,50 +121,87 @@ void discover_candidates(const HostIndex& H, const std::vector<char>& present, c
             c.pad_end = std::min(n, p.second + o.padding);
             R.regions.push_back(c);
         }
-        locus_regions[l].second = R.regions.size();
-    }
-    // reads over the regions: hits arrive grouped by read (any read order), sorted (prg, strand, start, k-mer node) within
-    struct Acc { uint32_t n = 0, lo = 0, hi = 0; uint8_t fwd = 0; };
-    std::vector<std::vector<ReadCoordinate>> per_region(R.regions.size());
-    std::vector<Acc> acc;
-    size_t i = 0;
-    while (i < hits.size()) {
-        size_t j = i;
-        while (j < hits.size() && hits[j].read == hits[i].read && hits[j].prg == hits[i].prg) ++j;
-        const uint32_t l = hits[i].prg;
-        const size_t r0 = l < P ? locus_regions[l].first : 0, r1 = l < P ? locus_regions[l].second : 0;
-        if (r1 > r0) {
-            acc.assign(r1 - r0, Acc());
-            for (size_t q = i; q < j; ++q) {
-                const uint32_t cs = hits[q].knode < cons_start[l].size() ? cons_start[l][hits[q].knode] : UINT32_MAX;
-                if (cs == UINT32_MAX) continue;
-                for (size_t rg = r0; rg < r1; ++rg) {
-                    const CandidateRegion& c = R.regions[rg];
-                    if (cs < c.pad_start || cs + H.k > c.pad_end) continue;
-                    Acc& a = acc[rg - r0];
-                    if (a.n == 0) {
-                        a.lo = hits[q].start;
-                        a.fwd = hits[q].fwd;
-                    }
-                    a.lo = std::min(a.lo, hits[q].start);
-                    a.hi = std::max(a.hi, hits[q].start + H.k);
-                    ++a.n;
-                }
-            }
-            for (size_t rg = r0; rg < r1; ++rg)
-                if (acc[rg - r0].n >= o.min_hits) per_region[rg].push_back(ReadCoordinate{hits[i].read, acc[rg - r0].lo, acc[rg - r0].hi, acc[rg - r0].fwd});
-        }
-        i = j;
-    }
-    for (size_t rg = 0; rg < R.regions.size(); ++rg) {
-        auto& v = per_region[rg];
-        std::sort(v.begin(), v.end(), [](const ReadCoordinate& a, const ReadCoordinate& b) { return a.read < b.read; });
-        R.regions[rg].read_off = R.reads.size();
-        R.regions[rg].n_reads = (uint32_t)v.size();
-        R.reads.insert(R.reads.end(), v.begin(), v.end());
     }
 }
 
+// R = cons[a, b) against the allele by global unit-cost edit distance; the traceback from the end extends an open gap while
+// that stays optimal (one indel stays one run), and otherwise prefers the diagonal, then a deletion (a base of R), then an
+// insertion.  Every maximal run of non-match columns is one variant.  A run with an empty side is anchored VCF-style by
+// the consensus base before it, or by the base after it when it starts at R[0].
+void allele_variants(const std::string& cons, uint32_t a, uint32_t b, const std::string& allele, std::vector<DenovoVariant>& out) {
+    const std::string R = cons.substr(a, b - a);
+    const std::string& A = allele;
+    const size_t n = R.size(), m = A.size(), W = m + 1;
+    std::vector<uint32_t> D((n + 1) * W);
+    for (size_t i = 0; i <= n; ++i) D[i * W] = (uint32_t)i;
+    for (size_t j = 0; j <= m; ++j) D[j] = (uint32_t)j;
+    for (size_t i = 1; i <= n; ++i)
+        for (size_t j = 1; j <= m; ++j)
+            D[i * W + j] = std::min({D[(i - 1) * W + j - 1] + (R[i - 1] != A[j - 1]), D[(i - 1) * W + j] + 1, D[i * W + j - 1] + 1});
+    struct Col {
+        int32_t i, j;  // the base of R / of the allele the column holds, -1 for a gap
+    };
+    std::vector<Col> cols;
+    char op = 0;  // the last column's kind: M(atch or substitution), D(eletion), I(nsertion)
+    for (size_t i = n, j = m; i || j;) {
+        const bool diag = i && j && D[i * W + j] == D[(i - 1) * W + j - 1] + (R[i - 1] != A[j - 1]);
+        const bool del = i && D[i * W + j] == D[(i - 1) * W + j] + 1;
+        const bool ins = j && D[i * W + j] == D[i * W + j - 1] + 1;
+        if (!((op == 'D' && del) || (op == 'I' && ins))) op = diag ? 'M' : del ? 'D' : 'I';  // else an open gap is extended
+        if (op != 'I') --i;
+        if (op != 'D') --j;
+        cols.push_back({op != 'I' ? (int32_t)i : -1, op != 'D' ? (int32_t)j : -1});
+    }
+    std::reverse(cols.begin(), cols.end());
+    auto match = [&](const Col& c) { return c.i >= 0 && c.j >= 0 && R[c.i] == A[c.j]; };
+    uint32_t ri = 0;  // bases of R before the column
+    for (size_t c = 0; c < cols.size();) {
+        if (match(cols[c])) {
+            ++ri;
+            ++c;
+            continue;
+        }
+        const uint32_t i0 = ri;
+        DenovoVariant v{a + i0 + 1, "", ""};
+        for (; c < cols.size() && !match(cols[c]); ++c) {
+            if (cols[c].i >= 0) {
+                v.ref += R[cols[c].i];
+                ++ri;
+            }
+            if (cols[c].j >= 0) v.alt += A[cols[c].j];
+        }
+        if (v.ref.empty() || v.alt.empty()) {
+            if (i0 == 0 && a + ri < cons.size()) {
+                v.ref += cons[a + ri];
+                v.alt += cons[a + ri];
+            } else if (a + i0 > 0) {
+                v.ref.insert(v.ref.begin(), cons[a + i0 - 1]);
+                v.alt.insert(v.alt.begin(), cons[a + i0 - 1]);
+                --v.pos;
+            }
+        }
+        out.push_back(std::move(v));
+    }
+}
+
+// pandora 0.10's discover/denovo_paths.txt [P]: the header, then per locus with variants its name, its ML local path (node
+// id, PRG-string interval, sequence) and its variants
+std::string denovo_paths_text(const HostIndex& H, const std::string& sample, const DiscoverResult& D,
+                              const std::vector<std::vector<DenovoVariant>>& variants) {
+    size_t n_loci = 0;
+    for (const auto& v : variants) n_loci += !v.empty();
+    std::string s = "1 samples\nSample " + sample + "\n" + std::to_string(n_loci) + " loci with denovo variants\n";
+    for (size_t l = 0; l < variants.size(); ++l) {
+        if (variants[l].empty()) continue;
+        const Locus& L = H.loci[l];
+        s += L.name + "\n" + std::to_string(D.local_path[l].size()) + " nodes\n";
+        for (uint32_t n : D.local_path[l])
+            s += "(" + std::to_string(n) + " [" + std::to_string(L.nodes[n].s) + ", " + std::to_string(L.nodes[n].e) + ") " + L.node_seq(n) + ")\n";
+        s += std::to_string(variants[l].size()) + " variants found\n";
+        for (const DenovoVariant& v : variants[l]) s += std::to_string(v.pos) + "\t" + v.ref + "\t" + v.alt + "\n";
+    }
+    return s;
+}
 
 // ============================================================================================
 // `pandora index` replacement (SURVEY.md §8f rank 3): drprg runs `pandora index -t T -w W -k K <prg>` when an index is

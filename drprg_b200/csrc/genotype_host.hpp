@@ -79,11 +79,6 @@ bool locus_coverage_outlier(const HostIndex& H, uint32_t locus, const std::vecto
                             const std::vector<uint32_t>& lpath, const int32_t* cov, uint32_t global_covg);
 
 // ---- discover's mapping front half from the map pass (discover.cpp, SURVEY 8f rank 1) ------------------------------
-struct RetainedHit {  // a kept hit of the sample, grouped by read, pandora order within a read
-    uint32_t read, start, knode;
-    uint16_t prg;
-    uint8_t fwd;
-};
 struct DiscoverOpts {  // pandora discover defaults (drprg overrides none of them)
     uint32_t covg_threshold = 3, min_len = 1, max_len = 30, padding = 22, min_hits = 2;
 };
@@ -98,13 +93,27 @@ struct CandidateRegion {
 struct DiscoverResult {
     std::vector<std::string> consensus;           // per locus: ML sequence (empty when the locus is absent)
     std::vector<std::vector<uint32_t>> coverage;  // per locus: per-base coverage along it
+    std::vector<std::vector<uint32_t>> local_path; // per locus: the local nodes the ML sequence spells
     std::vector<CandidateRegion> regions;         // ordered by locus, then position
     std::vector<ReadCoordinate> reads;            // per region, ordered by read id
 };
 std::vector<uint32_t> ml_path_base_coverage(const HostIndex& H, uint32_t locus, const std::vector<uint32_t>& kpath,
                                             const std::vector<uint32_t>& lpath, const int32_t* cov);
-void discover_candidates(const HostIndex& H, const std::vector<char>& present, const std::vector<std::vector<uint32_t>>& mlpaths,
-                         const int32_t* cov, const std::vector<RetainedHit>& hits, const DiscoverOpts& o, DiscoverResult& R);
+// the per-locus half: consensus, coverage, local path and candidate regions (reads left empty), and the consensus start of
+// every global k-mer node on the ML path of a locus with regions (UINT32_MAX elsewhere) for the region-read kernel
+void discover_regions(const HostIndex& H, const std::vector<char>& present, const std::vector<std::vector<uint32_t>>& mlpaths,
+                      const int32_t* cov, const DiscoverOpts& o, DiscoverResult& R, std::vector<uint32_t>& cons_start);
+// discover/denovo_paths.txt [P]: a de-novo allele replacing cons[a, b) as variants against the ML sequence (1-based pos,
+// anchored so that neither allele is empty), and the file's text for the loci with variants
+struct DenovoVariant {
+    uint32_t pos;
+    std::string ref, alt;
+    bool operator<(const DenovoVariant& o) const { return std::tie(pos, ref, alt) < std::tie(o.pos, o.ref, o.alt); }
+    bool operator==(const DenovoVariant& o) const { return pos == o.pos && ref == o.ref && alt == o.alt; }
+};
+void allele_variants(const std::string& cons, uint32_t a, uint32_t b, const std::string& allele, std::vector<DenovoVariant>& out);
+std::string denovo_paths_text(const HostIndex& H, const std::string& sample, const DiscoverResult& D,
+                              const std::vector<std::vector<DenovoVariant>>& variants /* per locus, sorted, distinct */);
 
 // pandora-compatible index files next to the PRG (`pandora index` replacement, SURVEY 8f rank 3): <prg>.k{K}.w{W}.idx and
 // kmer_prgs/NN/<locus>.k{K}.w{W}.gfa

@@ -190,13 +190,36 @@ void launch_format_g6_batch(const double* d_v, uint32_t n, char* d_out, uint8_t*
 // the likelihood / GT / GT_CONF kernel alone, on per-allele rows already in G.mean_fwd / G.mean_rev / G.gaps
 void launch_genotype_rows(const DevGenotype& G, ModelParams P, cudaStream_t st);
 
-// ---- discover: the bases of retained reads and the local assembler (assemble.cu) ------------------------------------
-// per active read of the last batch (n_active, lists of PostBuffers): a read with at least one kept hit gets its 2-bit words
-// copied to out_words[table[a].x ...] (table[a].y = its length in bases); table[a].x = UINT32_MAX for the other reads.  The
-// words wanted are counted in *d_cursor (zeroed by the caller) even past word_cap: the caller regrows and launches again.
+// ---- discover: retained hits and reads, region reads and the local assembler (assemble.cu) --------------------------
+// The kept hits of a sample on one GPU, appended batch after batch (hit retention on): per hit the global read id and the
+// grouped-hit key, per read with a kept hit one row {first hit, hit count}.  A read's hits keep their slice order.
+struct RetainStore {
+    uint32_t* hit_read;
+    unsigned long long* hit_key;
+    uint64_t hit_cap;
+    uint2* rows;
+    uint64_t row_cap;
+};
+enum : int { RT_WORDS = 0, RT_HITS = 1, RT_ROWS = 2, RT_COUNT = 3 };  // cursors of launch_retain_gather
+// per active read of the last batch (n_active, lists of PostBuffers), one warp each: a read with at least one kept hit takes
+// one row and appends its kept hits to the store, and its 2-bit words are copied to out_words.  table[row - row_base] =
+// {word offset (UINT32_MAX when the words did not fit), length in bases, global read id}.  d_cursor[RT_WORDS] (zero) and
+// d_cursor[RT_HITS / RT_ROWS] (the store's fill) count on past the capacities: the caller regrows, resets and launches again.
 void launch_retain_gather(const DevReads& R, const uint32_t* act_read, const uint32_t* act_base, const uint32_t* act_count,
-                          const uint8_t* gkept, uint32_t n_active, uint2* table, uint32_t* out_words, uint64_t word_cap,
-                          unsigned long long* d_cursor, cudaStream_t st);
+                          const unsigned long long* gkey, const uint8_t* gkept, uint32_t n_active, RetainStore S,
+                          uint64_t row_base, uint4* table, uint32_t* out_words, uint64_t word_cap, unsigned long long* d_cursor,
+                          cudaStream_t st);
+struct RegionRead {  // a read with at least min_hits kept hits inside a candidate region
+    uint32_t region, read, start, end, fwd;
+};
+// one warp per row of the store: for every (read, locus) group and every region of that locus (regions
+// [locus_region_off[l], locus_region_off[l + 1]), padded intervals pad[r]), the hits whose k-mer node has a consensus start
+// cs = cons_start[knode_base[l] + node] (UINT32_MAX: off the ML path) with pad.x <= cs and cs + k <= pad.y: their count, the
+// smallest start, the largest start + k and the strand of the first.  Groups with count >= min_hits go to out at slots
+// taken from *d_cursor (zeroed by the caller), which counts on past out_cap.
+void launch_region_reads(RetainStore S, uint32_t n_rows, const uint32_t* knode_base, const uint32_t* cons_start,
+                         const uint32_t* locus_region_off, uint32_t n_loci, const uint2* pad, uint32_t k, uint32_t min_hits,
+                         RegionRead* out, uint64_t out_cap, unsigned long long* d_cursor, cudaStream_t st);
 constexpr uint32_t DISCOVER_K = 11;             // de Bruijn k-mer size: 22-bit k-mers
 constexpr uint32_t KMER_ATTEMPTS = 10;          // anchor k-mers tried per flank
 constexpr uint32_t ASM_MAX_PATHS_LIMIT = 64;    // largest max_candidate_paths the walk's shared-memory store takes

@@ -54,6 +54,18 @@ class DenovoPath(C.Structure):
     _fields_ = [("region", C.c_uint32), ("a", C.c_uint32), ("b", C.c_uint32), ("length", C.c_uint32), ("offset", C.c_uint64)]
 
 
+class DiscoverStats(C.Structure):
+    _fields_ = [
+        ("n_reads", C.c_uint64), ("n_hits_kept", C.c_uint64), ("n_region_reads", C.c_uint64), ("n_regions", C.c_uint32),
+        ("n_assembled", C.c_uint32), ("n_no_anchor", C.c_uint32), ("n_too_many_paths", C.c_uint32), ("n_no_path", C.c_uint32),
+        ("n_loci_with_variants", C.c_uint32), ("n_variants", C.c_uint32), ("ms_ingest", C.c_double), ("ms_map", C.c_double),
+        ("ms_ml_path", C.c_double), ("ms_discover", C.c_double), ("ms_total", C.c_double),
+    ]
+
+    def asdict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # region status of discover_assemble (DRPRG_DENOVO_* of the header)
 ASSEMBLED, NO_ANCHOR, TOO_MANY_PATHS, NO_PATH = 0, 1, 2, 3
 
@@ -85,7 +97,7 @@ SYMBOLS = [
     "drprg_cuda_index_records", "drprg_cuda_index_min_path_length", "drprg_cuda_sketch_batch", "drprg_cuda_last_hits",
     "drprg_cuda_gt_params", "drprg_cuda_gt_mlpath", "drprg_cuda_gt_counts", "drprg_cuda_gt_records",
     "drprg_cuda_gt_alleles", "drprg_cuda_gt_allele_knodes", "drprg_cuda_genotype_rows", "drprg_cuda_gt_filter_stats", "drprg_cuda_set_minor_af", "drprg_cuda_retain_hits", "drprg_cuda_discover_candidates",
-    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover_paths",
+    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover", "drprg_cuda_discover_paths",
     "drprg_cuda_discover_region_status", "drprg_cuda_last_assemble_stats", "drprg_cuda_last_timings", "drprg_cuda_last_genotype_timings", "drprg_cuda_format_g6", "drprg_cuda_format_g6_device", "drprg_cuda_launch_count", "drprg_cuda_hash64", "drprg_cuda_hash64_inverse", "drprg_cuda_issue_peak",
 ]
 
@@ -487,6 +499,19 @@ class Index:
         o = np.zeros(4, np.float64)
         lib().drprg_cuda_last_assemble_stats(self.h, _p(o))
         return dict(regions_shared=int(o[0]), regions_global=int(o[1]), ms_shared=float(o[2]), ms_global=float(o[3]))
+
+    def discover(self, reads_path, outdir, opts=None, sample="sample", discover_opts=None, assemble_opts=None):
+        """`pandora discover` for one sample: maps the reads file (hit retention on for this call only), finds and assembles
+        the candidate regions and writes <outdir>/denovo_paths.txt; returns the stats dict.  discover_opts / assemble_opts:
+        keyword dicts of discover_candidates / discover_assemble."""
+        st = DiscoverStats()
+        o = opts or make_opts()
+        d = DiscoverOpts(**dict(dict(covg_threshold=0, min_len=0, max_len=0, padding=0xFFFFFFFF, min_hits=0), **(discover_opts or {})))
+        a = AssembleOpts(**dict(dict(min_dbg_dp=0, max_insertion=0xFFFFFFFF, max_candidate_paths=0), **(assemble_opts or {})))
+        rc = lib().drprg_cuda_discover(self.h, sample.encode(), str(reads_path).encode(), str(outdir).encode(), C.byref(o), C.byref(d),
+                                       C.byref(a), C.byref(st))
+        _check(rc, "drprg_cuda_discover")
+        return st.asdict()
 
     def set_minor_af(self, maf):
         lib().drprg_cuda_set_minor_af(self.h, C.c_float(maf))

@@ -1,8 +1,9 @@
 """Host-side mirror of the reference's adapter for this path: `Pandora::genotype_with`
 (/root/reference/src/lib.rs:580-642), `Pandora::vcf_filename` (:644-646) and `Pandora::index_with` (:479-510), same
 names, argument meaning and error behaviour, but backed by the CUDA library instead of a pandora subprocess.
-`discover_candidates` is the mapping front half of `Pandora::discover_with` (:513-578) taken from the map pass, and
-`discover_paths` its local assembly, on the GPU.
+`discover_with` is `Pandora::discover_with` (:513-578): one map pass, the local assembly on the GPU and
+discover/denovo_paths.txt.  `discover_candidates` and `discover_paths` return its intermediate results after a
+`genotype_with(..., retain_hits=True)`.
 
 The reference builds the argv  -t T -w W -k K -c C [-I] [-K]  (src/predict.rs:288-294) after the fixed
 `map --genotype --local --gt-conf 0 -v -o OUT -g 4411532 --max-covg 4294967295 --vcf-refs REF`
@@ -106,6 +107,33 @@ class Pandora:
             return ix.map_genotype(reads, vcf_ref, outdir, opts)
         except lib.DrprgCudaError as e:
             raise DependencyError(str(e)) from e
+
+    def discover_with(self, prg, query_idx, outdir, args=()):
+        """`pandora discover -g 4411532 --max-covg 4294967295 -v -o OUT -t T -w W -k K -c C [-I] [-K] <prg> <query.tsv>`
+        (src/lib.rs:513-578): query_idx holds one `sample<TAB>reads` line (a relative reads path is taken from the query
+        file's directory); writes OUT/denovo_paths.txt and returns its path; raises DependencyError where the reference
+        returns Err."""
+        o = self._parse_args(args)
+        try:
+            lines = [l for l in open(query_idx).read().splitlines() if l.strip()]
+        except OSError as e:
+            raise DependencyError(f"cannot read {query_idx}: {e}") from e
+        if len(lines) != 1:
+            raise DependencyError(f"{query_idx}: {len(lines)} samples; discover takes a query file with exactly one")
+        fields = lines[0].split("\t")
+        if len(fields) != 2:
+            raise DependencyError(f"{query_idx}: expected `sample<TAB>reads`")
+        sample, reads = fields
+        reads = os.path.join(os.path.dirname(os.path.abspath(str(query_idx))), reads)
+        os.makedirs(outdir, exist_ok=True)
+        try:
+            ix = self.load_index(prg, o["w"], o["k"])
+            opts = lib.make_opts(threads=o["threads"], min_cluster_size=o["c"], illumina=o["illumina"],
+                                 genome_size=MTB_GENOME_SIZE, gt_conf=0.0, debug=o["debug"])
+            ix.discover(reads, outdir, opts, sample=sample)
+        except lib.DrprgCudaError as e:
+            raise DependencyError(str(e)) from e
+        return os.path.join(str(outdir), "denovo_paths.txt")
 
     def discover_candidates(self, **opts):
         """After genotype_with(..., retain_hits=True): the inputs of pandora discover's local assembler (ML consensus and

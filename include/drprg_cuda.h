@@ -152,7 +152,9 @@ const char* drprg_cuda_vcf_view(drprg_index*, uint64_t* len);
  * (after drprg_cuda_genotype) returns what pandora's local assembler needs, from the pass that ran anyway: per present locus
  * the maximum-likelihood sequence and its per-base coverage, the candidate regions (runs of coverage < covg_threshold with a
  * length in [min_len, max_len], padded) and per region the reads with >= min_hits kept hits inside it (read id, span on the
- * read, strand).  Fields left 0 take pandora discover's defaults (3, 1, 30, 2); padding 0xffffffff = default 22. */
+ * read, strand).  Fields left 0 take pandora discover's defaults (3, 1, 30, 2); padding 0xffffffff = default 22.
+ * Retention keeps every kept hit (read id, hit key) in a store on its GPU, appended by a kernel at the end of each batch;
+ * the reads over the regions are found there by a kernel, only the result (a few thousand entries) comes to the host. */
 typedef struct {
     uint32_t covg_threshold, min_len, max_len, padding, min_hits;
 } drprg_discover_opts;
@@ -198,6 +200,29 @@ int drprg_cuda_discover_region_status(drprg_index*, uint8_t* status /* n_regions
 /* the last assembly's shape: regions counted in a shared-memory k-mer table, regions whose pileup needed a table in global
  * memory, and the device time in ms of the two kernel launches (CUDA events) — 4 doubles */
 int drprg_cuda_last_assemble_stats(drprg_index*, double* out4);
+
+/* `pandora discover` for one sample in one blocking call (drprg src/predict.rs:247-256 -> src/lib.rs:513-578): the reads file
+ * is mapped through the same ingest as drprg_cuda_map_genotype with hit retention switched on (the caller's setting is
+ * restored afterwards), genotyped without --vcf-refs (the ML path does not depend on them), its candidate regions are
+ * found and assembled as above, and <outdir>/denovo_paths.txt is written; no VCF.  The file [P: restates pandora 0.10's
+ * writer and make_prg update's reader]:
+ *     1 samples / Sample <sample> / <L> loci with denovo variants
+ *     then per locus with a variant, in PRG order: its name, "<M> nodes", one "(<node id> [<start>, <end>) <seq>)" line per
+ *     node of its ML local path (PRG-string coordinates, node ids = this library's local-node ranks), "<V> variants found",
+ *     and one "<pos>\t<ref>\t<alt>" line per variant.
+ * Variants: every de-novo allele is aligned to the consensus span it replaces (unit-cost edit distance; the traceback from
+ * the end extends an open gap while that stays optimal, else prefers substitution, then deletion, then insertion); each
+ * maximal run of non-match columns is one variant at its 1-based position on the ML sequence, a run with an empty side
+ * anchored by the consensus base before it (after it when it starts at the span's first base).  Per locus the union over its regions, distinct, sorted by (pos, ref, alt).
+ * NULL options take the defaults; refused on one-process-per-GPU handles. */
+typedef struct {
+    uint64_t n_reads, n_hits_kept, n_region_reads;
+    uint32_t n_regions, n_assembled, n_no_anchor, n_too_many_paths, n_no_path; /* region statuses: DRPRG_DENOVO_* */
+    uint32_t n_loci_with_variants, n_variants;
+    double ms_ingest, ms_map, ms_ml_path, ms_discover, ms_total; /* wall clock; discover = regions + assembly + file */
+} drprg_discover_stats;
+int drprg_cuda_discover(drprg_index*, const char* sample, const char* reads_path, const char* outdir, const drprg_map_opts*,
+                        const drprg_discover_opts*, const drprg_assemble_opts*, drprg_discover_stats* /* may be NULL */);
 
 /* ---- introspection / parity hooks (same .so, used by tests and bench) --------------------------- */
 /* pandora's hash64 on a 2k-bit k-mer and its inverse (the k-mer screen is built from the inverse): host functions */

@@ -1,25 +1,33 @@
-"""discover's local assembler at config-2 scale: the benchmark panel (workload.Config2) with a sample genome carrying
-20 variants the PRG does not know (a SNP, a 3 bp deletion or a 6 bp insertion in each of the first 20 loci), 1 M
-simulated 150 bp reads.  Reports, in one run on one GPU:
-  the card and its power limit; map_batch wall time with hit retention off and on, alternated, with spreads; the bytes the
-  retention keeps; the candidate regions and their assembly statuses; which k-mer table path the regions take and the
-  assembly kernels' device time (CUDA events inside the library); the oracle assembler's wall time on the same regions and
-  whether its results equal the GPU's; and how many planted variants come back as their true haplotype.
+"""`pandora discover` at config-2 scale: the benchmark panel (workload.Config2) with a sample genome carrying 20 variants
+the PRG does not know (a SNP, a 3 bp deletion or a 6 bp insertion in each of the first 20 loci), 1 M simulated 150 bp
+reads.  Reports, in one run on one GPU:
+  the card and its power limit; map_batch wall time with hit retention off and on, alternated, with spreads; the same at
+  config-3 size (--big-batches batches of 2 x --reads reads per sample, the 1 M reads twice over); the bytes the retention
+  keeps; the candidate regions and their assembly statuses; which k-mer table path the regions take and the assembly
+  kernels' device time (CUDA events inside the library); the oracle assembler's wall time on the same regions and whether
+  its results equal the GPU's; how many planted variants come back as their true haplotype; drprg_cuda_discover on the
+  reads as a plain and a gzip FASTQ with its stage split, alternated with drprg_cuda_map_genotype on the same file; whether
+  the file equals the test-side restatement (tests/denovo_paths_oracle.py) of the same ML paths, regions and oracle
+  alleles; and how many planted variants are records of the file.
 
-    python tools/discover_probe.py [--reads 1000000] [--reps 5] [--out LOG]
+    python tools/discover_probe.py [--reads 1000000] [--reps 5] [--big-batches 15] [--out LOG]
 """
 import argparse
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+sys.path[:0] = [ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle")]
 
 import denovo_oracle as A  # noqa: E402
+import denovo_paths_oracle as P  # noqa: E402
+import oracle_py as O  # noqa: E402
 from drprg_b200 import lib, sim, workload  # noqa: E402
 
 KINDS = ("snp", "del3", "ins6")
@@ -34,6 +42,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reads", type=int, default=1_000_000)
     ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--big-batches", type=int, default=15)
     ap.add_argument("--out", help="also write the report to this file")
     a = ap.parse_args()
     lines = []
@@ -65,6 +74,22 @@ def main():
                 ms[on].append((time.perf_counter() - t) * 1e3)
     log(f"map_batch ms, retention off: {spread(ms[False])}  (n={len(ms[False])})")
     log(f"map_batch ms, retention on:  {spread(ms[True])}  (n={len(ms[True])})")
+    big = gx.upload(np.concatenate([words, words]), None, np.concatenate([lens, lens]), total_bases=2 * int(o[-1]),
+                    stride_words=workload.STRIDE_WORDS)
+    ms = {False: [], True: []}
+    for rep in range(a.reps + 1):
+        for on in ((False, True) if rep % 2 == 0 else (True, False)):
+            gx.retain_hits(on)
+            gx.sample_begin(opts, workload.READ_LEN)
+            t = time.perf_counter()
+            for _ in range(a.big_batches):
+                gx.map_batch(big)
+            if rep:
+                ms[on].append((time.perf_counter() - t) * 1e3)
+    n_big = 2 * a.reads * a.big_batches
+    log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention off: {spread(ms[False])}  (n={len(ms[False])})")
+    log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention on:  {spread(ms[True])}  (n={len(ms[True])})")
+    del big
     # the last call above left retention on or off depending on the parity of reps: map once more with it on
     gx.retain_hits(True)
     gx.sample_begin(opts, workload.READ_LEN)
@@ -72,8 +97,8 @@ def main():
     h = gx.last_hits(nh)
     kept_reads = np.unique(h["read"][h["kept"] == 1])
     words_kept = int(((lens[kept_reads].astype(np.int64) + 15) // 16).sum())
-    log(f"retained: {len(kept_reads)} of {a.reads} reads ({100 * len(kept_reads) / a.reads:.2f} %), {4 * words_kept} bytes of "
-        f"2-bit words + {16 * len(kept_reads)} bytes of per-read entries")
+    log(f"retained: {nk} kept hits of {len(kept_reads)} of {a.reads} reads ({100 * len(kept_reads) / a.reads:.2f} %): {12 * nk} bytes "
+        f"of hits + {8 * len(kept_reads)} bytes of rows in the GPU's store, {4 * words_kept} bytes of 2-bit words on the host")
     gx.genotype(w.refs_path)
     loci, regions = gx.discover_candidates()
     n_region_reads = sum(len(r[5]) for r in regions)
@@ -116,6 +141,65 @@ def main():
                 found += 1
                 break
     log(f"planted variants recovered as their true haplotype: {found} of {len(variants)}")
+
+    # the whole discover call on files, next to the map call on the same file
+    gx.retain_hits(False)  # map_genotype runs with the caller's setting; discover switches retention on for itself
+    tmp = tempfile.mkdtemp(prefix="drprg_discover_probe_")
+    try:
+        text = None
+        for gz in (False, True):
+            fq = os.path.join(tmp, "reads.fq" + (".gz" if gz else ""))
+            sim.write_fastq_fast(fq, d, o, gz=gz)
+            runs = {"discover": [], "map": []}
+            for rep in range(a.reps + 1):
+                for what in (("discover", "map") if rep % 2 == 0 else ("map", "discover")):
+                    if what == "discover":
+                        st = gx.discover(fq, tmp, opts)
+                    else:
+                        st = gx.map_genotype(fq, w.refs_path, tmp, opts)
+                    if rep:
+                        runs[what].append(st)
+            kind = "gzip" if gz else "plain"
+            for key in ("ms_ingest", "ms_map", "ms_ml_path", "ms_discover", "ms_total"):
+                log(f"drprg_cuda_discover, {kind} FASTQ, {key}: {spread([r[key] for r in runs['discover']])}")
+            for key in ("ms_ingest", "ms_map", "ms_genotype", "ms_total"):
+                log(f"drprg_cuda_map_genotype, {kind} FASTQ, {key}: {spread([r[key] for r in runs['map']])}")
+            st = runs["discover"][-1]
+            log(f"drprg_cuda_discover, {kind} FASTQ: reads {st['n_reads']}, kept hits {st['n_hits_kept']}, regions {st['n_regions']}, "
+                f"region reads {st['n_region_reads']}, assembled {st['n_assembled']}, no anchor {st['n_no_anchor']}, too many paths "
+                f"{st['n_too_many_paths']}, no path {st['n_no_path']}, loci with variants {st['n_loci_with_variants']}, variants {st['n_variants']}")
+            t = open(os.path.join(tmp, "denovo_paths.txt")).read()
+            text = t if text is None else text
+            log(f"denovo_paths.txt of the {kind} FASTQ equals the plain one: {t == text}")
+    finally:
+        shutil.rmtree(tmp)
+    # the restatement from the ML paths and regions of the discover call's own genotyping (in-memory map above, same reads)
+    # and the oracle assembler's alleles: checks the variant form and the layout, not the map pass (the tests do that)
+    gx.retain_hits(True)
+    gx.sample_begin(opts, workload.READ_LEN)
+    gx.map_batch(batch)
+    gx.genotype(None)
+    loci, regions = gx.discover_candidates()
+    reads = {rd: d[int(o[rd]):int(o[rd + 1])].tobytes().decode() for r in regions for rd, _, _, _ in r[5]}
+    want = A.assemble(loci, regions, reads)
+    ox = O.Index(w.prg_path, w.w, w.k)
+    want_text = P.file_from(ox, open(w.prg_path).read().splitlines(), {l: gx.mlpath(l).tolist() for l in loci}, loci, regions, want)
+    same_file = want_text == text
+    log(f"denovo_paths.txt equals the restatement: {same_file}")
+    _, got = P.read_denovo_paths(text)
+    records = 0
+    for li, v, ref_len, alt, old in variants:
+        if gx.names[li] not in got:
+            continue
+        nodes, recs = got[gx.names[li]]
+        cons = "".join(q for _, _, _, q in nodes)
+        at = cons.find(old[v - 30:v]) + 30
+        if at < 30:
+            continue
+        planted = cons[:at] + alt + cons[at + ref_len:]
+        records += any(cons[p - 1:p - 1 + len(r)] == r and cons[:p - 1] + al + cons[p - 1 + len(r):] == planted for p, r, al in recs)
+    log(f"planted variants that are records of denovo_paths.txt (same edit of the ML sequence): {records} of {len(variants)}")
+    same = same and same_file
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
