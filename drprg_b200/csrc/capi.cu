@@ -1826,7 +1826,8 @@ void refuse_shard_handles(const drprg_index* X) {
 // `pandora discover` for one sample from the one map pass: map (hit retention on), ML path, candidate regions, local
 // assembly, and <outdir>/denovo_paths.txt from the de-novo alleles
 void run_discover(drprg_index* X, const char* sample_name, const char* reads_path, const char* outdir, const drprg_map_opts* o,
-                  const drprg_discover_opts* d, const drprg_assemble_opts* a, drprg_discover_stats* stats) {
+                  const drprg_discover_opts* d, const drprg_assemble_opts* a, drprg_discover_stats* stats,
+                  const Inflated* pre = nullptr) {
     need_device(X);
     refuse_shard_handles(X);
     const char* sample = sample_name ? sample_name : "sample";
@@ -1842,7 +1843,7 @@ void run_discover(drprg_index* X, const char* sample_name, const char* reads_pat
         }
     } guard{X, X->retain_hits};
     for (drprg_index* g : (X->gpus.empty() ? std::vector<drprg_index*>{X} : X->gpus)) g->retain_hits = true;
-    const FileMapped M = map_reads_file(X, reads_path, o, nullptr);
+    const FileMapped M = map_reads_file(X, reads_path, o, pre);
     const double t1 = now_ms();
     genotype(X, nullptr, sample);  // pandora discover takes no --vcf-refs: the ML path does not depend on them
     const double t2 = now_ms();
@@ -1885,6 +1886,48 @@ void run_discover(drprg_index* X, const char* sample_name, const char* reads_pat
     s.ms_total = t3 - t0;
     if (stats) *stats = s;
 }
+
+// The gzip look-ahead of the batch calls.  A gzip file is inflated on all host cores (gzip_inflate.cpp), and that is still
+// most of a sample's time: in a batch of 1 M-read samples on a 16-core host, 91 ms per sample from gzip files against
+// 7 ms (map) and 11 ms (discover) from plain ones (profiles/r7_batch_discover_n1.jsonl).  While sample i runs, the gzip
+// files of the next few samples are inflated on threads of their own.  They share the cores with each other and with
+// sample i's host work, so the look-ahead gains only the time the cores would otherwise be idle, such as sample i's GPU
+// work and its waits.
+class GzipLookahead {
+  public:
+    GzipLookahead(size_t n, const char* const* reads_paths, const drprg_map_opts* o)
+        : paths_(reads_paths), ahead_(n),
+          window_(std::max<size_t>(1, std::min<size_t>({n, (size_t)(o && o->threads ? o->threads : 1), (size_t)8}))) {
+        for (size_t i = 0; i < window_; ++i) start(i);
+    }
+    // the text of sample i (p == nullptr for a plain file); starts the look-ahead of sample i + window; throws the error of
+    // the inflate
+    Inflated take(size_t i) {
+        Inflated pre;
+        if (ahead_[i].valid()) pre = ahead_[i].get();
+        start(i + window_);
+        if (!pre.error.empty()) throw std::runtime_error(pre.error);
+        return pre;
+    }
+
+  private:
+    void start(size_t i) {
+        if (i >= ahead_.size() || !file_is_gzip(paths_[i])) return;
+        const std::string path = paths_[i];
+        ahead_[i] = std::async(std::launch::async, [path]() {
+            Inflated r;
+            try {
+                r.inflate(path);
+            } catch (const std::exception& e) {
+                r.error = e.what();
+            }
+            return r;
+        });
+    }
+    const char* const* paths_;
+    std::vector<std::future<Inflated>> ahead_;
+    const size_t window_;
+};
 }  // namespace
 
 #define API_BEGIN try {
@@ -1980,30 +2023,9 @@ int drprg_cuda_map_genotype(drprg_index* X, const char* reads_path, const char* 
 }
 int drprg_cuda_map_genotype_batch(drprg_index* X, size_t n, const char* const* reads_paths, const char* vcf_refs,
                                   const char* const* outdirs, const drprg_map_opts* o, drprg_map_stats* stats) {
-    API_BEGIN
-    // gzip inputs are inflate-bound (one zlib stream = one core, ~0.6 s per million reads): the next few samples are
-    // inflated on spare threads while the GPU works on the current one
-    const size_t window = std::max<size_t>(1, std::min<size_t>({n, (size_t)(o && o->threads ? o->threads : 1), (size_t)8}));
-    std::vector<std::future<Inflated>> ahead(n);
-    auto prefetch = [&](size_t i) {
-        if (i >= n || !file_is_gzip(reads_paths[i])) return;
-        const std::string path = reads_paths[i];
-        ahead[i] = std::async(std::launch::async, [path]() {
-            Inflated r;
-            try {
-                r.inflate(path);
-            } catch (const std::exception& e) {
-                r.error = e.what();
-            }
-            return r;
-        });
-    };
-    for (size_t i = 0; i < window; ++i) prefetch(i);
+    API_BEGIN GzipLookahead ahead(n, reads_paths, o);
     for (size_t i = 0; i < n; ++i) {
-        Inflated pre;
-        if (ahead[i].valid()) pre = ahead[i].get();
-        prefetch(i + window);
-        if (!pre.error.empty()) throw std::runtime_error(pre.error);
+        const Inflated pre = ahead.take(i);
         run_sample(X, reads_paths[i], vcf_refs, outdirs[i], o, stats ? stats + i : nullptr, pre.p ? &pre : nullptr);
     }
     return 0;
@@ -2498,6 +2520,25 @@ int drprg_cuda_discover_assemble(drprg_index* X, const drprg_assemble_opts* o, u
 int drprg_cuda_discover(drprg_index* X, const char* sample, const char* reads_path, const char* outdir, const drprg_map_opts* o,
                         const drprg_discover_opts* d, const drprg_assemble_opts* a, drprg_discover_stats* stats) {
     API_BEGIN run_discover(X, sample, reads_path, outdir, o, d, a, stats);
+    return 0;
+    API_END
+}
+int drprg_cuda_discover_batch(drprg_index* X, size_t n, const char* const* samples, const char* const* reads_paths,
+                              const char* const* outdirs, const drprg_map_opts* o, const drprg_discover_opts* d,
+                              const drprg_assemble_opts* a, drprg_discover_stats* stats) {
+    API_BEGIN need_device(X);
+    refuse_shard_handles(X);
+    if (n && (!reads_paths || !outdirs)) throw std::runtime_error("reads_paths and outdirs must hold n entries each");
+    GzipLookahead ahead(n, reads_paths, o);
+    for (size_t i = 0; i < n; ++i) {
+        try {
+            const Inflated pre = ahead.take(i);
+            run_discover(X, samples ? samples[i] : nullptr, reads_paths[i], outdirs[i], o, d, a, stats ? stats + i : nullptr,
+                         pre.p ? &pre : nullptr);
+        } catch (const std::exception& e) {
+            throw std::runtime_error("sample " + std::to_string(i) + " (" + reads_paths[i] + "): " + e.what());
+        }
+    }
     return 0;
     API_END
 }

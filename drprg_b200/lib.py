@@ -97,7 +97,7 @@ SYMBOLS = [
     "drprg_cuda_index_records", "drprg_cuda_index_min_path_length", "drprg_cuda_sketch_batch", "drprg_cuda_last_hits",
     "drprg_cuda_gt_params", "drprg_cuda_gt_mlpath", "drprg_cuda_gt_counts", "drprg_cuda_gt_records",
     "drprg_cuda_gt_alleles", "drprg_cuda_gt_allele_knodes", "drprg_cuda_genotype_rows", "drprg_cuda_gt_filter_stats", "drprg_cuda_set_minor_af", "drprg_cuda_retain_hits", "drprg_cuda_discover_candidates",
-    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover", "drprg_cuda_discover_paths",
+    "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover", "drprg_cuda_discover_batch", "drprg_cuda_discover_paths",
     "drprg_cuda_discover_region_status", "drprg_cuda_last_assemble_stats", "drprg_cuda_last_timings", "drprg_cuda_last_genotype_timings", "drprg_cuda_format_g6", "drprg_cuda_format_g6_device", "drprg_cuda_launch_count", "drprg_cuda_hash64", "drprg_cuda_hash64_inverse", "drprg_cuda_issue_peak",
 ]
 
@@ -132,6 +132,13 @@ def _p(a):
 def _check(rc, what):
     if rc != 0:
         raise DrprgCudaError(f"{what}: {lib().drprg_cuda_last_error().decode()}")
+
+
+def _discover_args(opts, discover_opts, assemble_opts):
+    """the three option structs of the discover calls; the keyword dicts override the defaults field by field"""
+    d = DiscoverOpts(**dict(dict(covg_threshold=0, min_len=0, max_len=0, padding=0xFFFFFFFF, min_hits=0), **(discover_opts or {})))
+    a = AssembleOpts(**dict(dict(min_dbg_dp=0, max_insertion=0xFFFFFFFF, max_candidate_paths=0), **(assemble_opts or {})))
+    return opts or make_opts(), d, a
 
 
 def pack_reads(data, off, stride_words=0):
@@ -505,13 +512,27 @@ class Index:
         the candidate regions and writes <outdir>/denovo_paths.txt; returns the stats dict.  discover_opts / assemble_opts:
         keyword dicts of discover_candidates / discover_assemble."""
         st = DiscoverStats()
-        o = opts or make_opts()
-        d = DiscoverOpts(**dict(dict(covg_threshold=0, min_len=0, max_len=0, padding=0xFFFFFFFF, min_hits=0), **(discover_opts or {})))
-        a = AssembleOpts(**dict(dict(min_dbg_dp=0, max_insertion=0xFFFFFFFF, max_candidate_paths=0), **(assemble_opts or {})))
+        o, d, a = _discover_args(opts, discover_opts, assemble_opts)
         rc = lib().drprg_cuda_discover(self.h, sample.encode(), str(reads_path).encode(), str(outdir).encode(), C.byref(o), C.byref(d),
                                        C.byref(a), C.byref(st))
         _check(rc, "drprg_cuda_discover")
         return st.asdict()
+
+    def discover_batch(self, samples, reads_paths, outdirs, opts=None, discover_opts=None, assemble_opts=None):
+        """`pandora discover` for several samples on this resident index (drprg_cuda_discover_batch): sample i as
+        discover(reads_paths[i], outdirs[i], sample=samples[i]) would run it, while the next gzip files are inflated ahead;
+        samples=None names every sample "sample".  Returns one stats dict per sample.  The first failing sample raises,
+        naming its index; the files of the samples before it stay."""
+        n = len(reads_paths)
+        if len(outdirs) != n or (samples is not None and len(samples) != n):
+            raise ValueError("samples, reads_paths and outdirs must have one entry per sample")
+        strs = lambda xs: (C.c_char_p * max(1, n))(*[str(x).encode() for x in xs])
+        st = (DiscoverStats * max(1, n))()
+        o, d, a = _discover_args(opts, discover_opts, assemble_opts)
+        rc = lib().drprg_cuda_discover_batch(self.h, C.c_size_t(n), None if samples is None else strs(samples), strs(reads_paths),
+                                             strs(outdirs), C.byref(o), C.byref(d), C.byref(a), st)
+        _check(rc, "drprg_cuda_discover_batch")
+        return [st[i].asdict() for i in range(n)]
 
     def set_minor_af(self, maf):
         lib().drprg_cuda_set_minor_af(self.h, C.c_float(maf))

@@ -92,7 +92,8 @@ int drprg_cuda_shard_done(drprg_index*, void* stream);
 int drprg_cuda_map_genotype(drprg_index*, const char* reads_path, const char* vcf_refs_fasta, const char* outdir,
                             const drprg_map_opts*, drprg_map_stats* out_stats /* may be NULL */);
 /* config 5: independent samples, one after another on this index's GPU (sample-sharding across GPUs is
- * one process per GPU, each calling this on its share) */
+ * one process per GPU, each calling this on its share); the gzip files of the next few samples are inflated on host
+ * threads of their own while a sample runs.  drprg_cuda_discover_batch is the same for the discover step. */
 int drprg_cuda_map_genotype_batch(drprg_index*, size_t n, const char* const* reads_paths, const char* vcf_refs_fasta,
                                   const char* const* outdirs, const drprg_map_opts*, drprg_map_stats* out_stats /* n or NULL */);
 
@@ -223,6 +224,16 @@ typedef struct {
 } drprg_discover_stats;
 int drprg_cuda_discover(drprg_index*, const char* sample, const char* reads_path, const char* outdir, const drprg_map_opts*,
                         const drprg_discover_opts*, const drprg_assemble_opts*, drprg_discover_stats* /* may be NULL */);
+/* `pandora discover` for n independent samples, one after another on this index (the discover half of config 5, next to
+ * drprg_cuda_map_genotype_batch): sample i gets exactly what drprg_cuda_discover(X, samples[i], reads_paths[i], outdirs[i],
+ * ...) gives it, <outdirs[i]>/denovo_paths.txt byte for byte and out_stats[i].  As in the map batch, the gzip files of the
+ * next few samples are inflated on host threads of their own while a sample runs.  The first failing sample stops the call:
+ * it returns non-zero, drprg_cuda_last_error() names the sample's index and reads path, and the files of the samples before
+ * it stay.  The caller's retention setting is restored.  n = 0 does nothing; n > 0 needs reads_paths and outdirs.  Refused
+ * on host-only and one-process-per-GPU handles; a drprg_cuda_index_load_multi handle maps each file on its root GPU. */
+int drprg_cuda_discover_batch(drprg_index*, size_t n, const char* const* samples /* NULL = "sample" each */,
+                              const char* const* reads_paths, const char* const* outdirs, const drprg_map_opts*,
+                              const drprg_discover_opts*, const drprg_assemble_opts*, drprg_discover_stats* out_stats /* n or NULL */);
 
 /* ---- introspection / parity hooks (same .so, used by tests and bench) --------------------------- */
 /* pandora's hash64 on a 2k-bit k-mer and its inverse (the k-mer screen is built from the inverse): host functions */
