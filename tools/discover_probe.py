@@ -9,10 +9,14 @@ reads.  Reports, in one run on one GPU:
   reads as a plain and a gzip FASTQ with its stage split, alternated with drprg_cuda_map_genotype on the same file; whether
   the file equals the test-side restatement (tests/denovo_paths_oracle.py) of the same ML paths, regions and oracle
   alleles; and how many planted variants are records of the file.
+With --nanopore the sample is config 4's shape instead: --reads reads (default 15 000, 34x) of ~10 kb (lognormal sigma 0.3)
+at 5 % error split 40/30/30 into substitutions, insertions and deletions, uploaded ragged and mapped without -I; the
+config-3 section is left out.
 
-    python tools/discover_probe.py [--reads 1000000] [--reps 5] [--big-batches 15] [--out LOG]
+    python tools/discover_probe.py [--reads 1000000] [--reps 5] [--big-batches 15] [--nanopore] [--out LOG]
 """
 import argparse
+import gzip
 import os
 import shutil
 import subprocess
@@ -38,13 +42,24 @@ def spread(v):
     return f"median {v[len(v) // 2]:.3f} min {v[0]:.3f} max {v[-1]:.3f}"
 
 
+def write_fastq_ragged(path, data, off, gz):
+    """reads of any length, gzip at level 1 (a 300x nanopore sample is ~2.6 GB of FASTQ)"""
+    with (gzip.open(path, "wb", compresslevel=1) if gz else open(path, "wb")) as f:
+        for i in range(0, len(off) - 1, 4096):
+            f.write(b"".join(b"@r%d\n%s\n+\n%s\n" % (j, s, b"I" * len(s))
+                             for j in range(i, min(i + 4096, len(off) - 1))
+                             for s in [data[int(off[j]):int(off[j + 1])].tobytes()]))
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--reads", type=int, default=1_000_000)
+    ap.add_argument("--reads", type=int, help="default 1 000 000 (150 bp) or, with --nanopore, 15 000")
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--big-batches", type=int, default=15)
+    ap.add_argument("--nanopore", action="store_true", help="config-4 reads: ~10 kb at 5 % error, no -I")
     ap.add_argument("--out", help="also write the report to this file")
     a = ap.parse_args()
+    a.reads = a.reads or (15_000 if a.nanopore else 1_000_000)
     lines = []
 
     def log(s):
@@ -57,42 +72,51 @@ def main():
     hap = sim.sample_haplotype(w.panel, workload.PANEL_SEED + 1, 0.10)
     seqs, variants = sim.insert_novel_variants(w.panel, hap, [KINDS[i % 3] for i in range(20)], seed=5)
     genome, _ = sim.make_genome(w.panel, seqs, size=workload.GENOME_SIZE, seed=workload.PANEL_SEED + 5)
-    d, o = sim.simulate_reads(genome, a.reads, workload.READ_LEN, seed=workload.PANEL_SEED + 2, sub_rate=0.002)
-    log(f"sample: {a.reads} reads of {workload.READ_LEN} bp, {len(variants)} planted variants, config-2 panel ({len(w.panel.loci)} loci)")
+    if a.nanopore:
+        d, o = sim.simulate_long_reads(genome, a.reads, mean_len=10_000, sigma=0.3, seed=workload.PANEL_SEED + 2, err=0.05,
+                                       mix=(0.4, 0.3, 0.3))
+        log(f"sample: {a.reads} nanopore reads, {int(o[-1])} bases ({o[-1] / workload.GENOME_SIZE:.1f}x), mean "
+            f"{o[-1] / a.reads:.0f} bp, 5 % error, {len(variants)} planted variants, config-2 panel ({len(w.panel.loci)} loci)")
+    else:
+        d, o = sim.simulate_reads(genome, a.reads, workload.READ_LEN, seed=workload.PANEL_SEED + 2, sub_rate=0.002)
+        log(f"sample: {a.reads} reads of {workload.READ_LEN} bp, {len(variants)} planted variants, config-2 panel ({len(w.panel.loci)} loci)")
+    first_len = int(o[1] - o[0])
+    stride = 0 if a.nanopore else workload.STRIDE_WORDS  # long reads go up ragged (word_off)
     gx = lib.Index(w.prg_path, w.w, w.k, device=0)
-    words, woff, lens = lib.pack_reads(d, o, workload.STRIDE_WORDS)
-    batch = gx.upload(words, woff, lens, total_bases=int(o[-1]), stride_words=workload.STRIDE_WORDS)
-    opts = lib.make_opts(illumina=True, genome_size=workload.GENOME_SIZE)
+    words, woff, lens = lib.pack_reads(d, o, stride)
+    batch = gx.upload(words, woff, lens, total_bases=int(o[-1]), stride_words=stride)
+    opts = lib.make_opts(illumina=not a.nanopore, genome_size=workload.GENOME_SIZE)
     ms = {False: [], True: []}
     for rep in range(a.reps + 1):  # the first round warms both arms up
         for on in ((False, True) if rep % 2 == 0 else (True, False)):
             gx.retain_hits(on)
-            gx.sample_begin(opts, workload.READ_LEN)
+            gx.sample_begin(opts, first_len)
             t = time.perf_counter()
             nh, nk = gx.map_batch(batch)  # returns after its stream has been synchronised
             if rep:
                 ms[on].append((time.perf_counter() - t) * 1e3)
     log(f"map_batch ms, retention off: {spread(ms[False])}  (n={len(ms[False])})")
     log(f"map_batch ms, retention on:  {spread(ms[True])}  (n={len(ms[True])})")
-    big = gx.upload(np.concatenate([words, words]), None, np.concatenate([lens, lens]), total_bases=2 * int(o[-1]),
-                    stride_words=workload.STRIDE_WORDS)
-    ms = {False: [], True: []}
-    for rep in range(a.reps + 1):
-        for on in ((False, True) if rep % 2 == 0 else (True, False)):
-            gx.retain_hits(on)
-            gx.sample_begin(opts, workload.READ_LEN)
-            t = time.perf_counter()
-            for _ in range(a.big_batches):
-                gx.map_batch(big)
-            if rep:
-                ms[on].append((time.perf_counter() - t) * 1e3)
-    n_big = 2 * a.reads * a.big_batches
-    log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention off: {spread(ms[False])}  (n={len(ms[False])})")
-    log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention on:  {spread(ms[True])}  (n={len(ms[True])})")
-    del big
+    if not a.nanopore:
+        big = gx.upload(np.concatenate([words, words]), None, np.concatenate([lens, lens]), total_bases=2 * int(o[-1]),
+                        stride_words=workload.STRIDE_WORDS)
+        ms = {False: [], True: []}
+        for rep in range(a.reps + 1):
+            for on in ((False, True) if rep % 2 == 0 else (True, False)):
+                gx.retain_hits(on)
+                gx.sample_begin(opts, first_len)
+                t = time.perf_counter()
+                for _ in range(a.big_batches):
+                    gx.map_batch(big)
+                if rep:
+                    ms[on].append((time.perf_counter() - t) * 1e3)
+        n_big = 2 * a.reads * a.big_batches
+        log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention off: {spread(ms[False])}  (n={len(ms[False])})")
+        log(f"{n_big} reads in {a.big_batches} batches of {2 * a.reads}, all map_batch calls ms, retention on:  {spread(ms[True])}  (n={len(ms[True])})")
+        del big
     # the last call above left retention on or off depending on the parity of reps: map once more with it on
     gx.retain_hits(True)
-    gx.sample_begin(opts, workload.READ_LEN)
+    gx.sample_begin(opts, first_len)
     nh, nk = gx.map_batch(batch)
     h = gx.last_hits(nh)
     kept_reads = np.unique(h["read"][h["kept"] == 1])
@@ -102,7 +126,8 @@ def main():
     gx.genotype(w.refs_path)
     loci, regions = gx.discover_candidates()
     n_region_reads = sum(len(r[5]) for r in regions)
-    log(f"candidate regions: {len(regions)}, region reads: {n_region_reads}")
+    log(f"candidate regions: {len(regions)}, region reads: {n_region_reads}, k-mer positions in the largest pileup: "
+        f"{max([sum(max(0, e - s - A.DISCOVER_K + 1) for _, s, e, _ in r[5]) for r in regions], default=0)}")
     kt = []
     for rep in range(a.reps + 1):
         status, paths = gx.discover_assemble()
@@ -149,7 +174,10 @@ def main():
         text = None
         for gz in (False, True):
             fq = os.path.join(tmp, "reads.fq" + (".gz" if gz else ""))
-            sim.write_fastq_fast(fq, d, o, gz=gz)
+            if a.nanopore:
+                write_fastq_ragged(fq, d, o, gz)
+            else:
+                sim.write_fastq_fast(fq, d, o, gz=gz)
             runs = {"discover": [], "map": []}
             for rep in range(a.reps + 1):
                 for what in (("discover", "map") if rep % 2 == 0 else ("map", "discover")):
@@ -176,7 +204,7 @@ def main():
     # the restatement from the ML paths and regions of the discover call's own genotyping (in-memory map above, same reads)
     # and the oracle assembler's alleles: checks the variant form and the layout, not the map pass (the tests do that)
     gx.retain_hits(True)
-    gx.sample_begin(opts, workload.READ_LEN)
+    gx.sample_begin(opts, first_len)
     gx.map_batch(batch)
     gx.genotype(None)
     loci, regions = gx.discover_candidates()
