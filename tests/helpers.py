@@ -4,6 +4,7 @@ import tempfile
 
 import numpy as np
 
+import oracle_py as O
 from drprg_b200 import sim
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -43,3 +44,32 @@ def long_reads_sample(panel, n_reads, seed=21, genome_size=200_000, mean_len=400
     g, placements = sim.make_genome(panel, [h[0] for h in hap], size=genome_size, seed=seed + 1, min_sep=3000)
     d, o = sim.simulate_long_reads(g, n_reads, mean_len=mean_len, seed=seed + 2)
     return d, o, g, placements
+
+
+def assert_genotype_equal(gx, ox, mr, oo, refs):
+    og = O.Genotype(ox, mr, oo, refs)
+    gx.genotype(refs)
+    gp, op = gx.params(), og.params()
+    for key in op:
+        assert gp[key] == op[key], (key, gp[key], op[key])
+    for l in range(ox.n_loci):
+        a, b = gx.mlpath(l), og.mlpath(l)
+        assert (a is None) == (b is None), l
+        if a is not None:
+            assert len(a) == len(b) and (a == b).all(), ("ml path", l)
+    gr, orr = gx.gt_records(), og.records()
+    for key in ("locus", "pos", "n_alleles", "gt", "mean_fwd", "mean_rev", "med_fwd", "med_rev", "sum_fwd", "sum_rev",
+                "n_knodes", "allele_knodes", "gaps"):
+        assert len(gr[key]) == len(orr[key]), key
+        assert (gr[key] == orr[key]).all(), key
+    # log-likelihoods: fp64 on both sides, 1e-9 relative (BASELINE.json north_star)
+    np.testing.assert_allclose(gr["lik"], orr["lik"], rtol=1e-9, atol=0)
+    np.testing.assert_allclose(gr["gt_conf"], orr["gt_conf"], rtol=1e-9, atol=1e-9)
+    strip = lambda t: [l for l in t.splitlines() if not l.startswith("##fileDate")]
+    assert strip(gx.vcf()) == strip(og.vcf())
+    assert bytes(gx.vcf_view()) == gx.vcf_bytes()  # the zero-copy view is the same text
+    # the filter / minor-allele statistics fused into the genotype kernel (SURVEY 8f rank 4) against the Rust restatement
+    import rust_filters
+    rust_filters.check_against(gx.filter_stats(), np.concatenate([[0], np.cumsum(gr["n_alleles"])]), gr["mean_fwd"], gr["mean_rev"],
+                               gr["gaps"], gr["gt"], gr["gt_conf"], 0.1 if oo.illumina else 1.0)
+    return og
