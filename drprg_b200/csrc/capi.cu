@@ -122,7 +122,7 @@ struct drprg_index {
     // device-resident index
     DevTable T{};
     DBuf<uint2> d_slots, d_recs;
-    DBuf<uint32_t> d_kfilter;
+    DBuf<uint32_t> d_kfilter, d_kfilter14;
     DBuf<uint32_t> d_filter, d_knode_base, d_edge_off, d_edges;
     DBuf<uint8_t> d_is_terminal, d_needs_mean;
     DBuf<uint32_t> d_locus_level_off, d_level_start, d_level_nodes, d_level_singles;
@@ -266,6 +266,57 @@ struct drprg_index {
 namespace {
 inline size_t accum_flag_offset(uint64_t n_accum) { return (size_t)((n_accum + 31) & ~31ull); }  // 128-byte aligned flag words
 
+// ~24 filter bits per entry, capped by the shared memory of one SM
+std::vector<uint32_t> screen_filter(const std::vector<uint32_t>& kmers, uint32_t k) {
+    uint32_t nw = (uint32_t)std::min<uint64_t>(SCREEN_MAX_FILTER_WORDS, std::max<uint64_t>(1024, (kmers.size() * 24 + 31) / 32));
+    nw = (nw + 3) & ~3u;
+    std::vector<uint32_t> f(nw, 0);
+    for (uint32_t x : kmers) screen_filter_insert(f.data(), nw, x, k);
+    return f;
+}
+
+// k-mer screen filters (k = 15): the k-mers behind the indexed hashes in both orientations (hash64 is invertible), and the
+// two 14-mers of each of them, which the screen tests at every other read position
+struct ScreenFilters {
+    std::vector<uint32_t> kfilter, kfilter14;  // both empty: the index keeps the sketch kernels
+};
+ScreenFilters build_screen_filters(const HostIndex& H) {
+    ScreenFilters F;
+    if (H.k != 15 || H.records.empty()) return F;
+    const uint64_t mask = (1ull << (2 * H.k)) - 1;
+    std::vector<uint32_t> kmers;
+    kmers.reserve(H.records.size() * 2);
+    for (size_t i = 0; i < H.records.size(); ++i) {
+        if (i && H.records[i - 1].hash == H.records[i].hash) continue;
+        const uint64_t y = hash64_inverse_host(H.records[i].hash, mask);
+        if (hash64_host(y, mask) != H.records[i].hash) throw std::runtime_error("hash64 inversion failed");
+        uint64_t rc = 0, t = y;
+        for (uint32_t b = 0; b < H.k; ++b) {
+            rc = (rc << 2) | (3 - (t & 3));
+            t >>= 2;
+        }
+        kmers.push_back((uint32_t)y);
+        kmers.push_back((uint32_t)rc);
+    }
+    std::sort(kmers.begin(), kmers.end());
+    kmers.erase(std::unique(kmers.begin(), kmers.end()), kmers.end());
+    std::vector<uint32_t> sub;
+    sub.reserve(kmers.size() * 2);
+    for (uint32_t x : kmers) {
+        sub.push_back(x >> 2);                              // bases 0..13
+        sub.push_back(x & ((1u << (2 * (H.k - 1))) - 1u));  // bases 1..14
+    }
+    std::sort(sub.begin(), sub.end());
+    sub.erase(std::unique(sub.begin(), sub.end()), sub.end());
+    // The filters are capped by one SM's shared memory (1.77 Mbit).  Beyond ~300 k k-mers (4x the Mtb-scale panel) more
+    // than a third of the 15-mer filter's bits are set, over 10 % of all read positions are flagged and resolving them
+    // costs as much as sketching every read: such an index keeps the sketch kernels.
+    if (kmers.size() > 300000) return F;
+    F.kfilter = screen_filter(kmers, H.k);
+    F.kfilter14 = screen_filter(sub, H.k - 1);
+    return F;
+}
+
 void upload_index(drprg_index* X) {
     const HostIndex& H = X->H;
     if (H.k > (uint32_t)K_MAX) throw std::runtime_error("k > 16 is not supported by the device kernels (2k must fit 32 bits)");
@@ -308,39 +359,14 @@ void upload_index(drprg_index* X) {
     X->table_slots = 1u << sb;
     X->filter_words = 1u << fb;
     X->T = DevTable{X->d_slots.p, sb, X->d_recs.p, X->d_filter.p, fb};
-    // ---- k-mer screen: the k-mers behind the indexed hashes, both orientations (hash64 is invertible)
-    if (H.k >= 8 && H.k <= 15 && distinct > 0) {
-        const uint64_t mask = (1ull << (2 * H.k)) - 1;
-        std::vector<uint32_t> kmers;
-        kmers.reserve(distinct * 2);
-        for (size_t i = 0; i < H.records.size(); ++i) {
-            if (i && H.records[i - 1].hash == H.records[i].hash) continue;
-            const uint64_t y = hash64_inverse_host(H.records[i].hash, mask);
-            if (hash64_host(y, mask) != H.records[i].hash) throw std::runtime_error("hash64 inversion failed");
-            uint64_t rc = 0, t = y;
-            for (uint32_t b = 0; b < H.k; ++b) {
-                rc = (rc << 2) | (3 - (t & 3));
-                t >>= 2;
-            }
-            kmers.push_back((uint32_t)y);
-            kmers.push_back((uint32_t)rc);
-        }
-        std::sort(kmers.begin(), kmers.end());
-        kmers.erase(std::unique(kmers.begin(), kmers.end()), kmers.end());
-        // The filter is capped by one SM's shared memory (1.77 Mbit).  Beyond ~300 k k-mers (4x the Mtb-scale panel) more
-        // than a third of its bits are set, over 10 % of all read positions are flagged and resolving them costs as much
-        // as sketching every read: such an index keeps the sketch kernels.
-        const bool screen_pays = kmers.size() <= 300000;
-        // ~24 filter bits per k-mer, capped by the shared memory of one SM
-        uint32_t nw = (uint32_t)std::min<uint64_t>(SCREEN_MAX_FILTER_WORDS, std::max<uint64_t>(1024, (kmers.size() * 24 + 31) / 32));
-        nw = (nw + 3) & ~3u;
-        std::vector<uint32_t> kfilter(nw, 0);
-        for (uint32_t x : kmers) screen_filter_insert(kfilter.data(), nw, x, H.k);
-        if (screen_pays) {
-            X->d_kfilter.assign(kfilter);
-            X->T.kfilter = X->d_kfilter.p;
-            X->T.kfilter_words = nw;
-        }
+    const ScreenFilters F = build_screen_filters(H);
+    if (!F.kfilter.empty()) {
+        X->d_kfilter.assign(F.kfilter);
+        X->d_kfilter14.assign(F.kfilter14);
+        X->T.kfilter = X->d_kfilter.p;
+        X->T.kfilter_words = (uint32_t)F.kfilter.size();
+        X->T.kfilter14 = X->d_kfilter14.p;
+        X->T.kfilter14_words = (uint32_t)F.kfilter14.size();
     }
     // ---- k-mer graphs
     const uint32_t N = H.total_knodes();
@@ -610,7 +636,7 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     // whole-genome reads give ~0.35 hits per 150 bp read; a targeted run overflows once, regrows to the exact count and is redone
     ensure_hit_capacity(X, std::max<uint64_t>(X->hi.cap, std::max<uint64_t>(1u << 20, B->total_bases / 256)));
     ensure_read_capacity(X, B->R.n_reads);
-    if (X->T.kfilter) {  // ~2 flagged positions per 150 bp read
+    if (X->T.kfilter) {  // ~0.6 queued candidates per whole-genome 150 bp read; room for ~8x that, reads on the panel queue more
         X->queue.ensure(std::max<uint64_t>(X->queue.cap, B->total_bases / 32 + (1u << 20)));
         X->queue_kmer.ensure(X->queue.cap);
     }
@@ -621,6 +647,7 @@ void map_batch(drprg_index* X, drprg_batch* B, cudaStream_t st, uint64_t* n_hits
     // skip their work, the accumulators are untouched) and the batch is redone with larger buffers.
     for (int attempt = 0;; ++attempt) {
         const uint64_t queue_cap = X->T.kfilter ? std::min(X->queue.cap, X->queue_kmer.cap) : 0;
+        if (queue_cap >= (1ull << 31)) throw std::runtime_error("k-mer screen queue beyond 2^31 entries");  // resolve stages 31-bit indices
         CK(cudaMemsetAsync(X->d_counters.p, 0, CTR_COUNT * sizeof(unsigned long long), st));
         CK(cudaEventRecord(X->ev[0].get(), st));
         for (int c = 0; c < B->n_chunks; ++c) {
@@ -2249,6 +2276,17 @@ int drprg_cuda_index_records(drprg_index* X, uint64_t* hash, uint32_t* prg, uint
 int drprg_cuda_index_min_path_length(drprg_index* X, uint32_t* out) {
     for (size_t l = 0; l < X->H.loci.size(); ++l) out[l] = X->H.loci[l].min_path_len;
     return 0;
+}
+int drprg_cuda_index_screen_filters(drprg_index* X, uint32_t* kfilter, uint32_t* kfilter_words, uint32_t* kfilter14,
+                                    uint32_t* kfilter14_words) {
+    API_BEGIN
+    const ScreenFilters F = build_screen_filters(X->H);
+    if (kfilter) std::copy(F.kfilter.begin(), F.kfilter.end(), kfilter);
+    if (kfilter14) std::copy(F.kfilter14.begin(), F.kfilter14.end(), kfilter14);
+    *kfilter_words = (uint32_t)F.kfilter.size();
+    *kfilter14_words = (uint32_t)F.kfilter14.size();
+    return 0;
+    API_END
 }
 
 int64_t drprg_cuda_sketch_batch(drprg_index* X, drprg_batch* B, void* stream, uint32_t* read, uint32_t* start, uint64_t* hash,

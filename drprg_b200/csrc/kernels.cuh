@@ -38,10 +38,14 @@ struct DevTable {
     const uint2* recs;       // {knode rank within locus, prg << 1 | strand}, grouped by hash
     const uint32_t* filter;  // blocked 2-bit Bloom pre-filter, 1 << filter_bits words
     uint32_t filter_bits;
-    // k-mer screen (k <= 15): every indexed minimizer k-mer in both orientations.  A read can only produce a hit if
+    // k-mer screen (k = 15): every indexed minimizer k-mer in both orientations.  A read can only produce a hit if
     // one of its forward k-mers is in this set, which is tested WITHOUT hashing (hash64 is a bijection).
-    const uint32_t* kfilter = nullptr;  // blocked 2-bit Bloom over k-mers, kfilter_words words (multiple of 4), copied to shared memory
+    const uint32_t* kfilter = nullptr;  // blocked 2-bit Bloom over those 15-mers, kfilter_words words (multiple of 4)
     uint32_t kfilter_words = 0;
+    // the same over both 14-mers of each of them, copied to shared memory: a read's indexed 15-mer at p contains the 14-mer
+    // at the even one of p, p + 1, so testing the 14-mers at even positions finds every candidate
+    const uint32_t* kfilter14 = nullptr;
+    uint32_t kfilter14_words = 0;
 };
 
 struct Hit128 {  // sort key: (hi, lo) ascending == pandora MinimizerHit order

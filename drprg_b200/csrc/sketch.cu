@@ -524,9 +524,11 @@ static bool launch_short(const DevReads& R, const DevTable& T, uint32_t w, uint3
 // one of the indexed k-mers or their reverse complements" — a set-membership test on the raw 2-bit k-mer
 // that needs no hash and no window logic.
 //   screen_kernel   streams every read once (a warp takes 32 reads at a time from a global ticket counter,
-//                   words in registers) and tests each k-mer against a blocked 2-bit Bloom filter held in
-//                   shared memory: one multiply, one LDS, two shifts, ~10 instructions per position.  The
-//                   flagged positions (~1 % false positives + the real ones) are appended to a queue.
+//                   words in registers) and tests the 14-mer at every EVEN position against a blocked 2-bit Bloom
+//                   filter of the indexed k-mers' 14-mers held in shared memory: one multiply, one LDS, two shifts,
+//                   ~10 instructions per tested position.  A flagged position's two candidate k-mers are tested
+//                   against the same kind of filter over the indexed k-mers themselves, and those that pass (~1.5 %
+//                   false positives + the real ones) are appended to a queue.
 //   resolve_kernel  persistent warps, several queued (read, position) pairs per lane: canonical hash of each k-mer,
 //                   index probes side by side (exact, drops the false positives), survivors collected in a per-warp
 //                   shared-memory ring and tested 32 at a time — a position is a (w,k)-minimizer with pandora's
@@ -550,6 +552,12 @@ void screen_filter_insert(uint32_t* filter, uint32_t n_words, uint32_t kmer, uin
 // shifts on the ALU pipe.  Measured 0.152 ms per million reads against 0.155 with the address step alone and 0.159 with
 // neither; a multiply-high for the second bit index as well never paid.
 struct ScreenConsts { uint32_t four, two; };
+// Every other position: a 15-mer at p contains the 14-mers at p and p + 1, and exactly one of those is even, so the 14-mers
+// at even positions q are tested against a filter of the indexed 15-mers' 14-mers (shared memory).  A flagged q stands for
+// two candidates, p = q - 1 and p = q, and is queued with the 16 bases q - 1 .. q + 14 that hold both; the resolve kernel
+// tests them against the 15-mer filter.  Half the positions are tested, and a 14-mer costs the same instructions as a
+// 15-mer did.
+constexpr uint32_t QUEUE_AT_NK = 1u << 31;
 template <int K, int CW>
 __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, DevTable T, uint32_t wk, ScreenConsts SC,
                                                                    unsigned long long* __restrict__ queue,
@@ -557,14 +565,15 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
                                                                    unsigned long long* __restrict__ queue_count,
                                                                    unsigned long long queue_cap,
                                                                    unsigned long long* __restrict__ ticket) {
-    static_assert(K >= 8 && K <= 15, "the filter bit choice needs >= 16 k-mer bits; 2k < 32");
-    constexpr int NF = (CW + 1) / 2;
+    static_assert(K == 15, "the screened 14-mers and the 16-mer of a flagged position are laid out for k = 15");
+    constexpr int KS = K - 1;
+    constexpr int NF = (CW + 3) / 4;  // flag words: a read word holds 8 even positions
     extern __shared__ uint32_t s_kf[];
     const int tid = threadIdx.x, lane = tid & 31;
-    for (uint32_t i = tid * 4; i < T.kfilter_words; i += SCREEN_THREADS * 4)
-        *reinterpret_cast<uint4*>(s_kf + i) = __ldg(reinterpret_cast<const uint4*>(T.kfilter + i));
+    for (uint32_t i = tid * 4; i < T.kfilter14_words; i += SCREEN_THREADS * 4)
+        *reinterpret_cast<uint4*>(s_kf + i) = __ldg(reinterpret_cast<const uint4*>(T.kfilter14 + i));
     __syncthreads();
-    const uint32_t n_fw = T.kfilter_words;
+    const uint32_t n_fw = T.kfilter14_words;
     const uint32_t s_base = (uint32_t)__cvta_generic_to_shared(s_kf);
     const unsigned long long n_items = R.seg_read ? R.n_segs : R.n_reads;
     const unsigned long long n_tiles = (n_items + 31) / 32;
@@ -588,12 +597,17 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
         if (len + 1 < wk) len = 0;  // too short or dropped: the sketch skips it too
         const uint32_t nk_read = len ? len - K + 1 : 0;
         const uint32_t seg_s = (have && R.seg_read) ? __ldg(R.seg_start + item) : 0u;
-        const uint32_t seg_e = R.seg_read ? min(seg_s + R.seg_len, nk_read) : nk_read;  // screen positions [seg_s, seg_e)
-        const uint32_t q0 = seg_s & ~15u;                                             // streamed from a word boundary
-        const uint32_t span = seg_e > seg_s ? seg_e - q0 : 0u;
+        const uint32_t seg_e = R.seg_read ? min(seg_s + R.seg_len, nk_read) : nk_read;
+        // test the even q in [seg_s, seg_e), and q = nk at the read's end: every even q in [0, nk] falls in exactly one
+        // segment, so every candidate p in [0, nk) is found once
+        const uint32_t q_end = seg_e + (seg_e == nk_read ? 1u : 0u);
+        const uint32_t q0 = seg_s & ~15u;  // streamed from a word boundary
+        const uint32_t span = seg_e > seg_s ? q_end - q0 : 0u;
         const uint32_t span_max = __reduce_max_sync(FULL, span);
         const uint32_t* wp = R.words + (have ? (R.stride_words ? r * R.stride_words : __ldg(R.word_off + r)) : 0ull) + (q0 >> 4);
         const uint32_t nwords = span ? ((len + 15) >> 4) - (q0 >> 4) : 0u;  // words that may be read from wp
+        // the word before the chunk: base q - 1 of a flagged q at a word boundary (none before the read's first base)
+        uint32_t prev = (span && q0) ? __ldg(wp - 1) : 0u;
 #pragma unroll 1
         for (uint32_t c0 = 0; c0 < span_max; c0 += CW * 16) {
             const uint32_t w0 = c0 >> 4;
@@ -617,40 +631,57 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
             for (int i = 0; i < CW; ++i) {
                 if (c0 + i * 16 < span_max) {  // warp-uniform: skip words past every lane's last position
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        // 32 bits ENDING at the last base of the k-mer that starts at base j of word i; the older
-                        // bases above bit 2K are removed by the multiply
-                        const int n = 64 - 2 * (j + K);
+                    for (int j = 0; j < 16; j += 2) {
+                        // 32 bits ENDING at the last base of the 14-mer that starts at base j of word i; the older
+                        // bases above bit 2KS are removed by the multiply
+                        const int n = 64 - 2 * (j + KS);
                         const uint32_t v = (n >= 32) ? (cw[i] >> ((n - 32) & 31)) : __funnelshift_r(cw[i + 1], cw[i], n & 31);
-                        const uint32_t p = v * (SCREEN_MUL << (32 - 2 * K));
+                        const uint32_t p = v * (SCREEN_MUL << (32 - 2 * KS));
                         uint32_t addr, word;
                         asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(addr) : "r"(__umulhi(p, n_fw)), "r"(SC.four), "r"(s_base));
                         asm("ld.shared.u32 %0, [%1];" : "=r"(word) : "r"(addr));
                         const uint32_t t = __funnelshift_r(word, 0u, v) & __funnelshift_r(word, 0u, p >> 11);
                         // the flag enters at the bottom of its word; the word is bit-reversed once at the end
-                        asm("mad.lo.u32 %0, %0, %1, %2;" : "+r"(f[i >> 1]) : "r"(SC.two), "r"(t & 1u));
+                        asm("mad.lo.u32 %0, %0, %1, %2;" : "+r"(f[i >> 2]) : "r"(SC.two), "r"(t & 1u));
                     }
                 } else {
-                    f[i >> 1] <<= 16;  // a skipped word still occupies its sixteen flag positions
+                    f[i >> 2] <<= 8;  // a skipped word still occupies its eight flag positions
                 }
             }
+            // bit t of f[i] now stands for q = q0 + c0 + 64 i + 2 t
 #pragma unroll
-            for (int i = 0; i < NF; ++i) f[i] = __brev((CW & 1) && i == NF - 1 ? f[i] << 16 : f[i]);
-            // keep the flags of positions inside [seg_s, seg_e), count them, reserve queue space per warp
-            uint32_t cnt = 0;
+            for (int i = 0; i < NF; ++i) f[i] = __brev((CW & 3) && i == NF - 1 ? f[i] << (32 - 8 * (CW & 3)) : f[i]);
             {
-                const uint32_t lo_cut = (c0 == 0) ? (seg_s - q0) : 0u;                          // < 16
-                const uint32_t hi_cut = span > c0 ? min(span - c0, (uint32_t)(CW * 16)) : 0u;  // valid positions in this chunk
+                // keep the flags of even q - q0 in [lo, span)
+                const uint32_t lo = (c0 == 0) ? (seg_s - q0 + 1) >> 1 : 0u;                              // < 8
+                const uint32_t hi = span > c0 ? (min(span - c0, (uint32_t)(CW * 16)) + 1) >> 1 : 0u;  // flags in this chunk
 #pragma unroll
                 for (int i = 0; i < NF; ++i) {
                     const uint32_t base = i * 32;
-                    const uint32_t hi_n = hi_cut > base ? min(hi_cut - base, 32u) : 0u;
+                    const uint32_t hi_n = hi > base ? min(hi - base, 32u) : 0u;
                     uint32_t m = hi_n >= 32u ? 0xffffffffu : ((1u << hi_n) - 1u);
-                    if (i == 0) m &= ~((1u << lo_cut) - 1u);
+                    if (i == 0) m &= ~((1u << lo) - 1u);
                     f[i] &= m;
-                    cnt += __popc(f[i]);
                 }
             }
+            // the 16 bases q - 1 .. q + 14 of flag t of f[i] (base -1 of a read reads as 0): they start 2 t + 15 bases into
+            // word 4 i - 1 of the chunk
+            auto bases16 = [&](int i, uint32_t t) {
+                uint32_t x[6];
+#pragma unroll
+                for (int m = 0; m < 6; ++m) {
+                    const int wi = 4 * i - 1 + m;
+                    x[m] = wi < 0 ? prev : cw[wi < CW + 2 ? wi : CW + 1];  // words past CW + 1 hold no flagged q
+                }
+                const uint32_t s = 2u * t + 15u, u = s >> 4;
+                const uint32_t a = u == 0 ? x[0] : u == 1 ? x[1] : u == 2 ? x[2] : u == 3 ? x[3] : x[4];
+                const uint32_t b = u == 0 ? x[1] : u == 1 ? x[2] : u == 2 ? x[3] : u == 3 ? x[4] : x[5];
+                return __funnelshift_l(b, a, 2u * (s & 15u));
+            };
+            uint32_t cnt = 0;
+#pragma unroll
+            for (int i = 0; i < NF; ++i) cnt += __popc(f[i]);
+            // count them, reserve queue space per warp
             const uint32_t total = __reduce_add_sync(FULL, cnt);
             if (total) {
                 unsigned long long o = 0;
@@ -672,27 +703,30 @@ __global__ void __launch_bounds__(SCREEN_THREADS, 1) screen_kernel(DevReads R, D
                     for (int i = 0; i < NF; ++i) {
                         uint32_t m = f[i];
                         while (m) {
-                            const uint32_t bit = __ffs(m) - 1;
+                            const uint32_t t = __ffs(m) - 1;
                             m &= m - 1u;
-                            *reinterpret_cast<uint2*>(qp++) = make_uint2(pos0 + i * 32 + bit, tag);  // read << 32 | position
-                            // the k-mer travels with the entry, so the resolve kernel's index probe needs no access to the read
-                            const bool up = bit >= 16u;
-                            const uint32_t a = up ? cw[2 * i + 1] : cw[2 * i], b = up ? cw[2 * i + 2] : cw[2 * i + 1];
-                            *kp++ = __funnelshift_l(b, a, 2u * (bit & 15u)) >> (32 - 2 * K);
+                            const uint32_t q = pos0 + i * 64 + 2 * t;
+                            // read << 32 | q, bit 31 set when q = nk (its candidate p = q is past the read's last k-mer)
+                            *reinterpret_cast<uint2*>(qp++) = make_uint2(q | (q == nk_read ? QUEUE_AT_NK : 0u), tag);
+                            // the bases travel with the entry, so the resolve kernel needs no access to the read for them
+                            *kp++ = bases16(i, t);
                         }
                     }
                 }
             }
+            prev = cw[CW - 1];
         }
         tile = next_tile;
         next_tile = __shfl_sync(FULL, after_next, 0);
     }
 }
 
-// Resolve the flagged (read, position) pairs: persistent warps, no CTA barrier.  A warp takes tiles of RESOLVE_PER_LANE
-// queue entries per lane (lane-strided, so the queue loads stay coalesced), computes the canonical hash of every queued
-// k-mer and issues the index probes of all of them before it uses any result: RESOLVE_PER_LANE independent L2 chains per
-// thread.  The probe is exact, so the Bloom filter's false positives (~80 % of the queue) end here.  The survivors are
+// Resolve the flagged positions: persistent warps, no CTA barrier.  A warp takes tiles of RESOLVE_ENTRIES_PER_LANE queue
+// entries per lane (lane-strided, so the queue loads stay coalesced) and tests both candidate 15-mers of each against the
+// 15-mer filter, all filter loads in flight together; ~12 % of the candidates pass and go by ballot to a stage in the
+// warp's shared memory.  Whenever it holds RESOLVE_TILE of them the warp computes their canonical hashes and issues the
+// index probes of all of them before it uses any result: RESOLVE_PER_LANE independent L2 chains per thread.  The probe
+// is exact, so the filters' false positives (~25 % of the staged candidates) end here.  The survivors are
 // appended by ballot to a ring in the warp's own shared memory; whenever it holds 32 of them the warp runs the minimizer
 // test restricted to those positions with every lane busy, and after its last tile it tests what is left.
 //   W > 0: compile-time window (2W-2+K bases around the position fit three aligned words): the words are fetched once,
@@ -702,6 +736,9 @@ constexpr int RESOLVE_WARPS = 8;
 constexpr int RESOLVE_PER_LANE = 4;
 constexpr uint32_t RESOLVE_TILE = 32 * RESOLVE_PER_LANE;
 constexpr int RESOLVE_RING = 31 + RESOLVE_TILE;  // < 32 untested survivors + one tile's
+constexpr int RESOLVE_ENTRIES_PER_LANE = RESOLVE_PER_LANE / 2;  // queue entries per lane and tile: two candidates each
+constexpr uint32_t RESOLVE_ENTRY_TILE = 32 * RESOLVE_ENTRIES_PER_LANE;
+constexpr int RESOLVE_STAGE = 2 * RESOLVE_TILE - 1;  // < RESOLVE_TILE candidates left + one tile's
 template <int W, int K>
 __global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R, DevTable T, uint32_t w_rt, uint32_t k_rt,
                                                                      const unsigned long long* __restrict__ queue,
@@ -715,8 +752,10 @@ __global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R,
                                                                      unsigned long long* __restrict__ out_count,
                                                                      unsigned long long cap) {
     static_assert(W == 0 || 2 * W - 2 + K <= 48, "window + k-mer must fit three aligned words");
+    static_assert(K == 15, "queue entries carry the 16 bases of two candidate 15-mers");
     __shared__ unsigned long long s_q[RESOLVE_WARPS][RESOLVE_RING];
     __shared__ uint32_t s_rec[RESOLVE_WARPS][RESOLVE_RING];
+    __shared__ uint32_t s_stage[RESOLVE_WARPS][RESOLVE_STAGE];
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicMax(queue_need, *queue_count);  // sticky over the chunks of a batch: the host regrows and redoes
     if (*queue_count > queue_cap) return;  // overflow: the queue has unwritten slots and the batch is redone anyway
     const unsigned long long n = *queue_count;
@@ -727,6 +766,7 @@ __global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R,
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     unsigned long long* ring_q = s_q[wid];
     uint32_t* ring_rec = s_rec[wid];
+    uint32_t* stage = s_stage[wid];
     auto canon_of = [&](uint32_t v, uint32_t& strand) {  // v: 32 bits starting at the k-mer's first base
         const uint32_t F = v & hm;
         uint32_t y = __brev(~v & hm);
@@ -735,28 +775,72 @@ __global__ void __launch_bounds__(RESOLVE_WARPS * 32) resolve_kernel(DevReads R,
         strand = hf <= hr ? 1u : 0u;
         return min(hf, hr);
     };
-    const unsigned long long n_tiles = (n + RESOLVE_TILE - 1) / RESOLVE_TILE;
+    const unsigned long long n_tiles = (n + RESOLVE_ENTRY_TILE - 1) / RESOLVE_ENTRY_TILE;
     const unsigned long long n_warps = (unsigned long long)gridDim.x * RESOLVE_WARPS;
+    uint32_t stage_n = 0;             // staged candidates (warp-uniform)
     uint32_t ring_n = 0;              // survivors in the ring (warp-uniform)
     unsigned long long n_surv = 0;    // survivors this warp found (warp-uniform)
     for (unsigned long long tile = (unsigned long long)blockIdx.x * RESOLVE_WARPS + wid;; tile += n_warps) {
         const bool more = tile < n_tiles;  // warp-uniform
         if (more) {
+            // both candidates of every entry against the 15-mer filter, all filter loads in flight together: candidate 2 i is
+            // p = q - 1 (the top 15 of the 16 bases), 2 i + 1 is p = q (the bottom 15)
+            uint32_t x[2 * RESOLVE_ENTRIES_PER_LANE], fw[2 * RESOLVE_ENTRIES_PER_LANE], ok = 0;
+#pragma unroll
+            for (int i = 0; i < RESOLVE_ENTRIES_PER_LANE; ++i) {
+                const unsigned long long e = tile * RESOLVE_ENTRY_TILE + i * 32 + lane;
+                uint32_t pw = 0, m = 0;
+                if (e < n) {
+                    pw = (uint32_t)queue[e];
+                    m = queue_kmer[e];
+                    ok |= (((pw & ~QUEUE_AT_NK) != 0u ? 1u : 0u) | (pw & QUEUE_AT_NK ? 0u : 2u)) << (2 * i);  // p = q - 1 needs q > 0, p = q needs q < nk
+                }
+                x[2 * i] = m >> 2;
+                x[2 * i + 1] = m & 0x3fffffffu;
+            }
+#pragma unroll
+            for (int j = 0; j < 2 * RESOLVE_ENTRIES_PER_LANE; ++j)
+                fw[j] = __ldg(T.kfilter + __umulhi(x[j] * (SCREEN_MUL << (32 - 2 * K)), T.kfilter_words));
+            // the candidates that pass go to the warp's stage as (queue index << 1 | which)
+#pragma unroll
+            for (int j = 0; j < 2 * RESOLVE_ENTRIES_PER_LANE; ++j) {
+                const uint32_t p = x[j] * (SCREEN_MUL << (32 - 2 * K));
+                const bool pass = (ok >> j & 1u) && (__funnelshift_r(fw[j], 0u, x[j]) & __funnelshift_r(fw[j], 0u, p >> 11) & 1u);
+                const uint32_t bal = __ballot_sync(FULL, pass);
+                if (pass) stage[stage_n + __popc(bal & ((1u << lane) - 1u))] =
+                    (uint32_t)(tile * RESOLVE_ENTRY_TILE + (j >> 1) * 32 + lane) << 1 | (uint32_t)(j & 1);
+                stage_n += __popc(bal);
+            }
+            __syncwarp();
+        }
+        // index probes of RESOLVE_TILE staged candidates (after the last tile also the rest): a tile adds at most that many
+        // to fewer than that many, so one round leaves fewer than RESOLVE_TILE again
+        if (stage_n >= RESOLVE_TILE || (!more && stage_n)) {
             unsigned long long q[RESOLVE_PER_LANE];
             uint32_t km[RESOLVE_PER_LANE], hv[RESOLVE_PER_LANE], slot[RESOLVE_PER_LANE], rec[RESOLVE_PER_LANE];
             uint32_t pending = 0;  // bit i: entry i still walks its probe chain
 #pragma unroll
             for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
-                const unsigned long long e = tile * RESOLVE_TILE + i * 32 + lane;
+                const uint32_t si = i * 32 + lane;
                 q[i] = 0;
                 km[i] = 0;
                 rec[i] = 0;
-                if (e < n) {
-                    q[i] = queue[e];
-                    km[i] = queue_kmer[e];
+                if (si < stage_n) {
+                    const uint32_t c = stage[si];
+                    const unsigned long long qe = queue[c >> 1];
+                    const uint32_t m = queue_kmer[c >> 1];
+                    const uint32_t pos = ((uint32_t)qe & ~QUEUE_AT_NK) - ((c & 1u) ^ 1u);
+                    q[i] = (qe & 0xffffffff00000000ull) | pos;
+                    km[i] = (c & 1u) ? m & 0x3fffffffu : m >> 2;
                     pending |= 1u << i;
                 }
             }
+            // the < RESOLVE_TILE candidates left move to the front of the stage (only after a full round: disjoint ranges)
+            const uint32_t taken = min(stage_n, RESOLVE_TILE);
+            __syncwarp();
+            for (uint32_t i = lane; taken + i < stage_n; i += 32) stage[i] = stage[taken + i];
+            __syncwarp();
+            stage_n -= taken;
 #pragma unroll
             for (int i = 0; i < RESOLVE_PER_LANE; ++i) {
                 uint32_t strand;
@@ -908,7 +992,7 @@ static void launch_screen(const DevReads& R, const DevTable& T, uint32_t wk, uns
     const unsigned long long n_items = R.seg_read ? R.n_segs : R.n_reads;
     const unsigned long long n_ctas = (n_items + SCREEN_THREADS - 1) / SCREEN_THREADS;
     const unsigned grid = (unsigned)std::min<unsigned long long>(n_ctas, (unsigned long long)sm_count);  // one persistent CTA per SM
-    screen_kernel<K, CW><<<grid, SCREEN_THREADS, (size_t)T.kfilter_words * 4, st>>>(R, T, wk, ScreenConsts{4u, 2u}, queue, queue_kmer, counters, queue_cap, counters + 1);
+    screen_kernel<K, CW><<<grid, SCREEN_THREADS, (size_t)T.kfilter14_words * 4, st>>>(R, T, wk, ScreenConsts{4u, 2u}, queue, queue_kmer, counters, queue_cap, counters + 1);
     ++g_launches;
 }
 
@@ -925,7 +1009,7 @@ static void launch_resolve(const DevReads& R, const DevTable& T, uint32_t w, con
     // persistent warps at full occupancy; the queue length is only known on the device, but it cannot exceed the number of
     // k-mer positions, which caps the grid of a small batch
     const unsigned long long positions = (R.seg_read ? R.n_segs * R.seg_len : R.n_reads * max_len) + 1;
-    const unsigned long long want = (positions + RESOLVE_TILE * RESOLVE_WARPS - 1) / (RESOLVE_TILE * RESOLVE_WARPS);
+    const unsigned long long want = (positions + RESOLVE_ENTRY_TILE * RESOLVE_WARPS - 1) / (RESOLVE_ENTRY_TILE * RESOLVE_WARPS);
     const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)per_sm * (unsigned)sm_count);
     resolve_kernel<W, K><<<grid, RESOLVE_WARPS * 32, 0, st>>>(R, T, w, K, queue, queue_kmer, counters, queue_cap,
                                                               counters + (CTR_QUEUE_NEED - CTR_QUEUE), counters + (CTR_SURVIVORS - CTR_QUEUE),
@@ -965,7 +1049,7 @@ void launch_sketch_lookup(const DevReads& R, const DevTable& T, uint32_t w, uint
         const char* e = getenv("DRPRG_SCREEN");  // DRPRG_SCREEN=0 sketches every read (A/B measurements, parity tests)
         return !e || atoi(e) != 0;
     }();
-    if (screen_on && d_queue && d_queue_kmer && T.kfilter && (max_len <= SHORT_READ_MAX || R.seg_read) && k == 15)
+    if (screen_on && d_queue && d_queue_kmer && T.kfilter && T.kfilter14 && (max_len <= SHORT_READ_MAX || R.seg_read) && k == 15)
         return launch_screened<15>(R, T, w, d_hi, d_lo, d_hit_count, hit_cap, sm_count, max_len, d_queue, d_queue_kmer, queue_cap, d_screen_counters, st);
     if ((max_len <= SHORT_READ_MAX || R.seg_read) && launch_short<true>(R, T, w, k, d_hi, d_lo, d_hit_count, hit_cap, sm_count, st)) return;
     sketch_kernel<true><<<grid_for(sm_count, R.n_reads), WARPS * 32, 0, st>>>(R, T, w, k, d_hi, d_lo, d_hit_count, hit_cap);

@@ -94,7 +94,7 @@ SYMBOLS = [
     "drprg_cuda_accum_device_ptr", "drprg_cuda_accum_download", "drprg_cuda_accum_upload", "drprg_cuda_genotype",
     "drprg_cuda_write_vcf", "drprg_cuda_vcf_text", "drprg_cuda_vcf_view", "drprg_cuda_index_info", "drprg_cuda_locus_name",
     "drprg_cuda_index_knode_base", "drprg_cuda_index_knodes", "drprg_cuda_index_edges", "drprg_cuda_index_paths",
-    "drprg_cuda_index_records", "drprg_cuda_index_min_path_length", "drprg_cuda_sketch_batch", "drprg_cuda_last_hits",
+    "drprg_cuda_index_records", "drprg_cuda_index_min_path_length", "drprg_cuda_index_screen_filters", "drprg_cuda_sketch_batch", "drprg_cuda_last_hits",
     "drprg_cuda_gt_params", "drprg_cuda_gt_mlpath", "drprg_cuda_gt_counts", "drprg_cuda_gt_records",
     "drprg_cuda_gt_alleles", "drprg_cuda_gt_allele_knodes", "drprg_cuda_genotype_rows", "drprg_cuda_gt_filter_stats", "drprg_cuda_set_minor_af", "drprg_cuda_retain_hits", "drprg_cuda_discover_candidates",
     "drprg_cuda_discover_regions", "drprg_cuda_discover_region_reads", "drprg_cuda_discover_consensus", "drprg_cuda_discover_coverage", "drprg_cuda_discover_assemble", "drprg_cuda_discover", "drprg_cuda_discover_batch", "drprg_cuda_discover_paths",

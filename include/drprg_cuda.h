@@ -252,6 +252,11 @@ int drprg_cuda_index_edges(drprg_index*, uint32_t* edges /* global ids */);
 int drprg_cuda_index_paths(drprg_index*, uint32_t* iv_start, uint32_t* iv_len);
 int drprg_cuda_index_records(drprg_index*, uint64_t* hash, uint32_t* prg, uint32_t* knode, uint8_t* strand);
 int drprg_cuda_index_min_path_length(drprg_index*, uint32_t* out /* n_loci */);
+/* the k-mer screen's Bloom filters as the index builds them (k = 15; empty otherwise): over the indexed 15-mers of both
+ * orientations and over their 14-mers, in screen_filter_insert's layout.  Pass NULL filters to learn the word counts;
+ * both are 0 when the index keeps the sketch kernels. */
+int drprg_cuda_index_screen_filters(drprg_index*, uint32_t* kfilter, uint32_t* kfilter_words, uint32_t* kfilter14,
+                                    uint32_t* kfilter14_words);
 /* S1 only: all (w,k)-minimizers of the batch, ordered (read, start); returns count (or <0) */
 int64_t drprg_cuda_sketch_batch(drprg_index*, drprg_batch*, void* stream, uint32_t* read, uint32_t* start,
                                 uint64_t* hash, uint8_t* strand, uint64_t cap);
